@@ -2,6 +2,7 @@
 """bench.py -- MSDeformAttn forward+backward throughput on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--mode model|uniform]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's CPU path on the host cores
 
@@ -42,7 +43,10 @@ FALLBACK_HBM_GBS = 6650.0         # /opt/skills/guides/B200_PROFILING.md fallbac
 def parse_args():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=50)
+    p.add_argument("--steps", type=int, default=50,
+                   help="timed steps of the measured metric (>= 1).  Two context figures of the GPU arm "
+                        "keep their own counts, reported in the JSON line: the e2e leg times "
+                        "max(4, min(K, 20)) steps, the CPU baseline 5")
     p.add_argument("--warmup", type=int, default=10)
     p.add_argument("--impl", default="b200", choices=["b200", "reference"])
     p.add_argument("--workload", default=DEFAULT_WORKLOAD)
@@ -51,7 +55,15 @@ def parse_args():
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--cpu-sample-batch", type=int, default=0,
                    help="images per CPU step; 0 = the workload's whole batch")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write rank 0's output and three gradients of the last "
+                        "step as DIR/<name>.npy (float32); see dump_outputs()")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        p.error("--dump-outputs writes what the GPU arm computed; it needs --impl b200")
+    return args
 
 
 def measured_peak():
@@ -225,9 +237,9 @@ def run_reference_arm(args):
     if rank != 0:
         return
     w = load_synthetic().WORKLOADS[args.workload]
-    # the whole batch of the workload per step (~0.4-0.6 s on the box's cores): K and W are honoured
-    # up to a cap that keeps the run within minutes
-    steps = max(1, min(args.steps, 60))
+    # the whole batch of the workload per step (~0.4-0.6 s on the host's cores): K is honoured, W is
+    # capped at 5 warm-up steps
+    steps = args.steps
     warmup = max(1, min(args.warmup, 5))
     batch = w.batch if args.cpu_sample_batch <= 0 else args.cpu_sample_batch
     base = cpu_reference_run(args.workload, args.mode, batch, steps, warmup)
@@ -322,6 +334,9 @@ def run_b200_arm(args):
         dist.barrier()
     torch.cuda.synchronize()
     launches = pkg.launch_count() - n0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"output": out, "grad_value": gv, "grad_sampling_loc": gl,
+                                         "grad_attn_weight": gw})
 
     step_ms = [m[0].elapsed_time(m[3]) for m in marks]
     fwd_ms = [m[0].elapsed_time(m[1]) for m in marks]
@@ -414,6 +429,33 @@ def run_b200_arm(args):
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 60 << 20      # keeps the .npy files of --dump-outputs, headers included, under 64 MB
+
+
+def dump_outputs(directory, arrays, seed=0):
+    """Write each [N, S, ...] device tensor of `arrays` as <directory>/<name>.npy in float32, flattened to
+    [rows, ...] with one row per (image, query).  When all rows of all tensors exceed DUMP_BYTES, every
+    tensor keeps the same rows: a sample drawn with a fixed seed, in ascending order.  The inputs of a
+    run depend only on its arguments, so two builds run alike write files that compare element by element."""
+    import numpy as np
+    import torch
+    rows = {t.shape[0] * t.shape[1] for t in arrays.values()}
+    assert len(rows) == 1, "every dumped tensor has one row per (image, query)"
+    rows = rows.pop()
+    row_bytes = sum(t[0, 0].numel() * 4 for t in arrays.values())
+    keep = min(rows, DUMP_BYTES // row_bytes)
+    idx = None
+    if keep < rows:
+        pick = np.sort(np.random.default_rng(seed).choice(rows, keep, replace=False))
+        idx = torch.from_numpy(pick).to(next(iter(arrays.values())).device)
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        flat = t.detach().reshape(rows, *t.shape[2:])
+        if idx is not None:
+            flat = flat.index_select(0, idx)
+        np.save(os.path.join(directory, name + ".npy"), flat.float().cpu().numpy())
 
 
 def reference_cuda_same_gpu(pkg, d, flush, iters=5):

@@ -42,6 +42,45 @@ def test_mirror_loads_reference_checkpoint_and_matches_reference_forward_cpu(pkg
     assert np.abs(srcs[2].grad.numpy() - g["grad_src2"]).max() <= 1e-10
 
 
+def redraw_attention_projections(layers, gen, dtype):
+    """What tests/golden/make_golden.py does to the reference's seeded init before it stores the weights:
+    sampling offsets and attention weights of every layer redrawn from `gen`, so that the locations leave
+    the integer pixel steps of the default init."""
+    with torch.no_grad():
+        for layer in layers:
+            a = layer.self_attn
+            a.sampling_offsets.weight.copy_(torch.randn(a.sampling_offsets.weight.shape, generator=gen, dtype=dtype) * 0.05)
+            a.sampling_offsets.bias.add_(torch.rand(a.sampling_offsets.bias.shape, generator=gen, dtype=dtype) * 0.6 + 0.2)
+            a.attention_weights.weight.copy_(torch.randn(a.attention_weights.weight.shape, generator=gen, dtype=dtype) * 0.1)
+
+
+def assert_state_equals_golden(module, g):
+    state = module.state_dict()
+    assert list(state) == [k[len("state::"):] for k in g if k.startswith("state::")]
+    for k, v in state.items():
+        assert np.array_equal(v.numpy(), g["state::" + k]), k
+
+
+def test_mirror_init_matches_reference_golden(pkg):
+    """The golden's weights are the reference encoder's init under torch.manual_seed(1234), redrawn as
+    above, and its inputs come from the same generator (make_golden.py encoder_golden): under the same
+    seed the mirror reproduces the parameter order and every tensor bit for bit, and its sine position
+    embedding reproduces the reference's `pos` inputs."""
+    g = load_golden("encoder_small")
+    torch.manual_seed(1234)
+    m = pkg.modules.MSDeformAttnTransformerEncoderOnly(
+        d_model=64, nhead=2, num_encoder_layers=2, dim_feedforward=128, dropout=0.0,
+        num_feature_levels=3, enc_n_points=4).double()
+    gen = torch.Generator().manual_seed(99)
+    redraw_attention_projections(m.encoder.layers, gen, torch.float64)
+    assert_state_equals_golden(m, g)
+    pe = pkg.pixel_decoder.PositionEmbeddingSine(32, normalize=True)
+    for i, (h, w) in enumerate(LEVELS):
+        src = torch.randn(2, 64, h, w, generator=gen, dtype=torch.float64)
+        assert np.array_equal(src.numpy(), g[f"src{i}"])
+        assert np.array_equal(pe(src).double().numpy(), g[f"pos{i}"])
+
+
 def test_reference_points_match_reference_formula(pkg):
     enc = pkg.modules.MSDeformAttnTransformerEncoder
     shapes = torch.tensor(LEVELS)
@@ -97,6 +136,34 @@ def test_mirror_init_and_forward_equal_live_reference(pkg, oracle):
         assert (r_attn(q, refp, x, shapes, lsi, mask) - m_attn(q, refp, x, shapes, lsi, mask)).abs().max() <= 1e-12
         box = torch.rand(2, 126, 3, 4, dtype=torch.float64)      # 4-d reference boxes (ms_deform_attn.py:113-115)
         assert (r_attn(q, box, x, shapes, lsi) - m_attn(q, box, x, shapes, lsi)).abs().max() <= 1e-12
+
+
+def test_module_padding_mask_and_box_reference_points(pkg, oracle):
+    """The two module inputs the encoder never passes: a padding mask zeroes the value rows it marks, so
+    those rows of `input_flatten` cannot reach the output; 4-d reference boxes (cx, cy, w, h) give
+    loc = (cx, cy) + offset / P * (w, h) / 2 (ms_deform_attn.py:113-115)."""
+    seen = {}
+
+    def core(value, shapes, lsi, loc, w, im2col_step):
+        seen["loc"] = loc
+        return oracle.core_grid_sample(value, shapes, loc, w)
+    torch.manual_seed(3)
+    attn = pkg.modules.MSDeformAttn(64, 3, 2, 4, core=core).double()
+    with torch.no_grad():
+        attn.sampling_offsets.weight.normal_(std=0.05)
+        q = torch.randn(2, 126, 64, dtype=torch.float64)
+        x = torch.randn(2, 126, 64, dtype=torch.float64)
+        shapes, lsi = torch.tensor(LEVELS), torch.tensor([0, 6, 30])
+        refp = torch.rand(2, 126, 3, 2, dtype=torch.float64)
+        mask = torch.rand(2, 126) > 0.8
+        y = attn(q, refp, x, shapes, lsi, mask)
+        assert torch.equal(attn(q, refp, x + 5.0 * mask[..., None], shapes, lsi, mask), y)
+        assert not torch.equal(attn(q, refp, x + 5.0 * ~mask[..., None], shapes, lsi, mask), y)
+        box = torch.rand(2, 126, 3, 4, dtype=torch.float64)
+        attn(q, box, x, shapes, lsi)
+        off = attn.sampling_offsets(q).view(2, 126, 2, 3, 4, 2)
+        want = box[:, :, None, :, None, :2] + off / 4 * box[:, :, None, :, None, 2:] * 0.5
+        assert (seen["loc"] - want).abs().max().item() <= 1e-15
 
 
 def test_module_refuses_cpu_without_injected_core(pkg):
