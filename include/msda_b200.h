@@ -207,7 +207,8 @@ int msda_b200_add_layernorm_backward_f32(const float *grad_y, const float *x, co
  *     if up != NULL:  y += bilinear up-sampling of up[N, C, up_h, up_w] to H x W, align_corners=False
  * `workspace` must hold msda_b200_group_norm_workspace_bytes(N, groups) bytes (per-group partial sums;
  * its contents are meaningless before and after the call).  Needs H*W (and, with `up`, W) to be a multiple of 4 and
- * 16-byte aligned x / y; MSDA_ERR_UNSUPPORTED otherwise.  Inference only (no backward).
+ * 16-byte aligned x / y; MSDA_ERR_UNSUPPORTED otherwise.  Training: the _train_f32 forwards and the backward
+ * entry points below.
  */
 int msda_b200_group_norm_nchw_f32(const float *x, const float *channel_bias, const float *gamma,
                                   const float *beta, float *y, int batch, int channels, int height,
@@ -225,6 +226,46 @@ int msda_b200_group_norm_nchw_to_rows_f32(const float *x, const float *channel_b
                                           const float *beta, float *y_rows, long long row_stride,
                                           long long image_stride, int batch, int channels, long long plane,
                                           int groups, float eps, int relu, void *workspace, void *stream);
+/*
+ * Training forwards: the two GroupNorms above with the same arguments, plus mean_rstd [batch, groups, 2], which
+ * receives (mean, rstd) of x + channel_bias per (image, group) as the backward needs them.  y / y_rows are
+ * bit-identical to those of the entry points above.
+ */
+int msda_b200_group_norm_nchw_train_f32(const float *x, const float *channel_bias, const float *gamma,
+                                        const float *beta, float *y, float *mean_rstd, int batch, int channels,
+                                        int height, int width, int groups, float eps, int relu, const float *up,
+                                        int up_h, int up_w, void *workspace, void *stream);
+int msda_b200_group_norm_nchw_to_rows_train_f32(const float *x, const float *channel_bias, const float *gamma,
+                                                const float *beta, float *y_rows, float *mean_rstd,
+                                                long long row_stride, long long image_stride, int batch,
+                                                int channels, long long plane, int groups, float eps, int relu,
+                                                void *workspace, void *stream);
+/*
+ * Backward of msda_b200_group_norm_nchw_train_f32 (torch autograd semantics) from grad_y, the forward's inputs and
+ * its mean_rstd.  Overwritten: grad_x [N, C, H, W]; grad_gamma [C] and grad_beta [C], summed over the batch;
+ * grad_channel_bias [C] (may be NULL: not computed); grad_up [N, C, up_h, up_w] (may be NULL: not computed), the
+ * adjoint of the forward's bilinear up-sampling applied to grad_y (the add comes after the ReLU, so grad_y is not
+ * masked there).  With relu, the mask is rebuilt from x with the forward's own float expression.  Deterministic (no
+ * floating-point atomics).  Three launches (reduce, per-group finalize, apply), a fourth for grad_up.
+ * `workspace` must hold msda_b200_group_norm_backward_workspace_bytes(N, C) bytes.  Shape and alignment
+ * requirements are the forward's (16-byte aligned grad_y / x / grad_x); MSDA_ERR_UNSUPPORTED otherwise.
+ */
+int msda_b200_group_norm_backward_nchw_f32(const float *grad_y, const float *x, const float *channel_bias,
+                                           const float *gamma, const float *beta, const float *mean_rstd,
+                                           float *grad_x, float *grad_gamma, float *grad_beta,
+                                           float *grad_channel_bias, float *grad_up, int batch, int channels,
+                                           int height, int width, int groups, int relu, int up_h, int up_w,
+                                           void *workspace, void *stream);
+long long msda_b200_group_norm_backward_workspace_bytes(int batch, int channels);
+/* Backward of msda_b200_group_norm_nchw_to_rows_train_f32: the same, with grad_y read from the rows layout
+ * (grad_y_rows[n * image_stride + pixel * row_stride + c]) and grad_x written NCHW.  Three launches; same workspace
+ * and the forward's requirements. */
+int msda_b200_group_norm_rows_backward_f32(const float *grad_y_rows, long long row_stride, long long image_stride,
+                                           const float *x, const float *channel_bias, const float *gamma,
+                                           const float *beta, const float *mean_rstd, float *grad_x,
+                                           float *grad_gamma, float *grad_beta, float *grad_channel_bias, int batch,
+                                           int channels, long long plane, int groups, int relu, void *workspace,
+                                           void *stream);
 /* x[n, c, :] += bias[c] in place over an NCHW fp32 map (plane = H*W, a multiple of 4; 16-byte aligned x):
  * the bias of the decoder's last 1x1 convolution (mask_features, msdeformattn.py:268-275, :381) at the
  * memory roofline instead of torch's broadcasting add. */

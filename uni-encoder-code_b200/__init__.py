@@ -16,7 +16,8 @@ import sys
 
 from . import _lib
 from ._lib import get_option, launch_count, set_option
-from .functions import AddLayerNormFunction, LinearTF32x3Function, MSDeformAttnFunction, MSDeformAttnFusedFunction
+from .functions import (AddLayerNormFunction, GroupNormFunction, GroupNormRowsFunction, LinearTF32x3Function,
+                        MSDeformAttnFunction, MSDeformAttnFusedFunction)
 from .ops import (add_layernorm, debug_indices, group_norm, linear_tf32x3, ms_deform_attn_backward, ms_deform_attn_forward,
                   ms_deform_attn_fused_backward, ms_deform_attn_fused_forward)
 from . import synthetic
@@ -25,6 +26,7 @@ from . import modules, pixel_decoder, sharding
 __all__ = [
     "ms_deform_attn_forward", "ms_deform_attn_backward", "MSDeformAttnFunction", "debug_indices",
     "ms_deform_attn_fused_forward", "ms_deform_attn_fused_backward", "MSDeformAttnFusedFunction", "linear_tf32x3", "add_layernorm", "group_norm", "LinearTF32x3Function", "AddLayerNormFunction",
+    "GroupNormFunction", "GroupNormRowsFunction",
     "install_dropin", "set_option", "get_option", "launch_count", "synthetic", "modules", "pixel_decoder", "sharding",
 ]
 

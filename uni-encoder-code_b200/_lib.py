@@ -42,6 +42,13 @@ SYMBOLS = {
                                                     ctypes.c_float, _I, _P, _P]),
     "msda_b200_add_channel_bias_nchw_f32": (_I, [_P, _P, _I, _I, ctypes.c_longlong, _P]),
     "msda_b200_group_norm_workspace_bytes": (ctypes.c_longlong, [_I, _I]),
+    "msda_b200_group_norm_nchw_train_f32": (_I, [_P] * 6 + [_I] * 5 + [ctypes.c_float, _I, _P, _I, _I, _P, _P]),
+    "msda_b200_group_norm_nchw_to_rows_train_f32": (_I, [_P] * 6 + [ctypes.c_longlong, ctypes.c_longlong, _I, _I,
+                                                          ctypes.c_longlong, _I, ctypes.c_float, _I, _P, _P]),
+    "msda_b200_group_norm_backward_nchw_f32": (_I, [_P] * 11 + [_I] * 8 + [_P, _P]),
+    "msda_b200_group_norm_backward_workspace_bytes": (ctypes.c_longlong, [_I, _I]),
+    "msda_b200_group_norm_rows_backward_f32": (_I, [_P, ctypes.c_longlong, ctypes.c_longlong] + [_P] * 9
+                                               + [_I, _I, ctypes.c_longlong, _I, _I, _P, _P]),
     "msda_b200_set_option": (_I, [ctypes.c_char_p, _I]),
     "msda_b200_get_option": (_I, [ctypes.c_char_p, ctypes.POINTER(_I)]),
 }

@@ -21,8 +21,11 @@
 // Algorithmic bytes: read x twice + write y once = 12 B per element (+ 1/4 of a read for the
 // up-sampled map); torch's sequence moves 12 (GroupNorm) + 4 + 12 (up-sample, add) = 28.
 //
-// Inference only (no backward); the reference semantics are torch.nn.functional.group_norm and
-// F.interpolate(mode="bilinear", align_corners=False).
+// Training: the same two launches also write (mean, rstd) per (image, group) when asked (y unchanged), and the
+// backward below takes three launches (reduce, per-group finalize, apply; a fourth for the gradient of the
+// up-sampled map): 20 B per element (+ 5 B for that gradient) against torch's ~40.  The reference semantics are
+// torch.nn.functional.group_norm and F.interpolate(mode="bilinear", align_corners=False), with torch autograd's
+// gradients.
 #include <cuda_runtime.h>
 #include <cstdint>
 
@@ -75,6 +78,14 @@ group_stats_kernel(const float *__restrict__ x, double *__restrict__ partial, lo
     }
 }
 
+// the apply kernels' per-channel affine y = x * sc + sf (before the ReLU).  The backward rebuilds the ReLU mask
+// from this very expression on the (mean, rstd) the forward wrote, so that it matches the forward bit for bit.
+__device__ __forceinline__ void gn_affine(float rstd, float gamma, float beta, float cbias, float mean, float &sc,
+                                          float &sf) {
+    sc = rstd * gamma;
+    sf = beta + (cbias - mean) * sc;
+}
+
 // source index of torch's bilinear up-sampling with align_corners=False
 // (area_pixel_compute_source_index: scale * (dst + 0.5) - 0.5, clamped at 0)
 __device__ __forceinline__ void up_index(int dst, float scale, int in_size, int &i0, int &i1, float &l1) {
@@ -90,7 +101,7 @@ __global__ void __launch_bounds__(256)
 group_apply_kernel(const float *__restrict__ x, const double *__restrict__ partial, const float *__restrict__ gamma,
                    const float *__restrict__ beta, float *__restrict__ y, int C, int H, int W, int cpg, float eps,
                    const float *__restrict__ up, int uh, int uw, float sh, float sw,
-                   const float *__restrict__ cbias) {
+                   const float *__restrict__ cbias, float *__restrict__ mean_rstd) {
     // blockIdx.x = image * C + channel (one plane), blockIdx.y = part of the plane
     const int plane = blockIdx.x, c = plane % C, ng = plane / cpg;      // ng = image * groups + group
     __shared__ float s_scale, s_shift;
@@ -106,9 +117,11 @@ group_apply_kernel(const float *__restrict__ x, const double *__restrict__ parti
         var = var < 0.0 ? 0.0 : var;
         const float mean = (float)(mean_k + K);
         const float rstd = (float)(1.0 / sqrt(var + (double)eps));
-        const float sc = rstd * gamma[c];
-        s_scale = sc;
-        s_shift = beta[c] + ((cbias ? __ldg(cbias + c) : 0.f) - mean) * sc;
+        gn_affine(rstd, gamma[c], beta[c], cbias ? __ldg(cbias + c) : 0.f, mean, s_scale, s_shift);
+        if (mean_rstd != nullptr && blockIdx.y == 0 && c == g0) {        // one writer per (image, group)
+            mean_rstd[2 * ng] = mean;
+            mean_rstd[2 * ng + 1] = rstd;
+        }
     }
     __syncthreads();
     const float sc = s_scale, sf = s_shift;
@@ -157,7 +170,8 @@ constexpr int kRowsTilesPerWarp = 4;      // 32-pixel tiles per warp and CTA
 __global__ void __launch_bounds__(kRowsWarps * 32)
 group_apply_rows_kernel(const float *__restrict__ x, const double *__restrict__ partial, const float *__restrict__ gamma,
                         const float *__restrict__ beta, float *__restrict__ y, int C, long long hw, int cpg, float eps,
-                        const float *__restrict__ cbias, long long row_stride, long long image_stride, int relu) {
+                        const float *__restrict__ cbias, long long row_stride, long long image_stride, int relu,
+                        float *__restrict__ mean_rstd) {
     // blockIdx.x = image * (C / 32) + channel block, blockIdx.y = pixel range
     __shared__ float s_scale[32], s_shift[32];
     __shared__ float s_tile[kRowsWarps][32 * 33];
@@ -175,9 +189,13 @@ group_apply_rows_kernel(const float *__restrict__ x, const double *__restrict__ 
         double var = b / cnt - mean_k * mean_k;
         var = var < 0.0 ? 0.0 : var;
         const float mean = (float)(mean_k + K);
-        const float sc = (float)(1.0 / sqrt(var + (double)eps)) * gamma[c];
-        s_scale[threadIdx.x] = sc;
-        s_shift[threadIdx.x] = beta[c] + ((cbias ? __ldg(cbias + c) : 0.f) - mean) * sc;
+        const float rstd = (float)(1.0 / sqrt(var + (double)eps));
+        gn_affine(rstd, gamma[c], beta[c], cbias ? __ldg(cbias + c) : 0.f, mean, s_scale[threadIdx.x],
+                  s_shift[threadIdx.x]);
+        if (mean_rstd != nullptr && blockIdx.y == 0 && c % cpg == 0) {
+            mean_rstd[2 * ng] = mean;
+            mean_rstd[2 * ng + 1] = rstd;
+        }
     }
     __syncthreads();
     float *tile = s_tile[warp];
@@ -213,7 +231,7 @@ group_apply_rows_kernel(const float *__restrict__ x, const double *__restrict__ 
 // workspace: N * groups * kGnSplit * 2 doubles
 cudaError_t launch_group_norm(const float *x, const float *cbias, const float *gamma, const float *beta, float *y,
                               int N, int C, int H, int W, int groups, float eps, int relu, const float *up, int uh,
-                              int uw, double *workspace, cudaStream_t stream, bool *handled) {
+                              int uw, double *workspace, float *mean_rstd, cudaStream_t stream, bool *handled) {
     *handled = false;
     const long long hw = (long long)H * W;
     // planes are walked as float4 (H*W % 4 == 0); only the up-sampled add needs 4 outputs of one row (W % 4 == 0)
@@ -240,7 +258,7 @@ cudaError_t launch_group_norm(const float *x, const float *cbias, const float *g
     if (parts > 64) parts = 64;
     const dim3 grid((unsigned)(N * C), (unsigned)parts);
     const float sh = up ? (float)uh / (float)H : 0.f, sw = up ? (float)uw / (float)W : 0.f;
-#define GN_APPLY(R, U) group_apply_kernel<R, U><<<grid, 256, 0, stream>>>(x, workspace, gamma, beta, y, C, H, W, cpg, eps, up, uh, uw, sh, sw, cbias)
+#define GN_APPLY(R, U) group_apply_kernel<R, U><<<grid, 256, 0, stream>>>(x, workspace, gamma, beta, y, C, H, W, cpg, eps, up, uh, uw, sh, sw, cbias, mean_rstd)
     if (up != nullptr) { if (relu) GN_APPLY(true, true); else GN_APPLY(false, true); }
     else { if (relu) GN_APPLY(true, false); else GN_APPLY(false, false); }
 #undef GN_APPLY
@@ -251,7 +269,8 @@ cudaError_t launch_group_norm(const float *x, const float *cbias, const float *g
 // GroupNorm of x[N, C, H*W] written as rows: y[n * image_stride + pixel * row_stride + c]
 cudaError_t launch_group_norm_rows(const float *x, const float *cbias, const float *gamma, const float *beta, float *y,
                                    int N, int C, long long hw, int groups, float eps, int relu, long long row_stride,
-                                   long long image_stride, double *workspace, cudaStream_t stream, bool *handled) {
+                                   long long image_stride, double *workspace, float *mean_rstd, cudaStream_t stream,
+                                   bool *handled) {
     *handled = false;
     if (groups <= 0 || C % groups != 0 || C % 32 != 0 || (hw & 3) || hw > 0x7fffffffLL || row_stride < C ||
         (row_stride & 3) || (image_stride & 3) || (long long)N * (C / 32) > 0x7fffffffLL ||
@@ -274,12 +293,434 @@ cudaError_t launch_group_norm_rows(const float *x, const float *cbias, const flo
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     group_apply_rows_kernel<<<dim3((unsigned)(N * (C / 32)), (unsigned)parts), kRowsWarps * 32, 0, stream>>>(
-        x, workspace, gamma, beta, y, C, hw, cpg, eps, cbias, row_stride, image_stride, relu);
+        x, workspace, gamma, beta, y, C, hw, cpg, eps, cbias, row_stride, image_stride, relu, mean_rstd);
     note_launch();
     return cudaGetLastError();
 }
 
 int group_norm_workspace_doubles(int N, int groups) { return N * groups * kGnSplit * 2; }
+
+// ------------------------------------------------------------------------------------------------ backward
+// With x' = x + cbias[c], xh = (x' - mean) * rstd, gy = grad_y * [ReLU mask] and m = cpg * H * W:
+//   reduce:   per (n, c) plane  A = sum gy,  B = sum gy * xh,  X = sum xh                  (reads grad_y, x)
+//   finalize: per (n, g)  a = sum_c gamma_c A,  b = sum_c gamma_c B;  per c  grad_beta = sum_n A,
+//             grad_gamma = sum_n B,  grad_cbias = sum_n rstd * (gamma_c A - a / cpg - X b / m)  (no pass over the map)
+//   apply:    grad_x = rstd * (gamma_c * gy - a / m - xh * b / m)                            (reads grad_y, x; writes grad_x)
+//   up:       grad_up = the adjoint of the forward's bilinear up-sampling applied to grad_y (unmasked: the add
+//             comes after the ReLU), gathered per source pixel          (reads grad_y, writes grad_up)
+// Partial sums go to fixed slots and are combined in fp64 in a fixed order: no atomics, the same bits every run.
+namespace {
+
+constexpr int kBwdMaxParts = 16;          // reduce-pass CTAs per plane (NCHW) or per 32-channel block (rows)
+constexpr int kBwdThreads = 256;
+
+// per-channel constants of the backward from the forward's (mean, rstd) of group ng
+struct GnChan {
+    float sc, sf;                         // the forward's affine (ReLU mask)
+    float mc, rstd;                       // xh = (x - mc) * rstd, mc = mean - cbias[c]
+};
+
+__device__ __forceinline__ GnChan gn_chan(const float *mean_rstd, long long ng, const float *gamma, const float *beta,
+                                          const float *cbias, int c) {
+    GnChan k;
+    const float mean = __ldg(mean_rstd + 2 * ng), rstd = __ldg(mean_rstd + 2 * ng + 1);
+    const float cb = cbias ? __ldg(cbias + c) : 0.f;
+    gn_affine(rstd, __ldg(gamma + c), __ldg(beta + c), cb, mean, k.sc, k.sf);
+    k.mc = mean - cb;
+    k.rstd = rstd;
+    return k;
+}
+
+// one element of the reduce pass
+__device__ __forceinline__ void gn_bwd_acc(float v, float g, const GnChan &k, bool relu, float &sa, float &sb,
+                                           float &sx) {
+    const float xh = (v - k.mc) * k.rstd;
+    if (relu && !(fmaf(v, k.sc, k.sf) > 0.f)) g = 0.f;
+    sa += g;
+    sb = fmaf(g, xh, sb);
+    sx += xh;
+}
+
+// one element of the apply pass: k1 = rstd * gamma_c, ka = -rstd * a / m, kb = -rstd * b / m
+__device__ __forceinline__ float gn_bwd_dx(float v, float g, const GnChan &k, bool relu, float k1, float ka, float kb) {
+    const float xh = (v - k.mc) * k.rstd;
+    if (relu && !(fmaf(v, k.sc, k.sf) > 0.f)) g = 0.f;
+    return fmaf(k1, g, fmaf(xh, kb, ka));
+}
+
+// blockDim.x = kBwdThreads; the CTA's three sums combined in fp64 and written to slot `out`
+__device__ __forceinline__ void gn_bwd_store_sums(double a, double b, double x, double *out) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        a += __shfl_xor_sync(kFullMask, a, o);
+        b += __shfl_xor_sync(kFullMask, b, o);
+        x += __shfl_xor_sync(kFullMask, x, o);
+    }
+    __shared__ double red[3][kBwdThreads / 32];
+    if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = a; red[1][threadIdx.x >> 5] = b; red[2][threadIdx.x >> 5] = x; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        a = b = x = 0.0;
+        for (int w = 0; w < kBwdThreads / 32; ++w) { a += red[0][w]; b += red[1][w]; x += red[2][w]; }
+        out[0] = a;
+        out[1] = b;
+        out[2] = x;
+    }
+}
+
+template <bool RELU>
+__global__ void __launch_bounds__(kBwdThreads)
+gn_bwd_reduce_kernel(const float *__restrict__ gy, const float *__restrict__ x, const float *__restrict__ mean_rstd,
+                     const float *__restrict__ gamma, const float *__restrict__ beta, const float *__restrict__ cbias,
+                     double *__restrict__ partial, int C, int cpg, long long hw4) {
+    // blockIdx.x = image * C + channel (one plane), blockIdx.y = part of the plane
+    const int plane = blockIdx.x, c = plane % C;
+    const GnChan k = gn_chan(mean_rstd, plane / cpg, gamma, beta, cbias, c);
+    const long long per = (hw4 + gridDim.y - 1) / gridDim.y;
+    const long long beg = (long long)blockIdx.y * per, end = min(beg + per, hw4);
+    const float4 *x4 = reinterpret_cast<const float4 *>(x) + (long long)plane * hw4;
+    const float4 *g4 = reinterpret_cast<const float4 *>(gy) + (long long)plane * hw4;
+    double da = 0.0, db = 0.0, dx = 0.0;           // fp32 within a float4, fp64 across them
+    for (long long i = beg + threadIdx.x; i < end; i += kBwdThreads) {
+        const float4 v = ldg_stream_f4(x4 + i), g = ldg_stream_f4(g4 + i);
+        float sa = 0.f, sb = 0.f, sx = 0.f;
+        gn_bwd_acc(v.x, g.x, k, RELU, sa, sb, sx);
+        gn_bwd_acc(v.y, g.y, k, RELU, sa, sb, sx);
+        gn_bwd_acc(v.z, g.z, k, RELU, sa, sb, sx);
+        gn_bwd_acc(v.w, g.w, k, RELU, sa, sb, sx);
+        da += (double)sa;
+        db += (double)sb;
+        dx += (double)sx;
+    }
+    gn_bwd_store_sums(da, db, dx, partial + ((long long)plane * kBwdMaxParts + blockIdx.y) * 3);
+}
+
+// one CTA per group: the parts of every (n, c) of the group -> abx, the (n, g) sums -> ab, the parameter gradients
+__global__ void __launch_bounds__(kBwdThreads)
+gn_bwd_finalize_kernel(const double *__restrict__ partial, int parts, const float *__restrict__ gamma,
+                       const float *__restrict__ mean_rstd, int N, int C, int cpg, long long hw,
+                       double *__restrict__ abx, double *__restrict__ ab, float *__restrict__ grad_gamma,
+                       float *__restrict__ grad_beta, float *__restrict__ grad_cbias) {
+    const int g = blockIdx.x, groups = C / cpg;
+    for (int i = threadIdx.x; i < N * cpg; i += kBwdThreads) {
+        const long long plane = (long long)(i / cpg) * C + g * cpg + i % cpg;
+        const double *p = partial + plane * kBwdMaxParts * 3;
+        double A = 0.0, B = 0.0, X = 0.0;
+        for (int k = 0; k < parts; ++k) { A += p[3 * k]; B += p[3 * k + 1]; X += p[3 * k + 2]; }
+        abx[plane * 3] = A;
+        abx[plane * 3 + 1] = B;
+        abx[plane * 3 + 2] = X;
+    }
+    __syncthreads();
+    for (int n = threadIdx.x; n < N; n += kBwdThreads) {
+        double a = 0.0, b = 0.0;
+        for (int j = 0; j < cpg; ++j) {
+            const int c = g * cpg + j;
+            const double *s = abx + ((long long)n * C + c) * 3;
+            a += (double)gamma[c] * s[0];
+            b += (double)gamma[c] * s[1];
+        }
+        ab[((long long)n * groups + g) * 2] = a;
+        ab[((long long)n * groups + g) * 2 + 1] = b;
+    }
+    __syncthreads();
+    const double m = (double)cpg * (double)hw;
+    for (int j = threadIdx.x; j < cpg; j += kBwdThreads) {
+        const int c = g * cpg + j;
+        double sg = 0.0, sb = 0.0, scb = 0.0;
+        for (int n = 0; n < N; ++n) {
+            const double *s = abx + ((long long)n * C + c) * 3;
+            const long long ng = (long long)n * groups + g;
+            sb += s[0];
+            sg += s[1];
+            if (grad_cbias)
+                scb += (double)mean_rstd[2 * ng + 1] *
+                       ((double)gamma[c] * s[0] - ab[2 * ng] / cpg - s[2] * ab[2 * ng + 1] / m);
+        }
+        grad_gamma[c] = (float)sg;
+        grad_beta[c] = (float)sb;
+        if (grad_cbias) grad_cbias[c] = (float)scb;
+    }
+}
+
+// the apply pass's per-channel factors from the finalized (n, g) sums
+__device__ __forceinline__ void gn_bwd_factors(const GnChan &k, float gamma, const double *ab, long long ng, double m,
+                                               float &k1, float &ka, float &kb) {
+    k1 = k.rstd * gamma;
+    ka = (float)(-(double)k.rstd * ab[2 * ng] / m);
+    kb = (float)(-(double)k.rstd * ab[2 * ng + 1] / m);
+}
+
+template <bool RELU>
+__global__ void __launch_bounds__(kBwdThreads)
+gn_bwd_apply_kernel(const float *__restrict__ gy, const float *__restrict__ x, const float *__restrict__ mean_rstd,
+                    const float *__restrict__ gamma, const float *__restrict__ beta, const float *__restrict__ cbias,
+                    const double *__restrict__ ab, float *__restrict__ gx, int C, int cpg, long long hw4) {
+    // blockIdx.x = image * C + channel (one plane), blockIdx.y = part of the plane
+    const int plane = blockIdx.x, c = plane % C;
+    __shared__ GnChan s_k;
+    __shared__ float s_f[3];
+    if (threadIdx.x == 0) {
+        s_k = gn_chan(mean_rstd, plane / cpg, gamma, beta, cbias, c);
+        gn_bwd_factors(s_k, __ldg(gamma + c), ab, plane / cpg, (double)cpg * (double)(hw4 * 4), s_f[0], s_f[1], s_f[2]);
+    }
+    __syncthreads();
+    const GnChan k = s_k;
+    const float k1 = s_f[0], ka = s_f[1], kb = s_f[2];
+    const long long per = (hw4 + gridDim.y - 1) / gridDim.y;
+    const long long beg = (long long)blockIdx.y * per, end = min(beg + per, hw4);
+    const float4 *x4 = reinterpret_cast<const float4 *>(x) + (long long)plane * hw4;
+    const float4 *g4 = reinterpret_cast<const float4 *>(gy) + (long long)plane * hw4;
+    float4 *o4 = reinterpret_cast<float4 *>(gx) + (long long)plane * hw4;
+    for (long long i = beg + threadIdx.x; i < end; i += kBwdThreads) {
+        const float4 v = ldg_stream_f4(x4 + i), g = ldg_stream_f4(g4 + i);
+        o4[i] = make_float4(gn_bwd_dx(v.x, g.x, k, RELU, k1, ka, kb), gn_bwd_dx(v.y, g.y, k, RELU, k1, ka, kb),
+                            gn_bwd_dx(v.z, g.z, k, RELU, k1, ka, kb), gn_bwd_dx(v.w, g.w, k, RELU, k1, ka, kb));
+    }
+}
+
+// destinations whose up_index names source s as i0 or i1: their source coordinate lies in [s - 1, s + 1) (for the
+// last source: everything clamped onto it), i.e. dst + 0.5 in [(s - 0.5) / scale, (s + 1.5) / scale).  One index of
+// slack on either side absorbs the rounding of this estimate; the exact test is up_index itself.
+__device__ __forceinline__ void up_range(int s, float scale, int in_size, int out_size, int &lo, int &hi) {
+    lo = max(0, (int)floorf(((float)s - 0.5f) / scale - 0.5f) - 1);
+    hi = s == in_size - 1 ? out_size : min(out_size, (int)ceilf(((float)s + 1.5f) / scale - 0.5f) + 1);
+}
+
+// grad_up[plane][sy][sx] = sum over the destination pixels that read source (sy, sx), with the forward's weights
+__global__ void __launch_bounds__(kBwdThreads)
+gn_bwd_up_kernel(const float *__restrict__ gy, float *__restrict__ gup, int H, int W, int uh, int uw, float sh,
+                 float sw) {
+    // blockIdx.x = plane, blockIdx.y = range of source pixels
+    const float *g = gy + (long long)blockIdx.x * H * W;
+    float *o = gup + (long long)blockIdx.x * uh * uw;
+    for (int s = blockIdx.y * kBwdThreads + threadIdx.x; s < uh * uw; s += gridDim.y * kBwdThreads) {
+        const int sy = s / uw, sx = s - sy * uw;
+        int r0, r1, q0, q1;
+        up_range(sy, sh, uh, H, r0, r1);
+        up_range(sx, sw, uw, W, q0, q1);
+        float acc = 0.f;
+        for (int dr = r0; dr < r1; ++dr) {
+            int y0, y1;
+            float ly;
+            up_index(dr, sh, uh, y0, y1, ly);
+            const float wy = (y0 == sy ? 1.f - ly : 0.f) + (y1 == sy ? ly : 0.f);
+            if (y0 != sy && y1 != sy) continue;
+            const float *row = g + (long long)dr * W;
+            float sum = 0.f;
+            for (int dc = q0; dc < q1; ++dc) {
+                int x0, x1;
+                float lx;
+                up_index(dc, sw, uw, x0, x1, lx);
+                if (x0 != sx && x1 != sx) continue;
+                const float wx = (x0 == sx ? 1.f - lx : 0.f) + (x1 == sx ? lx : 0.f);
+                sum = fmaf(wx, __ldg(row + dc), sum);
+            }
+            acc = fmaf(wy, sum, acc);
+        }
+        o[s] = acc;
+    }
+}
+
+// rows layout: grad_y[n * image_stride + pixel * row_stride + c], x and grad_x NCHW.  One CTA = 32 channels x a range
+// of pixels, as in the forward's rows kernel.  Reduce: a warp stages a 32-channel x 32-pixel tile of x in shared
+// memory and each lane (= one channel) walks the pixels, reading grad_y along the channels of one pixel (128 bytes
+// per warp load).
+__global__ void __launch_bounds__(kRowsWarps * 32)
+gn_bwd_rows_reduce_kernel(const float *__restrict__ gy, long long row_stride, long long image_stride,
+                          const float *__restrict__ x, const float *__restrict__ mean_rstd,
+                          const float *__restrict__ gamma, const float *__restrict__ beta,
+                          const float *__restrict__ cbias, double *__restrict__ partial, int C, long long hw, int cpg,
+                          int relu) {
+    // blockIdx.x = image * (C / 32) + channel block, blockIdx.y = part
+    __shared__ float s_tile[kRowsWarps][32 * 33];
+    __shared__ double s_red[3][kRowsWarps][32];
+    const int cblocks = C / 32, n = blockIdx.x / cblocks, c0 = (blockIdx.x % cblocks) * 32;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, c = c0 + lane;
+    const GnChan k = gn_chan(mean_rstd, (long long)n * (C / cpg) + c / cpg, gamma, beta, cbias, c);
+    float *tile = s_tile[warp];
+    const float *xin = x + ((long long)n * C + c0) * hw;
+    const float *gin = gy + (long long)n * image_stride + c;
+    double da = 0.0, db = 0.0, dx = 0.0;           // fp32 within a tile, fp64 across tiles
+    for (long long t = (long long)blockIdx.y * kRowsWarps + warp; t * 32 < hw; t += (long long)gridDim.y * kRowsWarps) {
+        const long long p0 = t * 32, p = p0 + lane;
+#pragma unroll 8
+        for (int j = 0; j < 32; ++j) tile[j * 33 + lane] = p < hw ? ldg_stream_f1(xin + (long long)j * hw + p) : 0.f;
+        __syncwarp();
+        const int np = (int)min(32LL, hw - p0);
+        float sa = 0.f, sb = 0.f, sx = 0.f;
+        for (int q = 0; q < np; ++q)
+            gn_bwd_acc(tile[lane * 33 + q], ldg_stream_f1(gin + (p0 + q) * row_stride), k, relu != 0, sa, sb, sx);
+        da += (double)sa;
+        db += (double)sb;
+        dx += (double)sx;
+        __syncwarp();
+    }
+    s_red[0][warp][lane] = da;
+    s_red[1][warp][lane] = db;
+    s_red[2][warp][lane] = dx;
+    __syncthreads();
+    if (warp == 0) {
+        double a = 0.0, b = 0.0, xs = 0.0;
+        for (int w = 0; w < kRowsWarps; ++w) { a += s_red[0][w][lane]; b += s_red[1][w][lane]; xs += s_red[2][w][lane]; }
+        double *out = partial + (((long long)n * C + c) * kBwdMaxParts + blockIdx.y) * 3;
+        out[0] = a;
+        out[1] = b;
+        out[2] = xs;
+    }
+}
+
+// apply: a warp turns a 32-pixel x 32-channel tile of grad_y (128-bit loads along the channels of one pixel) through
+// shared memory, then each lane (= one pixel) walks the channels: reads of x and writes of grad_x along the pixels
+__global__ void __launch_bounds__(kRowsWarps * 32)
+gn_bwd_rows_apply_kernel(const float *__restrict__ gy, long long row_stride, long long image_stride,
+                         const float *__restrict__ x, const float *__restrict__ mean_rstd,
+                         const float *__restrict__ gamma, const float *__restrict__ beta,
+                         const float *__restrict__ cbias, const double *__restrict__ ab, float *__restrict__ gx, int C,
+                         long long hw, int cpg, int relu) {
+    // blockIdx.x = image * (C / 32) + channel block, blockIdx.y = pixel range
+    __shared__ GnChan s_k[32];
+    __shared__ float s_k1[32], s_ka[32], s_kb[32];
+    __shared__ float s_tile[kRowsWarps][32 * 33];
+    const int cblocks = C / 32, n = blockIdx.x / cblocks, c0 = (blockIdx.x % cblocks) * 32;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x < 32) {
+        const int c = c0 + threadIdx.x;
+        const long long ng = (long long)n * (C / cpg) + c / cpg;
+        const GnChan k = gn_chan(mean_rstd, ng, gamma, beta, cbias, c);
+        s_k[threadIdx.x] = k;
+        gn_bwd_factors(k, __ldg(gamma + c), ab, ng, (double)cpg * (double)hw, s_k1[threadIdx.x], s_ka[threadIdx.x],
+                       s_kb[threadIdx.x]);
+    }
+    __syncthreads();
+    float *tile = s_tile[warp];
+    const float *xin = x + ((long long)n * C + c0) * hw;
+    float *gout = gx + ((long long)n * C + c0) * hw;
+    const float *gin = gy + (long long)n * image_stride + c0;
+    const int sub = lane >> 3, ch4 = (lane & 7) * 4;
+    const long long first = ((long long)blockIdx.y * kRowsWarps + warp) * kRowsTilesPerWarp;
+    for (int t = 0; t < kRowsTilesPerWarp; ++t) {
+        const long long p0 = (first + t) * 32;
+        if (p0 >= hw) break;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int pix = i * 4 + sub;
+            const float4 g = p0 + pix < hw ? ldg_stream_f4(reinterpret_cast<const float4 *>(gin + (p0 + pix) * row_stride + ch4))
+                                           : make_float4(0.f, 0.f, 0.f, 0.f);
+            tile[(ch4 + 0) * 33 + pix] = g.x;
+            tile[(ch4 + 1) * 33 + pix] = g.y;
+            tile[(ch4 + 2) * 33 + pix] = g.z;
+            tile[(ch4 + 3) * 33 + pix] = g.w;
+        }
+        __syncwarp();
+        const long long p = p0 + lane;
+        if (p < hw) {
+#pragma unroll 8
+            for (int j = 0; j < 32; ++j) {
+                const float v = ldg_stream_f1(xin + (long long)j * hw + p);
+                gout[(long long)j * hw + p] = gn_bwd_dx(v, tile[j * 33 + lane], s_k[j], relu != 0, s_k1[j], s_ka[j], s_kb[j]);
+            }
+        }
+        __syncwarp();
+    }
+}
+
+// workspace (doubles): reduce-pass slots [N*C][kBwdMaxParts][3], per-plane sums [N*C][3], per-group sums [N*C][2]
+// (groups <= C)
+struct GnBwdWs {
+    double *partial, *abx, *ab;
+    GnBwdWs(double *w, long long planes)
+        : partial(w), abx(w + planes * kBwdMaxParts * 3), ab(w + planes * (kBwdMaxParts * 3 + 3)) {}
+};
+
+}  // namespace
+
+long long group_norm_bwd_workspace_doubles(int N, int C) { return (long long)N * C * (kBwdMaxParts * 3 + 3 + 2); }
+
+cudaError_t launch_group_norm_bwd(const float *gy, const float *x, const float *cbias, const float *gamma,
+                                  const float *beta, const float *mean_rstd, float *gx, float *ggamma, float *gbeta,
+                                  float *gcbias, float *gup, int N, int C, int H, int W, int groups, int relu, int uh,
+                                  int uw, double *workspace, cudaStream_t stream, bool *handled) {
+    *handled = false;
+    const long long hw = (long long)H * W;
+    // the forward's requirements
+    if (groups <= 0 || C % groups != 0 || (hw & 3) || (gup != nullptr && (W & 3)) || hw > 0x7fffffffLL ||
+        (long long)N * C > 0x7fffffffLL || (long long)N * groups > 0x7fffffffLL)
+        return cudaSuccess;
+    if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(gy) | reinterpret_cast<uintptr_t>(gx)) & 15u)
+        return cudaSuccess;
+    if (gup != nullptr && (uh <= 0 || uw <= 0 || (long long)uh * uw > 0x7fffffffLL)) return cudaSuccess;
+    *handled = true;
+    const int cpg = C / groups;
+    const long long hw4 = hw >> 2;
+    const GnBwdWs ws(workspace, (long long)N * C);
+    int parts = (int)((hw4 + 4095) / 4096);
+    parts = parts < 1 ? 1 : parts > kBwdMaxParts ? kBwdMaxParts : parts;
+    const dim3 rgrid((unsigned)(N * C), (unsigned)parts);
+    if (relu) gn_bwd_reduce_kernel<true><<<rgrid, kBwdThreads, 0, stream>>>(gy, x, mean_rstd, gamma, beta, cbias, ws.partial, C, cpg, hw4);
+    else gn_bwd_reduce_kernel<false><<<rgrid, kBwdThreads, 0, stream>>>(gy, x, mean_rstd, gamma, beta, cbias, ws.partial, C, cpg, hw4);
+    note_launch();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    gn_bwd_finalize_kernel<<<groups, kBwdThreads, 0, stream>>>(ws.partial, parts, gamma, mean_rstd, N, C, cpg, hw,
+                                                               ws.abx, ws.ab, ggamma, gbeta, gcbias);
+    note_launch();
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    int aparts = (int)((hw4 + 8191) / 8192);
+    aparts = aparts < 1 ? 1 : aparts > 64 ? 64 : aparts;
+    const dim3 agrid((unsigned)(N * C), (unsigned)aparts);
+    if (relu) gn_bwd_apply_kernel<true><<<agrid, kBwdThreads, 0, stream>>>(gy, x, mean_rstd, gamma, beta, cbias, ws.ab, gx, C, cpg, hw4);
+    else gn_bwd_apply_kernel<false><<<agrid, kBwdThreads, 0, stream>>>(gy, x, mean_rstd, gamma, beta, cbias, ws.ab, gx, C, cpg, hw4);
+    note_launch();
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    if (gup != nullptr) {
+        const long long src = (long long)uh * uw;
+        long long uparts = (src + 4 * kBwdThreads - 1) / (4 * kBwdThreads);
+        uparts = uparts < 1 ? 1 : uparts > 64 ? 64 : uparts;
+        gn_bwd_up_kernel<<<dim3((unsigned)(N * C), (unsigned)uparts), kBwdThreads, 0, stream>>>(
+            gy, gup, H, W, uh, uw, (float)uh / (float)H, (float)uw / (float)W);
+        note_launch();
+        e = cudaGetLastError();
+    }
+    return e;
+}
+
+cudaError_t launch_group_norm_rows_bwd(const float *gy, long long row_stride, long long image_stride, const float *x,
+                                       const float *cbias, const float *gamma, const float *beta,
+                                       const float *mean_rstd, float *gx, float *ggamma, float *gbeta, float *gcbias,
+                                       int N, int C, long long hw, int groups, int relu, double *workspace,
+                                       cudaStream_t stream, bool *handled) {
+    *handled = false;
+    // the forward's requirements
+    if (groups <= 0 || C % groups != 0 || C % 32 != 0 || (hw & 3) || hw > 0x7fffffffLL || row_stride < C ||
+        (row_stride & 3) || (image_stride & 3) || (long long)N * (C / 32) > 0x7fffffffLL ||
+        (long long)N * groups > 0x7fffffffLL)
+        return cudaSuccess;
+    if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(gy) | reinterpret_cast<uintptr_t>(gx)) & 15u)
+        return cudaSuccess;
+    const long long per_cta = 32LL * kRowsWarps * kRowsTilesPerWarp;
+    const long long aparts = (hw + per_cta - 1) / per_cta;
+    if (aparts > 65535) return cudaSuccess;
+    *handled = true;
+    const int cpg = C / groups;
+    const GnBwdWs ws(workspace, (long long)N * C);
+    long long parts = (hw + 32LL * kRowsWarps - 1) / (32LL * kRowsWarps);
+    parts = parts > kBwdMaxParts ? kBwdMaxParts : parts;
+    const unsigned cblocks = (unsigned)(N * (C / 32));
+    gn_bwd_rows_reduce_kernel<<<dim3(cblocks, (unsigned)parts), kRowsWarps * 32, 0, stream>>>(
+        gy, row_stride, image_stride, x, mean_rstd, gamma, beta, cbias, ws.partial, C, hw, cpg, relu);
+    note_launch();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    gn_bwd_finalize_kernel<<<groups, kBwdThreads, 0, stream>>>(ws.partial, (int)parts, gamma, mean_rstd, N, C, cpg, hw,
+                                                               ws.abx, ws.ab, ggamma, gbeta, gcbias);
+    note_launch();
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    gn_bwd_rows_apply_kernel<<<dim3(cblocks, (unsigned)aparts), kRowsWarps * 32, 0, stream>>>(
+        gy, row_stride, image_stride, x, mean_rstd, gamma, beta, cbias, ws.ab, gx, C, hw, cpg, relu);
+    note_launch();
+    return cudaGetLastError();
+}
 
 // x[n, c, :, :] += bias[c] in place (the bias of a convolution run without one), 128-bit accesses
 namespace {

@@ -50,12 +50,20 @@ cudaError_t launch_linear_wgrad(const float *, const float *, float *, float *, 
                                 bool *handled);
 cudaError_t launch_transpose(const float *, float *, long long, int, cudaStream_t);
 cudaError_t launch_group_norm(const float *, const float *, const float *, const float *, float *, int, int, int, int,
-                              int, float, int, const float *, int, int, double *, cudaStream_t, bool *handled);
+                              int, float, int, const float *, int, int, double *, float *mean_rstd, cudaStream_t,
+                              bool *handled);
 cudaError_t launch_channel_bias(float *, const float *, int, int, long long, cudaStream_t, bool *handled);
 cudaError_t launch_group_norm_rows(const float *, const float *, const float *, const float *, float *, int, int,
-                                   long long, int, float, int, long long, long long, double *, cudaStream_t,
-                                   bool *handled);
+                                   long long, int, float, int, long long, long long, double *, float *mean_rstd,
+                                   cudaStream_t, bool *handled);
 int group_norm_workspace_doubles(int N, int groups);
+cudaError_t launch_group_norm_bwd(const float *, const float *, const float *, const float *, const float *,
+                                  const float *, float *, float *, float *, float *, float *, int, int, int, int, int,
+                                  int, int, int, double *, cudaStream_t, bool *handled);
+cudaError_t launch_group_norm_rows_bwd(const float *, long long, long long, const float *, const float *, const float *,
+                                       const float *, const float *, float *, float *, float *, float *, int, int,
+                                       long long, int, int, double *, cudaStream_t, bool *handled);
+long long group_norm_bwd_workspace_doubles(int N, int C);
 cudaError_t launch_debug_indices(const int64_t *, const int64_t *, const float *, const Dims &,
                                  int32_t *, int64_t *, cudaStream_t);
 
@@ -394,8 +402,8 @@ int msda_b200_group_norm_nchw_f32(const float *x, const float *channel_bias, con
     if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
     cudaError_t e = launch_group_norm(x, channel_bias, gamma, beta, y, batch, channels, height, width, groups, eps,
-                                      relu, up, up_h, up_w, static_cast<double *>(workspace), (cudaStream_t)stream,
-                                      &handled);
+                                      relu, up, up_h, up_w, static_cast<double *>(workspace), nullptr,
+                                      (cudaStream_t)stream, &handled);
     if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
     return (int)e;
 }
@@ -409,8 +417,75 @@ int msda_b200_group_norm_nchw_to_rows_f32(const float *x, const float *channel_b
         return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
     cudaError_t e = launch_group_norm_rows(x, channel_bias, gamma, beta, y_rows, batch, channels, plane, groups, eps,
-                                           relu, row_stride, image_stride, static_cast<double *>(workspace),
+                                           relu, row_stride, image_stride, static_cast<double *>(workspace), nullptr,
                                            (cudaStream_t)stream, &handled);
+    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
+    return (int)e;
+}
+
+int msda_b200_group_norm_nchw_train_f32(const float *x, const float *channel_bias, const float *gamma,
+                                        const float *beta, float *y, float *mean_rstd, int batch, int channels,
+                                        int height, int width, int groups, float eps, int relu, const float *up,
+                                        int up_h, int up_w, void *workspace, void *stream) {
+    if (!x || !gamma || !beta || !y || !mean_rstd || !workspace) return MSDA_ERR_NULL_POINTER;
+    if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    cudaError_t e = launch_group_norm(x, channel_bias, gamma, beta, y, batch, channels, height, width, groups, eps,
+                                      relu, up, up_h, up_w, static_cast<double *>(workspace), mean_rstd,
+                                      (cudaStream_t)stream, &handled);
+    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
+    return (int)e;
+}
+
+int msda_b200_group_norm_nchw_to_rows_train_f32(const float *x, const float *channel_bias, const float *gamma,
+                                                const float *beta, float *y_rows, float *mean_rstd,
+                                                long long row_stride, long long image_stride, int batch,
+                                                int channels, long long plane, int groups, float eps, int relu,
+                                                void *workspace, void *stream) {
+    if (!x || !gamma || !beta || !y_rows || !mean_rstd || !workspace) return MSDA_ERR_NULL_POINTER;
+    if (batch <= 0 || channels <= 0 || plane <= 0 || groups <= 0 || row_stride < channels || image_stride < 0)
+        return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    cudaError_t e = launch_group_norm_rows(x, channel_bias, gamma, beta, y_rows, batch, channels, plane, groups, eps,
+                                           relu, row_stride, image_stride, static_cast<double *>(workspace),
+                                           mean_rstd, (cudaStream_t)stream, &handled);
+    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
+    return (int)e;
+}
+
+int msda_b200_group_norm_backward_nchw_f32(const float *grad_y, const float *x, const float *channel_bias,
+                                           const float *gamma, const float *beta, const float *mean_rstd,
+                                           float *grad_x, float *grad_gamma, float *grad_beta,
+                                           float *grad_channel_bias, float *grad_up, int batch, int channels,
+                                           int height, int width, int groups, int relu, int up_h, int up_w,
+                                           void *workspace, void *stream) {
+    if (!grad_y || !x || !gamma || !beta || !mean_rstd || !grad_x || !grad_gamma || !grad_beta || !workspace)
+        return MSDA_ERR_NULL_POINTER;
+    if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    cudaError_t e = launch_group_norm_bwd(grad_y, x, channel_bias, gamma, beta, mean_rstd, grad_x, grad_gamma,
+                                          grad_beta, grad_channel_bias, grad_up, batch, channels, height, width, groups,
+                                          relu, up_h, up_w, static_cast<double *>(workspace), (cudaStream_t)stream,
+                                          &handled);
+    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
+    return (int)e;
+}
+
+int msda_b200_group_norm_rows_backward_f32(const float *grad_y_rows, long long row_stride, long long image_stride,
+                                           const float *x, const float *channel_bias, const float *gamma,
+                                           const float *beta, const float *mean_rstd, float *grad_x,
+                                           float *grad_gamma, float *grad_beta, float *grad_channel_bias, int batch,
+                                           int channels, long long plane, int groups, int relu, void *workspace,
+                                           void *stream) {
+    if (!grad_y_rows || !x || !gamma || !beta || !mean_rstd || !grad_x || !grad_gamma || !grad_beta || !workspace)
+        return MSDA_ERR_NULL_POINTER;
+    if (batch <= 0 || channels <= 0 || plane <= 0 || groups <= 0 || row_stride < channels || image_stride < 0)
+        return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    cudaError_t e = launch_group_norm_rows_bwd(grad_y_rows, row_stride, image_stride, x, channel_bias, gamma, beta,
+                                               mean_rstd, grad_x, grad_gamma, grad_beta, grad_channel_bias, batch,
+                                               channels, plane, groups, relu, static_cast<double *>(workspace),
+                                               (cudaStream_t)stream, &handled);
     if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
     return (int)e;
 }
@@ -428,6 +503,11 @@ int msda_b200_add_channel_bias_nchw_f32(float *x, const float *bias, int batch, 
 long long msda_b200_group_norm_workspace_bytes(int batch, int groups) {
     if (batch <= 0 || groups <= 0) return 0;
     return (long long)group_norm_workspace_doubles(batch, groups) * (long long)sizeof(double);
+}
+
+long long msda_b200_group_norm_backward_workspace_bytes(int batch, int channels) {
+    if (batch <= 0 || channels <= 0) return 0;
+    return group_norm_bwd_workspace_doubles(batch, channels) * (long long)sizeof(double);
 }
 
 int msda_b200_transpose_f32(const float *x, float *y, long long rows, int cols, void *stream) {

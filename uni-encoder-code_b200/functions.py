@@ -148,3 +148,87 @@ class AddLayerNormFunction(Function):
         x, residual, weight = ctx.saved_tensors
         gv, gg, gb = ops.add_layernorm_backward(grad_y.contiguous(), x, residual, weight, ctx.eps)
         return gv, gv, gg, gb, None
+
+
+def _aligned(t):
+    """`t` contiguous and 16-byte aligned (the kernels' 128-bit accesses); copies only when it is not."""
+    t = t.contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
+class GroupNormFunction(Function):
+    """``apply(x, weight, bias, channel_bias, up, groups, eps, relu)`` =
+    ``F.group_norm(x + channel_bias[None, :, None, None], groups, weight, bias, eps)`` [-> ``F.relu``]
+    [+ ``F.interpolate(up, size=x.shape[-2:], mode="bilinear", align_corners=False)``] -- the pixel decoder's
+    GroupNorm epilogues (msdeformattn.py:233-248, :369-379) -- with the fused kernels both ways: two launches forward
+    (ops.group_norm_train, bit-identical to ops.group_norm), three backward, four with the gradient of ``up``
+    (ops.group_norm_backward).  ``channel_bias`` and ``up`` may be None.  Saves x and the [N, groups, 2] statistics,
+    not the output; the ReLU mask is rebuilt from x with the forward's own arithmetic."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, channel_bias, up, groups, eps, relu):
+        y, mean_rstd = ops.group_norm_train(x, weight, bias, groups, eps, relu=relu, up=up, channel_bias=channel_bias)
+        ctx.save_for_backward(x, weight, bias, channel_bias, mean_rstd)
+        ctx.groups, ctx.relu = groups, bool(relu)
+        ctx.up_shape = tuple(up.shape[-2:]) if up is not None else None
+        return y
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_y):
+        x, weight, bias, channel_bias, mean_rstd = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        gx, gw, gb, gcb, gup = ops.group_norm_backward(
+            _aligned(grad_y), x, weight, bias, mean_rstd, ctx.groups, relu=ctx.relu, channel_bias=channel_bias,
+            up_shape=ctx.up_shape if need[4] else None, with_channel_bias=channel_bias is not None and need[3])
+        return (gx if need[0] else None, gw if need[1] else None, gb if need[2] else None, gcb, gup, None, None, None)
+
+
+class GroupNormRowsFunction(Function):
+    """``apply(groups, eps, x_0, weight_0, bias_0, channel_bias_0, x_1, ...)`` = the encoder input
+    ``torch.cat([F.group_norm(x_i + channel_bias_i, groups, weight_i, bias_i, eps).flatten(2).transpose(1, 2)], 1)``
+    ([N, sum of H_i * W_i, C]) of the pixel decoder's input projections (msdeformattn.py:341-345, :72-79) as ONE
+    autograd node: every level's GroupNorm writes its rows of the concatenated tensor (ops.group_norm_rows_train) and
+    its backward reads them back from the concatenated gradient (ops.group_norm_rows_backward), so neither the
+    transposing ``cat`` nor its backward runs.  ``channel_bias_i`` may be None.  Two launches per level forward,
+    three backward."""
+
+    @staticmethod
+    def supported(xs, norms) -> bool:
+        """Whether every level qualifies (ops.group_norm_supported, channels a multiple of 32, one batch size, width
+        and device).  The destination the forward allocates, a contiguous [N, S, C] tensor, then meets the rows
+        kernels' stride and alignment requirements at every level's first row."""
+        return (len(xs) > 0 and all(ops.group_norm_supported(x, n) and x.size(1) % 32 == 0 for x, n in zip(xs, norms))
+                and len({(x.size(0), x.size(1), x.device) for x in xs}) == 1)
+
+    @staticmethod
+    def forward(ctx, groups, eps, *level_args):
+        levels = [level_args[i:i + 4] for i in range(0, len(level_args), 4)]
+        x0 = levels[0][0]
+        sizes = [x.size(2) * x.size(3) for x, _, _, _ in levels]
+        out = x0.new_empty((x0.size(0), sum(sizes), x0.size(1)))
+        saved, start = [], 0
+        for (x, weight, bias, channel_bias), hw in zip(levels, sizes):
+            mean_rstd = ops.group_norm_rows_train(x, weight, bias, groups, eps, out[:, start:start + hw],
+                                                  channel_bias=channel_bias)
+            saved += [x, weight, bias, channel_bias, mean_rstd]
+            start += hw
+        ctx.save_for_backward(*saved)
+        ctx.groups, ctx.sizes = groups, sizes
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        grad_out = _aligned(grad_out)
+        saved, need = ctx.saved_tensors, ctx.needs_input_grad
+        grads, start = [None, None], 0
+        for i, hw in enumerate(ctx.sizes):
+            x, weight, bias, channel_bias, mean_rstd = saved[5 * i:5 * i + 5]
+            gx, gw, gb, gcb = ops.group_norm_rows_backward(
+                grad_out[:, start:start + hw], x, weight, bias, mean_rstd, ctx.groups, channel_bias=channel_bias,
+                with_channel_bias=channel_bias is not None and need[2 + 4 * i + 3])
+            k = 2 + 4 * i
+            grads += [gx if need[k] else None, gw if need[k + 1] else None, gb if need[k + 2] else None, gcb]
+            start += hw
+        return tuple(grads)

@@ -24,6 +24,7 @@ import torch.nn.functional as F
 from torch import nn
 
 from . import ops
+from .functions import GroupNormFunction, GroupNormRowsFunction
 from .modules import CoreFn, MSDeformAttnTransformerEncoderOnly, ShapeCache, _capturing
 
 
@@ -74,12 +75,16 @@ class _ConvNormAct(nn.Conv2d):
 
     def forward(self, x, up=None, fused_norm=False):
         """conv -> norm -> activation (-> + bilinear up-sampling of `up`, the FPN top-down add of
-        msdeformattn.py:372-376).  `fused_norm` (inference, GroupNorm, fp32 CUDA): the norm, the ReLU and
-        the up-sampled add run as one statistics + one apply kernel (ops.group_norm, SURVEY 8f.4)."""
+        msdeformattn.py:372-376).  `fused_norm` (GroupNorm, fp32 CUDA): the norm, the ReLU and the up-sampled add
+        run as one statistics + one apply kernel (ops.group_norm, SURVEY 8f.4); with autograd on through
+        GroupNormFunction, whose backward also runs on the library's kernels."""
         x = super().forward(x)
-        if fused_norm and not torch.is_grad_enabled() and self.activation in (None, F.relu) \
-                and ops.group_norm_supported(x, self.norm, up):
-            return ops.group_norm(x, self.norm, relu=self.activation is F.relu, up=up)
+        if fused_norm and self.activation in (None, F.relu) and ops.group_norm_supported(x, self.norm, up):
+            relu = self.activation is F.relu
+            if not torch.is_grad_enabled():
+                return ops.group_norm(x, self.norm, relu=relu, up=up)
+            return GroupNormFunction.apply(x, self.norm.weight, self.norm.bias, None, up, self.norm.num_groups,
+                                           self.norm.eps, relu)
         if self.norm is not None:
             x = self.norm(x)
         x = x if self.activation is None else self.activation(x)
@@ -163,7 +168,14 @@ class MSDeformAttnPixelDecoder(nn.Module):
             for h, w in levels:
                 starts.append(starts[-1] + h * w)
             rows_ok = fused_norm and not torch.is_grad_enabled()
-            for idx, name in enumerate(names):
+            if fused_norm and torch.is_grad_enabled():
+                # training: the convolutions without their bias, then ONE autograd node for the GroupNorms of all
+                # levels that writes the concatenated [N, S, C] encoder input (and reads its gradient) in place
+                src_flat = self._input_proj_train(features, names)
+                if src_flat is not None:
+                    pos = [self.pe_layer(features[name]) for name in names]
+                    rows_ok = True
+            for idx, name in enumerate(names if src_flat is None else []):
                 x = features[name].float()
                 proj = self.input_proj[idx]
                 if fused_norm and not torch.is_grad_enabled():
@@ -200,6 +212,26 @@ class MSDeformAttnPixelDecoder(nn.Module):
                                             fused_norm=fused_norm)
                 out.append(self.output_convs[idx](y, fused_norm=fused_norm))
             return self._mask_features(out[-1], fused_norm), out[0], out[:self.oneformer_num_feature_levels]
+
+    def _input_proj_train(self, features, names):
+        """The input projections under autograd as GroupNormRowsFunction, or None when a level does not qualify
+        (then every level takes torch's path: no level is written into a shared tensor on its own)."""
+        if any(not features[k].is_cuda or (features[k].shape[2] * features[k].shape[3]) % 4 for k in names) or \
+                any(proj[0].out_channels % 32 for proj in self.input_proj):
+            return None                                    # shapes the kernels do not cover: no convolution spent
+        ys, args = [], []
+        for idx, name in enumerate(names):
+            conv, norm = self.input_proj[idx]
+            if not isinstance(norm, nn.GroupNorm):
+                return None
+            ys.append(F.conv2d(features[name].float(), conv.weight, None, conv.stride, conv.padding, conv.dilation,
+                               conv.groups))
+            args += [ys[-1], norm.weight, norm.bias, conv.bias]
+        norms = [proj[1] for proj in self.input_proj]
+        if not GroupNormRowsFunction.supported(ys, norms) or \
+                len({(n.num_groups, n.eps) for n in norms}) != 1:
+            return None
+        return GroupNormRowsFunction.apply(norms[0].num_groups, norms[0].eps, *args)
 
     @staticmethod
     def _nchw(view, memory, fused_norm):
