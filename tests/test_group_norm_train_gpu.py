@@ -6,6 +6,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from test_pixel_decoder import build
+
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 EPS = 1e-5
@@ -217,10 +219,10 @@ def _train_step(pkg, m, feats, cots):
     return [o.detach() for o in outs], grads, fwd, bwd
 
 
-def test_decoder_training_step_on_the_group_norm_kernels_matches_the_torch_path(pkg, monkeypatch):
-    """One forward_features + backward of the full-width decoder with the GroupNorm kernels on against the same step
-    with them off (today's torch path): outputs, every parameter gradient and the feature gradients agree."""
-    m, feats = _full_width_decoder(pkg)
+def _steps_with_the_kernels_on_and_off(pkg, m, feats, monkeypatch):
+    """One forward_features + backward with the GroupNorm kernels on, the same step with them off (both predicates
+    patched to False: torch's path), and that torch step on features moved by ~1e-6.  -> (forward launches on - off,
+    backward launches on - off, worst output error, per-tensor gradient error, per-tensor spread of the moved step)."""
     flags = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.deterministic)
     torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.deterministic = True
@@ -243,13 +245,9 @@ def test_decoder_training_step_on_the_group_norm_kernels_matches_the_torch_path(
             _, again_g, _, _ = _train_step(pkg, m, moved, cots)
     finally:
         torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.deterministic = flags
-    # five GroupNorms: 2 launches each forward; backward 3 per input projection, 3 for the output convolution and
-    # 4 for the lateral (its up-sampled add)
-    assert fwd_on - fwd_off == 5 * 2 and bwd_on - bwd_off == 3 * 3 + 3 + 4
     worst_out = 0.0
     for a, b in zip(got, want):
         worst_out = max(worst_out, (a - b).abs().max().item() / max(1e-30, b.abs().max().item()))
-    assert worst_out <= 1e-4, worst_out
     assert set(got_g) == set(want_g) and "input_proj.0.0.bias" in got_g and "feat::res2" in got_g
 
     def rel(a, b):                      # per tensor: |a - b| / |b| (Frobenius norms)
@@ -259,6 +257,33 @@ def test_decoder_training_step_on_the_group_norm_kernels_matches_the_torch_path(
     top = sorted(err.items(), key=lambda kv: -kv[1])[:4]
     print(f"\ndecoder training step, GroupNorm kernels against torch: outputs {worst_out:.3g}, gradients {top}; "
           f"torch against torch on moved features: {sorted(spread.items(), key=lambda kv: -kv[1])[:4]}")
+    return fwd_on - fwd_off, bwd_on - bwd_off, worst_out, err, spread
+
+
+def test_decoder_training_step_on_the_group_norm_kernels_matches_the_torch_path(pkg, monkeypatch):
+    """One forward_features + backward of the full-width decoder with the GroupNorm kernels on against the same step
+    with them off (today's torch path): outputs, every parameter gradient and the feature gradients agree."""
+    m, feats = _full_width_decoder(pkg)
+    fwd, bwd, worst_out, err, spread = _steps_with_the_kernels_on_and_off(pkg, m, feats, monkeypatch)
+    # five GroupNorms: 2 launches each forward; backward 3 per input projection, 3 for the output convolution and
+    # 4 for the lateral (its up-sampled add)
+    assert fwd == 5 * 2 and bwd == 3 * 3 + 3 + 4
+    assert worst_out <= 1e-4, worst_out
     # observed on a B200: outputs 6.0e-07; gradients at most 1.5e-3 (layers.0.linear1.weight), torch on the moved
     # features at most 1.4e-3 (adapter_1.norm.weight); torch rerun on identical inputs 5e-7
-    assert max(err.values()) <= 3 * max(spread.values()) + 1e-5, top
+    assert max(err.values()) <= 3 * max(spread.values()) + 1e-5, sorted(err.items(), key=lambda kv: -kv[1])[:4]
+
+
+def test_decoder_training_step_with_a_level_the_kernels_do_not_cover(pkg, monkeypatch):
+    """The golden decoder's pyramid has a stride-32 level of 2 x 3 pixels, which no GroupNorm kernel covers: in
+    training too, the covered maps (the stride-8 and stride-16 input projections, the lateral and the output
+    convolution) run on the kernels and that level on torch's path, each input projection on its own."""
+    m, feats, _ = build(pkg, device="cuda:0", fused=True, linear="tf32x3")
+    m.train()
+    torch.manual_seed(5)
+    for proj in m.input_proj:                                  # a non-zero convolution bias, so that it gets tested
+        torch.nn.init.normal_(proj[0].bias, std=0.1)
+    fwd, bwd, worst_out, err, spread = _steps_with_the_kernels_on_and_off(pkg, m, feats, monkeypatch)
+    assert fwd == 4 * 2 and bwd == 3 * 2 + 3 + 4
+    assert worst_out <= 1e-4, worst_out
+    assert max(err.values()) <= 3 * max(spread.values()) + 1e-5, sorted(err.items(), key=lambda kv: -kv[1])[:4]

@@ -430,6 +430,20 @@ def test_group_norm_unsupported_shapes_fall_back_in_the_mirror(pkg):
     assert torch.allclose(a, b, atol=1e-6)
 
 
+@pytest.mark.parametrize("bias", ["float64", "cpu"])
+def test_group_norm_is_not_supported_without_an_fp32_bias_on_the_map_device(pkg, bias):
+    """The kernels read the GroupNorm's bias through a raw fp32 pointer on x's device: any other bias is refused
+    (the decoder then takes torch's path)."""
+    norm = torch.nn.GroupNorm(32, 64).to(DEV)
+    b = norm.bias.detach()
+    norm.bias = torch.nn.Parameter(b.double() if bias == "float64" else b.cpu())
+    x = torch.randn(2, 64, 8, 12, device=DEV)
+    assert not pkg.ops.group_norm_supported(x, norm)
+    assert not pkg.ops.group_norm_rows_supported(x, norm, torch.empty(2, 8 * 12, 64, device=DEV))
+    with pytest.raises(RuntimeError, match="group_norm needs"):
+        pkg.group_norm(x, norm)
+
+
 @pytest.mark.parametrize("shape,groups", [((2, 64, 12, 20), 32), ((3, 256, 8, 16), 32), ((1, 32, 4, 4), 8)])
 def test_group_norm_with_the_convolution_bias_folded_in(pkg, shape, groups):
     """ops.group_norm(x, norm, channel_bias=b) == norm(x + b[None, :, None, None]) (fp64 reference)."""

@@ -86,6 +86,31 @@ __device__ __forceinline__ void gn_affine(float rstd, float gamma, float beta, f
     sf = beta + (cbias - mean) * sc;
 }
 
+// Both apply kernels' first step: (mean, rstd) of group ng (= image * groups + group; N * groups fits 32 bits) from
+// the kGnSplit partials of the statistics pass, and channel c's affine (sc, sf).  With mean_rstd, the CTA of the
+// group's first channel and first part (blockIdx.y == 0 in both kernels) also stores (mean, rstd): one writer per group.
+__device__ __forceinline__ void gn_finalize(const double *__restrict__ partial, const float *__restrict__ x,
+                                            const float *__restrict__ cbias, const float *__restrict__ gamma,
+                                            const float *__restrict__ beta, int ng, int groups, int cpg, long long hw,
+                                            float eps, int c, float *__restrict__ mean_rstd, float &sc, float &sf) {
+    double a = 0.0, b = 0.0;
+    const double *p = partial + (long long)ng * kGnSplit * 2;
+    for (int k = 0; k < kGnSplit; ++k) { a += p[2 * k]; b += p[2 * k + 1]; }
+    const double n = (double)cpg * (double)hw;
+    const int g0 = (ng % groups) * cpg;                                  // the group's first channel
+    const double K = (double)(__ldg(x + (long long)ng * cpg * hw) + (cbias ? __ldg(cbias + g0) : 0.f));
+    const double mean_k = a / n;                                         // mean of (x + cbias - K)
+    double var = b / n - mean_k * mean_k;
+    var = var < 0.0 ? 0.0 : var;
+    const float mean = (float)(mean_k + K);
+    const float rstd = (float)(1.0 / sqrt(var + (double)eps));
+    gn_affine(rstd, gamma[c], beta[c], cbias ? __ldg(cbias + c) : 0.f, mean, sc, sf);
+    if (mean_rstd != nullptr && blockIdx.y == 0 && c == g0) {
+        mean_rstd[2 * ng] = mean;
+        mean_rstd[2 * ng + 1] = rstd;
+    }
+}
+
 // source index of torch's bilinear up-sampling with align_corners=False
 // (area_pixel_compute_source_index: scale * (dst + 0.5) - 0.5, clamped at 0)
 __device__ __forceinline__ void up_index(int dst, float scale, int in_size, int &i0, int &i1, float &l1) {
@@ -103,26 +128,11 @@ group_apply_kernel(const float *__restrict__ x, const double *__restrict__ parti
                    const float *__restrict__ up, int uh, int uw, float sh, float sw,
                    const float *__restrict__ cbias, float *__restrict__ mean_rstd) {
     // blockIdx.x = image * C + channel (one plane), blockIdx.y = part of the plane
-    const int plane = blockIdx.x, c = plane % C, ng = plane / cpg;      // ng = image * groups + group
+    const int plane = blockIdx.x, c = plane % C;
     __shared__ float s_scale, s_shift;
-    if (threadIdx.x == 0) {
-        double a = 0.0, b = 0.0;
-        const double *p = partial + (long long)ng * kGnSplit * 2;
-        for (int k = 0; k < kGnSplit; ++k) { a += p[2 * k]; b += p[2 * k + 1]; }
-        const double n = (double)cpg * H * W;
-        const int g0 = (ng % (C / cpg)) * cpg;                           // the group's first channel
-        const double K = (double)(__ldg(x + (long long)ng * cpg * H * W) + (cbias ? __ldg(cbias + g0) : 0.f));
-        const double mean_k = a / n;                                     // mean of (x + cbias - K)
-        double var = b / n - mean_k * mean_k;
-        var = var < 0.0 ? 0.0 : var;
-        const float mean = (float)(mean_k + K);
-        const float rstd = (float)(1.0 / sqrt(var + (double)eps));
-        gn_affine(rstd, gamma[c], beta[c], cbias ? __ldg(cbias + c) : 0.f, mean, s_scale, s_shift);
-        if (mean_rstd != nullptr && blockIdx.y == 0 && c == g0) {        // one writer per (image, group)
-            mean_rstd[2 * ng] = mean;
-            mean_rstd[2 * ng + 1] = rstd;
-        }
-    }
+    if (threadIdx.x == 0)
+        gn_finalize(partial, x, cbias, gamma, beta, plane / cpg, C / cpg, cpg, (long long)H * W, eps, c, mean_rstd,
+                    s_scale, s_shift);
     __syncthreads();
     const float sc = s_scale, sf = s_shift;
     const long long hw4 = ((long long)H * W) >> 2;
@@ -178,24 +188,9 @@ group_apply_rows_kernel(const float *__restrict__ x, const double *__restrict__ 
     const int cblocks = C / 32, n = blockIdx.x / cblocks, c0 = (blockIdx.x % cblocks) * 32;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (threadIdx.x < 32) {
-        const int c = c0 + threadIdx.x, groups = C / cpg, g = c / cpg;
-        const long long ng = (long long)n * groups + g;
-        double a = 0.0, b = 0.0;
-        const double *p = partial + ng * kGnSplit * 2;
-        for (int k = 0; k < kGnSplit; ++k) { a += p[2 * k]; b += p[2 * k + 1]; }
-        const double cnt = (double)cpg * (double)hw;
-        const double K = (double)(__ldg(x + ng * cpg * hw) + (cbias ? __ldg(cbias + g * cpg) : 0.f));
-        const double mean_k = a / cnt;
-        double var = b / cnt - mean_k * mean_k;
-        var = var < 0.0 ? 0.0 : var;
-        const float mean = (float)(mean_k + K);
-        const float rstd = (float)(1.0 / sqrt(var + (double)eps));
-        gn_affine(rstd, gamma[c], beta[c], cbias ? __ldg(cbias + c) : 0.f, mean, s_scale[threadIdx.x],
-                  s_shift[threadIdx.x]);
-        if (mean_rstd != nullptr && blockIdx.y == 0 && c % cpg == 0) {
-            mean_rstd[2 * ng] = mean;
-            mean_rstd[2 * ng + 1] = rstd;
-        }
+        const int c = c0 + threadIdx.x;
+        gn_finalize(partial, x, cbias, gamma, beta, n * (C / cpg) + c / cpg, C / cpg, cpg, hw, eps, c, mean_rstd,
+                    s_scale[threadIdx.x], s_shift[threadIdx.x]);
     }
     __syncthreads();
     float *tile = s_tile[warp];
@@ -226,23 +221,38 @@ group_apply_rows_kernel(const float *__restrict__ x, const double *__restrict__ 
     }
 }
 
-}  // namespace
-
-// workspace: N * groups * kGnSplit * 2 doubles
-cudaError_t launch_group_norm(const float *x, const float *cbias, const float *gamma, const float *beta, float *y,
-                              int N, int C, int H, int W, int groups, float eps, int relu, const float *up, int uh,
-                              int uw, double *workspace, float *mean_rstd, cudaStream_t stream, bool *handled) {
-    *handled = false;
+// What the NCHW kernels need, forward and backward: planes walked as float4 (H*W % 4 == 0; W % 4 == 0 as well with
+// the up-sampled map, whose add takes 4 outputs of one row), 32-bit plane and chunk counts, and 16-byte aligned maps
+// (`maps`: their addresses or-ed together)
+bool gn_nchw_ok(int N, int C, int H, int W, int groups, bool up, uintptr_t maps) {
     const long long hw = (long long)H * W;
-    // planes are walked as float4 (H*W % 4 == 0); only the up-sampled add needs 4 outputs of one row (W % 4 == 0)
-    if (groups <= 0 || C % groups != 0 || (hw & 3) || (up != nullptr && (W & 3)) || hw > 0x7fffffffLL ||
-        (long long)N * C > 0x7fffffffLL || (long long)N * groups > 0x7fffffffLL)
-        return cudaSuccess;
-    if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15u) return cudaSuccess;
-    if (up != nullptr && (uh <= 0 || uw <= 0)) return cudaSuccess;
+    return groups > 0 && C % groups == 0 && !(hw & 3) && !(up && (W & 3)) && hw <= 0x7fffffffLL &&
+           (long long)N * C <= 0x7fffffffLL && (long long)N * groups <= 0x7fffffffLL && !(maps & 15u);
+}
+
+// pixel ranges of the rows kernels' apply grid (blockIdx.y)
+long long gn_rows_parts(long long hw) {
+    const long long per_cta = 32LL * kRowsWarps * kRowsTilesPerWarp;
+    return (hw + per_cta - 1) / per_cta;
+}
+
+// What the rows kernels need, forward and backward: 32-channel blocks, planes of whole float4, rows of whole float4
+// (row and image strides), 16-byte aligned maps and rows (`maps`), and at most 65535 pixel ranges
+bool gn_rows_ok(int N, int C, long long hw, int groups, long long row_stride, long long image_stride, uintptr_t maps) {
+    return groups > 0 && C % groups == 0 && C % 32 == 0 && !(hw & 3) && hw <= 0x7fffffffLL && row_stride >= C &&
+           !(row_stride & 3) && !(image_stride & 3) && (long long)N * (C / 32) <= 0x7fffffffLL &&
+           (long long)N * groups <= 0x7fffffffLL && !(maps & 15u) && gn_rows_parts(hw) <= 65535;
+}
+
+uintptr_t addr(const void *p) { return reinterpret_cast<uintptr_t>(p); }
+
+// The first launch of both forward layouts: the kGnSplit partial sums of every (image, group) chunk of x (+ cbias).
+// Sets *handled unless the chunk is too long for the CBIAS variant's 32-bit channel lookup.
+cudaError_t launch_group_stats(const float *x, const float *cbias, int N, int C, long long hw, int groups,
+                               double *workspace, cudaStream_t stream, bool *handled) {
     const int cpg = C / groups;
     const long long chunk = (long long)cpg * hw;
-    if (cbias != nullptr && chunk > 0x7fffffffLL) return cudaSuccess;    // 32-bit channel lookup in the statistics pass
+    if (cbias != nullptr && chunk > 0x7fffffffLL) return cudaSuccess;
     *handled = true;
     const dim3 sgrid((unsigned)(N * groups), kGnSplit);
     if (cbias != nullptr)
@@ -250,13 +260,27 @@ cudaError_t launch_group_norm(const float *x, const float *cbias, const float *g
     else
         group_stats_kernel<false><<<sgrid, kGnThreads, 0, stream>>>(x, workspace, chunk, nullptr, groups, cpg, 1u);
     note_launch();
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
+    return cudaGetLastError();
+}
+
+}  // namespace
+
+// workspace: N * groups * kGnSplit * 2 doubles
+cudaError_t launch_group_norm(const float *x, const float *cbias, const float *gamma, const float *beta, float *y,
+                              int N, int C, int H, int W, int groups, float eps, int relu, const float *up, int uh,
+                              int uw, double *workspace, float *mean_rstd, cudaStream_t stream, bool *handled) {
+    *handled = false;
+    if (!gn_nchw_ok(N, C, H, W, groups, up != nullptr, addr(x) | addr(y)) || (up != nullptr && (uh <= 0 || uw <= 0)))
+        return cudaSuccess;
+    const long long hw = (long long)H * W;
+    cudaError_t e = launch_group_stats(x, cbias, N, C, hw, groups, workspace, stream, handled);
+    if (e != cudaSuccess || !*handled) return e;
     // parts per plane: enough CTAs for the whole GPU, each with a few thousand float4
     int parts = (int)((hw / 4 + 8191) / 8192);
     if (parts < 1) parts = 1;
     if (parts > 64) parts = 64;
     const dim3 grid((unsigned)(N * C), (unsigned)parts);
+    const int cpg = C / groups;
     const float sh = up ? (float)uh / (float)H : 0.f, sw = up ? (float)uw / (float)W : 0.f;
 #define GN_APPLY(R, U) group_apply_kernel<R, U><<<grid, 256, 0, stream>>>(x, workspace, gamma, beta, y, C, H, W, cpg, eps, up, uh, uw, sh, sw, cbias, mean_rstd)
     if (up != nullptr) { if (relu) GN_APPLY(true, true); else GN_APPLY(false, true); }
@@ -272,28 +296,11 @@ cudaError_t launch_group_norm_rows(const float *x, const float *cbias, const flo
                                    long long image_stride, double *workspace, float *mean_rstd, cudaStream_t stream,
                                    bool *handled) {
     *handled = false;
-    if (groups <= 0 || C % groups != 0 || C % 32 != 0 || (hw & 3) || hw > 0x7fffffffLL || row_stride < C ||
-        (row_stride & 3) || (image_stride & 3) || (long long)N * (C / 32) > 0x7fffffffLL ||
-        (long long)N * groups > 0x7fffffffLL)
-        return cudaSuccess;
-    if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15u) return cudaSuccess;
-    const int cpg = C / groups;
-    const long long chunk = (long long)cpg * hw;
-    if (cbias != nullptr && chunk > 0x7fffffffLL) return cudaSuccess;
-    const long long per_cta = 32LL * kRowsWarps * kRowsTilesPerWarp;
-    const long long parts = (hw + per_cta - 1) / per_cta;
-    if (parts > 65535) return cudaSuccess;
-    *handled = true;
-    const dim3 sgrid((unsigned)(N * groups), kGnSplit);
-    if (cbias != nullptr)
-        group_stats_kernel<true><<<sgrid, kGnThreads, 0, stream>>>(x, workspace, chunk, cbias, groups, cpg, (unsigned)(hw >> 2));
-    else
-        group_stats_kernel<false><<<sgrid, kGnThreads, 0, stream>>>(x, workspace, chunk, nullptr, groups, cpg, 1u);
-    note_launch();
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return e;
-    group_apply_rows_kernel<<<dim3((unsigned)(N * (C / 32)), (unsigned)parts), kRowsWarps * 32, 0, stream>>>(
-        x, workspace, gamma, beta, y, C, hw, cpg, eps, cbias, row_stride, image_stride, relu, mean_rstd);
+    if (!gn_rows_ok(N, C, hw, groups, row_stride, image_stride, addr(x) | addr(y))) return cudaSuccess;
+    cudaError_t e = launch_group_stats(x, cbias, N, C, hw, groups, workspace, stream, handled);
+    if (e != cudaSuccess || !*handled) return e;
+    group_apply_rows_kernel<<<dim3((unsigned)(N * (C / 32)), (unsigned)gn_rows_parts(hw)), kRowsWarps * 32, 0, stream>>>(
+        x, workspace, gamma, beta, y, C, hw, C / groups, eps, cbias, row_stride, image_stride, relu, mean_rstd);
     note_launch();
     return cudaGetLastError();
 }
@@ -642,17 +649,12 @@ cudaError_t launch_group_norm_bwd(const float *gy, const float *x, const float *
                                   float *gcbias, float *gup, int N, int C, int H, int W, int groups, int relu, int uh,
                                   int uw, double *workspace, cudaStream_t stream, bool *handled) {
     *handled = false;
-    const long long hw = (long long)H * W;
-    // the forward's requirements
-    if (groups <= 0 || C % groups != 0 || (hw & 3) || (gup != nullptr && (W & 3)) || hw > 0x7fffffffLL ||
-        (long long)N * C > 0x7fffffffLL || (long long)N * groups > 0x7fffffffLL)
+    if (!gn_nchw_ok(N, C, H, W, groups, gup != nullptr, addr(x) | addr(gy) | addr(gx)) ||
+        (gup != nullptr && (uh <= 0 || uw <= 0 || (long long)uh * uw > 0x7fffffffLL)))
         return cudaSuccess;
-    if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(gy) | reinterpret_cast<uintptr_t>(gx)) & 15u)
-        return cudaSuccess;
-    if (gup != nullptr && (uh <= 0 || uw <= 0 || (long long)uh * uw > 0x7fffffffLL)) return cudaSuccess;
     *handled = true;
     const int cpg = C / groups;
-    const long long hw4 = hw >> 2;
+    const long long hw = (long long)H * W, hw4 = hw >> 2;
     const GnBwdWs ws(workspace, (long long)N * C);
     int parts = (int)((hw4 + 4095) / 4096);
     parts = parts < 1 ? 1 : parts > kBwdMaxParts ? kBwdMaxParts : parts;
@@ -691,16 +693,7 @@ cudaError_t launch_group_norm_rows_bwd(const float *gy, long long row_stride, lo
                                        int N, int C, long long hw, int groups, int relu, double *workspace,
                                        cudaStream_t stream, bool *handled) {
     *handled = false;
-    // the forward's requirements
-    if (groups <= 0 || C % groups != 0 || C % 32 != 0 || (hw & 3) || hw > 0x7fffffffLL || row_stride < C ||
-        (row_stride & 3) || (image_stride & 3) || (long long)N * (C / 32) > 0x7fffffffLL ||
-        (long long)N * groups > 0x7fffffffLL)
-        return cudaSuccess;
-    if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(gy) | reinterpret_cast<uintptr_t>(gx)) & 15u)
-        return cudaSuccess;
-    const long long per_cta = 32LL * kRowsWarps * kRowsTilesPerWarp;
-    const long long aparts = (hw + per_cta - 1) / per_cta;
-    if (aparts > 65535) return cudaSuccess;
+    if (!gn_rows_ok(N, C, hw, groups, row_stride, image_stride, addr(x) | addr(gy) | addr(gx))) return cudaSuccess;
     *handled = true;
     const int cpg = C / groups;
     const GnBwdWs ws(workspace, (long long)N * C);
@@ -716,7 +709,7 @@ cudaError_t launch_group_norm_rows_bwd(const float *gy, long long row_stride, lo
                                                                ws.abx, ws.ab, ggamma, gbeta, gcbias);
     note_launch();
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    gn_bwd_rows_apply_kernel<<<dim3(cblocks, (unsigned)aparts), kRowsWarps * 32, 0, stream>>>(
+    gn_bwd_rows_apply_kernel<<<dim3(cblocks, (unsigned)gn_rows_parts(hw)), kRowsWarps * 32, 0, stream>>>(
         gy, row_stride, image_stride, x, mean_rstd, gamma, beta, cbias, ws.ab, gx, C, hw, cpg, relu);
     note_launch();
     return cudaGetLastError();

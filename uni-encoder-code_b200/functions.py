@@ -194,14 +194,6 @@ class GroupNormRowsFunction(Function):
     three backward."""
 
     @staticmethod
-    def supported(xs, norms) -> bool:
-        """Whether every level qualifies (ops.group_norm_supported, channels a multiple of 32, one batch size, width
-        and device).  The destination the forward allocates, a contiguous [N, S, C] tensor, then meets the rows
-        kernels' stride and alignment requirements at every level's first row."""
-        return (len(xs) > 0 and all(ops.group_norm_supported(x, n) and x.size(1) % 32 == 0 for x, n in zip(xs, norms))
-                and len({(x.size(0), x.size(1), x.device) for x in xs}) == 1)
-
-    @staticmethod
     def forward(ctx, groups, eps, *level_args):
         levels = [level_args[i:i + 4] for i in range(0, len(level_args), 4)]
         x0 = levels[0][0]

@@ -390,18 +390,104 @@ def add_layernorm(x, residual, weight, bias, eps=1e-5):
     return y
 
 
+def _vec_ok(t, x) -> bool:
+    return (isinstance(t, torch.Tensor) and t.device == x.device and t.dtype == torch.float32 and t.is_contiguous()
+            and t.shape == (x.size(1),))
+
+
+def _map_ok(x, weight, bias, groups, up=None) -> bool:
+    """What every GroupNorm kernel needs of an NCHW map: x contiguous fp32 on a CUDA device, 16-byte aligned, with H*W
+    a multiple of 4 (the planes are walked as float4); weight and bias contiguous fp32 [C] on x's device; C divisible
+    by groups; with `up` (the map the forward up-samples and adds): W a multiple of 4 as well, and `up` a contiguous
+    fp32 map with x's batch and channels on x's device."""
+    return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 4
+            and x.is_contiguous() and x.numel() > 0 and (x.size(2) * x.size(3)) % 4 == 0 and x.data_ptr() % 16 == 0
+            and isinstance(groups, int) and groups > 0 and x.size(1) % groups == 0 and _vec_ok(weight, x)
+            and _vec_ok(bias, x)
+            and (up is None or (isinstance(up, torch.Tensor) and up.dtype == torch.float32 and up.dim() == 4
+                                and up.is_contiguous() and up.device == x.device and up.shape[:2] == x.shape[:2]
+                                and x.size(3) % 4 == 0)))
+
+
+def _rows_view_ok(rows, x) -> bool:
+    """What the rows kernels need besides the map: C a multiple of 32, and `rows` an fp32 [N, H*W, C] view on x's device
+    with unit channel stride and 16-byte aligned rows (e.g. a level's slice of the concatenated [N, S, C] tensor)."""
+    return (x.size(1) % 32 == 0 and isinstance(rows, torch.Tensor) and rows.device == x.device
+            and rows.dtype == torch.float32 and rows.dim() == 3
+            and tuple(rows.shape) == (x.size(0), x.size(2) * x.size(3), x.size(1)) and rows.stride(2) == 1
+            and rows.stride(1) >= x.size(1) and rows.stride(1) % 4 == 0 and rows.stride(0) % 4 == 0
+            and rows.data_ptr() % 16 == 0)
+
+
+def _check_channel_bias(channel_bias, x):
+    if channel_bias is not None and not _vec_ok(channel_bias, x):
+        raise RuntimeError("channel_bias must be a contiguous fp32 [C] tensor on x's device")
+
+
+def _check_mean_rstd(mean_rstd, x, groups):
+    if not (isinstance(mean_rstd, torch.Tensor) and mean_rstd.device == x.device and mean_rstd.dtype == torch.float32
+            and mean_rstd.is_contiguous() and mean_rstd.shape == (x.size(0), groups, 2)):
+        raise RuntimeError("mean_rstd must be the contiguous fp32 [N, groups, 2] tensor of the training forward")
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+def _workspace(nbytes, x):
+    return torch.empty(int(nbytes), dtype=torch.uint8, device=x.device)
+
+
 def group_norm_supported(x, norm, up=None) -> bool:
-    """Whether the fused GroupNorm kernel covers `norm(x)` (x: NCHW fp32 CUDA, contiguous)."""
-    ok = (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 4
-          and x.is_contiguous() and x.numel() > 0 and isinstance(norm, torch.nn.GroupNorm) and norm.affine
-          and norm.weight is not None and norm.bias is not None and norm.weight.device == x.device
-          and norm.weight.dtype == torch.float32 and norm.weight.is_contiguous() and norm.bias.is_contiguous()
-          and x.size(1) == norm.num_channels and (x.size(2) * x.size(3)) % 4 == 0
-          and x.data_ptr() % 16 == 0)
-    if ok and up is not None:
-        ok = (up.is_cuda and up.dtype == torch.float32 and up.dim() == 4 and up.is_contiguous()
-              and up.device == x.device and up.shape[:2] == x.shape[:2] and x.size(3) % 4 == 0)
-    return ok
+    """Whether the fused GroupNorm kernels cover `norm(x)` (x: NCHW fp32 CUDA, contiguous; `norm` an affine
+    nn.GroupNorm whose parameters are contiguous fp32 [C] tensors on x's device)."""
+    return isinstance(norm, torch.nn.GroupNorm) and _map_ok(x, norm.weight, norm.bias, norm.num_groups, up)
+
+
+def group_norm_rows_supported(x, norm, out_rows) -> bool:
+    """Whether `group_norm_rows` covers these tensors: the map as for `group_norm`, channels a multiple of 32, and
+    `out_rows` an fp32 [N, H*W, C] view with unit channel stride (a slice of the concatenated [N, S, C] tensor)."""
+    return group_norm_supported(x, norm) and _rows_view_ok(out_rows, x)
+
+
+def _group_norm_nchw(name, x, weight, bias, groups, eps, relu, up, channel_bias, stats):
+    """The NCHW forward -> (y, mean_rstd [N, groups, 2] when `stats`, else None)."""
+    if not _map_ok(x, weight, bias, groups, up):
+        raise RuntimeError(f"{name} needs a contiguous NCHW fp32 CUDA map with H*W (and, with `up`, W) a multiple of 4, "
+                           "contiguous fp32 [C] weight and bias on the same device, C divisible by groups and, if "
+                           "given, a contiguous `up` map with the same batch and channels")
+    _check_channel_bias(channel_bias, x)
+    N, C, H, W = x.shape
+    y = torch.empty_like(x)
+    mean_rstd = torch.empty(N, groups, 2, dtype=torch.float32, device=x.device) if stats else None
+    with torch.cuda.device(x.device):
+        ws = _workspace(_lib.lib.msda_b200_group_norm_workspace_bytes(N, groups), x)
+        head = (x.data_ptr(), _ptr(channel_bias), weight.data_ptr(), bias.data_ptr(), y.data_ptr())
+        tail = (N, C, H, W, groups, float(eps), int(bool(relu)), _ptr(up), up.size(2) if up is not None else 0,
+                up.size(3) if up is not None else 0, ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)
+        rc = (_lib.lib.msda_b200_group_norm_nchw_train_f32(*head, mean_rstd.data_ptr(), *tail) if stats
+              else _lib.lib.msda_b200_group_norm_nchw_f32(*head, *tail))
+    _lib.check(rc, name)
+    return y, mean_rstd
+
+
+def _group_norm_rows(name, x, weight, bias, groups, eps, out_rows, channel_bias, relu, stats):
+    """The rows forward: writes out_rows -> mean_rstd [N, groups, 2] when `stats`, else None."""
+    if not (_map_ok(x, weight, bias, groups) and _rows_view_ok(out_rows, x)):
+        raise RuntimeError(f"{name} needs what group_norm needs, channels % 32 == 0 and an fp32 [N, H*W, C] "
+                           "destination view with unit channel stride on the same device")
+    _check_channel_bias(channel_bias, x)
+    N, C, H, W = x.shape
+    mean_rstd = torch.empty(N, groups, 2, dtype=torch.float32, device=x.device) if stats else None
+    with torch.cuda.device(x.device):
+        ws = _workspace(_lib.lib.msda_b200_group_norm_workspace_bytes(N, groups), x)
+        head = (x.data_ptr(), _ptr(channel_bias), weight.data_ptr(), bias.data_ptr(), out_rows.data_ptr())
+        tail = (out_rows.stride(1), out_rows.stride(0), N, C, H * W, groups, float(eps), int(bool(relu)), ws.data_ptr(),
+                torch.cuda.current_stream(x.device).cuda_stream)
+        rc = (_lib.lib.msda_b200_group_norm_nchw_to_rows_train_f32(*head, mean_rstd.data_ptr(), *tail) if stats
+              else _lib.lib.msda_b200_group_norm_nchw_to_rows_f32(*head, *tail))
+    _lib.check(rc, name)
+    return mean_rstd
 
 
 def group_norm(x, norm, relu=False, up=None, channel_bias=None):
@@ -411,37 +497,8 @@ def group_norm(x, norm, relu=False, up=None, channel_bias=None):
     pixel decoder's input projections and FPN level (msdeformattn.py:233-248, :369-379) -- in two passes
     over x (statistics, apply) instead of torch's four to six kernels.  No autograd: training goes through
     functions.GroupNormFunction (group_norm_train / group_norm_backward)."""
-    if not group_norm_supported(x, norm, up):
-        raise RuntimeError("group_norm needs a contiguous NCHW fp32 CUDA map with H*W (and, with `up`, W) a multiple of 4, "
-                           "an affine nn.GroupNorm on the same device and, if given, a contiguous `up` map "
-                           "with the same batch and channels")
-    N, C, H, W = x.shape
-    if channel_bias is not None and not (channel_bias.is_cuda and channel_bias.device == x.device
-                                         and channel_bias.dtype == torch.float32 and channel_bias.is_contiguous()
-                                         and channel_bias.shape == (C,)):
-        raise RuntimeError("channel_bias must be a contiguous fp32 [C] tensor on x's device")
-    y = torch.empty_like(x)
-    with torch.cuda.device(x.device):
-        ws = torch.empty(int(_lib.lib.msda_b200_group_norm_workspace_bytes(N, norm.num_groups)), dtype=torch.uint8,
-                         device=x.device)
-        rc = _lib.lib.msda_b200_group_norm_nchw_f32(
-            x.data_ptr(), channel_bias.data_ptr() if channel_bias is not None else None,
-            norm.weight.data_ptr(), norm.bias.data_ptr(), y.data_ptr(), N, C, H, W, norm.num_groups,
-            float(norm.eps), int(bool(relu)), up.data_ptr() if up is not None else None,
-            up.size(2) if up is not None else 0, up.size(3) if up is not None else 0, ws.data_ptr(),
-            torch.cuda.current_stream(x.device).cuda_stream)
-    _lib.check(rc, "group_norm")
-    return y
-
-
-def group_norm_rows_supported(x, norm, out_rows) -> bool:
-    """Whether `group_norm_rows` covers these tensors: the map as for `group_norm`, channels a multiple of 32, and
-    `out_rows` an fp32 [N, H*W, C] view with unit channel stride (a slice of the concatenated [N, S, C] tensor)."""
-    return (group_norm_supported(x, norm) and x.size(1) % 32 == 0 and isinstance(out_rows, torch.Tensor)
-            and out_rows.is_cuda and out_rows.device == x.device and out_rows.dtype == torch.float32
-            and out_rows.dim() == 3 and tuple(out_rows.shape) == (x.size(0), x.size(2) * x.size(3), x.size(1))
-            and out_rows.stride(2) == 1 and out_rows.stride(1) >= x.size(1) and out_rows.stride(1) % 4 == 0
-            and out_rows.stride(0) % 4 == 0 and out_rows.data_ptr() % 16 == 0)
+    return _group_norm_nchw("group_norm", x, norm.weight, norm.bias, norm.num_groups, norm.eps, relu, up, channel_bias,
+                            False)[0]
 
 
 def group_norm_rows(x, norm, out_rows, channel_bias=None, relu=False):
@@ -449,31 +506,14 @@ def group_norm_rows(x, norm, out_rows, channel_bias=None, relu=False):
     straight into the ``[N, pixels, C]`` layout of the deformable encoder (``src.flatten(2).transpose(1, 2)``),
     e.g. into the level's rows of the concatenated tensor.  No autograd: training goes through
     functions.GroupNormRowsFunction (group_norm_rows_train / group_norm_rows_backward).  Returns out_rows."""
-    if not group_norm_rows_supported(x, norm, out_rows):
-        raise RuntimeError("group_norm_rows needs what group_norm needs, channels % 32 == 0 and an fp32 [N, H*W, C] "
-                           "destination view with unit channel stride on the same device")
-    N, C, H, W = x.shape
-    if channel_bias is not None and not (channel_bias.is_cuda and channel_bias.device == x.device
-                                         and channel_bias.dtype == torch.float32 and channel_bias.is_contiguous()
-                                         and channel_bias.shape == (C,)):
-        raise RuntimeError("channel_bias must be a contiguous fp32 [C] tensor on x's device")
-    with torch.cuda.device(x.device):
-        ws = torch.empty(int(_lib.lib.msda_b200_group_norm_workspace_bytes(N, norm.num_groups)), dtype=torch.uint8,
-                         device=x.device)
-        rc = _lib.lib.msda_b200_group_norm_nchw_to_rows_f32(
-            x.data_ptr(), channel_bias.data_ptr() if channel_bias is not None else None, norm.weight.data_ptr(),
-            norm.bias.data_ptr(), out_rows.data_ptr(), out_rows.stride(1), out_rows.stride(0), N, C, H * W,
-            norm.num_groups, float(norm.eps), int(bool(relu)), ws.data_ptr(),
-            torch.cuda.current_stream(x.device).cuda_stream)
-    _lib.check(rc, "group_norm_rows")
+    _group_norm_rows("group_norm_rows", x, norm.weight, norm.bias, norm.num_groups, norm.eps, out_rows, channel_bias,
+                     relu, False)
     return out_rows
 
 
 def channel_bias_supported(x, bias) -> bool:
-    return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 4
-            and x.is_contiguous() and x.numel() > 0 and (x.size(2) * x.size(3)) % 4 == 0 and x.data_ptr() % 16 == 0
-            and isinstance(bias, torch.Tensor) and bias.device == x.device and bias.dtype == torch.float32
-            and bias.is_contiguous() and bias.shape == (x.size(1),))
+    # the map predicate with the bias in the place of both affine parameters (one group)
+    return _map_ok(x, bias, bias, 1)
 
 
 def add_channel_bias_(x, bias):
@@ -550,56 +590,17 @@ def add_layernorm_backward(grad_y, x, residual, weight, eps=1e-5):
 
 
 # ---------------------------------------------------------------- GroupNorm training (forward + backward)
-def _gn_params_ok(x, weight, bias, groups) -> bool:
-    """x: contiguous NCHW fp32 CUDA map as group_norm needs; weight / bias: contiguous fp32 [C] on x's device."""
-    def vec_ok(t):
-        return (isinstance(t, torch.Tensor) and t.device == x.device and t.dtype == torch.float32
-                and t.is_contiguous() and t.shape == (x.size(1),))
-    return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 4
-            and x.is_contiguous() and x.numel() > 0 and (x.size(2) * x.size(3)) % 4 == 0 and x.data_ptr() % 16 == 0
-            and isinstance(groups, int) and groups > 0 and x.size(1) % groups == 0 and vec_ok(weight) and vec_ok(bias))
-
-
-def _check_channel_bias(channel_bias, x):
-    if channel_bias is not None and not (channel_bias.is_cuda and channel_bias.device == x.device
-                                         and channel_bias.dtype == torch.float32 and channel_bias.is_contiguous()
-                                         and channel_bias.shape == (x.size(1),)):
-        raise RuntimeError("channel_bias must be a contiguous fp32 [C] tensor on x's device")
-
-
-def _up_ok(x, up) -> bool:
-    return (isinstance(up, torch.Tensor) and up.is_cuda and up.dtype == torch.float32 and up.dim() == 4
-            and up.is_contiguous() and up.device == x.device and up.shape[:2] == x.shape[:2] and x.size(3) % 4 == 0)
-
-
 def group_norm_train(x, weight, bias, groups, eps, relu=False, up=None, channel_bias=None):
     """Training forward of ``group_norm``: ``(y, mean_rstd)`` with ``y`` bit-identical to ``group_norm`` on the same
     inputs and ``mean_rstd`` [N, groups, 2] the (mean, rstd) of ``x + channel_bias`` that the backward needs.  The
     affine parameters are passed as tensors (weight, bias [C]) so that autograd can follow them."""
-    if not (_gn_params_ok(x, weight, bias, groups) and (up is None or _up_ok(x, up))):
-        raise RuntimeError("group_norm_train needs a contiguous NCHW fp32 CUDA map with H*W (and, with `up`, W) a multiple "
-                           "of 4, contiguous fp32 [C] weight and bias on the same device, C divisible by groups and, if "
-                           "given, a contiguous `up` map with the same batch and channels")
-    _check_channel_bias(channel_bias, x)
-    N, C, H, W = x.shape
-    y = torch.empty_like(x)
-    mean_rstd = torch.empty(N, groups, 2, dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        ws = torch.empty(int(_lib.lib.msda_b200_group_norm_workspace_bytes(N, groups)), dtype=torch.uint8,
-                         device=x.device)
-        rc = _lib.lib.msda_b200_group_norm_nchw_train_f32(
-            x.data_ptr(), channel_bias.data_ptr() if channel_bias is not None else None, weight.data_ptr(),
-            bias.data_ptr(), y.data_ptr(), mean_rstd.data_ptr(), N, C, H, W, groups, float(eps), int(bool(relu)),
-            up.data_ptr() if up is not None else None, up.size(2) if up is not None else 0,
-            up.size(3) if up is not None else 0, ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)
-    _lib.check(rc, "group_norm_train")
-    return y, mean_rstd
+    return _group_norm_nchw("group_norm_train", x, weight, bias, groups, eps, relu, up, channel_bias, True)
 
 
-def _check_mean_rstd(mean_rstd, x, groups):
-    if not (isinstance(mean_rstd, torch.Tensor) and mean_rstd.device == x.device and mean_rstd.dtype == torch.float32
-            and mean_rstd.is_contiguous() and mean_rstd.shape == (x.size(0), groups, 2)):
-        raise RuntimeError("mean_rstd must be the contiguous fp32 [N, groups, 2] tensor of the training forward")
+def group_norm_rows_train(x, weight, bias, groups, eps, out_rows, channel_bias=None, relu=False):
+    """Training forward of ``group_norm_rows``: writes ``out_rows`` (bit-identical to ``group_norm_rows``) and returns
+    ``mean_rstd`` [N, groups, 2]."""
+    return _group_norm_rows("group_norm_rows_train", x, weight, bias, groups, eps, out_rows, channel_bias, relu, True)
 
 
 def group_norm_backward(grad_y, x, weight, bias, mean_rstd, groups, relu=False, channel_bias=None, up_shape=None,
@@ -608,9 +609,9 @@ def group_norm_backward(grad_y, x, weight, bias, mean_rstd, groups, relu=False, 
     ``grad_y`` and the forward's inputs and ``mean_rstd``.  ``grad_channel_bias`` is computed when
     ``with_channel_bias`` (else None); ``grad_up`` [N, C, *up_shape] when ``up_shape`` (the up-sampled map's (h, w))
     is given (else None).  Three launches, four with ``grad_up``; deterministic."""
-    if not (_gn_params_ok(x, weight, bias, groups) and isinstance(grad_y, torch.Tensor) and grad_y.shape == x.shape
-            and grad_y.device == x.device and grad_y.dtype == torch.float32 and grad_y.is_contiguous()
-            and grad_y.data_ptr() % 16 == 0 and (up_shape is None or x.size(3) % 4 == 0)):
+    # grad_y: a map like x; with up_shape, the forward's `up` requirement on W
+    if not (_map_ok(x, weight, bias, groups) and _map_ok(grad_y, weight, bias, groups) and grad_y.shape == x.shape
+            and (up_shape is None or x.size(3) % 4 == 0)):
         raise RuntimeError("group_norm_backward needs contiguous NCHW fp32 CUDA grad_y and x of the same shape with H*W "
                            "(and, with up_shape, W) a multiple of 4, and contiguous fp32 [C] weight and bias")
     _check_channel_bias(channel_bias, x)
@@ -621,43 +622,14 @@ def group_norm_backward(grad_y, x, weight, bias, mean_rstd, groups, relu=False, 
     gcb = torch.empty_like(bias) if with_channel_bias else None
     gup = torch.empty(N, C, int(up_shape[0]), int(up_shape[1]), dtype=x.dtype, device=x.device) if up_shape else None
     with torch.cuda.device(x.device):
-        ws = torch.empty(int(_lib.lib.msda_b200_group_norm_backward_workspace_bytes(N, C)), dtype=torch.uint8,
-                         device=x.device)
+        ws = _workspace(_lib.lib.msda_b200_group_norm_backward_workspace_bytes(N, C), x)
         rc = _lib.lib.msda_b200_group_norm_backward_nchw_f32(
-            grad_y.data_ptr(), x.data_ptr(), channel_bias.data_ptr() if channel_bias is not None else None,
-            weight.data_ptr(), bias.data_ptr(), mean_rstd.data_ptr(), gx.data_ptr(), gw.data_ptr(), gb.data_ptr(),
-            gcb.data_ptr() if gcb is not None else None, gup.data_ptr() if gup is not None else None, N, C, H, W,
+            grad_y.data_ptr(), x.data_ptr(), _ptr(channel_bias), weight.data_ptr(), bias.data_ptr(),
+            mean_rstd.data_ptr(), gx.data_ptr(), gw.data_ptr(), gb.data_ptr(), _ptr(gcb), _ptr(gup), N, C, H, W,
             groups, int(bool(relu)), gup.size(2) if gup is not None else 0, gup.size(3) if gup is not None else 0,
             ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)
     _lib.check(rc, "group_norm_backward")
     return gx, gw, gb, gcb, gup
-
-
-def _rows_ok(rows, x) -> bool:
-    return (isinstance(rows, torch.Tensor) and rows.is_cuda and rows.device == x.device and rows.dtype == torch.float32
-            and rows.dim() == 3 and tuple(rows.shape) == (x.size(0), x.size(2) * x.size(3), x.size(1))
-            and rows.stride(2) == 1 and rows.stride(1) >= x.size(1) and rows.stride(1) % 4 == 0
-            and rows.stride(0) % 4 == 0 and rows.data_ptr() % 16 == 0)
-
-
-def group_norm_rows_train(x, weight, bias, groups, eps, out_rows, channel_bias=None, relu=False):
-    """Training forward of ``group_norm_rows``: writes ``out_rows`` (bit-identical to ``group_norm_rows``) and returns
-    ``mean_rstd`` [N, groups, 2]."""
-    if not (_gn_params_ok(x, weight, bias, groups) and x.size(1) % 32 == 0 and _rows_ok(out_rows, x)):
-        raise RuntimeError("group_norm_rows_train needs what group_norm_train needs, channels % 32 == 0 and an fp32 "
-                           "[N, H*W, C] destination view with unit channel stride on the same device")
-    _check_channel_bias(channel_bias, x)
-    N, C, H, W = x.shape
-    mean_rstd = torch.empty(N, groups, 2, dtype=torch.float32, device=x.device)
-    with torch.cuda.device(x.device):
-        ws = torch.empty(int(_lib.lib.msda_b200_group_norm_workspace_bytes(N, groups)), dtype=torch.uint8,
-                         device=x.device)
-        rc = _lib.lib.msda_b200_group_norm_nchw_to_rows_train_f32(
-            x.data_ptr(), channel_bias.data_ptr() if channel_bias is not None else None, weight.data_ptr(),
-            bias.data_ptr(), out_rows.data_ptr(), mean_rstd.data_ptr(), out_rows.stride(1), out_rows.stride(0), N, C,
-            H * W, groups, float(eps), int(bool(relu)), ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)
-    _lib.check(rc, "group_norm_rows_train")
-    return mean_rstd
 
 
 def group_norm_rows_backward(grad_rows, x, weight, bias, mean_rstd, groups, relu=False, channel_bias=None,
@@ -665,7 +637,7 @@ def group_norm_rows_backward(grad_rows, x, weight, bias, mean_rstd, groups, relu
     """Gradients of ``group_norm_rows_train``: ``(grad_x, grad_weight, grad_bias, grad_channel_bias)`` with ``grad_rows``
     an fp32 [N, H*W, C] view in the rows layout (e.g. the level's slice of the concatenated gradient) and grad_x NCHW.
     Three launches; deterministic."""
-    if not (_gn_params_ok(x, weight, bias, groups) and x.size(1) % 32 == 0 and _rows_ok(grad_rows, x)):
+    if not (_map_ok(x, weight, bias, groups) and _rows_view_ok(grad_rows, x)):
         raise RuntimeError("group_norm_rows_backward needs what group_norm_backward needs, channels % 32 == 0 and an "
                            "fp32 [N, H*W, C] grad_rows view with unit channel stride on the same device")
     _check_channel_bias(channel_bias, x)
@@ -675,12 +647,10 @@ def group_norm_rows_backward(grad_rows, x, weight, bias, mean_rstd, groups, relu
     gw, gb = torch.empty_like(weight), torch.empty_like(bias)
     gcb = torch.empty_like(bias) if with_channel_bias else None
     with torch.cuda.device(x.device):
-        ws = torch.empty(int(_lib.lib.msda_b200_group_norm_backward_workspace_bytes(N, C)), dtype=torch.uint8,
-                         device=x.device)
+        ws = _workspace(_lib.lib.msda_b200_group_norm_backward_workspace_bytes(N, C), x)
         rc = _lib.lib.msda_b200_group_norm_rows_backward_f32(
-            grad_rows.data_ptr(), grad_rows.stride(1), grad_rows.stride(0), x.data_ptr(),
-            channel_bias.data_ptr() if channel_bias is not None else None, weight.data_ptr(), bias.data_ptr(),
-            mean_rstd.data_ptr(), gx.data_ptr(), gw.data_ptr(), gb.data_ptr(), gcb.data_ptr() if gcb is not None else None,
-            N, C, H * W, groups, int(bool(relu)), ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)
+            grad_rows.data_ptr(), grad_rows.stride(1), grad_rows.stride(0), x.data_ptr(), _ptr(channel_bias),
+            weight.data_ptr(), bias.data_ptr(), mean_rstd.data_ptr(), gx.data_ptr(), gw.data_ptr(), gb.data_ptr(),
+            _ptr(gcb), N, C, H * W, groups, int(bool(relu)), ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)
     _lib.check(rc, "group_norm_rows_backward")
     return gx, gw, gb, gcb

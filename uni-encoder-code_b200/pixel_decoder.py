@@ -75,22 +75,33 @@ class _ConvNormAct(nn.Conv2d):
 
     def forward(self, x, up=None, fused_norm=False):
         """conv -> norm -> activation (-> + bilinear up-sampling of `up`, the FPN top-down add of
-        msdeformattn.py:372-376).  `fused_norm` (GroupNorm, fp32 CUDA): the norm, the ReLU and the up-sampled add
-        run as one statistics + one apply kernel (ops.group_norm, SURVEY 8f.4); with autograd on through
-        GroupNormFunction, whose backward also runs on the library's kernels."""
+        msdeformattn.py:372-376).  `fused_norm` (GroupNorm): the norm, the ReLU and the up-sampled add through
+        `_group_norm`."""
         x = super().forward(x)
-        if fused_norm and self.activation in (None, F.relu) and ops.group_norm_supported(x, self.norm, up):
-            relu = self.activation is F.relu
-            if not torch.is_grad_enabled():
-                return ops.group_norm(x, self.norm, relu=relu, up=up)
-            return GroupNormFunction.apply(x, self.norm.weight, self.norm.bias, None, up, self.norm.num_groups,
-                                           self.norm.eps, relu)
+        if fused_norm and isinstance(self.norm, nn.GroupNorm) and self.activation in (None, F.relu):
+            return _group_norm(self.norm, x, relu=self.activation is F.relu, up=up)
         if self.norm is not None:
             x = self.norm(x)
         x = x if self.activation is None else self.activation(x)
         if up is not None:
             x = x + F.interpolate(up, size=x.shape[-2:], mode="bilinear", align_corners=False)
         return x
+
+
+def _group_norm(norm: nn.GroupNorm, x, relu=False, up=None, channel_bias=None):
+    """``norm(x + channel_bias[None, :, None, None])`` [-> ReLU] [+ bilinear up-sampling of `up`] (`channel_bias`: the
+    bias of the convolution that produced x and ran without it).  Where ops.group_norm_supported holds, one statistics
+    + one apply kernel (SURVEY 8f.4): ops.group_norm with autograd off, GroupNormFunction, whose backward also runs on
+    the library's kernels, with it on; torch otherwise."""
+    if ops.group_norm_supported(x, norm, up):
+        if not torch.is_grad_enabled():
+            return ops.group_norm(x, norm, relu=relu, up=up, channel_bias=channel_bias)
+        return GroupNormFunction.apply(x, norm.weight, norm.bias, channel_bias, up, norm.num_groups, norm.eps, relu)
+    x = norm(x if channel_bias is None else x + channel_bias.view(1, -1, 1, 1))
+    x = F.relu(x) if relu else x
+    if up is not None:
+        x = x + F.interpolate(up, size=x.shape[-2:], mode="bilinear", align_corners=False)
+    return x
 
 
 def _norm(kind, channels):
@@ -158,52 +169,12 @@ class MSDeformAttnPixelDecoder(nn.Module):
         """-> (mask_features [N, mask_dim, H/4, W/4], lowest-resolution map, 3 multi-scale maps),
         as msdeformattn.py:336-386 (autocast disabled, inputs promoted to fp32)."""
         with torch.autocast(device_type=next(iter(features.values())).device.type, enabled=False):
-            srcs, pos = [], []
             fused_norm = self.linear == "tf32x3"        # the inference kernels of SURVEY 8f.3 / 8f.4
             names = self.transformer_in_features[::-1]
             levels = [(int(features[k].shape[2]), int(features[k].shape[3])) for k in names]
-            # inference kernels: every input projection's GroupNorm writes its rows of the concatenated
-            # [N, S, C] tensor directly (no transposing `cat` afterwards) when all levels qualify
-            src_flat, starts = None, [0]
-            for h, w in levels:
-                starts.append(starts[-1] + h * w)
-            rows_ok = fused_norm and not torch.is_grad_enabled()
-            if fused_norm and torch.is_grad_enabled():
-                # training: the convolutions without their bias, then ONE autograd node for the GroupNorms of all
-                # levels that writes the concatenated [N, S, C] encoder input (and reads its gradient) in place
-                src_flat = self._input_proj_train(features, names)
-                if src_flat is not None:
-                    pos = [self.pe_layer(features[name]) for name in names]
-                    rows_ok = True
-            for idx, name in enumerate(names if src_flat is None else []):
-                x = features[name].float()
-                proj = self.input_proj[idx]
-                if fused_norm and not torch.is_grad_enabled():
-                    # the convolution runs without its bias (torch adds it in a separate pass over the map);
-                    # the GroupNorm kernels add it on the fly
-                    y = F.conv2d(x, proj[0].weight, None, proj[0].stride, proj[0].padding, proj[0].dilation,
-                                 proj[0].groups)
-                    if rows_ok and src_flat is None:
-                        src_flat = y.new_empty((y.shape[0], starts[-1], y.shape[1]))
-                    rows = src_flat[:, starts[idx]:starts[idx + 1]] if rows_ok else None
-                    if rows_ok and ops.group_norm_rows_supported(y, proj[1], rows):
-                        ops.group_norm_rows(y, proj[1], rows, channel_bias=proj[0].bias)
-                        srcs.append(None)
-                    else:
-                        if ops.group_norm_supported(y, proj[1]):
-                            z = ops.group_norm(y, proj[1], channel_bias=proj[0].bias)
-                        else:
-                            z = proj[1](y if proj[0].bias is None else y + proj[0].bias.view(1, -1, 1, 1))
-                        srcs.append(z)
-                        if rows_ok:                                   # keep the rows complete: this level through torch
-                            rows.copy_(z.flatten(2).transpose(1, 2))
-                else:
-                    srcs.append(proj[1](proj[0](x)))
-                pos.append(self.pe_layer(x))
-            if rows_ok:
-                memory, _, _, _ = self.transformer(None, pos, src_flat=src_flat, levels=levels)
-            else:
-                memory, _, _, _ = self.transformer(srcs, pos)
+            srcs, src_flat = self._input_proj([features[k].float() for k in names], levels, fused_norm)
+            pos = [self.pe_layer(features[k]) for k in names]
+            memory, _, _, _ = self.transformer(srcs, pos, src_flat=src_flat, levels=levels)
             n = memory.shape[0]
             out: List[torch.Tensor] = [z.transpose(1, 2).reshape(n, -1, h, w) for z, (h, w) in
                                        zip(memory.split([h * w for h, w in levels], dim=1), levels)]
@@ -213,25 +184,33 @@ class MSDeformAttnPixelDecoder(nn.Module):
                 out.append(self.output_convs[idx](y, fused_norm=fused_norm))
             return self._mask_features(out[-1], fused_norm), out[0], out[:self.oneformer_num_feature_levels]
 
-    def _input_proj_train(self, features, names):
-        """The input projections under autograd as GroupNormRowsFunction, or None when a level does not qualify
-        (then every level takes torch's path: no level is written into a shared tensor on its own)."""
-        if any(not features[k].is_cuda or (features[k].shape[2] * features[k].shape[3]) % 4 for k in names) or \
-                any(proj[0].out_channels % 32 for proj in self.input_proj):
-            return None                                    # shapes the kernels do not cover: no convolution spent
-        ys, args = [], []
-        for idx, name in enumerate(names):
-            conv, norm = self.input_proj[idx]
-            if not isinstance(norm, nn.GroupNorm):
-                return None
-            ys.append(F.conv2d(features[name].float(), conv.weight, None, conv.stride, conv.padding, conv.dilation,
-                               conv.groups))
-            args += [ys[-1], norm.weight, norm.bias, conv.bias]
-        norms = [proj[1] for proj in self.input_proj]
-        if not GroupNormRowsFunction.supported(ys, norms) or \
-                len({(n.num_groups, n.eps) for n in norms}) != 1:
-            return None
-        return GroupNormRowsFunction.apply(norms[0].num_groups, norms[0].eps, *args)
+    def _input_proj(self, xs, levels, fused_norm):
+        """The input projections of the encoder's levels -> (srcs, None): the per-level NCHW maps, which the encoder
+        concatenates; or (None, src_flat): that concatenated [N, S, C] tensor, written directly.  With `fused_norm` the
+        convolutions run without their bias (torch adds it in a separate pass over the map) and the GroupNorms add it
+        on the fly.  When ops.group_norm_rows_supported holds for every level, each level's GroupNorm writes its rows
+        of src_flat (no transposing `cat`): ops.group_norm_rows with autograd off, ONE GroupNormRowsFunction node for
+        all levels with it on.  Otherwise every level goes through `_group_norm`."""
+        if not fused_norm:
+            return [proj[1](proj[0](x)) for proj, x in zip(self.input_proj, xs)], None
+        convs, norms = [proj[0] for proj in self.input_proj], [proj[1] for proj in self.input_proj]
+        ys = [F.conv2d(x, c.weight, None, c.stride, c.padding, c.dilation, c.groups) for c, x in zip(convs, xs)]
+        starts = [0]
+        for h, w in levels:
+            starts.append(starts[-1] + h * w)
+        src_flat = ys[0].new_empty((ys[0].shape[0], starts[-1], ys[0].shape[1]))
+        rows = [src_flat[:, a:b] for a, b in zip(starts, starts[1:])]
+        if not (all(ops.group_norm_rows_supported(y, n, r) for y, n, r in zip(ys, norms, rows))
+                and len({(n.num_groups, n.eps) for n in norms}) == 1):
+            return [_group_norm(n, y, channel_bias=c.bias) for n, y, c in zip(norms, ys, convs)], None
+        if not torch.is_grad_enabled():
+            for y, n, c, r in zip(ys, norms, convs, rows):
+                ops.group_norm_rows(y, n, r, channel_bias=c.bias)
+            return None, src_flat
+        del src_flat, rows                             # GroupNormRowsFunction allocates its own output
+        return None, GroupNormRowsFunction.apply(norms[0].num_groups, norms[0].eps,
+                                                 *[t for y, n, c in zip(ys, norms, convs)
+                                                   for t in (y, n.weight, n.bias, c.bias)])
 
     @staticmethod
     def _nchw(view, memory, fused_norm):
