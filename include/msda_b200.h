@@ -101,6 +101,39 @@ int msda_b200_backward_f64(const double *grad_output, const double *value,
                            double *grad_attn_weight, void *stream);
 
 /*
+ * Deterministic backwards: the same gradients with no order-dependent floating-point sums, so bit-identical
+ * inputs give bit-identical outputs on the same device (what torch.use_deterministic_algorithms asks for).
+ * Same arguments as the entries above plus `workspace`, device scratch of
+ * msda_b200_backward_deterministic_workspace_bytes(...) bytes (value_bytes = 4 for the f32 entries, 8 for f64;
+ * 16-byte aligned; contents meaningless before and after; 0 = shape not covered: more than 2^31 - 1 corner
+ * records, i.e. batch * num_query * num_heads * num_levels * num_point * 4, or batch * spatial_size * num_heads
+ * >= 2^31 -- split the batch).  grad_value is fully overwritten (no zero-fill needed).  The backward kernel of
+ * the path writes one {grad_value row, weight} record per (sampling point, corner) into a fixed slot, a stable
+ * radix sort (CUB) orders the records by row, and one warp per row adds its records up in slot order -- the
+ * order of a sequential loop over query, head, level, point, corner.  grad_sampling_loc / grad_attn_weight are
+ * computed exactly as by the default entries.  No host read-back or allocation: CUDA-graph capturable.
+ * msda_b200_launch_count counts four launches per call: the records kernel, the sort (as one launch, however many
+ * kernels CUB runs for it), the bucket bounds and the gather.
+ */
+long long msda_b200_backward_deterministic_workspace_bytes(int batch, int spatial_size, int num_heads,
+                                                          int channels, int num_levels, int num_query,
+                                                          int num_point, int value_bytes);
+int msda_b200_backward_deterministic_f32(const float *grad_output, const float *value,
+                                         const int64_t *spatial_shapes, const int64_t *level_start,
+                                         const float *sampling_loc, const float *attn_weight,
+                                         int batch, int spatial_size, int num_heads, int channels,
+                                         int num_levels, int num_query, int num_point,
+                                         float *grad_value, float *grad_sampling_loc,
+                                         float *grad_attn_weight, void *workspace, void *stream);
+int msda_b200_backward_deterministic_f64(const double *grad_output, const double *value,
+                                         const int64_t *spatial_shapes, const int64_t *level_start,
+                                         const double *sampling_loc, const double *attn_weight,
+                                         int batch, int spatial_size, int num_heads, int channels,
+                                         int num_levels, int num_query, int num_point,
+                                         double *grad_value, double *grad_sampling_loc,
+                                         double *grad_attn_weight, void *workspace, void *stream);
+
+/*
  * Fused producers (SURVEY.md 8f.1): the same op with the three elementwise steps of its caller
  * folded into the kernels -- ops/modules/ms_deform_attn.py:105-112:
  *     attention_weights = softmax(attn_logits over num_levels*num_point)
@@ -147,6 +180,17 @@ int msda_b200_fused_backward_f32(const float *grad_output, const float *value,
                                  int num_levels, int num_query, int num_point, float *grad_value,
                                  float *grad_sampling_offsets, float *grad_attn_logits,
                                  void *stream);
+/* Deterministic twin of the fused backward: the records carry the in-kernel softmax and locations, exactly as
+ * the fused forward used them.  Workspace and guarantees as for msda_b200_backward_deterministic_f32
+ * (value_bytes = 4). */
+int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const float *value,
+                                               const int64_t *spatial_shapes, const int64_t *level_start,
+                                               const float *reference_points, long long ref_batch_stride,
+                                               const float *sampling_offsets, const float *attn_logits,
+                                               int batch, int spatial_size, int num_heads, int channels,
+                                               int num_levels, int num_query, int num_point, float *grad_value,
+                                               float *grad_sampling_offsets, float *grad_attn_logits,
+                                               void *workspace, void *stream);
 
 /*
  * Next component on the path's caller side (SURVEY.md section 8f.3): the fp32 nn.Linear layers around
@@ -166,6 +210,13 @@ int msda_b200_fused_backward_f32(const float *grad_output, const float *value,
 int msda_b200_linear_f32(const float *x, const float *weight, const float *bias, float *y,
                          int rows, int out_features, int in_features, int relu, float *workspace,
                          void *stream);
+/* Deterministic twin (same arguments): never spreads a tile's reduction over CTAs, so the result does not
+ * depend on scheduling.  Where msda_b200_linear_f32 uses split-K, one CTA per output tile computes the same
+ * chunks of the reduction in order and adds them in chunk order (same accuracy); elsewhere the result is
+ * bit-identical to msda_b200_linear_f32. */
+int msda_b200_linear_deterministic_f32(const float *x, const float *weight, const float *bias, float *y,
+                                       int rows, int out_features, int in_features, int relu,
+                                       float *workspace, void *stream);
 
 /*
  * The same GEMM for a weight that does not change between calls (inference): msda_b200_split_weight_f32 writes
@@ -177,6 +228,9 @@ int msda_b200_split_weight_f32(const float *weight, float *split_weight, int out
                                void *stream);
 int msda_b200_linear_presplit_f32(const float *x, const float *split_weight, const float *bias, float *y,
                                   int rows, int out_features, int in_features, int relu, void *stream);
+int msda_b200_linear_presplit_deterministic_f32(const float *x, const float *split_weight, const float *bias,
+                                                float *y, int rows, int out_features, int in_features, int relu,
+                                                void *stream);
 
 /*
  * y[rows, cols] = LayerNorm(x + residual) * gamma + beta over the last dimension (eps inside the square
@@ -196,6 +250,14 @@ int msda_b200_add_layernorm_f32(const float *x, const float *residual, const flo
 int msda_b200_add_layernorm_backward_f32(const float *grad_y, const float *x, const float *residual,
                                          const float *gamma, float *grad_v, float *grad_gamma,
                                          float *grad_beta, long long rows, int cols, float eps, void *stream);
+/* Deterministic twin: every CTA stores its grad_gamma / grad_beta partials in `workspace`
+ * (msda_b200_add_layernorm_backward_deterministic_workspace_bytes(rows, cols) bytes, computed for the current
+ * device) and a second launch adds them in CTA order.  grad_v is bit-identical to the entry above. */
+int msda_b200_add_layernorm_backward_deterministic_f32(const float *grad_y, const float *x, const float *residual,
+                                                       const float *gamma, float *grad_v, float *grad_gamma,
+                                                       float *grad_beta, long long rows, int cols, float eps,
+                                                       void *workspace, void *stream);
+long long msda_b200_add_layernorm_backward_deterministic_workspace_bytes(long long rows, int cols);
 
 /*
  * GroupNorm over an NCHW fp32 map with the pixel decoder's epilogues fused in (SURVEY 8f.4;
@@ -282,6 +344,13 @@ int msda_b200_add_channel_bias_nchw_f32(float *x, const float *bias, int batch, 
  */
 int msda_b200_linear_wgrad_f32(const float *grad_y, const float *x, float *grad_weight, float *grad_bias,
                                long long rows, int out_features, int in_features, void *stream);
+/* Deterministic twin: each work item (a chunk of rows of one output tile) stores its partial tile and bias in
+ * `workspace` (msda_b200_linear_wgrad_deterministic_workspace_bytes(rows, out_features, in_features) bytes, one
+ * grad_weight + grad_bias per row chunk) and a second launch adds the chunks in order. */
+int msda_b200_linear_wgrad_deterministic_f32(const float *grad_y, const float *x, float *grad_weight,
+                                             float *grad_bias, long long rows, int out_features, int in_features,
+                                             void *workspace, void *stream);
+long long msda_b200_linear_wgrad_deterministic_workspace_bytes(long long rows, int out_features, int in_features);
 
 /* y[cols, rows] = x[rows, cols]^T, fp32 (operand preparation for weight-gradient GEMMs). */
 int msda_b200_transpose_f32(const float *x, float *y, long long rows, int cols, void *stream);

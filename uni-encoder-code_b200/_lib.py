@@ -26,16 +26,26 @@ SYMBOLS = {
     "msda_b200_forward_f64": (_I, [_P] * 5 + _DIMS + [_P, _P]),
     "msda_b200_backward_f32": (_I, [_P] * 6 + _DIMS + [_P, _P, _P, _P]),
     "msda_b200_backward_f64": (_I, [_P] * 6 + _DIMS + [_P, _P, _P, _P]),
+    "msda_b200_backward_deterministic_workspace_bytes": (ctypes.c_longlong, _DIMS + [_I]),
+    "msda_b200_backward_deterministic_f32": (_I, [_P] * 6 + _DIMS + [_P, _P, _P, _P, _P]),
+    "msda_b200_backward_deterministic_f64": (_I, [_P] * 6 + _DIMS + [_P, _P, _P, _P, _P]),
     "msda_b200_debug_indices_f32": (_I, [_P] * 3 + _DIMS + [_P, _P, _P]),
     "msda_b200_fused_forward_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P, _P]),
     "msda_b200_fused_forward_strided_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _P, _I, _P, _I, _P, _P] + _DIMS + [_P, _P]),
     "msda_b200_fused_backward_f32": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P, _P, _P, _P]),
+    "msda_b200_fused_backward_deterministic_f32": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P] * 5),
     "msda_b200_linear_f32": (_I, [_P] * 4 + [_I] * 4 + [_P, _P]),
+    "msda_b200_linear_deterministic_f32": (_I, [_P] * 4 + [_I] * 4 + [_P, _P]),
     "msda_b200_split_weight_f32": (_I, [_P, _P, _I, _I, _P]),
     "msda_b200_linear_presplit_f32": (_I, [_P] * 4 + [_I] * 4 + [_P]),
+    "msda_b200_linear_presplit_deterministic_f32": (_I, [_P] * 4 + [_I] * 4 + [_P]),
     "msda_b200_add_layernorm_f32": (_I, [_P] * 5 + [ctypes.c_longlong, _I, ctypes.c_float, _P]),
     "msda_b200_add_layernorm_backward_f32": (_I, [_P] * 7 + [ctypes.c_longlong, _I, ctypes.c_float, _P]),
+    "msda_b200_add_layernorm_backward_deterministic_f32": (_I, [_P] * 7 + [ctypes.c_longlong, _I, ctypes.c_float, _P, _P]),
+    "msda_b200_add_layernorm_backward_deterministic_workspace_bytes": (ctypes.c_longlong, [ctypes.c_longlong, _I]),
     "msda_b200_linear_wgrad_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _I, _I, _P]),
+    "msda_b200_linear_wgrad_deterministic_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _I, _I, _P, _P]),
+    "msda_b200_linear_wgrad_deterministic_workspace_bytes": (ctypes.c_longlong, [ctypes.c_longlong, _I, _I]),
     "msda_b200_transpose_f32": (_I, [_P, _P, ctypes.c_longlong, _I, _P]),
     "msda_b200_group_norm_nchw_f32": (_I, [_P] * 5 + [_I] * 5 + [ctypes.c_float, _I, _P, _I, _I, _P, _P]),
     "msda_b200_group_norm_nchw_to_rows_f32": (_I, [_P] * 5 + [ctypes.c_longlong, ctypes.c_longlong, _I, _I, ctypes.c_longlong, _I,

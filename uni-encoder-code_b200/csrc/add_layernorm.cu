@@ -112,7 +112,9 @@ cudaError_t launch_add_layernorm(const float *x, const float *res, const float *
 //     grad_gamma = sum_rows grad_y * xhat,   grad_beta = sum_rows grad_y
 // v, mean and rstd are recomputed from x and residual (one extra read of residual instead of a stored copy
 // of v).  One warp per row as in the forward; each warp keeps its partial grad_gamma / grad_beta in
-// registers over all its rows and adds them to the zero-filled outputs once at the end.
+// registers over all its rows and adds them to the zero-filled outputs once at the end -- or, in the
+// deterministic entry, stores the CTA's partials in a workspace that a second launch sums in CTA order (the
+// grid is a fixed function of rows and SM count).
 // ---------------------------------------------------------------------------
 namespace msda {
 namespace {
@@ -121,7 +123,7 @@ template <int V>
 __global__ void __launch_bounds__(256)
 add_layernorm_bwd_kernel(const float4 *__restrict__ gy, const float4 *__restrict__ x, const float4 *__restrict__ res,
                          const float4 *__restrict__ gamma, float4 *__restrict__ gv, float *__restrict__ ggamma,
-                         float *__restrict__ gbeta, long long rows, float eps) {
+                         float *__restrict__ gbeta, long long rows, float eps, float *__restrict__ partials) {
     constexpr int C4 = 32 * V;
     const int lane = threadIdx.x & 31;
     const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
@@ -201,33 +203,66 @@ add_layernorm_bwd_kernel(const float4 *__restrict__ gy, const float4 *__restrict
             a += part[0][k][c];
             b += part[1][k][c];
         }
-        asm volatile("red.global.add.f32 [%0], %1;" ::"l"(ggamma + c), "f"(a) : "memory");
-        asm volatile("red.global.add.f32 [%0], %1;" ::"l"(gbeta + c), "f"(b) : "memory");
+        if (partials != nullptr) {        // [2][gridDim.x][C]
+            partials[(long long)blockIdx.x * (128 * V) + c] = a;
+            partials[((long long)gridDim.x + blockIdx.x) * (128 * V) + c] = b;
+        } else {
+            asm volatile("red.global.add.f32 [%0], %1;" ::"l"(ggamma + c), "f"(a) : "memory");
+            asm volatile("red.global.add.f32 [%0], %1;" ::"l"(gbeta + c), "f"(b) : "memory");
+        }
     }
+}
+
+// deterministic entry: grad_gamma / grad_beta = the CTAs' partials summed in CTA order
+__global__ void __launch_bounds__(256)
+add_layernorm_bwd_sum_kernel(const float *__restrict__ partials, float *__restrict__ ggamma, float *__restrict__ gbeta,
+                             int ctas, int cols) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= 2 * cols) return;
+    const int which = i / cols, c = i - which * cols;
+    const float *p = partials + (long long)which * ctas * cols + c;
+    float s = 0.f;
+    for (int k = 0; k < ctas; ++k) s += p[(long long)k * cols];
+    (which == 0 ? ggamma : gbeta)[c] = s;
+}
+
+long long bwd_ctas(long long rows) {
+    long long blocks = (rows + 7) / 8;
+    const long long cap = (long long)sm_count() * 4;      // few CTAs: each ends with 2 x C reductions
+    return blocks > cap ? cap : blocks;
 }
 
 template <int V>
 cudaError_t launch_bwd(const float *gy, const float *x, const float *res, const float *gamma, float *gv,
-                       float *ggamma, float *gbeta, long long rows, float eps, cudaStream_t stream) {
-    cudaError_t e = cudaMemsetAsync(ggamma, 0, 128 * V * sizeof(float), stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(gbeta, 0, 128 * V * sizeof(float), stream);
-    if (e != cudaSuccess) return e;
-    long long blocks = (rows + 7) / 8;
-    const long long cap = (long long)sm_count() * 4;      // few CTAs: each ends with 2 x C reductions
-    if (blocks > cap) blocks = cap;
+                       float *ggamma, float *gbeta, long long rows, float eps, cudaStream_t stream, float *partials) {
+    if (partials == nullptr) {
+        cudaError_t e = cudaMemsetAsync(ggamma, 0, 128 * V * sizeof(float), stream);
+        if (e == cudaSuccess) e = cudaMemsetAsync(gbeta, 0, 128 * V * sizeof(float), stream);
+        if (e != cudaSuccess) return e;
+    }
+    const long long blocks = bwd_ctas(rows);
     add_layernorm_bwd_kernel<V><<<(unsigned)blocks, 256, 0, stream>>>(
         reinterpret_cast<const float4 *>(gy), reinterpret_cast<const float4 *>(x),
         reinterpret_cast<const float4 *>(res), reinterpret_cast<const float4 *>(gamma),
-        reinterpret_cast<float4 *>(gv), ggamma, gbeta, rows, eps);
+        reinterpret_cast<float4 *>(gv), ggamma, gbeta, rows, eps, partials);
+    note_launch();
+    if (partials == nullptr) return cudaGetLastError();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    add_layernorm_bwd_sum_kernel<<<(2 * 128 * V + 255) / 256, 256, 0, stream>>>(partials, ggamma, gbeta, (int)blocks,
+                                                                              128 * V);
     note_launch();
     return cudaGetLastError();
 }
 
 }  // namespace
 
+// floats of the deterministic entry's workspace: grad_gamma and grad_beta partials of every CTA
+long long add_layernorm_bwd_partials(long long rows, int cols) { return 2 * bwd_ctas(rows) * cols; }
+
 cudaError_t launch_add_layernorm_bwd(const float *gy, const float *x, const float *res, const float *gamma, float *gv,
                                      float *ggamma, float *gbeta, long long rows, int cols, float eps,
-                                     cudaStream_t stream, bool *handled) {
+                                     cudaStream_t stream, bool *handled, float *partials) {
     *handled = true;
     const uintptr_t bits = reinterpret_cast<uintptr_t>(gy) | reinterpret_cast<uintptr_t>(x) |
                            reinterpret_cast<uintptr_t>(res) | reinterpret_cast<uintptr_t>(gamma) |
@@ -237,8 +272,8 @@ cudaError_t launch_add_layernorm_bwd(const float *gy, const float *x, const floa
         return cudaSuccess;
     }
     switch (cols) {
-        case 128: return launch_bwd<1>(gy, x, res, gamma, gv, ggamma, gbeta, rows, eps, stream);
-        case 256: return launch_bwd<2>(gy, x, res, gamma, gv, ggamma, gbeta, rows, eps, stream);
+        case 128: return launch_bwd<1>(gy, x, res, gamma, gv, ggamma, gbeta, rows, eps, stream, partials);
+        case 256: return launch_bwd<2>(gy, x, res, gamma, gv, ggamma, gbeta, rows, eps, stream, partials);
         default: *handled = false; return cudaSuccess;
     }
 }

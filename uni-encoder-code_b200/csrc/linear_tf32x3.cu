@@ -81,12 +81,16 @@ struct LinCfg {
 // k_chunks > 1 (split-K): an output tile is computed by k_chunks CTAs-worth of work, each over kb_per_chunk
 //         k-blocks, and added into y (zeroed by the launcher) with red.global.add -- for GEMMs with few
 //         output tiles and a very long reduction (weight gradients: reduction over the rows).
+//         ordered != 0 (deterministic entries): the launcher starts one CTA per output tile and the items are
+//         numbered chunk-slowest, so CTA b walks the chunks of tile b in order; its epilogue stores chunk 0 and
+//         adds every later chunk to what the same thread stored before -- the chunks' sums are added in chunk
+//         order, with the accuracy of the chunked accumulation and without reductions in scheduling order.
 template <int BN, int STAGES, int NBUF, int NACC, bool WSPLIT>
 __global__ void __launch_bounds__(kThreads, 1)
 linear_tf32x3_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_wh,
                      const __grid_constant__ CUtensorMap map_wl, const float *__restrict__ bias,
                      float *__restrict__ y, int M, int N, int K, int relu, int whatif, int k_chunks,
-                     int kb_per_chunk) {
+                     int kb_per_chunk, int ordered) {
     using Cfg = LinCfg<BN, STAGES, NBUF, NACC>;
     extern __shared__ uint8_t smem_dyn[];
     const uint32_t base = (smem_u32(smem_dyn) + 1023u) & ~1023u;         // 128-byte swizzle: 1024-byte aligned tiles
@@ -108,12 +112,13 @@ linear_tf32x3_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_con
                dbg_no_x = whatif & 16;
     const int kblocks_all = K / kBK;
     const int n_tiles = (N + BN - 1) / BN;
-    // work items: (row block, column block, k chunk), chunk fastest
-    const long long tiles = (long long)((M + kBM - 1) / kBM) * n_tiles * k_chunks;
+    // work items: (row block, column block, k chunk), chunk fastest (ordered: chunk slowest)
+    const long long out_tiles = (long long)((M + kBM - 1) / kBM) * n_tiles;
+    const long long tiles = out_tiles * k_chunks;
     // item -> (m0, n0, first k-block, number of k-blocks, rotation of the k order)
     auto decode = [&](long long t, int &m0, int &n0, int &kb0, int &nkb, int &rot) {
-        const int chunk = (int)(t % k_chunks);
-        const long long o = t / k_chunks;
+        const int chunk = ordered ? (int)(t / out_tiles) : (int)(t % k_chunks);
+        const long long o = ordered ? t % out_tiles : t / k_chunks;
         m0 = (int)(o / n_tiles) * kBM;
         n0 = (int)(o % n_tiles) * BN;
         kb0 = chunk * kb_per_chunk;
@@ -305,6 +310,16 @@ linear_tf32x3_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_con
                         float o = tile[r * 33 + lane] + b;
                         if (relu) o = fmaxf(o, 0.f);
                         if (row < M && col + lane < N && !dbg_no_store) y[(long long)row * N + col + lane] = o;
+                    }
+                } else if (ordered) {              // this thread stored the tile's earlier chunks of these elements
+#pragma unroll 8
+                    for (int r = 0; r < 32; ++r) {
+                        const int row = m0 + q * 32 + r;
+                        const float o = tile[r * 33 + lane] + b;
+                        if (row < M && col + lane < N) {
+                            float *p = y + (long long)row * N + col + lane;
+                            *p = kb0 == 0 ? o : *p + o;
+                        }
                     }
                 } else {
 #pragma unroll 8
@@ -621,7 +636,7 @@ __global__ void split_weight_kernel(const float4 *__restrict__ w, float4 *__rest
 // ---- host side ----
 template <int BN, int STAGES, int NBUF, int NACC, bool WSPLIT>
 cudaError_t launch_linear(const float *x, const float *w, const float *bias, float *y, int M, int N, int K,
-                          int relu, float *workspace, cudaStream_t stream) {
+                          int relu, float *workspace, cudaStream_t stream, bool deterministic) {
     using Cfg = LinCfg<BN, STAGES, NBUF, NACC>;
     auto kern = linear_tf32x3_kernel<BN, STAGES, NBUF, NACC, WSPLIT>;
     static std::atomic<bool> attr_set[msda::kMaxDevices];
@@ -648,7 +663,8 @@ cudaError_t launch_linear(const float *x, const float *w, const float *bias, flo
             reinterpret_cast<const float4 *>(w), reinterpret_cast<float4 *>(whi), reinterpret_cast<float4 *>(wlo), n4);
         note_launch();
     }
-    // split-K when the output has too few tiles to occupy the GPU and the reduction is long
+    // split-K when the output has too few tiles to occupy the GPU and the reduction is long (deterministic
+    // entries: the same chunks, walked in order by one CTA per tile, see the kernel)
     const long long out_tiles = (long long)((M + kBM - 1) / kBM) * ((N + BN - 1) / BN);
     const int kblocks = K / kBK;
     int k_chunks = 1;
@@ -659,14 +675,17 @@ cudaError_t launch_linear(const float *x, const float *w, const float *bias, flo
     }
     const int kb_per_chunk = (kblocks + k_chunks - 1) / k_chunks;
     k_chunks = (kblocks + kb_per_chunk - 1) / kb_per_chunk;
-    if (k_chunks > 1) {
+    const int ordered = deterministic && k_chunks > 1;
+    if (k_chunks > 1 && !ordered) {
         cudaError_t e = cudaMemsetAsync(y, 0, (size_t)M * N * sizeof(float), stream);
         if (e != cudaSuccess) return e;
     }
     const long long tiles = out_tiles * k_chunks;
-    const long long grid = tiles < sm_count() ? tiles : sm_count();     // persistent: one CTA per SM
+    // persistent: one CTA per SM; ordered: one CTA per output tile (out_tiles * 2 <= SMs here)
+    const long long grid = ordered ? out_tiles : (tiles < sm_count() ? tiles : sm_count());
     kern<<<(unsigned)grid, kThreads, Cfg::kSmem, stream>>>(mx, mwh, mwl, bias, y, M, N, K, relu,
-                                                           whatif_value(OPT_WHATIF_LINEAR), k_chunks, kb_per_chunk);
+                                                           whatif_value(OPT_WHATIF_LINEAR), k_chunks, kb_per_chunk,
+                                                           ordered);
     note_launch();
     return cudaGetLastError();
 }
@@ -727,9 +746,11 @@ cudaError_t launch_split_weight(const float *w, float *split, int N, int K, cuda
     return cudaGetLastError();
 }
 
-// y[M, N] = x[M, K] * w[N, K]^T + bias[N]; K % 32 == 0, 16-byte aligned rows; workspace: 2*N*K floats
+// y[M, N] = x[M, K] * w[N, K]^T + bias[N]; K % 32 == 0, 16-byte aligned rows; workspace: 2*N*K floats.
+// deterministic: every output tile is reduced by one CTA, split-K chunks in chunk order (bit-identical to the
+// default outside split-K shapes)
 cudaError_t launch_linear_tf32x3(const float *x, const float *w, const float *bias, float *y, int M, int N, int K,
-                                 int relu, float *workspace, cudaStream_t stream, bool *handled) {
+                                 int relu, float *workspace, cudaStream_t stream, bool *handled, bool deterministic) {
     *handled = true;
     if (M <= 0 || N <= 0 || K <= 0 || K % kBK != 0 || N % 4 != 0 ||
         (reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(w) | reinterpret_cast<uintptr_t>(workspace) |
@@ -746,8 +767,8 @@ cudaError_t launch_linear_tf32x3(const float *x, const float *w, const float *bi
     const int variant = option_value(OPT_LINEAR_VARIANT);
     if (workspace == nullptr) {
         // one-shot weight: split inside the kernel; long reductions (the use case) -> four accumulators
-        if (narrow) return launch_linear<96, 3, 1, 4, true>(x, w, bias, y, M, N, K, relu, workspace, stream);
-        return launch_linear<128, 3, 1, 4, true>(x, w, bias, y, M, N, K, relu, workspace, stream);
+        if (narrow) return launch_linear<96, 3, 1, 4, true>(x, w, bias, y, M, N, K, relu, workspace, stream, deterministic);
+        return launch_linear<128, 3, 1, 4, true>(x, w, bias, y, M, N, K, relu, workspace, stream, deterministic);
     }
     // default: A operand in tensor memory (fastest; {main, small} accumulators, drained into registers every
     // 256 of the reduction so that the truncating accumulation never sees more than 64 MMAs per accumulator)
@@ -758,11 +779,11 @@ cudaError_t launch_linear_tf32x3(const float *x, const float *w, const float *bi
     // both operands in shared memory, the products spread over four accumulators (one set: the epilogue is
     // not overlapped) -- the long-reduction kernel before the chunked accumulation above
     if (variant == 2) {
-        if (narrow) return launch_linear<96, 3, 1, 4, false>(x, w, bias, y, M, N, K, relu, workspace, stream);
-        return launch_linear<128, 3, 1, 4, false>(x, w, bias, y, M, N, K, relu, workspace, stream);
+        if (narrow) return launch_linear<96, 3, 1, 4, false>(x, w, bias, y, M, N, K, relu, workspace, stream, deterministic);
+        return launch_linear<128, 3, 1, 4, false>(x, w, bias, y, M, N, K, relu, workspace, stream, deterministic);
     }
-    if (narrow) return launch_linear<96, 3, 2, 2, false>(x, w, bias, y, M, N, K, relu, workspace, stream);
-    return launch_linear<128, 3, 2, 2, false>(x, w, bias, y, M, N, K, relu, workspace, stream);
+    if (narrow) return launch_linear<96, 3, 2, 2, false>(x, w, bias, y, M, N, K, relu, workspace, stream, deterministic);
+    return launch_linear<128, 3, 2, 2, false>(x, w, bias, y, M, N, K, relu, workspace, stream, deterministic);
 }
 
 }  // namespace msda

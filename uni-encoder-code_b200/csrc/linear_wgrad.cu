@@ -13,7 +13,8 @@
 //     swizzled B tiles B_hi / B_lo in shared memory (what a K-major TMA load would have produced);
 // and the MMA thread issues x-like products from there: A_hi * [B_hi; B_lo]^T -> {main, small}, A_lo * B_hi^T ->
 // small.  An output tile (128 x BN of grad_W) is computed by several work items, each over a chunk of the rows
-// (split-K), and added into the zero-filled output with red.global.add.
+// (split-K), and added into the zero-filled output with red.global.add -- or, in the deterministic entry, stored
+// as the chunk's partial tile in a workspace whose chunks a second launch adds up in chunk order.
 #include "tc_common.cuh"
 
 namespace msda {
@@ -44,7 +45,7 @@ template <int BN>
 __global__ void __launch_bounds__(kThreads, 1)
 linear_wgrad_kernel(const __grid_constant__ CUtensorMap map_gy, const __grid_constant__ CUtensorMap map_x,
                     float *__restrict__ grad_w, float *__restrict__ grad_b, long long rows, int out_f, int in_f,
-                    int chunks, int kb_per_chunk) {
+                    int chunks, int kb_per_chunk, float *__restrict__ partials) {
     using Cfg = WgCfg<BN>;
     extern __shared__ uint8_t smem_dyn[];
     const uint32_t base = (smem_u32(smem_dyn) + 1023u) & ~1023u;
@@ -186,8 +187,12 @@ linear_wgrad_kernel(const __grid_constant__ CUtensorMap map_gy, const __grid_con
                 mbar_arrive(ready(s));
             }
             // bias gradient: every (out tile, chunk) contributes once (taken from the first in-tile)
-            if (grad_b != nullptr && k0 == 0 && n0 + col < out_f)
-                asm volatile("red.global.add.f32 [%0], %1;" ::"l"(grad_b + n0 + col), "f"(bsum) : "memory");
+            if (grad_b != nullptr && k0 == 0 && n0 + col < out_f) {
+                if (partials != nullptr)
+                    partials[(long long)chunks * out_f * in_f + (long long)(kb0 / kb_per_chunk) * out_f + n0 + col] = bsum;
+                else
+                    asm volatile("red.global.add.f32 [%0], %1;" ::"l"(grad_b + n0 + col), "f"(bsum) : "memory");
+            }
         }
     } else {
         // ---- epilogue warps: accumulators -> registers (set handed back at once) -> transposes -> reductions ----
@@ -198,6 +203,7 @@ linear_wgrad_kernel(const __grid_constant__ CUtensorMap map_gy, const __grid_con
             int n0, k0, kb0, nkb;
             decode(t, n0, k0, kb0, nkb);
             const uint32_t acc = tmem_base + ((uint32_t)(q * 32) << 16);
+            float *chunk_out = partials != nullptr ? partials + (long long)(kb0 / kb_per_chunk) * out_f * in_f : nullptr;
             mbar_wait(acc_full, it & 1);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             constexpr int kStep = kEpiWarps / 4, kMaxBlk = (BN / 32 + kStep - 1) / kStep;
@@ -228,8 +234,10 @@ linear_wgrad_kernel(const __grid_constant__ CUtensorMap map_gy, const __grid_con
                 for (int r = 0; r < 32; ++r) {
                     const int n = n0 + q * 32 + r;
                     const float o = tile[r * 33 + lane];
-                    if (n < out_f && colk + lane < in_f)
-                        asm volatile("red.global.add.f32 [%0], %1;" ::"l"(grad_w + (long long)n * in_f + colk + lane), "f"(o));
+                    if (n < out_f && colk + lane < in_f) {
+                        if (chunk_out != nullptr) chunk_out[(long long)n * in_f + colk + lane] = o;
+                        else asm volatile("red.global.add.f32 [%0], %1;" ::"l"(grad_w + (long long)n * in_f + colk + lane), "f"(o));
+                    }
                 }
                 __syncwarp();
             }
@@ -241,12 +249,46 @@ linear_wgrad_kernel(const __grid_constant__ CUtensorMap map_gy, const __grid_con
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
 }
 
+// deterministic entry: out[i] = sum of the chunks' partials in chunk order (grad_w, then grad_b)
+__global__ void __launch_bounds__(256)
+linear_wgrad_sum_kernel(const float *__restrict__ partials, float *__restrict__ grad_w, float *__restrict__ grad_b,
+                        int chunks, long long nw, int nb) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nw + (grad_b != nullptr ? nb : 0);
+         i += (long long)gridDim.x * blockDim.x) {
+        const bool is_w = i < nw;
+        const float *p = is_w ? partials + i : partials + (long long)chunks * nw + (i - nw);
+        const long long stride = is_w ? nw : nb;
+        float s = 0.f;
+        for (int c = 0; c < chunks; ++c) s += p[c * stride];
+        if (is_w) grad_w[i] = s;
+        else grad_b[i - nw] = s;
+    }
+}
+
+// rows per work item: the tensor core truncates when it adds into the fp32 accumulators, so the error
+// grows with the number of MMAs per accumulator -- 16 k-blocks (512 rows, 64 MMAs) per item keep it at
+// the level of an fp32 SIMT GEMM (73 k-blocks measured 5x that); more items than 2 per SM are welcome
+int wgrad_kb_per_chunk(long long rows) {
+    const int kblocks = (int)((rows + kBK - 1) / kBK);
+    int kb_per_chunk = option_value(OPT_WGRAD_CHUNK) > 0 ? option_value(OPT_WGRAD_CHUNK) : 16;   // "wgrad_chunk" option
+    if (kb_per_chunk < 1) kb_per_chunk = 1;
+    if (kb_per_chunk > kblocks) kb_per_chunk = kblocks;
+    return kb_per_chunk;
+}
+
 }  // namespace
 
+// floats of the deterministic entry's workspace: one partial grad_w and grad_b per row chunk
+long long linear_wgrad_partials(long long rows, int out_f, int in_f) {
+    const long long kblocks = (rows + kBK - 1) / kBK, kbpc = wgrad_kb_per_chunk(rows);
+    return (kblocks + kbpc - 1) / kbpc * ((long long)out_f * in_f + out_f);
+}
+
 // grad_w[out_f, in_f] = grad_y[rows, out_f]^T x[rows, in_f]; grad_b[out_f] (optional) = column sums of grad_y.
-// Both outputs are zero-filled here.  out_f % 4 == 0, in_f % 4 == 0, 16-byte aligned operands.
+// Both outputs are overwritten: zero-filled and reduced into, or, with `partials` (linear_wgrad_partials floats),
+// summed from the per-chunk partial tiles in chunk order.  out_f % 4 == 0, in_f % 4 == 0, 16-byte aligned operands.
 cudaError_t launch_linear_wgrad(const float *grad_y, const float *x, float *grad_w, float *grad_b, long long rows,
-                                int out_f, int in_f, cudaStream_t stream, bool *handled) {
+                                int out_f, int in_f, cudaStream_t stream, bool *handled, float *partials) {
     *handled = true;
     if (rows <= 0 || out_f <= 0 || in_f <= 0 || out_f % 4 != 0 || in_f % 4 != 0 || rows > 0x7fffffffLL ||
         (reinterpret_cast<uintptr_t>(grad_y) | reinterpret_cast<uintptr_t>(x)) % 16 != 0) {
@@ -270,22 +312,26 @@ cudaError_t launch_linear_wgrad(const float *grad_y, const float *x, float *grad
     CUtensorMap mgy, mx;
     if (!make_map_plain(&mgy, grad_y, rows, out_f, kBK, kBM) || !make_map_plain(&mx, x, rows, in_f, kBK, BN))
         return cudaErrorInvalidValue;
-    cudaError_t e = cudaMemsetAsync(grad_w, 0, (size_t)out_f * in_f * sizeof(float), stream);
-    if (e == cudaSuccess && grad_b != nullptr) e = cudaMemsetAsync(grad_b, 0, (size_t)out_f * sizeof(float), stream);
-    if (e != cudaSuccess) return e;
+    if (partials == nullptr) {
+        cudaError_t e = cudaMemsetAsync(grad_w, 0, (size_t)out_f * in_f * sizeof(float), stream);
+        if (e == cudaSuccess && grad_b != nullptr) e = cudaMemsetAsync(grad_b, 0, (size_t)out_f * sizeof(float), stream);
+        if (e != cudaSuccess) return e;
+    }
     const int kblocks = (int)((rows + kBK - 1) / kBK);
     const long long out_tiles = (long long)((out_f + kBM - 1) / kBM) * ((in_f + BN - 1) / BN);
-    // rows per work item: the tensor core truncates when it adds into the fp32 accumulators, so the error
-    // grows with the number of MMAs per accumulator -- 16 k-blocks (512 rows, 64 MMAs) per item keep it at
-    // the level of an fp32 SIMT GEMM (73 k-blocks measured 5x that); more items than 2 per SM are welcome
-    int kb_per_chunk = option_value(OPT_WGRAD_CHUNK) > 0 ? option_value(OPT_WGRAD_CHUNK) : 16;   // "wgrad_chunk" option
-    if (kb_per_chunk < 1) kb_per_chunk = 1;
-    if (kb_per_chunk > kblocks) kb_per_chunk = kblocks;
+    const int kb_per_chunk = wgrad_kb_per_chunk(rows);
     const long long chunks = (kblocks + kb_per_chunk - 1) / kb_per_chunk;
     const long long items = out_tiles * chunks;
     const long long grid = items < sm_count() ? items : sm_count();
     kern<<<(unsigned)grid, kThreads, Cfg::kSmem, stream>>>(mgy, mx, grad_w, grad_b, rows, out_f, in_f, (int)chunks,
-                                                           kb_per_chunk);
+                                                           kb_per_chunk, partials);
+    note_launch();
+    if (partials == nullptr) return cudaGetLastError();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    const long long nw = (long long)out_f * in_f, total = nw + (grad_b != nullptr ? out_f : 0);
+    const long long blocks = (total + 255) / 256 < (long long)sm_count() * 8 ? (total + 255) / 256 : (long long)sm_count() * 8;
+    linear_wgrad_sum_kernel<<<(unsigned)blocks, 256, 0, stream>>>(partials, grad_w, grad_b, (int)chunks, nw, out_f);
     note_launch();
     return cudaGetLastError();
 }

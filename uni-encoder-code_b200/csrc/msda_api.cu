@@ -33,6 +33,12 @@ cudaError_t launch_bwd_d32_fused(const float *, const float *, const int64_t *, 
 cudaError_t launch_bwd_sorted_fused(const float *, const float *, const int64_t *, const int64_t *,
                                     const float *, long long, const float *, const float *,
                                     const Dims &, float *, float *, float *, cudaStream_t, bool *handled, int gate);
+cudaError_t launch_bwd_d32_records(const float *, const float *, const int64_t *, const int64_t *, const float *,
+                                   long long, const float *, const float *, const Dims &, float *, float *,
+                                   const DetRecords &, cudaStream_t, bool *handled);
+template <typename T>
+cudaError_t launch_bwd_generic_records(const T *, const T *, const int64_t *, const int64_t *, const T *, const T *,
+                                       const Dims &, T *, T *, const DetRecords &, cudaStream_t);
 template <typename T>
 cudaError_t launch_fwd_generic(const T *, const int64_t *, const int64_t *, const T *, const T *,
                                const Dims &, T *, cudaStream_t);
@@ -40,14 +46,16 @@ template <typename T>
 cudaError_t launch_bwd_generic(const T *, const T *, const int64_t *, const int64_t *, const T *,
                                const T *, const Dims &, T *, T *, T *, cudaStream_t);
 cudaError_t launch_linear_tf32x3(const float *, const float *, const float *, float *, int, int, int, int,
-                                 float *, cudaStream_t, bool *handled);
+                                 float *, cudaStream_t, bool *handled, bool deterministic);
 cudaError_t launch_split_weight(const float *, float *, int, int, cudaStream_t, bool *handled);
 cudaError_t launch_add_layernorm(const float *, const float *, const float *, const float *, float *, long long,
                                  int, float, cudaStream_t, bool *handled);
 cudaError_t launch_add_layernorm_bwd(const float *, const float *, const float *, const float *, float *, float *,
-                                     float *, long long, int, float, cudaStream_t, bool *handled);
+                                     float *, long long, int, float, cudaStream_t, bool *handled, float *partials);
+long long add_layernorm_bwd_partials(long long rows, int cols);
 cudaError_t launch_linear_wgrad(const float *, const float *, float *, float *, long long, int, int, cudaStream_t,
-                                bool *handled);
+                                bool *handled, float *partials);
+long long linear_wgrad_partials(long long rows, int out_f, int in_f);
 cudaError_t launch_transpose(const float *, float *, long long, int, cudaStream_t);
 cudaError_t launch_group_norm(const float *, const float *, const float *, const float *, float *, int, int, int, int,
                               int, float, int, const float *, int, int, double *, float *mean_rstd, cudaStream_t,
@@ -112,6 +120,36 @@ static int option_index(const char *name) {
     if (!strcmp(name, "whatif_linear")) return OPT_WHATIF_LINEAR;
 #endif
     return -1;
+}
+
+// Deterministic backwards (msda_det.cu): the records kernel of the path, then sort, bounds and gather.
+template <typename T>
+static int backward_deterministic(const T *grad_output, const T *value, const int64_t *spatial_shapes,
+                                  const int64_t *level_start, const T *sampling_loc, const T *attn_weight,
+                                  const Dims &d, T *grad_value, T *grad_sampling_loc, T *grad_attn_weight,
+                                  void *workspace, cudaStream_t st) {
+    if (!grad_output || !value || !spatial_shapes || !level_start || !sampling_loc || !attn_weight ||
+        !grad_value || !grad_sampling_loc || !grad_attn_weight || !workspace)
+        return MSDA_ERR_NULL_POINTER;
+    if (int rc = check_dims(d)) return rc;
+    DetLayout l;
+    if (!det_layout(d, (int)sizeof(T), &l)) return MSDA_ERR_BAD_SHAPE;
+    if (!aligned16(workspace)) return MSDA_ERR_UNSUPPORTED;
+    const DetRecords rec = det_records(workspace, l);
+    bool handled = false;
+    cudaError_t e = cudaSuccess;
+    if constexpr (sizeof(T) == 4) {
+        const bool fast_ok = aligned16(value) && aligned16(grad_output) && aligned8(sampling_loc) &&
+                             aligned8(grad_sampling_loc);
+        if (option_value(OPT_BWD_VARIANT) != 63 && fast_ok)
+            e = launch_bwd_d32_records(grad_output, value, spatial_shapes, level_start, nullptr, 0, sampling_loc,
+                                       attn_weight, d, grad_sampling_loc, grad_attn_weight, rec, st, &handled);
+    }
+    if (e == cudaSuccess && !handled)
+        e = launch_bwd_generic_records<T>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
+                                          d, grad_sampling_loc, grad_attn_weight, rec, st);
+    if (e == cudaSuccess) e = launch_det_reduce<T>(l, workspace, grad_output, grad_value, d, st);
+    return (int)e;
 }
 
 }  // namespace msda
@@ -329,13 +367,89 @@ int msda_b200_fused_backward_f32(const float *grad_output, const float *value,
     return (int)e;
 }
 
+long long msda_b200_backward_deterministic_workspace_bytes(int batch, int spatial_size, int num_heads, int channels,
+                                                          int num_levels, int num_query, int num_point,
+                                                          int value_bytes) {
+    const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
+    DetLayout l;
+    if (check_dims(d) != MSDA_OK || (value_bytes != 4 && value_bytes != 8) || !det_layout(d, value_bytes, &l)) return 0;
+    return (long long)l.total;
+}
+
+int msda_b200_backward_deterministic_f32(const float *grad_output, const float *value,
+                                         const int64_t *spatial_shapes, const int64_t *level_start,
+                                         const float *sampling_loc, const float *attn_weight, int batch,
+                                         int spatial_size, int num_heads, int channels, int num_levels,
+                                         int num_query, int num_point, float *grad_value,
+                                         float *grad_sampling_loc, float *grad_attn_weight, void *workspace,
+                                         void *stream) {
+    const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
+    return backward_deterministic<float>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight, d,
+                                         grad_value, grad_sampling_loc, grad_attn_weight, workspace,
+                                         (cudaStream_t)stream);
+}
+
+int msda_b200_backward_deterministic_f64(const double *grad_output, const double *value,
+                                         const int64_t *spatial_shapes, const int64_t *level_start,
+                                         const double *sampling_loc, const double *attn_weight, int batch,
+                                         int spatial_size, int num_heads, int channels, int num_levels,
+                                         int num_query, int num_point, double *grad_value,
+                                         double *grad_sampling_loc, double *grad_attn_weight, void *workspace,
+                                         void *stream) {
+    const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
+    return backward_deterministic<double>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
+                                          d, grad_value, grad_sampling_loc, grad_attn_weight, workspace,
+                                          (cudaStream_t)stream);
+}
+
+int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const float *value,
+                                               const int64_t *spatial_shapes, const int64_t *level_start,
+                                               const float *reference_points, long long ref_batch_stride,
+                                               const float *sampling_offsets, const float *attn_logits, int batch,
+                                               int spatial_size, int num_heads, int channels, int num_levels,
+                                               int num_query, int num_point, float *grad_value,
+                                               float *grad_sampling_offsets, float *grad_attn_logits,
+                                               void *workspace, void *stream) {
+    if (!grad_output || !value || !spatial_shapes || !level_start || !reference_points ||
+        !sampling_offsets || !attn_logits || !grad_value || !grad_sampling_offsets || !grad_attn_logits || !workspace)
+        return MSDA_ERR_NULL_POINTER;
+    const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
+    if (int rc = check_dims(d)) return rc;
+    if (ref_batch_stride != 0 && ref_batch_stride != (long long)num_query * num_levels * 2)
+        return MSDA_ERR_BAD_SHAPE;
+    DetLayout l;
+    if (!det_layout(d, 4, &l)) return MSDA_ERR_BAD_SHAPE;
+    const bool aligned = aligned16(value) && aligned16(grad_output) && aligned16(workspace) &&
+                         aligned8(sampling_offsets) && aligned8(grad_sampling_offsets) && aligned8(reference_points);
+    if (!aligned) return MSDA_ERR_UNSUPPORTED;
+    cudaStream_t st = (cudaStream_t)stream;
+    bool handled = false;
+    cudaError_t e = launch_bwd_d32_records(grad_output, value, spatial_shapes, level_start, reference_points,
+                                           ref_batch_stride, sampling_offsets, attn_logits, d, grad_sampling_offsets,
+                                           grad_attn_logits, det_records(workspace, l), st, &handled);
+    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
+    if (e == cudaSuccess) e = launch_det_reduce<float>(l, workspace, grad_output, grad_value, d, st);
+    return (int)e;
+}
+
 int msda_b200_linear_f32(const float *x, const float *weight, const float *bias, float *y, int rows,
                          int out_features, int in_features, int relu, float *workspace, void *stream) {
     if (!x || !weight || !y) return MSDA_ERR_NULL_POINTER;
     if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
     cudaError_t e = launch_linear_tf32x3(x, weight, bias, y, rows, out_features, in_features, relu,
-                                         workspace, (cudaStream_t)stream, &handled);
+                                         workspace, (cudaStream_t)stream, &handled, false);
+    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
+    return (int)e;
+}
+
+int msda_b200_linear_deterministic_f32(const float *x, const float *weight, const float *bias, float *y, int rows,
+                                       int out_features, int in_features, int relu, float *workspace, void *stream) {
+    if (!x || !weight || !y) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    cudaError_t e = launch_linear_tf32x3(x, weight, bias, y, rows, out_features, in_features, relu,
+                                         workspace, (cudaStream_t)stream, &handled, true);
     if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
     return (int)e;
 }
@@ -357,7 +471,18 @@ int msda_b200_linear_presplit_f32(const float *x, const float *split_weight, con
     bool handled = false;
     // the kernel only reads the split weight
     cudaError_t e = launch_linear_tf32x3(x, nullptr, bias, y, rows, out_features, in_features, relu,
-                                         const_cast<float *>(split_weight), (cudaStream_t)stream, &handled);
+                                         const_cast<float *>(split_weight), (cudaStream_t)stream, &handled, false);
+    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
+    return (int)e;
+}
+
+int msda_b200_linear_presplit_deterministic_f32(const float *x, const float *split_weight, const float *bias, float *y,
+                                                int rows, int out_features, int in_features, int relu, void *stream) {
+    if (!x || !split_weight || !y) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    cudaError_t e = launch_linear_tf32x3(x, nullptr, bias, y, rows, out_features, in_features, relu,
+                                         const_cast<float *>(split_weight), (cudaStream_t)stream, &handled, true);
     if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
     return (int)e;
 }
@@ -379,9 +504,27 @@ int msda_b200_add_layernorm_backward_f32(const float *grad_y, const float *x, co
     if (rows <= 0 || cols <= 0) return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
     cudaError_t e = launch_add_layernorm_bwd(grad_y, x, residual, gamma, grad_v, grad_gamma, grad_beta, rows, cols,
-                                             eps, (cudaStream_t)stream, &handled);
+                                             eps, (cudaStream_t)stream, &handled, nullptr);
     if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
     return (int)e;
+}
+
+int msda_b200_add_layernorm_backward_deterministic_f32(const float *grad_y, const float *x, const float *residual,
+                                                       const float *gamma, float *grad_v, float *grad_gamma,
+                                                       float *grad_beta, long long rows, int cols, float eps,
+                                                       void *workspace, void *stream) {
+    if (!grad_y || !x || !gamma || !grad_v || !grad_gamma || !grad_beta || !workspace) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || cols <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    cudaError_t e = launch_add_layernorm_bwd(grad_y, x, residual, gamma, grad_v, grad_gamma, grad_beta, rows, cols,
+                                             eps, (cudaStream_t)stream, &handled, static_cast<float *>(workspace));
+    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
+    return (int)e;
+}
+
+long long msda_b200_add_layernorm_backward_deterministic_workspace_bytes(long long rows, int cols) {
+    if (rows <= 0 || cols <= 0) return 0;
+    return add_layernorm_bwd_partials(rows, cols) * (long long)sizeof(float);
 }
 
 int msda_b200_linear_wgrad_f32(const float *grad_y, const float *x, float *grad_weight, float *grad_bias,
@@ -390,9 +533,26 @@ int msda_b200_linear_wgrad_f32(const float *grad_y, const float *x, float *grad_
     if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
     cudaError_t e = launch_linear_wgrad(grad_y, x, grad_weight, grad_bias, rows, out_features, in_features,
-                                        (cudaStream_t)stream, &handled);
+                                        (cudaStream_t)stream, &handled, nullptr);
     if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
     return (int)e;
+}
+
+int msda_b200_linear_wgrad_deterministic_f32(const float *grad_y, const float *x, float *grad_weight, float *grad_bias,
+                                             long long rows, int out_features, int in_features, void *workspace,
+                                             void *stream) {
+    if (!grad_y || !x || !grad_weight || !workspace) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    cudaError_t e = launch_linear_wgrad(grad_y, x, grad_weight, grad_bias, rows, out_features, in_features,
+                                        (cudaStream_t)stream, &handled, static_cast<float *>(workspace));
+    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
+    return (int)e;
+}
+
+long long msda_b200_linear_wgrad_deterministic_workspace_bytes(long long rows, int out_features, int in_features) {
+    if (rows <= 0 || out_features <= 0 || in_features <= 0) return 0;
+    return linear_wgrad_partials(rows, out_features, in_features) * (long long)sizeof(float);
 }
 
 int msda_b200_group_norm_nchw_f32(const float *x, const float *channel_bias, const float *gamma, const float *beta,

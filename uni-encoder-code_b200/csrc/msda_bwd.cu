@@ -53,17 +53,19 @@ struct BwdCfg {
 };
 
 // BATCH = record pairs whose 2*BATCH value loads are in flight together (register budget)
+// RECORDS: deterministic mode (msda_det.cu) -- grad_value is not touched; each corner's {destination row,
+// weight} goes to its fixed slot of `det` instead (chunk lane 0 of each corner group writes it)
 // FUSED: `loc` / `attw` are the raw sampling offsets / attention logits and `grad_loc` / `grad_attw`
 // receive the gradients with respect to THEM (offset gradient = location gradient / (W, H);
 // softmax backward folded in), see phase1_records() in msda_common.cuh.
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED>
+template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED, bool RECORDS>
 __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
 msda_bwd_d32_kernel(const float *__restrict__ grad_out, const float *__restrict__ value,
                     const int64_t *__restrict__ shapes, const int64_t *__restrict__ lstart,
                     const float *__restrict__ loc, const float *__restrict__ attw,
                     const Producers pr, const Dims d, const int flags,
                     float *__restrict__ grad_value, float *__restrict__ grad_loc,
-                    float *__restrict__ grad_attw, const int gate) {
+                    float *__restrict__ grad_attw, const int gate, const DetRecords det) {
     using Cfg = BwdCfg<LP, WARPS, TILE_W, QPW>;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ LevelTable lt;
@@ -114,6 +116,9 @@ msda_bwd_d32_kernel(const float *__restrict__ grad_out, const float *__restrict_
             const long long qrow = (n * d.Lq + q0 + qi) * M + m;
             const float4 go = ldg_stream_f4(reinterpret_cast<const float4 *>(grad_out) + qrow * 8 + chunk);
             const uint4 *rq = plane + qi * Cfg::kPairs;
+            // RECORDS: this query-head's first slot, and the first grad_value row of image n
+            const uint32_t slot0 = (uint32_t)qrow * (uint32_t)(LP * 4) + (uint32_t)corner;
+            const uint32_t key0 = (uint32_t)n * (uint32_t)d.S * (uint32_t)M;
             float dpart[LP];
 #pragma unroll
             for (int pb = 0; pb < Cfg::kPairs; pb += BATCH) {
@@ -135,7 +140,18 @@ msda_bwd_d32_kernel(const float *__restrict__ grad_out, const float *__restrict_
                     if (pb + j < Cfg::kPairs) {
                         const int sp = 2 * (pb + j);
                         const float wa = __uint_as_float(e[j].y), wc = __uint_as_float(e[j].w);
-                        if (pb + j >= drop_pairs) {
+                        if (RECORDS) {
+                            if (chunk == 0) {
+                                const uint32_t sa = slot0 + (uint32_t)sp * 4u, sc = sa + 4u;
+                                // record offsets are (pixel*M + m)*8 float4 from the image start
+                                det.key[sa] = e[j].x != kNoCorner ? key0 + (e[j].x >> 3) : det.sentinel;
+                                det.key[sc] = e[j].z != kNoCorner ? key0 + (e[j].z >> 3) : det.sentinel;
+                                det.slot_id[sa] = sa;
+                                det.slot_id[sc] = sc;
+                                static_cast<float *>(det.w)[sa] = wa;
+                                static_cast<float *>(det.w)[sc] = wc;
+                            }
+                        } else if (pb + j >= drop_pairs) {
                             red_add_f4_if(gvb, e[j].x, make_float4(wa * go.x, wa * go.y, wa * go.z, wa * go.w));
                             red_add_f4_if(gvb, e[j].z, make_float4(wc * go.x, wc * go.y, wc * go.z, wc * go.w));
                         }
@@ -244,14 +260,15 @@ msda_bwd_d32_kernel(const float *__restrict__ grad_out, const float *__restrict_
 // ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED = false>
+template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED = false, bool RECORDS = false>
 static cudaError_t launch_bwd_cfg(const float *grad_out, const float *value, const int64_t *shapes,
                                   const int64_t *lstart, const float *loc, const float *attw,
                                   const Dims &d, float *grad_value, float *grad_loc,
                                   float *grad_attw, cudaStream_t stream,
-                                  Producers pr = Producers{nullptr, 0, 0, 0, nullptr, nullptr}, int gate = GATE_NONE) {
+                                  Producers pr = Producers{nullptr, 0, 0, 0, nullptr, nullptr}, int gate = GATE_NONE,
+                                  DetRecords det = DetRecords{nullptr, nullptr, nullptr, 0}) {
     using Cfg = BwdCfg<LP, WARPS, TILE_W, QPW>;
-    auto kern = msda_bwd_d32_kernel<LP, WARPS, TILE_W, MIN_CTAS, BATCH, QPW, FUSED>;
+    auto kern = msda_bwd_d32_kernel<LP, WARPS, TILE_W, MIN_CTAS, BATCH, QPW, FUSED, RECORDS>;
     // the opt-in shared-memory size is a per-device function attribute: set it (and query the
     // occupancy) once per device; the values are immutable afterwards
     static std::atomic<int> ctas_per_sm_of[kMaxDevices];
@@ -278,7 +295,7 @@ static cudaError_t launch_bwd_cfg(const float *grad_out, const float *value, con
     const int flags = (option_value(OPT_TILE_ORDER) != 1 ? 1 : 0) | (whatif_value(OPT_WHATIF_DROP_REDS) << 1);
     kern<<<(unsigned)blocks, WARPS * 32, Cfg::kSmem, stream>>>(grad_out, value, shapes, lstart, loc,
                                                               attw, pr, d, flags, grad_value,
-                                                              grad_loc, grad_attw, gate);
+                                                              grad_loc, grad_attw, gate, det);
     note_launch();
     return cudaGetLastError();
 }
@@ -347,6 +364,34 @@ cudaError_t launch_bwd_d32_fused(const float *grad_out, const float *value, cons
         default: *handled = false; return cudaSuccess;
     }
 #undef MSDA_BWD_FUSED
+}
+
+// Deterministic mode: the records kernel of the default CTA shape (16 warps, 8x16 tiles), plain or fused
+// (ref != nullptr: `loc` / `attw` are the raw offsets / logits).  Same domain as the two launchers above.
+cudaError_t launch_bwd_d32_records(const float *grad_out, const float *value, const int64_t *shapes,
+                                   const int64_t *lstart, const float *ref, long long ref_bstride,
+                                   const float *loc, const float *attw, const Dims &d, float *gl, float *gw,
+                                   const DetRecords &det, cudaStream_t st, bool *handled) {
+    *handled = true;
+    if (d.D != 32 || (long long)d.S * d.M * 8 >= 0x7fffffffLL) {
+        *handled = false;
+        return cudaSuccess;
+    }
+    const Producers none{nullptr, 0, 0, 0, nullptr, nullptr}, fused{ref, ref_bstride};
+#define MSDA_BWD_REC(LPV)                                                                                          \
+    (ref != nullptr                                                                                                \
+         ? launch_bwd_cfg<LPV, 16, 16, 2, 1, 8, true, true>(grad_out, value, shapes, lstart, loc, attw, d, nullptr, \
+                                                            gl, gw, st, fused, GATE_NONE, det)                     \
+         : launch_bwd_cfg<LPV, 16, 16, 2, 1, 8, false, true>(grad_out, value, shapes, lstart, loc, attw, d, nullptr,\
+                                                             gl, gw, st, none, GATE_NONE, det))
+    switch (d.L * d.P) {
+        case 4: return MSDA_BWD_REC(4);
+        case 8: return MSDA_BWD_REC(8);
+        case 12: return MSDA_BWD_REC(12);
+        case 16: return MSDA_BWD_REC(16);
+        default: *handled = false; return cudaSuccess;
+    }
+#undef MSDA_BWD_REC
 }
 
 }  // namespace msda

@@ -529,6 +529,32 @@ struct Dims {
     int N, S, M, D, L, Lq, P;
 };
 
+// Deterministic backward (msda_det.cu): instead of reducing into grad_value, the backward kernels
+// write one record per (sampling point, corner) into the fixed slot
+//     ((((n*Lq + q)*M + m)*L + l)*P + p)*4 + corner
+// key[slot] = destination grad_value row (n*S + pixel)*M + m, or `sentinel` (= N*S*M) for a corner that
+// does not contribute; slot_id[slot] = slot (the values the stable sort carries); w[slot] = bilinear corner
+// weight * attention weight (of the value type: float or double; 0 for the sentinel).
+struct DetRecords {
+    uint32_t *key;
+    uint32_t *slot_id;
+    void *w;
+    uint32_t sentinel;
+};
+// the deterministic backward's workspace (msda_det.cu)
+struct DetLayout {
+    long long records;          // N*Lq*M*L*P*4
+    uint32_t rows;              // N*S*M: grad_value rows, also the sentinel key
+    int end_bit;                // bit width of `rows`
+    size_t keys_a, keys_b, ids_a, ids_b, w, start, temp;   // byte offsets into the workspace
+    size_t temp_bytes, total;
+};
+bool det_layout(const Dims &d, int value_bytes, DetLayout *out);
+DetRecords det_records(void *ws, const DetLayout &l);
+template <typename T>
+cudaError_t launch_det_reduce(const DetLayout &l, void *ws, const T *grad_out, T *grad_value, const Dims &d,
+                              cudaStream_t stream);
+
 void note_launch();                   // increments the library launch counter
 int sm_count();                       // SMs of the current device (cached)
 int option_value(int which);          // tuning knobs, see msda_api.cu

@@ -8,7 +8,9 @@
 //
 // One warp per (image, query, head) row; lanes stride over channels, so a corner
 // row is read as one coalesced segment.  grad_sampling_loc / grad_attn_weight are
-// warp-shuffle sums (no shared memory, no barrier); grad_value uses scalar atomics.
+// warp-shuffle sums (no shared memory, no barrier); grad_value uses scalar atomics, or, in the
+// deterministic mode (RECORDS, msda_det.cu), is left alone while lanes 0-3 write the four corner records
+// of every point.
 #include "msda_common.cuh"
 
 namespace msda {
@@ -70,13 +72,13 @@ msda_fwd_generic_kernel(const T *__restrict__ value, const int64_t *__restrict__
     }
 }
 
-template <typename T>
+template <typename T, bool RECORDS>
 __global__ void __launch_bounds__(256)
 msda_bwd_generic_kernel(const T *__restrict__ grad_out, const T *__restrict__ value,
                         const int64_t *__restrict__ shapes, const int64_t *__restrict__ lstart,
                         const T *__restrict__ loc, const T *__restrict__ attw, const Dims d,
                         T *__restrict__ grad_value, T *__restrict__ grad_loc,
-                        T *__restrict__ grad_attw) {
+                        T *__restrict__ grad_attw, const DetRecords det) {
     __shared__ LevelTable lt;
     fill_level_table(lt, shapes, lstart, d.L, d.P, d.S, d.Lq, 8, 1, 8, 0);
     __syncthreads();
@@ -96,6 +98,18 @@ msda_bwd_generic_kernel(const T *__restrict__ grad_out, const T *__restrict__ va
                 const long long s = (row * d.L + l) * d.P + p;
                 const Geom<T> g = decompose(loc[2 * s], loc[2 * s + 1], H, W);
                 T gx = 0, gy = 0, ga = 0;
+                if (RECORDS && lane < 4) {          // lane k: corner k (also of an invalid point: cmask == 0)
+                    const int k = lane;
+                    const bool live = g.cmask >> k & 1;
+                    const T hh = 1 - g.lh, hw = 1 - g.lw;
+                    const T cw = k == 0 ? hh * hw : k == 1 ? hh * g.lw : k == 2 ? g.lh * hw : g.lh * g.lw;
+                    // element offset / D = destination row (n*S + pixel)*M + m
+                    const long long o = lvl + (((long long)g.h_low + (k >> 1)) * W + g.w_low + (k & 1)) * pix;
+                    const uint32_t slot = (uint32_t)(4 * s + k);
+                    det.key[slot] = live ? (uint32_t)(o / d.D) : det.sentinel;
+                    det.slot_id[slot] = slot;
+                    static_cast<T *>(det.w)[slot] = live ? cw * attw[s] : (T)0;
+                }
                 if (g.valid) {
                     const T a = attw[s];
                     const T hh = 1 - g.lh, hw = 1 - g.lw;
@@ -119,7 +133,7 @@ msda_bwd_generic_kernel(const T *__restrict__ grad_out, const T *__restrict__ va
                                 sh += dh[k] * v;
                                 sw += dw[k] * v;
                                 val += cw[k] * v;
-                                atomicAdd(grad_value + o, cw[k] * tgv);
+                                if (!RECORDS) atomicAdd(grad_value + o, cw[k] * tgv);
                             }
                         }
                         ga += tg * val;
@@ -194,8 +208,20 @@ cudaError_t launch_bwd_generic(const T *grad_out, const T *value, const int64_t 
                                const int64_t *lstart, const T *loc, const T *attw, const Dims &d,
                                T *gv, T *gl, T *gw, cudaStream_t stream) {
     const long long rows = (long long)d.N * d.Lq * d.M;
-    msda_bwd_generic_kernel<T><<<grid_for(rows, 8), 256, 0, stream>>>(grad_out, value, shapes, lstart,
-                                                                       loc, attw, d, gv, gl, gw);
+    msda_bwd_generic_kernel<T, false><<<grid_for(rows, 8), 256, 0, stream>>>(
+        grad_out, value, shapes, lstart, loc, attw, d, gv, gl, gw, DetRecords{nullptr, nullptr, nullptr, 0});
+    note_launch();
+    return cudaGetLastError();
+}
+
+// deterministic mode: grad_loc / grad_attw as above, the corner records into `det` (grad_value untouched)
+template <typename T>
+cudaError_t launch_bwd_generic_records(const T *grad_out, const T *value, const int64_t *shapes,
+                                       const int64_t *lstart, const T *loc, const T *attw, const Dims &d,
+                                       T *gl, T *gw, const DetRecords &det, cudaStream_t stream) {
+    const long long rows = (long long)d.N * d.Lq * d.M;
+    msda_bwd_generic_kernel<T, true><<<grid_for(rows, 8), 256, 0, stream>>>(grad_out, value, shapes, lstart,
+                                                                             loc, attw, d, nullptr, gl, gw, det);
     note_launch();
     return cudaGetLastError();
 }
@@ -221,5 +247,13 @@ template cudaError_t launch_bwd_generic<double>(const double *, const double *, 
                                                 const int64_t *, const double *, const double *,
                                                 const Dims &, double *, double *, double *,
                                                 cudaStream_t);
+template cudaError_t launch_bwd_generic_records<float>(const float *, const float *, const int64_t *,
+                                                       const int64_t *, const float *, const float *,
+                                                       const Dims &, float *, float *, const DetRecords &,
+                                                       cudaStream_t);
+template cudaError_t launch_bwd_generic_records<double>(const double *, const double *, const int64_t *,
+                                                        const int64_t *, const double *, const double *,
+                                                        const Dims &, double *, double *, const DetRecords &,
+                                                        cudaStream_t);
 
 }  // namespace msda

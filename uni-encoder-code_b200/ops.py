@@ -53,6 +53,32 @@ class _timed:
 
 _FWD = {torch.float32: _lib.lib.msda_b200_forward_f32, torch.float64: _lib.lib.msda_b200_forward_f64}
 _BWD = {torch.float32: _lib.lib.msda_b200_backward_f32, torch.float64: _lib.lib.msda_b200_backward_f64}
+_BWD_DET = {torch.float32: _lib.lib.msda_b200_backward_deterministic_f32,
+            torch.float64: _lib.lib.msda_b200_backward_deterministic_f64}
+
+# With torch.use_deterministic_algorithms(True) every backward here takes its deterministic entry point.  The
+# MSDA backwards then sort one record per (sampling point, corner): the batch is processed in chunks of whole
+# images of at most this many records (20 bytes each in fp32, plus the sort's scratch), which bounds the
+# workspace and keeps the record slots 32-bit.  Chunks write disjoint grad_value rows, so the chunking cannot
+# change a bit of the result.
+DETERMINISTIC_RECORD_LIMIT = 1 << 25
+
+
+def _deterministic() -> bool:
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def _image_chunks(N, records_per_image):
+    step = max(1, min(N, DETERMINISTIC_RECORD_LIMIT // records_per_image))
+    return [(n0, min(N, n0 + step)) for n0 in range(0, N, step)]
+
+
+def _det_workspace(images, S, M, D, L, Lq, P, dtype, device):
+    nbytes = _lib.lib.msda_b200_backward_deterministic_workspace_bytes(images, S, M, D, L, Lq, P,
+                                                                       torch.empty((), dtype=dtype).element_size())
+    if nbytes <= 0:
+        raise RuntimeError("deterministic MSDA backward: one image has more than 2^31 - 1 corner records")
+    return torch.empty(int(nbytes), dtype=torch.uint8, device=device)
 
 
 def _check_common(named, im2col_step, opname):
@@ -127,6 +153,9 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
     if N * Lq * M * D == 0 or S == 0 or L * P == 0:
         # nothing to sample: all three gradients stay at the reference's zero fill (cu:126-128)
         return [torch.zeros_like(value), torch.zeros_like(sampling_loc), torch.zeros_like(attn_weight)]
+    if _deterministic():
+        return _ms_deform_attn_backward_deterministic(value, spatial_shapes, level_start_index, sampling_loc,
+                                                      attn_weight, grad_output, N, S, M, D, L, Lq, P)
     with torch.cuda.device(value.device):
         grad_value = torch.zeros_like(value)            # accumulated by reductions (cu:126)
         grad_loc = torch.empty_like(sampling_loc)       # fully overwritten (cf. cu:127)
@@ -138,6 +167,26 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
                 N, S, M, D, L, Lq, P, grad_value.data_ptr(), grad_loc.data_ptr(), grad_w.data_ptr(),
                 torch.cuda.current_stream().cuda_stream)
     _lib.check(rc, "ms_deform_attn_backward")
+    return [grad_value, grad_loc, grad_w]
+
+
+def _ms_deform_attn_backward_deterministic(value, shapes, lsi, loc, w, grad_output, N, S, M, D, L, Lq, P):
+    """ms_deform_attn_backward through msda_b200_backward_deterministic_f32/_f64, in chunks of whole images."""
+    chunks = _image_chunks(N, Lq * M * L * P * 4)
+    with torch.cuda.device(value.device):
+        grad_value = torch.empty_like(value)            # fully overwritten by the gather
+        grad_loc = torch.empty_like(loc)
+        grad_w = torch.empty_like(w)
+        ws = _det_workspace(max(b - a for a, b in chunks), S, M, D, L, Lq, P, value.dtype, value.device)
+        stream = torch.cuda.current_stream().cuda_stream
+        with _timed("backward"):
+            for a, b in chunks:
+                rc = _BWD_DET[value.dtype](
+                    grad_output[a:b].data_ptr(), value[a:b].data_ptr(), shapes.data_ptr(), lsi.data_ptr(),
+                    loc[a:b].data_ptr(), w[a:b].data_ptr(), b - a, S, M, D, L, Lq, P,
+                    grad_value[a:b].data_ptr(), grad_loc[a:b].data_ptr(), grad_w[a:b].data_ptr(), ws.data_ptr(),
+                    stream)
+                _lib.check(rc, "ms_deform_attn_backward (deterministic)")
     return [grad_value, grad_loc, grad_w]
 
 
@@ -271,6 +320,10 @@ def ms_deform_attn_fused_backward(value, spatial_shapes, level_start_index, refe
     """[grad_value, grad_sampling_offsets, grad_attn_logits] (msda_b200_fused_backward_f32)."""
     N, S, M, D, L, Lq, P, rs = _check_fused(value, spatial_shapes, level_start_index, reference_points,
                                             sampling_offsets, attn_logits, [("grad_output", grad_output)])
+    if _deterministic():
+        return _ms_deform_attn_fused_backward_deterministic(value, spatial_shapes, level_start_index, reference_points,
+                                                            sampling_offsets, attn_logits, grad_output, rs,
+                                                            N, S, M, D, L, Lq, P)
     with torch.cuda.device(value.device):
         grad_value = torch.zeros_like(value)
         grad_off = torch.empty_like(sampling_offsets)
@@ -283,6 +336,28 @@ def ms_deform_attn_fused_backward(value, spatial_shapes, level_start_index, refe
                 grad_value.data_ptr(), grad_off.data_ptr(), grad_logits.data_ptr(),
                 torch.cuda.current_stream().cuda_stream)
     _lib.check(rc, "ms_deform_attn_fused_backward")
+    return [grad_value, grad_off, grad_logits]
+
+
+def _ms_deform_attn_fused_backward_deterministic(value, shapes, lsi, ref, off, logits, grad_output, rs,
+                                                 N, S, M, D, L, Lq, P):
+    """ms_deform_attn_fused_backward through msda_b200_fused_backward_deterministic_f32, in chunks of whole images."""
+    chunks = _image_chunks(N, Lq * M * L * P * 4)
+    with torch.cuda.device(value.device):
+        grad_value = torch.empty_like(value)
+        grad_off = torch.empty_like(off)
+        grad_logits = torch.empty_like(logits)
+        ws = _det_workspace(max(b - a for a, b in chunks), S, M, D, L, Lq, P, value.dtype, value.device)
+        stream = torch.cuda.current_stream().cuda_stream
+        with _timed("backward"):
+            for a, b in chunks:
+                ref_a = ref[a:b] if rs != 0 and ref.size(0) == N else ref    # rs == 0: one set shared by the batch
+                rc = _lib.lib.msda_b200_fused_backward_deterministic_f32(
+                    grad_output[a:b].data_ptr(), value[a:b].data_ptr(), shapes.data_ptr(), lsi.data_ptr(),
+                    ref_a.data_ptr(), rs, off[a:b].data_ptr(), logits[a:b].data_ptr(), b - a, S, M, D, L, Lq, P,
+                    grad_value[a:b].data_ptr(), grad_off[a:b].data_ptr(), grad_logits[a:b].data_ptr(), ws.data_ptr(),
+                    stream)
+                _lib.check(rc, "ms_deform_attn_fused_backward (deterministic)")
     return [grad_value, grad_off, grad_logits]
 
 
@@ -338,8 +413,10 @@ def linear_tf32x3(x, weight, bias=None, relu=False, split_weight_in_kernel=False
         if not (presplit.is_cuda and presplit.device == x.device and presplit.dtype == torch.float32
                 and presplit.is_contiguous() and presplit.numel() == 2 * out_f * in_f):
             raise RuntimeError("presplit must be split_weight(weight) on x's device")
+        fn = (_lib.lib.msda_b200_linear_presplit_deterministic_f32 if _deterministic()
+              else _lib.lib.msda_b200_linear_presplit_f32)
         with torch.cuda.device(x.device):
-            rc = _lib.lib.msda_b200_linear_presplit_f32(x.data_ptr(), presplit.data_ptr(),
+            rc = fn(x.data_ptr(), presplit.data_ptr(),
                                                         bias.data_ptr() if bias is not None else None, y.data_ptr(),
                                                         rows, out_f, in_f, 1 if relu else 0,
                                                         torch.cuda.current_stream(x.device).cuda_stream)
@@ -347,8 +424,9 @@ def linear_tf32x3(x, weight, bias=None, relu=False, split_weight_in_kernel=False
         return y
     workspace = None if split_weight_in_kernel else \
         torch.empty(2 * out_f * in_f, dtype=torch.float32, device=x.device)
+    fn = _lib.lib.msda_b200_linear_deterministic_f32 if _deterministic() else _lib.lib.msda_b200_linear_f32
     with torch.cuda.device(x.device):
-        rc = _lib.lib.msda_b200_linear_f32(x.data_ptr(), weight.data_ptr(),
+        rc = fn(x.data_ptr(), weight.data_ptr(),
                                            bias.data_ptr() if bias is not None else None, y.data_ptr(),
                                            rows, out_f, in_f, 1 if relu else 0,
                                            workspace.data_ptr() if workspace is not None else None,
@@ -562,11 +640,16 @@ def linear_wgrad(grad_y, x, with_bias=True):
                            "out % 4 == 0 and in % 4 == 0")
     gw = torch.empty(grad_y.size(1), x.size(1), dtype=torch.float32, device=x.device)
     gb = torch.empty(grad_y.size(1), dtype=torch.float32, device=x.device) if with_bias else None
+    rows, out_f, in_f = grad_y.size(0), grad_y.size(1), x.size(1)
     with torch.cuda.device(x.device):
-        rc = _lib.lib.msda_b200_linear_wgrad_f32(grad_y.data_ptr(), x.data_ptr(), gw.data_ptr(),
-                                                 gb.data_ptr() if gb is not None else None, grad_y.size(0),
-                                                 grad_y.size(1), x.size(1),
-                                                 torch.cuda.current_stream(x.device).cuda_stream)
+        stream = torch.cuda.current_stream(x.device).cuda_stream
+        if _deterministic():      # per-chunk partial tiles, added in chunk order
+            ws = _workspace(_lib.lib.msda_b200_linear_wgrad_deterministic_workspace_bytes(rows, out_f, in_f), x)
+            rc = _lib.lib.msda_b200_linear_wgrad_deterministic_f32(grad_y.data_ptr(), x.data_ptr(), gw.data_ptr(),
+                                                                   _ptr(gb), rows, out_f, in_f, ws.data_ptr(), stream)
+        else:
+            rc = _lib.lib.msda_b200_linear_wgrad_f32(grad_y.data_ptr(), x.data_ptr(), gw.data_ptr(), _ptr(gb), rows,
+                                                     out_f, in_f, stream)
     _lib.check(rc, "linear_wgrad")
     return gw, gb
 
@@ -580,11 +663,16 @@ def add_layernorm_backward(grad_y, x, residual, weight, eps=1e-5):
     gv = torch.empty_like(x)
     gg, gb = torch.empty_like(weight), torch.empty_like(weight)
     cols = x.size(-1)
+    rows = x.numel() // cols
     with torch.cuda.device(x.device):
-        rc = _lib.lib.msda_b200_add_layernorm_backward_f32(
-            grad_y.data_ptr(), x.data_ptr(), residual.data_ptr() if residual is not None else None,
-            weight.data_ptr(), gv.data_ptr(), gg.data_ptr(), gb.data_ptr(), x.numel() // cols, cols, float(eps),
-            torch.cuda.current_stream(x.device).cuda_stream)
+        args = (grad_y.data_ptr(), x.data_ptr(), _ptr(residual), weight.data_ptr(), gv.data_ptr(), gg.data_ptr(),
+                gb.data_ptr(), rows, cols, float(eps))
+        stream = torch.cuda.current_stream(x.device).cuda_stream
+        if _deterministic():      # per-CTA partials of grad_weight / grad_bias, added in CTA order
+            ws = _workspace(_lib.lib.msda_b200_add_layernorm_backward_deterministic_workspace_bytes(rows, cols), x)
+            rc = _lib.lib.msda_b200_add_layernorm_backward_deterministic_f32(*args, ws.data_ptr(), stream)
+        else:
+            rc = _lib.lib.msda_b200_add_layernorm_backward_f32(*args, stream)
     _lib.check(rc, "add_layernorm_backward")
     return gv, gg, gb
 
