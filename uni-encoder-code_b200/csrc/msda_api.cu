@@ -4,6 +4,11 @@
 // (ms_deform_attn_cuda.cu:25-85, 88-158): argument validation and kernel choice.
 // Tensor-level checks (contiguity, device, dtype, im2col_step divisibility) live in
 // the Python shim because they need tensor metadata; this layer sees raw pointers.
+//
+// The plain and the fused-producer MSDA entries differ only in the Producers they hand to the
+// launchers (reference points == nullptr: plain), so each backward has one body for both:
+// backward_f32() (kernel choice and "bwd_variant") and backward_deterministic().  Entries that
+// come as a default and a deterministic / training twin forward to one static body each.
 #include <atomic>
 #include <cstdint>
 #include <cstring>
@@ -14,28 +19,15 @@
 namespace msda {
 
 // implemented in the kernel translation units
-cudaError_t launch_fwd_d32(const float *, const int64_t *, const int64_t *, const float *,
-                           const float *, const Dims &, float *, cudaStream_t, bool *handled);
-cudaError_t launch_bwd_d32(const float *, const float *, const int64_t *, const int64_t *,
-                           const float *, const float *, const Dims &, float *, float *, float *,
-                           cudaStream_t, bool *handled, int gate);
-cudaError_t launch_bwd_sorted(const float *, const float *, const int64_t *, const int64_t *,
-                              const float *, const float *, const Dims &, float *, float *, float *,
-                              cudaStream_t, bool *handled, int gate);
+cudaError_t launch_fwd_d32(const float *, const int64_t *, const int64_t *, const float *, const float *,
+                           const Producers &, const Dims &, float *, cudaStream_t, bool *handled);
+cudaError_t launch_bwd_d32(const float *, const float *, const int64_t *, const int64_t *, const float *,
+                           const float *, const Producers &, const Dims &, float *, float *, float *,
+                           const DetRecords *, int gate, cudaStream_t, bool *handled);
+cudaError_t launch_bwd_sorted(const float *, const float *, const int64_t *, const int64_t *, const float *,
+                              const float *, const Producers &, const Dims &, float *, float *, float *, int gate,
+                              cudaStream_t, bool *handled);
 bool bwd_sorted_applies(const float *value, const float *grad_value, const Dims &);
-cudaError_t launch_fwd_d32_fused(const float *, const int64_t *, const int64_t *, const float *,
-                                 long long, const float *, const float *, const Dims &, float *,
-                                 cudaStream_t, bool *handled, int off_qstride = 0, int logit_qstride = 0,
-                                 const float *off_table = nullptr, const float *logit_table = nullptr);
-cudaError_t launch_bwd_d32_fused(const float *, const float *, const int64_t *, const int64_t *,
-                                 const float *, long long, const float *, const float *,
-                                 const Dims &, float *, float *, float *, cudaStream_t, bool *handled, int gate);
-cudaError_t launch_bwd_sorted_fused(const float *, const float *, const int64_t *, const int64_t *,
-                                    const float *, long long, const float *, const float *,
-                                    const Dims &, float *, float *, float *, cudaStream_t, bool *handled, int gate);
-cudaError_t launch_bwd_d32_records(const float *, const float *, const int64_t *, const int64_t *, const float *,
-                                   long long, const float *, const float *, const Dims &, float *, float *,
-                                   const DetRecords &, cudaStream_t, bool *handled);
 template <typename T>
 cudaError_t launch_bwd_generic_records(const T *, const T *, const int64_t *, const int64_t *, const T *, const T *,
                                        const Dims &, T *, T *, const DetRecords &, cudaStream_t);
@@ -94,10 +86,12 @@ int sm_count() {
     return v;
 }
 
-static int check_dims(const Dims &d) {
+// ref_bstride: the fused entries' reference-point batch stride, 0 (shared by the batch) or Lq*L*2
+static int check_dims(const Dims &d, long long ref_bstride = 0) {
     if (d.N <= 0 || d.S <= 0 || d.M <= 0 || d.D <= 0 || d.L <= 0 || d.Lq <= 0 || d.P <= 0)
         return MSDA_ERR_BAD_SHAPE;
     if (d.L > MSDA_MAX_LEVELS) return MSDA_ERR_UNSUPPORTED;
+    if (ref_bstride != 0 && ref_bstride != (long long)d.Lq * d.L * 2) return MSDA_ERR_BAD_SHAPE;
     return MSDA_OK;
 }
 
@@ -106,6 +100,11 @@ static int check_dims(const Dims &d) {
 // which accept any alignment like the reference's scalar kernels do
 static bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static bool aligned8(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
+
+// the return code of a launcher that reports through `handled` whether it covers the problem
+static int launch_rc(cudaError_t e, bool handled) {
+    return e == cudaSuccess && !handled ? MSDA_ERR_UNSUPPORTED : (int)e;
+}
 
 static int option_index(const char *name) {
     if (!name) return -1;
@@ -122,16 +121,55 @@ static int option_index(const char *name) {
     return -1;
 }
 
-// Deterministic backwards (msda_det.cu): the records kernel of the path, then sort, bounds and gather.
-template <typename T>
-static int backward_deterministic(const T *grad_output, const T *value, const int64_t *spatial_shapes,
-                                  const int64_t *level_start, const T *sampling_loc, const T *attn_weight,
-                                  const Dims &d, T *grad_value, T *grad_sampling_loc, T *grad_attn_weight,
-                                  void *workspace, cudaStream_t st) {
-    if (!grad_output || !value || !spatial_shapes || !level_start || !sampling_loc || !attn_weight ||
-        !grad_value || !grad_sampling_loc || !grad_attn_weight || !workspace)
+// The fp32 backward, plain (pr.ref == nullptr: `loc` / `attw` are the sampling locations and attention weights)
+// or fused (`loc` / `attw` are the raw sampling offsets and attention logits, and the gradients are taken with
+// respect to them).  Where no 32-channel kernel covers the problem (shape, or a view that is not aligned) the plain
+// op takes the generic kernel and the fused one returns MSDA_ERR_UNSUPPORTED.  "bwd_variant":
+//   0 (default): where the queries are the value pixels (encoder self-attention) the in-SM merging kernel (points
+//       near their query) and the per-row reduction kernel (points anywhere) are both launched; every CTA of both
+//       runs the same probe of the sampling locations first and the kernel the verdict goes against returns at
+//       once (msda_common.cuh);
+//   20..39: merging kernel forced (plain: and its tuning variants); 1..8: CTA shapes of the plain per-row kernel;
+//   63: generic kernel (plain only, tests)
+static int backward_f32(const float *grad_output, const float *value, const int64_t *shapes, const int64_t *lstart,
+                        const float *loc, const float *attw, const Producers &pr, const Dims &d, float *gv,
+                        float *gl, float *gw, cudaStream_t st) {
+    if (!grad_output || !value || !shapes || !lstart || !loc || !attw || !gv || !gl || !gw)
         return MSDA_ERR_NULL_POINTER;
-    if (int rc = check_dims(d)) return rc;
+    if (int rc = check_dims(d, pr.ref_bstride)) return rc;
+    const bool fused = pr.ref != nullptr;
+    const int variant = option_value(OPT_BWD_VARIANT);
+    const bool aligned = aligned16(value) && aligned16(grad_output) && aligned16(gv) && aligned8(loc) &&
+                         aligned8(gl) && aligned8(pr.ref);
+    bool handled = false;
+    cudaError_t e = cudaSuccess;
+    if (aligned && (fused || variant != 63)) {
+        int gate = GATE_NONE;
+        if ((variant == 0 || (variant >= 20 && variant < 40)) && bwd_sorted_applies(value, gv, d)) {
+            e = launch_bwd_sorted(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw,
+                                  variant == 0 ? GATE_RUN_IF_LOCAL : GATE_NONE, st, &handled);
+            if (variant == 0) {                  // the per-row kernel follows, gated the other way
+                handled = false;
+                gate = GATE_RUN_IF_SPREAD;
+            }
+        }
+        if (e == cudaSuccess && !handled)
+            e = launch_bwd_d32(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, nullptr, gate, st,
+                               &handled);
+    }
+    if (e != cudaSuccess || handled || fused) return launch_rc(e, handled);
+    return (int)launch_bwd_generic<float>(grad_output, value, shapes, lstart, loc, attw, d, gv, gl, gw, st);
+}
+
+// Deterministic backward (msda_det.cu), plain or fused as in backward_f32 (fp64: plain only): the records kernel
+// of the path, then sort, bounds and gather into grad_value.
+template <typename T>
+static int backward_deterministic(const T *grad_output, const T *value, const int64_t *shapes, const int64_t *lstart,
+                                  const T *loc, const T *attw, const Producers &pr, const Dims &d, T *gv, T *gl,
+                                  T *gw, void *workspace, cudaStream_t st) {
+    if (!grad_output || !value || !shapes || !lstart || !loc || !attw || !gv || !gl || !gw || !workspace)
+        return MSDA_ERR_NULL_POINTER;
+    if (int rc = check_dims(d, pr.ref_bstride)) return rc;
     DetLayout l;
     if (!det_layout(d, (int)sizeof(T), &l)) return MSDA_ERR_BAD_SHAPE;
     if (!aligned16(workspace)) return MSDA_ERR_UNSUPPORTED;
@@ -139,17 +177,92 @@ static int backward_deterministic(const T *grad_output, const T *value, const in
     bool handled = false;
     cudaError_t e = cudaSuccess;
     if constexpr (sizeof(T) == 4) {
-        const bool fast_ok = aligned16(value) && aligned16(grad_output) && aligned8(sampling_loc) &&
-                             aligned8(grad_sampling_loc);
-        if (option_value(OPT_BWD_VARIANT) != 63 && fast_ok)
-            e = launch_bwd_d32_records(grad_output, value, spatial_shapes, level_start, nullptr, 0, sampling_loc,
-                                       attn_weight, d, grad_sampling_loc, grad_attn_weight, rec, st, &handled);
+        const bool aligned = aligned16(value) && aligned16(grad_output) && aligned8(loc) && aligned8(gl) &&
+                             aligned8(pr.ref);
+        if (aligned && (pr.ref != nullptr || option_value(OPT_BWD_VARIANT) != 63))
+            e = launch_bwd_d32(grad_output, value, shapes, lstart, loc, attw, pr, d, nullptr, gl, gw, &rec,
+                               GATE_NONE, st, &handled);
     }
-    if (e == cudaSuccess && !handled)
-        e = launch_bwd_generic_records<T>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
-                                          d, grad_sampling_loc, grad_attn_weight, rec, st);
-    if (e == cudaSuccess) e = launch_det_reduce<T>(l, workspace, grad_output, grad_value, d, st);
+    if (e == cudaSuccess && !handled) {
+        if (pr.ref != nullptr) return MSDA_ERR_UNSUPPORTED;
+        e = launch_bwd_generic_records<T>(grad_output, value, shapes, lstart, loc, attw, d, gl, gw, rec, st);
+    }
+    if (e == cudaSuccess) e = launch_det_reduce<T>(l, workspace, grad_output, gv, d, st);
     return (int)e;
+}
+
+// the bodies of the entries that come in a default and a deterministic (or training) form: `deterministic` /
+// `train` select the form's null-pointer rule, the workspace / mean_rstd pointer selects the launch
+static int linear(const float *x, const float *weight, const float *bias, float *y, int rows, int out_f, int in_f,
+                  int relu, float *workspace, void *stream, bool deterministic) {
+    if (!x || !weight || !y) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || out_f <= 0 || in_f <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_linear_tf32x3(x, weight, bias, y, rows, out_f, in_f, relu, workspace,
+                                               (cudaStream_t)stream, &handled, deterministic);
+    return launch_rc(e, handled);
+}
+
+static int linear_presplit(const float *x, const float *split_weight, const float *bias, float *y, int rows,
+                           int out_f, int in_f, int relu, void *stream, bool deterministic) {
+    if (!x || !split_weight || !y) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || out_f <= 0 || in_f <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    // the kernel only reads the split weight
+    const cudaError_t e = launch_linear_tf32x3(x, nullptr, bias, y, rows, out_f, in_f, relu,
+                                               const_cast<float *>(split_weight), (cudaStream_t)stream, &handled,
+                                               deterministic);
+    return launch_rc(e, handled);
+}
+
+static int add_layernorm_backward(const float *grad_y, const float *x, const float *residual, const float *gamma,
+                                  float *grad_v, float *grad_gamma, float *grad_beta, long long rows, int cols,
+                                  float eps, void *workspace, void *stream, bool deterministic) {
+    if (!grad_y || !x || !gamma || !grad_v || !grad_gamma || !grad_beta || (deterministic && !workspace))
+        return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || cols <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_add_layernorm_bwd(grad_y, x, residual, gamma, grad_v, grad_gamma, grad_beta, rows,
+                                                   cols, eps, (cudaStream_t)stream, &handled,
+                                                   static_cast<float *>(workspace));
+    return launch_rc(e, handled);
+}
+
+static int linear_wgrad(const float *grad_y, const float *x, float *grad_weight, float *grad_bias, long long rows,
+                        int out_f, int in_f, void *workspace, void *stream, bool deterministic) {
+    if (!grad_y || !x || !grad_weight || (deterministic && !workspace)) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || out_f <= 0 || in_f <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_linear_wgrad(grad_y, x, grad_weight, grad_bias, rows, out_f, in_f,
+                                              (cudaStream_t)stream, &handled, static_cast<float *>(workspace));
+    return launch_rc(e, handled);
+}
+
+static int group_norm_nchw(const float *x, const float *channel_bias, const float *gamma, const float *beta, float *y,
+                           float *mean_rstd, int batch, int channels, int height, int width, int groups, float eps,
+                           int relu, const float *up, int up_h, int up_w, void *workspace, void *stream, bool train) {
+    if (!x || !gamma || !beta || !y || (train && !mean_rstd) || !workspace) return MSDA_ERR_NULL_POINTER;
+    if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_group_norm(x, channel_bias, gamma, beta, y, batch, channels, height, width, groups,
+                                            eps, relu, up, up_h, up_w, static_cast<double *>(workspace), mean_rstd,
+                                            (cudaStream_t)stream, &handled);
+    return launch_rc(e, handled);
+}
+
+static int group_norm_nchw_to_rows(const float *x, const float *channel_bias, const float *gamma, const float *beta,
+                                   float *y_rows, float *mean_rstd, long long row_stride, long long image_stride,
+                                   int batch, int channels, long long plane, int groups, float eps, int relu,
+                                   void *workspace, void *stream, bool train) {
+    if (!x || !gamma || !beta || !y_rows || (train && !mean_rstd) || !workspace) return MSDA_ERR_NULL_POINTER;
+    if (batch <= 0 || channels <= 0 || plane <= 0 || groups <= 0 || row_stride < channels || image_stride < 0)
+        return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_group_norm_rows(x, channel_bias, gamma, beta, y_rows, batch, channels, plane, groups,
+                                                 eps, relu, row_stride, image_stride,
+                                                 static_cast<double *>(workspace), mean_rstd, (cudaStream_t)stream,
+                                                 &handled);
+    return launch_rc(e, handled);
 }
 
 }  // namespace msda
@@ -203,7 +316,7 @@ int msda_b200_forward_f32(const float *value, const int64_t *spatial_shapes,
     cudaError_t e = cudaSuccess;
     const bool fast_ok = aligned16(value) && aligned16(output) && aligned8(sampling_loc);
     if (option_value(OPT_FWD_VARIANT) != 63 && fast_ok)   // 63 forces the generic kernel (tests)
-        e = launch_fwd_d32(value, spatial_shapes, level_start, sampling_loc, attn_weight, d, output, st,
+        e = launch_fwd_d32(value, spatial_shapes, level_start, sampling_loc, attn_weight, Producers{}, d, output, st,
                            &handled);
     if (e == cudaSuccess && !handled)
         e = launch_fwd_generic<float>(value, spatial_shapes, level_start, sampling_loc, attn_weight, d,
@@ -230,41 +343,9 @@ int msda_b200_backward_f32(const float *grad_output, const float *value,
                            int spatial_size, int num_heads, int channels, int num_levels,
                            int num_query, int num_point, float *grad_value,
                            float *grad_sampling_loc, float *grad_attn_weight, void *stream) {
-    if (!grad_output || !value || !spatial_shapes || !level_start || !sampling_loc || !attn_weight ||
-        !grad_value || !grad_sampling_loc || !grad_attn_weight)
-        return MSDA_ERR_NULL_POINTER;
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    if (int rc = check_dims(d)) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    bool handled = false;
-    cudaError_t e = cudaSuccess;
-    const int variant = option_value(OPT_BWD_VARIANT);
-    const bool fast_ok = aligned16(value) && aligned16(grad_output) && aligned16(grad_value) &&
-                         aligned8(sampling_loc) && aligned8(grad_sampling_loc);
-    // 0 (default): where the queries are the value pixels (encoder self-attention) the in-SM merging
-    //     kernel (points near their query) and the per-row reduction kernel (points anywhere) are both
-    //     launched; every CTA of both runs the same probe of the sampling locations first and the
-    //     kernel the verdict goes against returns at once (msda_common.cuh);
-    // 20..39: merging kernel forced (and its tuning variants); 1..8: CTA shapes of the per-row
-    //     reduction kernel; 63: generic kernel (tests)
-    int gate = GATE_NONE;
-    if (variant == 0 && fast_ok && bwd_sorted_applies(value, grad_value, d)) {
-        e = launch_bwd_sorted(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
-                              d, grad_value, grad_sampling_loc, grad_attn_weight, st, &handled, GATE_RUN_IF_LOCAL);
-        handled = false;                     // the per-row kernel follows, gated the other way
-        gate = GATE_RUN_IF_SPREAD;
-    } else if (variant >= 20 && variant < 40 && fast_ok) {
-        e = launch_bwd_sorted(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
-                              d, grad_value, grad_sampling_loc, grad_attn_weight, st, &handled, GATE_NONE);
-    }
-    if (e == cudaSuccess && !handled && variant != 63 && fast_ok)
-        e = launch_bwd_d32(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
-                           d, grad_value, grad_sampling_loc, grad_attn_weight, st, &handled, gate);
-    if (e == cudaSuccess && !handled)
-        e = launch_bwd_generic<float>(grad_output, value, spatial_shapes, level_start, sampling_loc,
-                                      attn_weight, d, grad_value, grad_sampling_loc,
-                                      grad_attn_weight, st);
-    return (int)e;
+    return backward_f32(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight, Producers{}, d,
+                        grad_value, grad_sampling_loc, grad_attn_weight, (cudaStream_t)stream);
 }
 
 int msda_b200_backward_f64(const double *grad_output, const double *value,
@@ -295,9 +376,7 @@ int msda_b200_fused_forward_strided_f32(const float *value, const int64_t *spati
         !attn_logits || !output)
         return MSDA_ERR_NULL_POINTER;
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    if (int rc = check_dims(d)) return rc;
-    if (ref_batch_stride != 0 && ref_batch_stride != (long long)num_query * num_levels * 2)
-        return MSDA_ERR_BAD_SHAPE;
+    if (int rc = check_dims(d, ref_batch_stride)) return rc;
     const long long packed = (long long)num_heads * num_levels * num_point;
     if (offsets_row_stride < 2 * packed || logits_row_stride < packed || (offsets_row_stride & 1))
         return MSDA_ERR_BAD_SHAPE;
@@ -305,13 +384,14 @@ int msda_b200_fused_forward_strided_f32(const float *value, const int64_t *spati
     if (!aligned16(value) || !aligned16(output) || !aligned8(sampling_offsets) || !aligned8(reference_points) ||
         !aligned8(offsets_table))
         return MSDA_ERR_UNSUPPORTED;
+    // the kernel reads packed rows (row strides 2*M*L*P and M*L*P) as stride 0
+    const bool rows_packed = offsets_row_stride == 2 * packed && logits_row_stride == packed;
+    const Producers pr{reference_points, ref_batch_stride, rows_packed ? 0 : offsets_row_stride,
+                       rows_packed ? 0 : logits_row_stride, offsets_table, logits_table};
     bool handled = false;
-    cudaError_t e = launch_fwd_d32_fused(value, spatial_shapes, level_start, reference_points,
-                                         ref_batch_stride, sampling_offsets, attn_logits, d, output,
-                                         (cudaStream_t)stream, &handled, offsets_row_stride, logits_row_stride,
-                                         offsets_table, logits_table);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    const cudaError_t e = launch_fwd_d32(value, spatial_shapes, level_start, sampling_offsets, attn_logits, pr, d,
+                                         output, (cudaStream_t)stream, &handled);
+    return launch_rc(e, handled);
 }
 
 int msda_b200_fused_forward_f32(const float *value, const int64_t *spatial_shapes,
@@ -335,36 +415,11 @@ int msda_b200_fused_backward_f32(const float *grad_output, const float *value,
                                  int spatial_size, int num_heads, int channels, int num_levels,
                                  int num_query, int num_point, float *grad_value,
                                  float *grad_sampling_offsets, float *grad_attn_logits, void *stream) {
-    if (!grad_output || !value || !spatial_shapes || !level_start || !reference_points ||
-        !sampling_offsets || !attn_logits || !grad_value || !grad_sampling_offsets || !grad_attn_logits)
-        return MSDA_ERR_NULL_POINTER;
+    if (!reference_points) return MSDA_ERR_NULL_POINTER;      // (it selects the fused form)
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    if (int rc = check_dims(d)) return rc;
-    if (ref_batch_stride != 0 && ref_batch_stride != (long long)num_query * num_levels * 2)
-        return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = cudaSuccess;
-    const int variant = option_value(OPT_BWD_VARIANT);
-    const bool aligned = aligned16(value) && aligned16(grad_output) && aligned16(grad_value) &&
-                         aligned8(sampling_offsets) && aligned8(grad_sampling_offsets) && aligned8(reference_points);
-    if (!aligned) return MSDA_ERR_UNSUPPORTED;
-    // as in msda_b200_backward_f32: merging kernel and per-row kernel behind the same location probe
-    // (here on the raw offsets), or one of them forced by "bwd_variant" (20..39 / 1..8)
-    int gate = GATE_NONE;
-    if ((variant == 0 || (variant >= 20 && variant < 40)) && bwd_sorted_applies(value, grad_value, d)) {
-        e = launch_bwd_sorted_fused(grad_output, value, spatial_shapes, level_start, reference_points,
-                                    ref_batch_stride, sampling_offsets, attn_logits, d, grad_value,
-                                    grad_sampling_offsets, grad_attn_logits, (cudaStream_t)stream, &handled,
-                                    variant == 0 ? GATE_RUN_IF_LOCAL : GATE_NONE);
-        if (variant == 0 && handled) { handled = false; gate = GATE_RUN_IF_SPREAD; }
-    }
-    if (e == cudaSuccess && !handled)
-        e = launch_bwd_d32_fused(grad_output, value, spatial_shapes, level_start,
-                                 reference_points, ref_batch_stride, sampling_offsets,
-                                 attn_logits, d, grad_value, grad_sampling_offsets,
-                                 grad_attn_logits, (cudaStream_t)stream, &handled, gate);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return backward_f32(grad_output, value, spatial_shapes, level_start, sampling_offsets, attn_logits,
+                        Producers{reference_points, ref_batch_stride}, d, grad_value, grad_sampling_offsets,
+                        grad_attn_logits, (cudaStream_t)stream);
 }
 
 long long msda_b200_backward_deterministic_workspace_bytes(int batch, int spatial_size, int num_heads, int channels,
@@ -384,8 +439,8 @@ int msda_b200_backward_deterministic_f32(const float *grad_output, const float *
                                          float *grad_sampling_loc, float *grad_attn_weight, void *workspace,
                                          void *stream) {
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    return backward_deterministic<float>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight, d,
-                                         grad_value, grad_sampling_loc, grad_attn_weight, workspace,
+    return backward_deterministic<float>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
+                                         Producers{}, d, grad_value, grad_sampling_loc, grad_attn_weight, workspace,
                                          (cudaStream_t)stream);
 }
 
@@ -398,7 +453,7 @@ int msda_b200_backward_deterministic_f64(const double *grad_output, const double
                                          void *stream) {
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
     return backward_deterministic<double>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
-                                          d, grad_value, grad_sampling_loc, grad_attn_weight, workspace,
+                                          Producers{}, d, grad_value, grad_sampling_loc, grad_attn_weight, workspace,
                                           (cudaStream_t)stream);
 }
 
@@ -410,48 +465,21 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
                                                int num_query, int num_point, float *grad_value,
                                                float *grad_sampling_offsets, float *grad_attn_logits,
                                                void *workspace, void *stream) {
-    if (!grad_output || !value || !spatial_shapes || !level_start || !reference_points ||
-        !sampling_offsets || !attn_logits || !grad_value || !grad_sampling_offsets || !grad_attn_logits || !workspace)
-        return MSDA_ERR_NULL_POINTER;
+    if (!reference_points) return MSDA_ERR_NULL_POINTER;      // (it selects the fused form)
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    if (int rc = check_dims(d)) return rc;
-    if (ref_batch_stride != 0 && ref_batch_stride != (long long)num_query * num_levels * 2)
-        return MSDA_ERR_BAD_SHAPE;
-    DetLayout l;
-    if (!det_layout(d, 4, &l)) return MSDA_ERR_BAD_SHAPE;
-    const bool aligned = aligned16(value) && aligned16(grad_output) && aligned16(workspace) &&
-                         aligned8(sampling_offsets) && aligned8(grad_sampling_offsets) && aligned8(reference_points);
-    if (!aligned) return MSDA_ERR_UNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
-    bool handled = false;
-    cudaError_t e = launch_bwd_d32_records(grad_output, value, spatial_shapes, level_start, reference_points,
-                                           ref_batch_stride, sampling_offsets, attn_logits, d, grad_sampling_offsets,
-                                           grad_attn_logits, det_records(workspace, l), st, &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    if (e == cudaSuccess) e = launch_det_reduce<float>(l, workspace, grad_output, grad_value, d, st);
-    return (int)e;
+    return backward_deterministic<float>(grad_output, value, spatial_shapes, level_start, sampling_offsets,
+                                         attn_logits, Producers{reference_points, ref_batch_stride}, d, grad_value,
+                                         grad_sampling_offsets, grad_attn_logits, workspace, (cudaStream_t)stream);
 }
 
 int msda_b200_linear_f32(const float *x, const float *weight, const float *bias, float *y, int rows,
                          int out_features, int in_features, int relu, float *workspace, void *stream) {
-    if (!x || !weight || !y) return MSDA_ERR_NULL_POINTER;
-    if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_linear_tf32x3(x, weight, bias, y, rows, out_features, in_features, relu,
-                                         workspace, (cudaStream_t)stream, &handled, false);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return linear(x, weight, bias, y, rows, out_features, in_features, relu, workspace, stream, false);
 }
 
 int msda_b200_linear_deterministic_f32(const float *x, const float *weight, const float *bias, float *y, int rows,
                                        int out_features, int in_features, int relu, float *workspace, void *stream) {
-    if (!x || !weight || !y) return MSDA_ERR_NULL_POINTER;
-    if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_linear_tf32x3(x, weight, bias, y, rows, out_features, in_features, relu,
-                                         workspace, (cudaStream_t)stream, &handled, true);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return linear(x, weight, bias, y, rows, out_features, in_features, relu, workspace, stream, true);
 }
 
 int msda_b200_split_weight_f32(const float *weight, float *split_weight, int out_features, int in_features,
@@ -459,32 +487,19 @@ int msda_b200_split_weight_f32(const float *weight, float *split_weight, int out
     if (!weight || !split_weight) return MSDA_ERR_NULL_POINTER;
     if (out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
-    cudaError_t e = launch_split_weight(weight, split_weight, out_features, in_features, (cudaStream_t)stream, &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    const cudaError_t e = launch_split_weight(weight, split_weight, out_features, in_features, (cudaStream_t)stream,
+                                              &handled);
+    return launch_rc(e, handled);
 }
 
 int msda_b200_linear_presplit_f32(const float *x, const float *split_weight, const float *bias, float *y, int rows,
                                   int out_features, int in_features, int relu, void *stream) {
-    if (!x || !split_weight || !y) return MSDA_ERR_NULL_POINTER;
-    if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    // the kernel only reads the split weight
-    cudaError_t e = launch_linear_tf32x3(x, nullptr, bias, y, rows, out_features, in_features, relu,
-                                         const_cast<float *>(split_weight), (cudaStream_t)stream, &handled, false);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return linear_presplit(x, split_weight, bias, y, rows, out_features, in_features, relu, stream, false);
 }
 
 int msda_b200_linear_presplit_deterministic_f32(const float *x, const float *split_weight, const float *bias, float *y,
                                                 int rows, int out_features, int in_features, int relu, void *stream) {
-    if (!x || !split_weight || !y) return MSDA_ERR_NULL_POINTER;
-    if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_linear_tf32x3(x, nullptr, bias, y, rows, out_features, in_features, relu,
-                                         const_cast<float *>(split_weight), (cudaStream_t)stream, &handled, true);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return linear_presplit(x, split_weight, bias, y, rows, out_features, in_features, relu, stream, true);
 }
 
 int msda_b200_add_layernorm_f32(const float *x, const float *residual, const float *gamma, const float *beta,
@@ -492,34 +507,24 @@ int msda_b200_add_layernorm_f32(const float *x, const float *residual, const flo
     if (!x || !gamma || !beta || !y) return MSDA_ERR_NULL_POINTER;
     if (rows <= 0 || cols <= 0) return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
-    cudaError_t e = launch_add_layernorm(x, residual, gamma, beta, y, rows, cols, eps, (cudaStream_t)stream, &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    const cudaError_t e = launch_add_layernorm(x, residual, gamma, beta, y, rows, cols, eps, (cudaStream_t)stream,
+                                               &handled);
+    return launch_rc(e, handled);
 }
 
 int msda_b200_add_layernorm_backward_f32(const float *grad_y, const float *x, const float *residual,
                                          const float *gamma, float *grad_v, float *grad_gamma, float *grad_beta,
                                          long long rows, int cols, float eps, void *stream) {
-    if (!grad_y || !x || !gamma || !grad_v || !grad_gamma || !grad_beta) return MSDA_ERR_NULL_POINTER;
-    if (rows <= 0 || cols <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_add_layernorm_bwd(grad_y, x, residual, gamma, grad_v, grad_gamma, grad_beta, rows, cols,
-                                             eps, (cudaStream_t)stream, &handled, nullptr);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return add_layernorm_backward(grad_y, x, residual, gamma, grad_v, grad_gamma, grad_beta, rows, cols, eps, nullptr,
+                                  stream, false);
 }
 
 int msda_b200_add_layernorm_backward_deterministic_f32(const float *grad_y, const float *x, const float *residual,
                                                        const float *gamma, float *grad_v, float *grad_gamma,
                                                        float *grad_beta, long long rows, int cols, float eps,
                                                        void *workspace, void *stream) {
-    if (!grad_y || !x || !gamma || !grad_v || !grad_gamma || !grad_beta || !workspace) return MSDA_ERR_NULL_POINTER;
-    if (rows <= 0 || cols <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_add_layernorm_bwd(grad_y, x, residual, gamma, grad_v, grad_gamma, grad_beta, rows, cols,
-                                             eps, (cudaStream_t)stream, &handled, static_cast<float *>(workspace));
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return add_layernorm_backward(grad_y, x, residual, gamma, grad_v, grad_gamma, grad_beta, rows, cols, eps,
+                                  workspace, stream, true);
 }
 
 long long msda_b200_add_layernorm_backward_deterministic_workspace_bytes(long long rows, int cols) {
@@ -529,25 +534,13 @@ long long msda_b200_add_layernorm_backward_deterministic_workspace_bytes(long lo
 
 int msda_b200_linear_wgrad_f32(const float *grad_y, const float *x, float *grad_weight, float *grad_bias,
                                long long rows, int out_features, int in_features, void *stream) {
-    if (!grad_y || !x || !grad_weight) return MSDA_ERR_NULL_POINTER;
-    if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_linear_wgrad(grad_y, x, grad_weight, grad_bias, rows, out_features, in_features,
-                                        (cudaStream_t)stream, &handled, nullptr);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return linear_wgrad(grad_y, x, grad_weight, grad_bias, rows, out_features, in_features, nullptr, stream, false);
 }
 
 int msda_b200_linear_wgrad_deterministic_f32(const float *grad_y, const float *x, float *grad_weight, float *grad_bias,
                                              long long rows, int out_features, int in_features, void *workspace,
                                              void *stream) {
-    if (!grad_y || !x || !grad_weight || !workspace) return MSDA_ERR_NULL_POINTER;
-    if (rows <= 0 || out_features <= 0 || in_features <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_linear_wgrad(grad_y, x, grad_weight, grad_bias, rows, out_features, in_features,
-                                        (cudaStream_t)stream, &handled, static_cast<float *>(workspace));
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return linear_wgrad(grad_y, x, grad_weight, grad_bias, rows, out_features, in_features, workspace, stream, true);
 }
 
 long long msda_b200_linear_wgrad_deterministic_workspace_bytes(long long rows, int out_features, int in_features) {
@@ -558,43 +551,24 @@ long long msda_b200_linear_wgrad_deterministic_workspace_bytes(long long rows, i
 int msda_b200_group_norm_nchw_f32(const float *x, const float *channel_bias, const float *gamma, const float *beta,
                                   float *y, int batch, int channels, int height, int width, int groups, float eps,
                                   int relu, const float *up, int up_h, int up_w, void *workspace, void *stream) {
-    if (!x || !gamma || !beta || !y || !workspace) return MSDA_ERR_NULL_POINTER;
-    if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_group_norm(x, channel_bias, gamma, beta, y, batch, channels, height, width, groups, eps,
-                                      relu, up, up_h, up_w, static_cast<double *>(workspace), nullptr,
-                                      (cudaStream_t)stream, &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return group_norm_nchw(x, channel_bias, gamma, beta, y, nullptr, batch, channels, height, width, groups, eps, relu,
+                           up, up_h, up_w, workspace, stream, false);
 }
 
 int msda_b200_group_norm_nchw_to_rows_f32(const float *x, const float *channel_bias, const float *gamma,
                                           const float *beta, float *y_rows, long long row_stride,
                                           long long image_stride, int batch, int channels, long long plane,
                                           int groups, float eps, int relu, void *workspace, void *stream) {
-    if (!x || !gamma || !beta || !y_rows || !workspace) return MSDA_ERR_NULL_POINTER;
-    if (batch <= 0 || channels <= 0 || plane <= 0 || groups <= 0 || row_stride < channels || image_stride < 0)
-        return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_group_norm_rows(x, channel_bias, gamma, beta, y_rows, batch, channels, plane, groups, eps,
-                                           relu, row_stride, image_stride, static_cast<double *>(workspace), nullptr,
-                                           (cudaStream_t)stream, &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return group_norm_nchw_to_rows(x, channel_bias, gamma, beta, y_rows, nullptr, row_stride, image_stride, batch,
+                                   channels, plane, groups, eps, relu, workspace, stream, false);
 }
 
 int msda_b200_group_norm_nchw_train_f32(const float *x, const float *channel_bias, const float *gamma,
                                         const float *beta, float *y, float *mean_rstd, int batch, int channels,
                                         int height, int width, int groups, float eps, int relu, const float *up,
                                         int up_h, int up_w, void *workspace, void *stream) {
-    if (!x || !gamma || !beta || !y || !mean_rstd || !workspace) return MSDA_ERR_NULL_POINTER;
-    if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_group_norm(x, channel_bias, gamma, beta, y, batch, channels, height, width, groups, eps,
-                                      relu, up, up_h, up_w, static_cast<double *>(workspace), mean_rstd,
-                                      (cudaStream_t)stream, &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return group_norm_nchw(x, channel_bias, gamma, beta, y, mean_rstd, batch, channels, height, width, groups, eps,
+                           relu, up, up_h, up_w, workspace, stream, true);
 }
 
 int msda_b200_group_norm_nchw_to_rows_train_f32(const float *x, const float *channel_bias, const float *gamma,
@@ -602,15 +576,8 @@ int msda_b200_group_norm_nchw_to_rows_train_f32(const float *x, const float *cha
                                                 long long row_stride, long long image_stride, int batch,
                                                 int channels, long long plane, int groups, float eps, int relu,
                                                 void *workspace, void *stream) {
-    if (!x || !gamma || !beta || !y_rows || !mean_rstd || !workspace) return MSDA_ERR_NULL_POINTER;
-    if (batch <= 0 || channels <= 0 || plane <= 0 || groups <= 0 || row_stride < channels || image_stride < 0)
-        return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    cudaError_t e = launch_group_norm_rows(x, channel_bias, gamma, beta, y_rows, batch, channels, plane, groups, eps,
-                                           relu, row_stride, image_stride, static_cast<double *>(workspace),
-                                           mean_rstd, (cudaStream_t)stream, &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    return group_norm_nchw_to_rows(x, channel_bias, gamma, beta, y_rows, mean_rstd, row_stride, image_stride, batch,
+                                   channels, plane, groups, eps, relu, workspace, stream, true);
 }
 
 int msda_b200_group_norm_backward_nchw_f32(const float *grad_y, const float *x, const float *channel_bias,
@@ -623,12 +590,11 @@ int msda_b200_group_norm_backward_nchw_f32(const float *grad_y, const float *x, 
         return MSDA_ERR_NULL_POINTER;
     if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
-    cudaError_t e = launch_group_norm_bwd(grad_y, x, channel_bias, gamma, beta, mean_rstd, grad_x, grad_gamma,
-                                          grad_beta, grad_channel_bias, grad_up, batch, channels, height, width, groups,
-                                          relu, up_h, up_w, static_cast<double *>(workspace), (cudaStream_t)stream,
-                                          &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    const cudaError_t e = launch_group_norm_bwd(grad_y, x, channel_bias, gamma, beta, mean_rstd, grad_x, grad_gamma,
+                                                grad_beta, grad_channel_bias, grad_up, batch, channels, height, width,
+                                                groups, relu, up_h, up_w, static_cast<double *>(workspace),
+                                                (cudaStream_t)stream, &handled);
+    return launch_rc(e, handled);
 }
 
 int msda_b200_group_norm_rows_backward_f32(const float *grad_y_rows, long long row_stride, long long image_stride,
@@ -642,12 +608,11 @@ int msda_b200_group_norm_rows_backward_f32(const float *grad_y_rows, long long r
     if (batch <= 0 || channels <= 0 || plane <= 0 || groups <= 0 || row_stride < channels || image_stride < 0)
         return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
-    cudaError_t e = launch_group_norm_rows_bwd(grad_y_rows, row_stride, image_stride, x, channel_bias, gamma, beta,
-                                               mean_rstd, grad_x, grad_gamma, grad_beta, grad_channel_bias, batch,
-                                               channels, plane, groups, relu, static_cast<double *>(workspace),
-                                               (cudaStream_t)stream, &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    const cudaError_t e = launch_group_norm_rows_bwd(grad_y_rows, row_stride, image_stride, x, channel_bias, gamma,
+                                                     beta, mean_rstd, grad_x, grad_gamma, grad_beta, grad_channel_bias,
+                                                     batch, channels, plane, groups, relu,
+                                                     static_cast<double *>(workspace), (cudaStream_t)stream, &handled);
+    return launch_rc(e, handled);
 }
 
 int msda_b200_add_channel_bias_nchw_f32(float *x, const float *bias, int batch, int channels, long long plane,
@@ -655,9 +620,8 @@ int msda_b200_add_channel_bias_nchw_f32(float *x, const float *bias, int batch, 
     if (!x || !bias) return MSDA_ERR_NULL_POINTER;
     if (batch <= 0 || channels <= 0 || plane <= 0) return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
-    cudaError_t e = launch_channel_bias(x, bias, batch, channels, plane, (cudaStream_t)stream, &handled);
-    if (e == cudaSuccess && !handled) return MSDA_ERR_UNSUPPORTED;
-    return (int)e;
+    const cudaError_t e = launch_channel_bias(x, bias, batch, channels, plane, (cudaStream_t)stream, &handled);
+    return launch_rc(e, handled);
 }
 
 long long msda_b200_group_norm_workspace_bytes(int batch, int groups) {

@@ -258,140 +258,69 @@ msda_bwd_d32_kernel(const float *__restrict__ grad_out, const float *__restrict_
 }
 
 // ---------------------------------------------------------------------------
-// host side
+// host side: launch_bwd_d32() serves the plain op, the fused producers (Producers::ref set) and
+// the deterministic records (msda_det.cu), the last two in the default CTA shape only
 // ---------------------------------------------------------------------------
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED = false, bool RECORDS = false>
+template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED, bool RECORDS>
 static cudaError_t launch_bwd_cfg(const float *grad_out, const float *value, const int64_t *shapes,
-                                  const int64_t *lstart, const float *loc, const float *attw,
-                                  const Dims &d, float *grad_value, float *grad_loc,
-                                  float *grad_attw, cudaStream_t stream,
-                                  Producers pr = Producers{nullptr, 0, 0, 0, nullptr, nullptr}, int gate = GATE_NONE,
-                                  DetRecords det = DetRecords{nullptr, nullptr, nullptr, 0}) {
+                                  const int64_t *lstart, const float *loc, const float *attw, const Producers &pr,
+                                  const Dims &d, float *grad_value, float *grad_loc, float *grad_attw,
+                                  const DetRecords &det, int gate, cudaStream_t stream) {
     using Cfg = BwdCfg<LP, WARPS, TILE_W, QPW>;
-    auto kern = msda_bwd_d32_kernel<LP, WARPS, TILE_W, MIN_CTAS, BATCH, QPW, FUSED, RECORDS>;
-    // the opt-in shared-memory size is a per-device function attribute: set it (and query the
-    // occupancy) once per device; the values are immutable afterwards
-    static std::atomic<int> ctas_per_sm_of[kMaxDevices];
-    cudaError_t e = cudaSuccess;
-    const int dev = device_slot(&e);
-    if (dev < 0) return e;
-    int ctas_per_sm = ctas_per_sm_of[dev].load(std::memory_order_acquire);
-    if (ctas_per_sm == 0) {
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmem);
-        if (e != cudaSuccess) return e;
-        int nb = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, WARPS * 32, Cfg::kSmem);
-        if (e != cudaSuccess) return e;
-        ctas_per_sm = nb > 0 ? nb : 1;
-        ctas_per_sm_of[dev].store(ctas_per_sm, std::memory_order_release);
-    }
-    int per_sm = ctas_per_sm;
-    const int cap = option_value(OPT_CTAS_PER_SM);
-    if (cap > 0 && cap < per_sm) per_sm = cap;
-    long long blocks = (long long)sm_count() * per_sm;
-    const long long items_ub = (long long)d.N * d.M * d.Lq;
-    if (blocks > items_ub) blocks = items_ub;
-    if (blocks < 1) blocks = 1;
+    constexpr auto kern = msda_bwd_d32_kernel<LP, WARPS, TILE_W, MIN_CTAS, BATCH, QPW, FUSED, RECORDS>;
+    cudaError_t e;
+    const int blocks = persistent_blocks<kern>(WARPS * 32, Cfg::kSmem, d, &e);
+    if (blocks == 0) return e;
     const int flags = (option_value(OPT_TILE_ORDER) != 1 ? 1 : 0) | (whatif_value(OPT_WHATIF_DROP_REDS) << 1);
-    kern<<<(unsigned)blocks, WARPS * 32, Cfg::kSmem, stream>>>(grad_out, value, shapes, lstart, loc,
-                                                              attw, pr, d, flags, grad_value,
-                                                              grad_loc, grad_attw, gate, det);
+    kern<<<blocks, WARPS * 32, Cfg::kSmem, stream>>>(grad_out, value, shapes, lstart, loc, attw, pr, d, flags,
+                                                     grad_value, grad_loc, grad_attw, gate, det);
     note_launch();
     return cudaGetLastError();
 }
 
 template <int LP>
 static cudaError_t launch_bwd_lp(const float *grad_out, const float *value, const int64_t *shapes,
-                                 const int64_t *lstart, const float *loc, const float *attw,
-                                 const Dims &d, float *gv, float *gl, float *gw, cudaStream_t st,
-                                 int gate) {
+                                 const int64_t *lstart, const float *loc, const float *attw, const Producers &pr,
+                                 const Dims &d, float *gv, float *gl, float *gw, const DetRecords *det, int gate,
+                                 cudaStream_t st) {
     // variant = (warps, query tile width, min CTAs per SM -> register budget, load batch in pairs,
     //            queries per warp)
-#define MSDA_BWD(W, TW, C, B, Q) \
-    launch_bwd_cfg<LP, W, TW, C, B, Q>(grad_out, value, shapes, lstart, loc, attw, d, gv, gl, gw, st, \
-                                       Producers{nullptr, 0, 0, 0, nullptr, nullptr}, gate)
+#define MSDA_BWD(W, TW, C, B, Q, F, R) \
+    launch_bwd_cfg<LP, W, TW, C, B, Q, F, R>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, \
+                                             R ? *det : DetRecords{}, gate, st)
+    // fused producers and the deterministic records: the default shape only
+    if (det != nullptr)
+        return pr.ref != nullptr ? MSDA_BWD(16, 16, 2, 1, 8, true, true) : MSDA_BWD(16, 16, 2, 1, 8, false, true);
+    if (pr.ref != nullptr) return MSDA_BWD(16, 16, 2, 1, 8, true, false);
     switch (option_value(OPT_BWD_VARIANT)) {
-        case 1: return MSDA_BWD(8, 8, 4, 1, 8);     //  8 warps, tile  8x8
-        case 3: return MSDA_BWD(32, 16, 1, 1, 8);   // 32 warps, tile 16x16, one CTA per SM
-        case 4: return MSDA_BWD(16, 16, 2, 2, 8);   // 16 warps, 4 loads in flight (spills at 64 regs)
-        case 5: return MSDA_BWD(16, 16, 2, 1, 4);   // 16 warps, tile  4x16, 4 queries per warp (76 KB smem per SM)
-        case 6: return MSDA_BWD(8, 8, 2, 6, 8);     //  8 warps, 114 regs, 12 loads in flight
-        case 7: return MSDA_BWD(16, 8, 2, 1, 4);    // 16 warps, tile  8x8,  4 queries per warp
-        case 8: return MSDA_BWD(32, 16, 1, 1, 4);   // 32 warps, tile  8x16, 4 queries per warp, one CTA per SM
+        case 1: return MSDA_BWD(8, 8, 4, 1, 8, false, false);     //  8 warps, tile  8x8
+        case 3: return MSDA_BWD(32, 16, 1, 1, 8, false, false);   // 32 warps, tile 16x16, one CTA per SM
+        case 4: return MSDA_BWD(16, 16, 2, 2, 8, false, false);   // 16 warps, 4 loads in flight (spills at 64 regs)
+        case 5: return MSDA_BWD(16, 16, 2, 1, 4, false, false);   // 16 warps, tile  4x16, 4 queries per warp (76 KB smem per SM)
+        case 6: return MSDA_BWD(8, 8, 2, 6, 8, false, false);     //  8 warps, 114 regs, 12 loads in flight
+        case 7: return MSDA_BWD(16, 8, 2, 1, 4, false, false);    // 16 warps, tile  8x8,  4 queries per warp
+        case 8: return MSDA_BWD(32, 16, 1, 1, 4, false, false);   // 32 warps, tile  8x16, 4 queries per warp, one CTA per SM
         case 2:
-        default: return MSDA_BWD(16, 16, 2, 1, 8);  // 16 warps, tile  8x16, 8 queries per warp (147 KB smem per SM)
+        default: return MSDA_BWD(16, 16, 2, 1, 8, false, false);  // 16 warps, tile  8x16, 8 queries per warp (147 KB smem per SM)
     }
 #undef MSDA_BWD
 }
 
-cudaError_t launch_bwd_d32(const float *grad_out, const float *value, const int64_t *shapes,
-                           const int64_t *lstart, const float *loc, const float *attw, const Dims &d,
-                           float *gv, float *gl, float *gw, cudaStream_t stream, bool *handled,
-                           int gate) {
-    *handled = true;
-    const int LP = d.L * d.P;
-    if (d.D != 32 || (long long)d.S * d.M * 8 >= 0x7fffffffLL) {
-        *handled = false;
-        return cudaSuccess;
+// pr.ref == nullptr: plain; otherwise fused producers, gradients w.r.t. the raw sampling offsets (`loc`) and
+// attention logits (`attw`).  det != nullptr: deterministic mode (msda_det.cu), grad_value `gv` is not touched and
+// the corner records go to `det`.  `gate`: see msda_bwd_sorted.cu.  `handled` = false: the problem is outside
+// d32_applies() and nothing was launched.
+cudaError_t launch_bwd_d32(const float *grad_out, const float *value, const int64_t *shapes, const int64_t *lstart,
+                           const float *loc, const float *attw, const Producers &pr, const Dims &d, float *gv,
+                           float *gl, float *gw, const DetRecords *det, int gate, cudaStream_t st, bool *handled) {
+    *handled = d32_applies(d);
+    if (!*handled) return cudaSuccess;
+    switch (d.L * d.P) {       // 4, 8, 12 or 16 (d32_applies)
+        case 4: return launch_bwd_lp<4>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        case 8: return launch_bwd_lp<8>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        case 12: return launch_bwd_lp<12>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        default: return launch_bwd_lp<16>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
     }
-    switch (LP) {
-        case 4: return launch_bwd_lp<4>(grad_out, value, shapes, lstart, loc, attw, d, gv, gl, gw, stream, gate);
-        case 8: return launch_bwd_lp<8>(grad_out, value, shapes, lstart, loc, attw, d, gv, gl, gw, stream, gate);
-        case 12: return launch_bwd_lp<12>(grad_out, value, shapes, lstart, loc, attw, d, gv, gl, gw, stream, gate);
-        case 16: return launch_bwd_lp<16>(grad_out, value, shapes, lstart, loc, attw, d, gv, gl, gw, stream, gate);
-        default: *handled = false; return cudaSuccess;
-    }
-}
-
-// Fused producers: gradients w.r.t. the raw sampling offsets and attention logits.
-cudaError_t launch_bwd_d32_fused(const float *grad_out, const float *value, const int64_t *shapes,
-                                 const int64_t *lstart, const float *ref, long long ref_bstride,
-                                 const float *off, const float *logits, const Dims &d, float *gv,
-                                 float *g_off, float *g_logits, cudaStream_t st, bool *handled, int gate) {
-    *handled = true;
-    const Producers pr{ref, ref_bstride};
-    if (d.D != 32 || (long long)d.S * d.M * 8 >= 0x7fffffffLL) {
-        *handled = false;
-        return cudaSuccess;
-    }
-#define MSDA_BWD_FUSED(LPV) \
-    launch_bwd_cfg<LPV, 16, 16, 2, 1, 8, true>(grad_out, value, shapes, lstart, off, logits, d, gv, g_off, g_logits, st, pr, gate)
-    switch (d.L * d.P) {
-        case 4: return MSDA_BWD_FUSED(4);
-        case 8: return MSDA_BWD_FUSED(8);
-        case 12: return MSDA_BWD_FUSED(12);
-        case 16: return MSDA_BWD_FUSED(16);
-        default: *handled = false; return cudaSuccess;
-    }
-#undef MSDA_BWD_FUSED
-}
-
-// Deterministic mode: the records kernel of the default CTA shape (16 warps, 8x16 tiles), plain or fused
-// (ref != nullptr: `loc` / `attw` are the raw offsets / logits).  Same domain as the two launchers above.
-cudaError_t launch_bwd_d32_records(const float *grad_out, const float *value, const int64_t *shapes,
-                                   const int64_t *lstart, const float *ref, long long ref_bstride,
-                                   const float *loc, const float *attw, const Dims &d, float *gl, float *gw,
-                                   const DetRecords &det, cudaStream_t st, bool *handled) {
-    *handled = true;
-    if (d.D != 32 || (long long)d.S * d.M * 8 >= 0x7fffffffLL) {
-        *handled = false;
-        return cudaSuccess;
-    }
-    const Producers none{nullptr, 0, 0, 0, nullptr, nullptr}, fused{ref, ref_bstride};
-#define MSDA_BWD_REC(LPV)                                                                                          \
-    (ref != nullptr                                                                                                \
-         ? launch_bwd_cfg<LPV, 16, 16, 2, 1, 8, true, true>(grad_out, value, shapes, lstart, loc, attw, d, nullptr, \
-                                                            gl, gw, st, fused, GATE_NONE, det)                     \
-         : launch_bwd_cfg<LPV, 16, 16, 2, 1, 8, false, true>(grad_out, value, shapes, lstart, loc, attw, d, nullptr,\
-                                                             gl, gw, st, none, GATE_NONE, det))
-    switch (d.L * d.P) {
-        case 4: return MSDA_BWD_REC(4);
-        case 8: return MSDA_BWD_REC(8);
-        case 12: return MSDA_BWD_REC(12);
-        case 16: return MSDA_BWD_REC(16);
-        default: *handled = false; return cudaSuccess;
-    }
-#undef MSDA_BWD_REC
 }
 
 }  // namespace msda

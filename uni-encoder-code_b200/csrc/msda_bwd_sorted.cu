@@ -755,113 +755,76 @@ msda_bwd_sorted_kernel(const float *__restrict__ grad_out, const float *__restri
 }
 
 // ---------------------------------------------------------------------------
-// host side
+// host side: launch_bwd_sorted() serves the plain op and the fused producers (Producers::ref set),
+// the latter in the default shapes only
 // ---------------------------------------------------------------------------
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int TILE_Q, int SLOTS, int GW, bool FUSED = false>
+template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int TILE_Q, int SLOTS, int GW, bool FUSED>
 static cudaError_t launch_bwd_sorted_cfg(const float *grad_out, const float *value, const int64_t *shapes,
                                          const int64_t *lstart, const float *loc, const float *attw,
-                                         const Dims &d, float *gv, float *gl, float *gw, cudaStream_t stream,
-                                         int gate, Producers pr = Producers{nullptr, 0, 0, 0, nullptr, nullptr}) {
+                                         const Producers &pr, const Dims &d, float *gv, float *gl, float *gw,
+                                         int gate, cudaStream_t stream) {
     using Cfg = SortCfg<LP, WARPS, TILE_W, TILE_Q, SLOTS>;
-    auto kern = msda_bwd_sorted_kernel<LP, WARPS, TILE_W, MIN_CTAS, TILE_Q, SLOTS, GW, FUSED>;
+    constexpr auto kern = msda_bwd_sorted_kernel<LP, WARPS, TILE_W, MIN_CTAS, TILE_Q, SLOTS, GW, FUSED>;
     constexpr size_t kSmemBytes = Cfg::kSmem + (FUSED ? (size_t)Cfg::kPoints * sizeof(float) : 0);
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return e;
-    if (dev < 0 || dev >= kMaxDevices) return cudaErrorInvalidDevice;
-    static std::atomic<int> ctas_per_sm_of[kMaxDevices];
-    int per_sm = ctas_per_sm_of[dev].load(std::memory_order_acquire);
-    if (per_sm == 0) {
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-        if (e != cudaSuccess) return e;
-        int nb = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, WARPS * 32, kSmemBytes);
-        if (e != cudaSuccess) return e;
-        per_sm = nb > 0 ? nb : 1;
-        ctas_per_sm_of[dev].store(per_sm, std::memory_order_release);
-    }
-    const int cap = option_value(OPT_CTAS_PER_SM);
-    if (cap > 0 && cap < per_sm) per_sm = cap;
-    long long blocks = (long long)sm_count() * per_sm;
-    const long long items_ub = (long long)d.N * d.M * d.Lq;
-    if (blocks > items_ub) blocks = items_ub;
-    if (blocks < 1) blocks = 1;
+    cudaError_t e;
+    const int blocks = persistent_blocks<kern>(WARPS * 32, kSmemBytes, d, &e);
+    if (blocks == 0) return e;
     const int flags = option_value(OPT_TILE_ORDER) != 1 ? 1 : 0;
-    kern<<<(unsigned)blocks, WARPS * 32, kSmemBytes, stream>>>(grad_out, value, shapes, lstart, loc, attw, pr, d,
-                                                              flags, gv, gl, gw, gate);
+    kern<<<blocks, WARPS * 32, kSmemBytes, stream>>>(grad_out, value, shapes, lstart, loc, attw, pr, d, flags, gv,
+                                                     gl, gw, gate);
     note_launch();
     return cudaGetLastError();
 }
 
 // whether launch_bwd_sorted() covers this problem (shape + alignment)
 bool bwd_sorted_applies(const float *value, const float *gv, const Dims &d) {
-    const int LP = d.L * d.P;
     // rows of value / grad_value must be 128-byte aligned (the merge loop addresses the two halves
     // of a row as p and p ^ 64); torch allocations are, odd views take the other kernel
     const bool rows_aligned = ((reinterpret_cast<uintptr_t>(value) | reinterpret_cast<uintptr_t>(gv)) & 127u) == 0;
-    return d.D == 32 && d.Lq == d.S && (long long)d.S < (long long)kNoKey && rows_aligned &&
-           (long long)d.S * d.M * 8 < 0x7fffffffLL && (LP == 4 || LP == 8 || LP == 12 || LP == 16);
+    return d32_applies(d) && d.Lq == d.S && (long long)d.S < (long long)kNoKey && rows_aligned;
 }
 
-// `handled` = false: shape outside this kernel's domain (the caller falls back to msda_bwd.cu)
+// pr.ref == nullptr: plain; otherwise fused producers, gradients w.r.t. the raw sampling offsets (`loc`) and
+// attention logits (`attw`), default shapes only.  `handled` = false: shape outside this kernel's domain (the
+// caller falls back to msda_bwd.cu)
 cudaError_t launch_bwd_sorted(const float *grad_out, const float *value, const int64_t *shapes,
-                              const int64_t *lstart, const float *loc, const float *attw, const Dims &d,
-                              float *gv, float *gl, float *gw, cudaStream_t stream, bool *handled,
-                              int gate) {
-    *handled = true;
-    const int LP = d.L * d.P;
-    if (!bwd_sorted_applies(value, gv, d)) {
-        *handled = false;
-        return cudaSuccess;
-    }
+                              const int64_t *lstart, const float *loc, const float *attw, const Producers &pr,
+                              const Dims &d, float *gv, float *gl, float *gw, int gate, cudaStream_t stream,
+                              bool *handled) {
+    *handled = bwd_sorted_applies(value, gv, d);
+    if (!*handled) return cudaSuccess;
     // (warps, tile width, min CTAs per SM, queries per tile, window slots, lanes per record)
-#define MSDA_SORTED(LPV, W, TW, C, TQ, SL, GWV) \
-    launch_bwd_sorted_cfg<LPV, W, TW, C, TQ, SL, GWV>(grad_out, value, shapes, lstart, loc, attw, d, gv, gl, gw, stream, gate)
+#define MSDA_SORTED(LPV, W, TW, C, TQ, SL, GWV, F) \
+    launch_bwd_sorted_cfg<LPV, W, TW, C, TQ, SL, GWV, F>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, \
+                                                         gw, gate, stream)
+    if (pr.ref != nullptr) {
+        switch (d.L * d.P) {   // 4, 8, 12 or 16 (d32_applies)
+            case 4: return MSDA_SORTED(4, 16, 16, 2, 128, 4096, 4, true);
+            case 8: return MSDA_SORTED(8, 16, 16, 2, 128, 4096, 4, true);
+            case 12: return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 4, true);
+            default: return MSDA_SORTED(16, 16, 16, 1, 128, 4096, 4, true);
+        }
+    }
     const int variant = option_value(OPT_BWD_VARIANT);
-    switch (LP) {
-        case 4: return MSDA_SORTED(4, 16, 16, 2, 128, 4096, 8);
-        case 8: return MSDA_SORTED(8, 16, 16, 2, 128, 4096, 8);
+    switch (d.L * d.P) {
+        case 4: return MSDA_SORTED(4, 16, 16, 2, 128, 4096, 8, false);
+        case 8: return MSDA_SORTED(8, 16, 16, 2, 128, 4096, 8, false);
         case 12:
             switch (variant) {      // tuning variants kept for tools/sweep.py (profiles/r2_sweep.md)
-                case 21: return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 8);   // 8 lanes per record (16 bytes each)
-                case 24: return MSDA_SORTED(12, 12, 16, 2, 128, 4096, 4);   // 12 warps, 80 registers
-                case 25: return MSDA_SORTED(12, 8, 8, 4, 64, 2048, 4);      // 64-query tiles, 4 CTAs of 8 warps
+                case 21: return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 8, false);   // 8 lanes per record (16 bytes each)
+                case 24: return MSDA_SORTED(12, 12, 16, 2, 128, 4096, 4, false);   // 12 warps, 80 registers
+                case 25: return MSDA_SORTED(12, 8, 8, 4, 64, 2048, 4, false);      // 64-query tiles, 4 CTAs of 8 warps
                 case 27:
-                    if (d.S < 0x1ffff) return MSDA_SORTED(12, 32, 16, 1, 256, 4096, 8);
-                    return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 4);
-                case 26:                                                    // 256-query tiles (16 x 16), one CTA of 32 warps:
-                    if (d.S < 0x1ffff) return MSDA_SORTED(12, 32, 16, 1, 256, 4096, 4);   // -2 % at configs[1], +2 % at 1024x2048
-                    return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 4);
-                default: return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 4);   // 128-query tiles, 2 CTAs of 16 warps, 4 lanes per record
+                    if (d.S < 0x1ffff) return MSDA_SORTED(12, 32, 16, 1, 256, 4096, 8, false);
+                    return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 4, false);
+                case 26:                                                           // 256-query tiles (16 x 16), one CTA of 32 warps:
+                    if (d.S < 0x1ffff) return MSDA_SORTED(12, 32, 16, 1, 256, 4096, 4, false);   // -2 % at configs[1], +2 % at 1024x2048
+                    return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 4, false);
+                default: return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 4, false);   // 128-query tiles, 2 CTAs of 16 warps, 4 lanes per record
             }
-        case 16: return MSDA_SORTED(16, 16, 16, 1, 128, 4096, 8);
-        default: *handled = false; return cudaSuccess;
+        default: return MSDA_SORTED(16, 16, 16, 1, 128, 4096, 8, false);
     }
 #undef MSDA_SORTED
-}
-
-// Fused producers: gradients w.r.t. the raw sampling offsets and attention logits (default shape only).
-cudaError_t launch_bwd_sorted_fused(const float *grad_out, const float *value, const int64_t *shapes,
-                                    const int64_t *lstart, const float *ref, long long ref_bstride,
-                                    const float *off, const float *logits, const Dims &d, float *gv,
-                                    float *g_off, float *g_logits, cudaStream_t stream, bool *handled, int gate) {
-    *handled = true;
-    if (!bwd_sorted_applies(value, gv, d)) {
-        *handled = false;
-        return cudaSuccess;
-    }
-    const Producers pr{ref, ref_bstride};
-#define MSDA_SORTED_FUSED(LPV, C) \
-    launch_bwd_sorted_cfg<LPV, 16, 16, C, 128, 4096, 4, true>(grad_out, value, shapes, lstart, off, logits, d, gv, \
-                                                                 g_off, g_logits, stream, gate, pr)
-    switch (d.L * d.P) {
-        case 4: return MSDA_SORTED_FUSED(4, 2);
-        case 8: return MSDA_SORTED_FUSED(8, 2);
-        case 12: return MSDA_SORTED_FUSED(12, 2);
-        case 16: return MSDA_SORTED_FUSED(16, 1);
-        default: *handled = false; return cudaSuccess;
-    }
-#undef MSDA_SORTED_FUSED
 }
 
 }  // namespace msda

@@ -317,7 +317,7 @@ __device__ __forceinline__ float div_by_size(float a, float b, float rb) {
 }
 
 struct Producers {
-    const float *ref;          // FUSED only
+    const float *ref;          // FUSED only; the host launchers pick the plain kernels when it is null
     long long ref_bstride;     // elements between images in `ref` (0: shared by the batch)
     // FUSED forward only: floats between consecutive queries' rows of the raw offsets / logits (0: packed,
     // M*L*P*2 and M*L*P) -- lets both live in one [rows, M*L*P*3] projection output
@@ -577,6 +577,40 @@ inline int device_slot(cudaError_t *err) {
     if (*err != cudaSuccess) return -1;
     if (dev < 0 || dev >= kMaxDevices) { *err = cudaErrorInvalidDevice; return -1; }
     return dev;
+}
+
+// Domain of the 32-channel kernels (msda_fwd.cu, msda_bwd.cu, msda_bwd_sorted.cu): D == 32, an instantiated
+// point count L*P, and float4 offsets into an image of value / grad_value that fit in 31 bits.
+inline bool d32_applies(const Dims &d) {
+    const int lp = d.L * d.P;
+    return d.D == 32 && (long long)d.S * d.M * 8 < 0x7fffffffLL && (lp == 4 || lp == 8 || lp == 12 || lp == 16);
+}
+
+// Grid of the persistent kernel `Kern`: as many CTAs as fit on an SM (capped by "ctas_per_sm") on every SM, but
+// no more than N*M*Lq (every work item holds at least one query).  The opt-in shared-memory size is a per-device
+// function attribute: it is set, and the occupancy queried, once per device and kernel instance; the values are
+// immutable afterwards.  Returns 0 with *err set when a CUDA call fails.
+template <auto Kern>
+int persistent_blocks(int threads, size_t smem, const Dims &d, cudaError_t *err) {
+    static std::atomic<int> ctas_per_sm_of[kMaxDevices];
+    const int dev = device_slot(err);
+    if (dev < 0) return 0;
+    int per_sm = ctas_per_sm_of[dev].load(std::memory_order_acquire);
+    if (per_sm == 0) {
+        *err = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (*err != cudaSuccess) return 0;
+        int nb = 0;
+        *err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, Kern, threads, smem);
+        if (*err != cudaSuccess) return 0;
+        per_sm = nb > 0 ? nb : 1;
+        ctas_per_sm_of[dev].store(per_sm, std::memory_order_release);
+    }
+    const int cap = option_value(OPT_CTAS_PER_SM);
+    if (cap > 0 && cap < per_sm) per_sm = cap;
+    long long blocks = (long long)sm_count() * per_sm;
+    const long long items_ub = (long long)d.N * d.M * d.Lq;
+    if (blocks > items_ub) blocks = items_ub;
+    return blocks < 1 ? 1 : (int)blocks;
 }
 
 }  // namespace msda

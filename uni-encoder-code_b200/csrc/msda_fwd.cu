@@ -124,111 +124,58 @@ msda_fwd_d32_kernel(const float *__restrict__ value, const int64_t *__restrict__
 }
 
 // ---------------------------------------------------------------------------
-// host side
+// host side: launch_fwd_d32() serves the plain op and the fused producers (Producers::ref set),
+// the latter in the default CTA shape only
 // ---------------------------------------------------------------------------
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED = false>
+template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
 static cudaError_t launch_fwd_cfg(const float *value, const int64_t *shapes, const int64_t *lstart,
-                                  const float *loc, const float *attw, const Dims &d,
-                                  float *out, cudaStream_t stream, Producers pr = Producers{nullptr, 0, 0, 0, nullptr, nullptr}) {
+                                  const float *loc, const float *attw, const Producers &pr, const Dims &d,
+                                  float *out, cudaStream_t stream) {
     using Cfg = FwdCfg<LP, WARPS, TILE_W, QPW>;
-    auto kern = msda_fwd_d32_kernel<LP, WARPS, TILE_W, MIN_CTAS, QPW, FUSED>;
-    // the opt-in shared-memory size is a per-device function attribute: set it (and query the
-    // occupancy) once per device; the values are immutable afterwards
-    static std::atomic<int> ctas_per_sm_of[kMaxDevices];
-    cudaError_t e = cudaSuccess;
-    const int dev = device_slot(&e);
-    if (dev < 0) return e;
-    int ctas_per_sm = ctas_per_sm_of[dev].load(std::memory_order_acquire);
-    if (ctas_per_sm == 0) {
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmem);
-        if (e != cudaSuccess) return e;
-        int nb = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, WARPS * 32, Cfg::kSmem);
-        if (e != cudaSuccess) return e;
-        ctas_per_sm = nb > 0 ? nb : 1;
-        ctas_per_sm_of[dev].store(ctas_per_sm, std::memory_order_release);
-    }
-    int per_sm = ctas_per_sm;
-    const int cap = option_value(OPT_CTAS_PER_SM);
-    if (cap > 0 && cap < per_sm) per_sm = cap;
-    // every group holds at least one query, so items <= N*M*Lq
-    long long blocks = (long long)sm_count() * per_sm;
-    const long long items_ub = (long long)d.N * d.M * d.Lq;
-    if (blocks > items_ub) blocks = items_ub;
-    if (blocks < 1) blocks = 1;
+    constexpr auto kern = msda_fwd_d32_kernel<LP, WARPS, TILE_W, MIN_CTAS, QPW, FUSED>;
+    cudaError_t e;
+    const int blocks = persistent_blocks<kern>(WARPS * 32, Cfg::kSmem, d, &e);
+    if (blocks == 0) return e;
     const int want_spatial = option_value(OPT_TILE_ORDER) != 1;
-    kern<<<(unsigned)blocks, WARPS * 32, Cfg::kSmem, stream>>>(value, shapes, lstart, loc, attw, pr, d,
-                                                              want_spatial, out);
+    kern<<<blocks, WARPS * 32, Cfg::kSmem, stream>>>(value, shapes, lstart, loc, attw, pr, d, want_spatial, out);
     note_launch();
     return cudaGetLastError();
 }
 
 template <int LP>
 static cudaError_t launch_fwd_lp(const float *value, const int64_t *shapes, const int64_t *lstart,
-                                 const float *loc, const float *attw, const Dims &d, float *out,
-                                 cudaStream_t stream) {
+                                 const float *loc, const float *attw, const Producers &pr, const Dims &d,
+                                 float *out, cudaStream_t stream) {
     // variant = (warps, query tile width, min CTAs per SM -> register budget, queries per warp)
-#define MSDA_FWD(W, TW, C, Q) launch_fwd_cfg<LP, W, TW, C, Q>(value, shapes, lstart, loc, attw, d, out, stream)
+#define MSDA_FWD(W, TW, C, Q, F) launch_fwd_cfg<LP, W, TW, C, Q, F>(value, shapes, lstart, loc, attw, pr, d, out, stream)
+    if (pr.ref != nullptr) return MSDA_FWD(16, 16, 2, 8, true);   // fused producers: the default shape only
     switch (option_value(OPT_FWD_VARIANT)) {
-        case 1: return MSDA_FWD(8, 8, 4, 8);     //  8 warps, tile  8x8
-        case 3: return MSDA_FWD(32, 16, 1, 8);   // 32 warps, tile 16x16, one CTA per SM
-        case 4: return MSDA_FWD(16, 8, 2, 8);    // 16 warps, tile 16x8
-        case 5: return MSDA_FWD(16, 16, 2, 4);   // 16 warps, tile  4x16, 4 queries per warp (50 KB smem per SM)
-        case 6: return MSDA_FWD(16, 8, 2, 4);    // 16 warps, tile  8x8,  4 queries per warp
-        case 7: return MSDA_FWD(32, 16, 1, 4);   // 32 warps, tile  8x16, 4 queries per warp, one CTA per SM
-        case 8: return MSDA_FWD(16, 16, 3, 4);   // 16 warps, tile  4x16, 48 warps per SM (40 regs)
+        case 1: return MSDA_FWD(8, 8, 4, 8, false);     //  8 warps, tile  8x8
+        case 3: return MSDA_FWD(32, 16, 1, 8, false);   // 32 warps, tile 16x16, one CTA per SM
+        case 4: return MSDA_FWD(16, 8, 2, 8, false);    // 16 warps, tile 16x8
+        case 5: return MSDA_FWD(16, 16, 2, 4, false);   // 16 warps, tile  4x16, 4 queries per warp (50 KB smem per SM)
+        case 6: return MSDA_FWD(16, 8, 2, 4, false);    // 16 warps, tile  8x8,  4 queries per warp
+        case 7: return MSDA_FWD(32, 16, 1, 4, false);   // 32 warps, tile  8x16, 4 queries per warp, one CTA per SM
+        case 8: return MSDA_FWD(16, 16, 3, 4, false);   // 16 warps, tile  4x16, 48 warps per SM (40 regs)
         case 2:
-        default: return MSDA_FWD(16, 16, 2, 8);  // 16 warps, tile  8x16, 8 queries per warp (98 KB smem per SM)
+        default: return MSDA_FWD(16, 16, 2, 8, false);  // 16 warps, tile  8x16, 8 queries per warp (98 KB smem per SM)
     }
 #undef MSDA_FWD
 }
 
-// `handled` tells the caller whether this specialised path took the problem
-// (otherwise the generic kernel is used).
-cudaError_t launch_fwd_d32(const float *value, const int64_t *shapes, const int64_t *lstart,
-                           const float *loc, const float *attw, const Dims &d, float *out,
-                           cudaStream_t stream, bool *handled) {
-    *handled = true;
-    const int LP = d.L * d.P;
-    if (d.D != 32 || (long long)d.S * d.M * 8 >= 0x7fffffffLL) {
-        *handled = false;
-        return cudaSuccess;
-    }
-    switch (LP) {
-        case 4: return launch_fwd_lp<4>(value, shapes, lstart, loc, attw, d, out, stream);
-        case 8: return launch_fwd_lp<8>(value, shapes, lstart, loc, attw, d, out, stream);
-        case 12: return launch_fwd_lp<12>(value, shapes, lstart, loc, attw, d, out, stream);
-        case 16: return launch_fwd_lp<16>(value, shapes, lstart, loc, attw, d, out, stream);
-        default: *handled = false; return cudaSuccess;
-    }
-}
-
-// Fused producers (SURVEY 8f.1): `off` = raw sampling offsets, `logits` = raw attention logits,
-// `ref` = reference points [N or 1, Lq, L, 2].  Only the default CTA shape is instantiated.
-cudaError_t launch_fwd_d32_fused(const float *value, const int64_t *shapes, const int64_t *lstart,
-                                 const float *ref, long long ref_bstride, const float *off,
-                                 const float *logits, const Dims &d, float *out, cudaStream_t stream,
-                                 bool *handled, int off_qstride, int logit_qstride, const float *off_table,
-                                 const float *logit_table) {
-    *handled = true;
-    const int lp = d.L * d.P;
-    if (off_qstride == d.M * lp * 2 && logit_qstride == d.M * lp) off_qstride = logit_qstride = 0;   // packed
-    const Producers pr{ref, ref_bstride, off_qstride, logit_qstride, off_table, logit_table};
-    if ((off_qstride != 0) != (logit_qstride != 0) || (off_qstride & 1) || off_qstride < 0 || logit_qstride < 0 ||
-        (off_table != nullptr) != (logit_table != nullptr)) {
-        *handled = false;
-        return cudaSuccess;
-    }
-    if (d.D != 32 || (long long)d.S * d.M * 8 >= 0x7fffffffLL) {
-        *handled = false;
-        return cudaSuccess;
-    }
-    switch (d.L * d.P) {
-        case 4: return launch_fwd_cfg<4, 16, 16, 2, 8, true>(value, shapes, lstart, off, logits, d, out, stream, pr);
-        case 8: return launch_fwd_cfg<8, 16, 16, 2, 8, true>(value, shapes, lstart, off, logits, d, out, stream, pr);
-        case 12: return launch_fwd_cfg<12, 16, 16, 2, 8, true>(value, shapes, lstart, off, logits, d, out, stream, pr);
-        case 16: return launch_fwd_cfg<16, 16, 16, 2, 8, true>(value, shapes, lstart, off, logits, d, out, stream, pr);
-        default: *handled = false; return cudaSuccess;
+// pr.ref == nullptr: plain, `loc` / `attw` are the sampling locations and attention weights.  Otherwise fused
+// producers (SURVEY 8f.1): `loc` = raw sampling offsets, `attw` = raw attention logits, `pr.ref` = reference
+// points [N or 1, Lq, L, 2].  `handled` = false: the problem is outside d32_applies() and nothing was launched.
+cudaError_t launch_fwd_d32(const float *value, const int64_t *shapes, const int64_t *lstart, const float *loc,
+                           const float *attw, const Producers &pr, const Dims &d, float *out, cudaStream_t stream,
+                           bool *handled) {
+    *handled = d32_applies(d);
+    if (!*handled) return cudaSuccess;
+    switch (d.L * d.P) {       // 4, 8, 12 or 16 (d32_applies)
+        case 4: return launch_fwd_lp<4>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        case 8: return launch_fwd_lp<8>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        case 12: return launch_fwd_lp<12>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        default: return launch_fwd_lp<16>(value, shapes, lstart, loc, attw, pr, d, out, stream);
     }
 }
 

@@ -81,9 +81,11 @@ def _det_workspace(images, S, M, D, L, Lq, P, dtype, device):
     return torch.empty(int(nbytes), dtype=torch.uint8, device=device)
 
 
-def _check_common(named, im2col_step, opname):
-    value = named[0][1]
-    if not isinstance(value, torch.Tensor) or not value.is_cuda:
+def _require_cuda_contiguous(named):
+    """The reference's input checks over (name, tensor) pairs: every tensor contiguous and on the device of the
+    first one, which must be a CUDA tensor."""
+    first, anchor = named[0]
+    if not isinstance(anchor, torch.Tensor) or not anchor.is_cuda:
         raise RuntimeError("Not implemented on the CPU")                     # ms_deform_attn.h:43,65
     for name, t in named:
         if not t.is_contiguous():
@@ -91,8 +93,13 @@ def _check_common(named, im2col_step, opname):
     for name, t in named:
         if not t.is_cuda:
             raise RuntimeError(f"{name} must be a CUDA tensor")              # cu:39-43
-        if t.device != value.device:
-            raise RuntimeError(f"{name} is on {t.device}, value is on {value.device}")
+        if t.device != anchor.device:
+            raise RuntimeError(f"{name} is on {t.device}, {first} is on {anchor.device}")
+
+
+def _check_common(named, im2col_step, opname):
+    _require_cuda_contiguous(named)
+    value = named[0][1]
     if value.dtype not in _FWD:
         raise RuntimeError(f'"{opname}" not implemented for \'{value.dtype}\'')   # cu:69,139
     _, shapes, lsi, loc, w = (t for _, t in named[:5])
@@ -154,8 +161,9 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
         # nothing to sample: all three gradients stay at the reference's zero fill (cu:126-128)
         return [torch.zeros_like(value), torch.zeros_like(sampling_loc), torch.zeros_like(attn_weight)]
     if _deterministic():
-        return _ms_deform_attn_backward_deterministic(value, spatial_shapes, level_start_index, sampling_loc,
-                                                      attn_weight, grad_output, N, S, M, D, L, Lq, P)
+        return _backward_deterministic(_BWD_DET[value.dtype], "ms_deform_attn_backward (deterministic)", value,
+                                       spatial_shapes, level_start_index, (sampling_loc, attn_weight), grad_output,
+                                       (N, S, M, D, L, Lq, P))
     with torch.cuda.device(value.device):
         grad_value = torch.zeros_like(value)            # accumulated by reductions (cu:126)
         grad_loc = torch.empty_like(sampling_loc)       # fully overwritten (cf. cu:127)
@@ -170,24 +178,27 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
     return [grad_value, grad_loc, grad_w]
 
 
-def _ms_deform_attn_backward_deterministic(value, shapes, lsi, loc, w, grad_output, N, S, M, D, L, Lq, P):
-    """ms_deform_attn_backward through msda_b200_backward_deterministic_f32/_f64, in chunks of whole images."""
+def _backward_deterministic(fn, opname, value, shapes, lsi, producers, grad_output, dims, ref=None, rs=0):
+    """A deterministic backward entry ``fn`` (msda_b200_backward_deterministic_f32/_f64, or with ``ref`` the fused
+    msda_b200_fused_backward_deterministic_f32) in chunks of whole images -> [grad_value, *grads of producers].
+    ``producers``: (sampling_loc, attn_weight), or for the fused op (sampling_offsets, attn_logits)."""
+    N, S, M, D, L, Lq, P = dims
     chunks = _image_chunks(N, Lq * M * L * P * 4)
     with torch.cuda.device(value.device):
         grad_value = torch.empty_like(value)            # fully overwritten by the gather
-        grad_loc = torch.empty_like(loc)
-        grad_w = torch.empty_like(w)
+        grads = [torch.empty_like(t) for t in producers]
         ws = _det_workspace(max(b - a for a, b in chunks), S, M, D, L, Lq, P, value.dtype, value.device)
         stream = torch.cuda.current_stream().cuda_stream
         with _timed("backward"):
             for a, b in chunks:
-                rc = _BWD_DET[value.dtype](
-                    grad_output[a:b].data_ptr(), value[a:b].data_ptr(), shapes.data_ptr(), lsi.data_ptr(),
-                    loc[a:b].data_ptr(), w[a:b].data_ptr(), b - a, S, M, D, L, Lq, P,
-                    grad_value[a:b].data_ptr(), grad_loc[a:b].data_ptr(), grad_w[a:b].data_ptr(), ws.data_ptr(),
-                    stream)
-                _lib.check(rc, "ms_deform_attn_backward (deterministic)")
-    return [grad_value, grad_loc, grad_w]
+                fused = ()
+                if ref is not None:                     # rs == 0: one set of reference points shared by the batch
+                    fused = ((ref[a:b] if rs != 0 and ref.size(0) == N else ref).data_ptr(), rs)
+                rc = fn(grad_output[a:b].data_ptr(), value[a:b].data_ptr(), shapes.data_ptr(), lsi.data_ptr(), *fused,
+                        *(t[a:b].data_ptr() for t in producers), b - a, S, M, D, L, Lq, P, grad_value[a:b].data_ptr(),
+                        *(g[a:b].data_ptr() for g in grads), ws.data_ptr(), stream)
+                _lib.check(rc, opname)
+    return [grad_value, *grads]
 
 
 def debug_indices(value_shape, spatial_shapes, level_start_index, sampling_loc):
@@ -229,13 +240,7 @@ def fused_supported(value, reference_points, sampling_offsets, attn_logits):
 def _check_fused(value, shapes, lsi, ref, off, logits, extra=()):
     named = [("value", value), ("spatial_shapes", shapes), ("level_start_index", lsi),
              ("reference_points", ref), ("sampling_offsets", off), ("attn_logits", logits)] + list(extra)
-    if not value.is_cuda:
-        raise RuntimeError("Not implemented on the CPU")
-    for name, t in named:
-        if not t.is_contiguous():
-            raise RuntimeError(f"{name} tensor has to be contiguous")
-        if not t.is_cuda or t.device != value.device:
-            raise RuntimeError(f"{name} must be a CUDA tensor on {value.device}")
+    _require_cuda_contiguous(named)
     if not fused_supported(value, ref, off, logits):
         raise RuntimeError("fused MSDA covers fp32, 32 channels per head, L*P in {4,8,12,16}, 2-d "
                            "reference points only; compose the unfused op for other shapes")
@@ -253,17 +258,27 @@ def _check_fused(value, shapes, lsi, ref, off, logits, extra=()):
 
 def ms_deform_attn_fused_forward(value, spatial_shapes, level_start_index, reference_points,
                                  sampling_offsets, attn_logits):
-    """output [N, Lq, M*D] from raw offsets / logits (msda_b200_fused_forward_f32)."""
+    """output [N, Lq, M*D] from raw offsets / logits (msda_b200_fused_forward_strided_f32 on packed rows)."""
     N, S, M, D, L, Lq, P, rs = _check_fused(value, spatial_shapes, level_start_index, reference_points,
                                             sampling_offsets, attn_logits)
+    return _fused_forward("ms_deform_attn_fused_forward", value, spatial_shapes, level_start_index, reference_points,
+                          rs, sampling_offsets, 2 * M * L * P, attn_logits, M * L * P, None, None,
+                          (N, S, M, D, L, Lq, P))
+
+
+def _fused_forward(opname, value, shapes, lsi, ref, rs, off, off_stride, logits, logit_stride, off_table, logit_table,
+                   dims):
+    """msda_b200_fused_forward_strided_f32 on checked tensors; ``off`` / ``logits`` rows ``off_stride`` /
+    ``logit_stride`` floats apart, ``off_table`` / ``logit_table`` (both or neither) the per-query additive tables."""
+    N, S, M, D, L, Lq, P = dims
     with torch.cuda.device(value.device):
         output = torch.empty((N, Lq, M * D), dtype=value.dtype, device=value.device)
         with _timed("forward"):
-            rc = _lib.lib.msda_b200_fused_forward_f32(
-                value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
-                reference_points.data_ptr(), rs, sampling_offsets.data_ptr(), attn_logits.data_ptr(),
-                N, S, M, D, L, Lq, P, output.data_ptr(), torch.cuda.current_stream().cuda_stream)
-    _lib.check(rc, "ms_deform_attn_fused_forward")
+            rc = _lib.lib.msda_b200_fused_forward_strided_f32(
+                value.data_ptr(), shapes.data_ptr(), lsi.data_ptr(), ref.data_ptr(), rs, off.data_ptr(), off_stride,
+                logits.data_ptr(), logit_stride, _ptr(off_table), _ptr(logit_table), N, S, M, D, L, Lq, P,
+                output.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    _lib.check(rc, opname)
     return output
 
 
@@ -289,30 +304,16 @@ def ms_deform_attn_fused_forward_packed(value, spatial_shapes, level_start_index
         named.append(("query_table", query_table))
         if tuple(query_table.shape) != (Lq, width) or query_table.dtype != torch.float32:
             raise RuntimeError(f"query_table must be a float32 [Lq, {width}] tensor")
-    if not value.is_cuda:
-        raise RuntimeError("Not implemented on the CPU")
-    for name, t in named:
-        if not t.is_contiguous():
-            raise RuntimeError(f"{name} tensor has to be contiguous")
-        if not t.is_cuda or t.device != value.device:
-            raise RuntimeError(f"{name} must be a CUDA tensor on {value.device}")
+    _require_cuda_contiguous(named)
     if not fused_supported(value, reference_points, off.view(N, Lq, M, L, P, 2), logits) \
             or tuple(reference_points.shape[1:]) != (Lq, L, 2) or spatial_shapes.size(0) != L \
             or projections.dtype != torch.float32 or reference_points.dtype != torch.float32:
         raise RuntimeError("fused MSDA covers fp32, 32 channels per head, L*P in {4,8,12,16}, 2-d "
                            "reference points only; compose the unfused op for other shapes")
     rs = 0 if reference_points.size(0) == 1 and N > 1 else Lq * L * 2
-    with torch.cuda.device(value.device):
-        output = torch.empty((N, Lq, M * D), dtype=value.dtype, device=value.device)
-        with _timed("forward"):
-            rc = _lib.lib.msda_b200_fused_forward_strided_f32(
-                value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
-                reference_points.data_ptr(), rs, off.data_ptr(), width, logits.data_ptr(), width,
-                query_table.data_ptr() if query_table is not None else None,
-                query_table[:, 2 * M * L * P:].data_ptr() if query_table is not None else None,
-                N, S, M, D, L, Lq, P, output.data_ptr(), torch.cuda.current_stream().cuda_stream)
-    _lib.check(rc, "ms_deform_attn_fused_forward_packed")
-    return output
+    return _fused_forward("ms_deform_attn_fused_forward_packed", value, spatial_shapes, level_start_index,
+                          reference_points, rs, off, width, logits, width, query_table,
+                          query_table[:, 2 * M * L * P:] if query_table is not None else None, (N, S, M, D, L, Lq, P))
 
 
 def ms_deform_attn_fused_backward(value, spatial_shapes, level_start_index, reference_points,
@@ -321,9 +322,10 @@ def ms_deform_attn_fused_backward(value, spatial_shapes, level_start_index, refe
     N, S, M, D, L, Lq, P, rs = _check_fused(value, spatial_shapes, level_start_index, reference_points,
                                             sampling_offsets, attn_logits, [("grad_output", grad_output)])
     if _deterministic():
-        return _ms_deform_attn_fused_backward_deterministic(value, spatial_shapes, level_start_index, reference_points,
-                                                            sampling_offsets, attn_logits, grad_output, rs,
-                                                            N, S, M, D, L, Lq, P)
+        return _backward_deterministic(_lib.lib.msda_b200_fused_backward_deterministic_f32,
+                                       "ms_deform_attn_fused_backward (deterministic)", value, spatial_shapes,
+                                       level_start_index, (sampling_offsets, attn_logits), grad_output,
+                                       (N, S, M, D, L, Lq, P), reference_points, rs)
     with torch.cuda.device(value.device):
         grad_value = torch.zeros_like(value)
         grad_off = torch.empty_like(sampling_offsets)
@@ -336,28 +338,6 @@ def ms_deform_attn_fused_backward(value, spatial_shapes, level_start_index, refe
                 grad_value.data_ptr(), grad_off.data_ptr(), grad_logits.data_ptr(),
                 torch.cuda.current_stream().cuda_stream)
     _lib.check(rc, "ms_deform_attn_fused_backward")
-    return [grad_value, grad_off, grad_logits]
-
-
-def _ms_deform_attn_fused_backward_deterministic(value, shapes, lsi, ref, off, logits, grad_output, rs,
-                                                 N, S, M, D, L, Lq, P):
-    """ms_deform_attn_fused_backward through msda_b200_fused_backward_deterministic_f32, in chunks of whole images."""
-    chunks = _image_chunks(N, Lq * M * L * P * 4)
-    with torch.cuda.device(value.device):
-        grad_value = torch.empty_like(value)
-        grad_off = torch.empty_like(off)
-        grad_logits = torch.empty_like(logits)
-        ws = _det_workspace(max(b - a for a, b in chunks), S, M, D, L, Lq, P, value.dtype, value.device)
-        stream = torch.cuda.current_stream().cuda_stream
-        with _timed("backward"):
-            for a, b in chunks:
-                ref_a = ref[a:b] if rs != 0 and ref.size(0) == N else ref    # rs == 0: one set shared by the batch
-                rc = _lib.lib.msda_b200_fused_backward_deterministic_f32(
-                    grad_output[a:b].data_ptr(), value[a:b].data_ptr(), shapes.data_ptr(), lsi.data_ptr(),
-                    ref_a.data_ptr(), rs, off[a:b].data_ptr(), logits[a:b].data_ptr(), b - a, S, M, D, L, Lq, P,
-                    grad_value[a:b].data_ptr(), grad_off[a:b].data_ptr(), grad_logits[a:b].data_ptr(), ws.data_ptr(),
-                    stream)
-                _lib.check(rc, "ms_deform_attn_fused_backward (deterministic)")
     return [grad_value, grad_off, grad_logits]
 
 
@@ -395,13 +375,9 @@ def linear_tf32x3(x, weight, bias=None, relu=False, split_weight_in_kernel=False
     the affected rows, but an infinite input may come out as NaN where F.linear returns +-inf (the
     error-compensated split forms inf - inf and inf * w_lo of either sign).  ``split_weight_in_kernel``: no pre-pass over
     (and no workspace for) the weight -- for a one-shot "weight" such as transposed activations."""
-    if not x.is_cuda:
-        raise RuntimeError("Not implemented on the CPU")
-    for name, t in (("x", x), ("weight", weight)) + ((("bias", bias),) if bias is not None else ()):
-        if not t.is_contiguous():
-            raise RuntimeError(f"{name} tensor has to be contiguous")
-        if not t.is_cuda or t.device != x.device:
-            raise RuntimeError(f"{name} must be a CUDA tensor on {x.device}")
+    named = [("x", x), ("weight", weight)] + ([("bias", bias)] if bias is not None else [])
+    _require_cuda_contiguous(named)
+    for name, t in named:
         if t.dtype != torch.float32:
             raise RuntimeError(f"{name} must be float32")
     if not linear_tf32x3_supported(x, weight) or (bias is not None and bias.shape != (weight.size(0),)):
