@@ -104,7 +104,8 @@ int msda_b200_backward_f64(const double *grad_output, const double *value,
  * Deterministic backwards: the same gradients with no order-dependent floating-point sums, so bit-identical
  * inputs give bit-identical outputs on the same device (what torch.use_deterministic_algorithms asks for).
  * Same arguments as the entries above plus `workspace`, device scratch of
- * msda_b200_backward_deterministic_workspace_bytes(...) bytes (value_bytes = 4 for the f32 entries, 8 for f64;
+ * msda_b200_backward_deterministic_workspace_bytes(...) bytes (value_bytes = 4 for the f32 entries, 8 for f64,
+ * 2 for the bf16 / f16 ones below;
  * 16-byte aligned; contents meaningless before and after; 0 = shape not covered: more than 2^31 - 1 corner
  * records, i.e. batch * num_query * num_heads * num_levels * num_point * 4, or batch * spatial_size * num_heads
  * >= 2^31 -- split the batch).  grad_value is fully overwritten (no zero-fill needed).  The backward kernel of
@@ -132,6 +133,56 @@ int msda_b200_backward_deterministic_f64(const double *grad_output, const double
                                          int num_levels, int num_query, int num_point,
                                          double *grad_value, double *grad_sampling_loc,
                                          double *grad_attn_weight, void *workspace, void *stream);
+
+/*
+ * Mixed precision (torch.autocast): value, output, grad_output and grad_value are bfloat16 (_bf16) or IEEE
+ * half (_f16), passed as uint16_t bit patterns, one type per call; sampling_loc, attn_weight and their
+ * gradients stay float.  Every sum is fp32 with the geometry of the f32 entries; the only 16-bit rounding is
+ * the final store of output / grad_value (round to nearest even; fp16 overflow gives +-inf).  The results
+ * therefore equal the f32 entries applied to the widened 16-bit inputs, up to that one rounding.  Same
+ * kernel choice and "bwd_variant" meanings as the f32 entries (each kernel in its default shape); any
+ * channels, levels and points (shapes outside the 32-channel kernels take the generic ones).
+ *
+ * msda_b200_backward_{bf16,f16}: `grad_value_accum` is caller-provided device scratch of
+ * batch * spatial_size * num_heads * channels floats, ZERO-FILLED before the call (16-byte aligned for the
+ * fastest path); the kernels reduce into it in fp32 and one more launch rounds it into grad_value.  Its
+ * contents afterwards are the fp32 grad_value.
+ * msda_b200_backward_deterministic_{bf16,f16}: as the f32 twin, workspace of
+ * msda_b200_backward_deterministic_workspace_bytes(..., value_bytes = 2) bytes (the records carry fp32
+ * weights); the gather sums in fp32 and writes the 16-bit grad_value directly (no accumulation buffer).
+ */
+int msda_b200_forward_bf16(const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start,
+                           const float *sampling_loc, const float *attn_weight, int batch, int spatial_size,
+                           int num_heads, int channels, int num_levels, int num_query, int num_point,
+                           uint16_t *output, void *stream);
+int msda_b200_forward_f16(const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start,
+                          const float *sampling_loc, const float *attn_weight, int batch, int spatial_size,
+                          int num_heads, int channels, int num_levels, int num_query, int num_point,
+                          uint16_t *output, void *stream);
+int msda_b200_backward_bf16(const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes,
+                            const int64_t *level_start, const float *sampling_loc, const float *attn_weight,
+                            int batch, int spatial_size, int num_heads, int channels, int num_levels,
+                            int num_query, int num_point, float *grad_value_accum, uint16_t *grad_value,
+                            float *grad_sampling_loc, float *grad_attn_weight, void *stream);
+int msda_b200_backward_f16(const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes,
+                           const int64_t *level_start, const float *sampling_loc, const float *attn_weight,
+                           int batch, int spatial_size, int num_heads, int channels, int num_levels,
+                           int num_query, int num_point, float *grad_value_accum, uint16_t *grad_value,
+                           float *grad_sampling_loc, float *grad_attn_weight, void *stream);
+int msda_b200_backward_deterministic_bf16(const uint16_t *grad_output, const uint16_t *value,
+                                          const int64_t *spatial_shapes, const int64_t *level_start,
+                                          const float *sampling_loc, const float *attn_weight, int batch,
+                                          int spatial_size, int num_heads, int channels, int num_levels,
+                                          int num_query, int num_point, uint16_t *grad_value,
+                                          float *grad_sampling_loc, float *grad_attn_weight, void *workspace,
+                                          void *stream);
+int msda_b200_backward_deterministic_f16(const uint16_t *grad_output, const uint16_t *value,
+                                         const int64_t *spatial_shapes, const int64_t *level_start,
+                                         const float *sampling_loc, const float *attn_weight, int batch,
+                                         int spatial_size, int num_heads, int channels, int num_levels,
+                                         int num_query, int num_point, uint16_t *grad_value,
+                                         float *grad_sampling_loc, float *grad_attn_weight, void *workspace,
+                                         void *stream);
 
 /*
  * Fused producers (SURVEY.md 8f.1): the same op with the three elementwise steps of its caller

@@ -1,0 +1,211 @@
+"""Mixed-precision MSDA on the B200: the bf16 / fp16 op against fp32, and the pixel decoder under autocast.
+
+    python tools/bench_mixed.py [--parts a,b,c] [--steps 20] [--out DIR]
+
+DIR defaults to $BENCH_OUT/mixed, and BENCH_OUT to bench_out/ in the repository (git-ignored).
+
+(a) the op alone at BASELINE configs[1] (512x1024, batch 8) and at the configs[2] shape (1024x2048, batch 8):
+    forward, backward (gated default, merging kernel forced, per-row kernel forced) and forward + backward, for
+    fp32, bf16 and fp16 on the same seeded inputs (value / grad_output rounded once to the 16-bit type), the three
+    types alternating in one process.  Every timed call follows a 256 MB write that evicts the 126 MB L2; the
+    events bracket the call only.  Times are of the Python-level call, so the 16-bit backward includes the
+    zero-fill of its fp32 accumulation buffer (torch) and the conversion launch.  Algorithmic bytes from shapes:
+    value / output / grad_output / grad_value once each at their element size, locations and weights (12 bytes a
+    point) and their gradients once -- per query at configs[1] 3 200 (fp32) / 2 176 (16-bit) forward and
+    5 376 / 3 840 backward; the accumulation buffer's zero-fill and conversion read (4 + 4 bytes per value
+    element) are reported separately.
+(b) the decoder forward (forward_features, no autograd) at the configs[2] shape with a Swin-T pyramid: the fastest
+    fp32 setting (fused=True, linear="tf32x3") against amp=True under bf16 autocast.
+(c) the decoder training step (forward_features -> loss -> backward -> AdamW) at 512x1024, batch 16, as
+    tools/bench_decoder_train.py: fp32 linear="tf32x3" against amp=True with bf16, and with fp16 + GradScaler.
+
+Every JSON line carries the card's name and power limit (read-only nvidia-smi query).
+"""
+import argparse
+import contextlib
+import json
+import os
+import statistics
+import sys
+
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+from __graft_entry__ import load_package  # noqa: E402
+from bench_decoder_train import card, timed  # noqa: E402
+
+DTYPES = {"fp32": torch.float32, "bf16": torch.bfloat16, "fp16": torch.float16}
+SWIN_T = {"res2": (96, 4), "res3": (192, 8), "res4": (384, 16), "res5": (768, 32)}
+
+
+def op_bytes(inp, esize):
+    N, S, M, D = inp["value"].shape
+    Lq, L, P = inp["sampling_locations"].shape[1], inp["sampling_locations"].shape[3], inp["sampling_locations"].shape[4]
+    rows_v, rows_q, pts = N * S * M * D, N * Lq * M * D, N * Lq * M * L * P
+    return {"forward": rows_v * esize + rows_q * esize + pts * 12,
+            "backward": 2 * rows_v * esize + rows_q * esize + 2 * pts * 12,
+            "accum_zero_fill": rows_v * 4 if esize == 2 else 0, "accum_conversion_read": rows_v * 4 if esize == 2 else 0,
+            "queries": N * Lq}
+
+
+def part_a(pkg, args, emit):
+    dev = torch.device("cuda", 0)
+    dtypes = {k: DTYPES[k] for k in args.dtypes.split(",")}
+    ops = args.ops.split(",")
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    for name in ("cityscapes_512x1024_b8", "cityscapes_1024x2048_b8"):
+        base = pkg.synthetic.make_workload_inputs(name, mode="model", seed=1, device=dev)
+        inputs = {}
+        for tag, dt in dtypes.items():
+            d = dict(base)
+            if dt != torch.float32:
+                d["value"], d["grad_output"] = base["value"].to(dt), base["grad_output"].to(dt)
+            else:   # the same values as the 16-bit arms see: rounded through bf16 once
+                d["value"], d["grad_output"] = base["value"].bfloat16().float(), base["grad_output"].bfloat16().float()
+            inputs[tag] = d
+        del base
+
+        def calls(tag):
+            d = inputs[tag]
+            a = (d["value"], d["spatial_shapes"], d["level_start_index"], d["sampling_locations"], d["attention_weights"])
+            fwd = pkg.ms_deform_attn_forward if tag == "fp32" else pkg.ms_deform_attn_mixed_forward
+            bwd = pkg.ms_deform_attn_backward if tag == "fp32" else pkg.ms_deform_attn_mixed_backward
+            return {"forward": lambda: fwd(*a, 128),
+                    "backward": lambda: bwd(*a, d["grad_output"], 128),
+                    "fwd+bwd": lambda: (fwd(*a, 128), bwd(*a, d["grad_output"], 128))}
+
+        arms = [(op, variant) for op, variant in (("forward", 0), ("backward", 0), ("backward", 20), ("backward", 2),
+                                                  ("fwd+bwd", 0)) if op in ops]
+        times = {(tag, op, v): [] for tag in dtypes for op, v in arms}
+        fns = {tag: calls(tag) for tag in dtypes}
+        for tag in dtypes:                                  # warm-up of every shape and arm
+            for op, v in arms:
+                pkg.set_option("bwd_variant", v)
+                for _ in range(2):
+                    fns[tag][op]()
+        pkg.set_option("bwd_variant", 0)
+        torch.cuda.synchronize()
+        for _ in range(args.steps):
+            for op, v in arms:
+                pkg.set_option("bwd_variant", v)
+                for tag in dtypes:                          # the types alternate
+                    flush.zero_()
+                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                    e0.record()
+                    fns[tag][op]()
+                    e1.record()
+                    e1.synchronize()
+                    times[(tag, op, v)].append(e0.elapsed_time(e1))
+        pkg.set_option("bwd_variant", 0)
+        for (tag, op, v), ts in times.items():
+            b = op_bytes(inputs[tag], inputs[tag]["value"].element_size())
+            nbytes = b["forward"] * (op != "backward") + b["backward"] * (op != "forward")
+            ms = statistics.median(ts)
+            emit({"part": "a", "label": args.label, "workload": name, "dtype": tag, "op": op,
+                  "bwd_variant": {0: "gated default", 20: "merging forced", 2: "per-row forced"}[v],
+                  "ms_median": ms, "ms_min": min(ts), "ms_max": max(ts), "timed_calls": len(ts),
+                  "algorithmic_bytes": nbytes, "algorithmic_bytes_per_query": nbytes / b["queries"],
+                  "accum_zero_fill_bytes": b["accum_zero_fill"] if op != "forward" else 0,
+                  "accum_conversion_read_bytes": b["accum_conversion_read"] if op != "forward" else 0,
+                  "algorithmic_GBs": nbytes / ms / 1e6, "l2": "evicted before every call (256 MB write)"})
+        del inputs, fns
+        torch.cuda.empty_cache()
+
+
+def _decoder(pkg, fused, linear, amp, train):
+    torch.manual_seed(0)
+    m = pkg.pixel_decoder.MSDeformAttnPixelDecoder(
+        SWIN_T, transformer_dropout=0.1 if train else 0.0, transformer_nheads=8, transformer_dim_feedforward=1024,
+        transformer_enc_layers=6, conv_dim=256, mask_dim=256, norm="GN", transformer_in_features=["res3", "res4", "res5"],
+        common_stride=4, fused=fused, linear=linear, amp=amp).cuda()
+    return m.train() if train else m.eval()
+
+
+def _feats(batch, h, w, seed):
+    gen = torch.Generator(device="cuda").manual_seed(seed)
+    return {k: torch.randn(batch, c, h // s, w // s, device="cuda", generator=gen) for k, (c, s) in SWIN_T.items()}
+
+
+def part_b(pkg, args, emit):
+    feats = _feats(8, 1024, 2048, 3)
+    arms = [("fp32 fused tf32x3", dict(fused=True, linear="tf32x3", amp=False), None),
+            ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16)]
+    models = {tag: _decoder(pkg, train=False, **kw) for tag, kw, _ in arms}
+    res = {tag: [] for tag, _, _ in arms}
+    for _ in range(args.repeats):
+        for tag, _, dt in arms:
+            ctx = torch.autocast("cuda", dtype=dt) if dt is not None else contextlib.nullcontext()
+
+            def fwd(m=models[tag], ctx=ctx):
+                with torch.no_grad(), ctx:
+                    m.forward_features(feats)
+            res[tag].append(timed(fwd, max(2, args.steps // 4), 2))
+    for tag, _, _ in arms:
+        emit({"part": "b", "what": "pixel-decoder forward_features, no autograd, 1024x2048, batch 8, Swin-T pyramid, "
+                                   "6 encoder layers", "arm": tag, "ms": min(res[tag]), "ms_all_repeats": res[tag]})
+
+
+def part_c(pkg, args, emit):
+    feats = _feats(16, 512, 1024, 2)
+    arms = [("fp32 fused tf32x3", dict(fused=True, linear="tf32x3", amp=False), None),
+            ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16),
+            ("amp fp16 + GradScaler", dict(fused=True, linear="torch", amp=True), torch.float16)]
+    for tag, kw, dt in arms:
+        m = _decoder(pkg, train=True, **kw)
+        opt = torch.optim.AdamW(m.parameters(), lr=1e-4)
+        scaler = torch.amp.GradScaler("cuda") if dt == torch.float16 else None
+        ctx = (lambda: torch.autocast("cuda", dtype=dt)) if dt is not None else contextlib.nullcontext
+
+        def step():
+            opt.zero_grad(set_to_none=True)
+            with ctx():
+                mask, low, multi = m.forward_features(feats)
+                loss = sum(o.float().square().mean() for o in (mask, low, *multi))
+            if scaler is None:
+                loss.backward()
+                opt.step()
+            else:
+                scaler.scale(loss).backward()
+                scaler.step(opt)
+                scaler.update()
+        ms = timed(step, args.steps // 2, args.warmup)
+        emit({"part": "c", "what": "pixel-decoder training step (forward_features + loss + backward + AdamW), "
+                                   "512x1024, batch 16, Swin-T pyramid, 6 encoder layers", "arm": tag, "ms": ms,
+              "images_per_s": 16 / ms * 1e3, "peak_mem_gib": torch.cuda.max_memory_allocated() / 2 ** 30})
+        del m, opt
+        torch.cuda.empty_cache()
+        torch.cuda.reset_peak_memory_stats()
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--parts", default="a,b,c")
+    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dtypes", default="fp32,bf16,fp16", help="part (a): element types of value")
+    ap.add_argument("--ops", default="forward,backward,fwd+bwd", help="part (a): calls timed")
+    ap.add_argument("--label", default="", help="part (a): recorded in every line (e.g. the library build)")
+    ap.add_argument("--repeats", type=int, default=3, help="part (b): alternating repeats of each arm (min reported)")
+    ap.add_argument("--out", default=os.path.join(os.environ.get("BENCH_OUT") or os.path.join(ROOT, "bench_out"),
+                                                  "mixed"))
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        sys.exit("bench_mixed.py measures on a CUDA device; none is available")
+    pkg = load_package()
+    os.makedirs(args.out, exist_ok=True)
+    info = card()
+    path = os.path.join(args.out, "mixed.jsonl")
+
+    def emit(rec):
+        rec = {**info, **rec}
+        print(json.dumps(rec), flush=True)
+        with open(path, "a") as f:
+            f.write(json.dumps(rec) + "\n")
+    for part in args.parts.split(","):
+        {"a": part_a, "b": part_b, "c": part_c}[part](pkg, args, emit)
+
+
+if __name__ == "__main__":
+    main()

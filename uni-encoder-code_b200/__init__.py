@@ -7,6 +7,7 @@ is missing -- there is no CPU or PyTorch fallback anywhere in the package.
 Public surface (names mirror the reference, see INTEGRATION.md):
     ms_deform_attn_forward / ms_deform_attn_backward   (ops/src/vision.cpp:18-21)
     MSDeformAttnFunction                               (ops/functions/ms_deform_attn_func.py:35-52)
+    MSDeformAttnMixedFunction -- the same op for bf16 / fp16 value rows (torch.autocast)
     install_dropin()  -- makes ``import MultiScaleDeformableAttention`` resolve to the shim
 """
 from __future__ import annotations
@@ -17,9 +18,10 @@ import sys
 from . import _lib
 from ._lib import get_option, launch_count, set_option
 from .functions import (AddLayerNormFunction, GroupNormFunction, GroupNormRowsFunction, LinearTF32x3Function,
-                        MSDeformAttnFunction, MSDeformAttnFusedFunction)
+                        MSDeformAttnFunction, MSDeformAttnFusedFunction, MSDeformAttnMixedFunction)
 from .ops import (add_layernorm, debug_indices, group_norm, linear_tf32x3, ms_deform_attn_backward, ms_deform_attn_forward,
-                  ms_deform_attn_fused_backward, ms_deform_attn_fused_forward)
+                  ms_deform_attn_fused_backward, ms_deform_attn_fused_forward, ms_deform_attn_mixed_backward,
+                  ms_deform_attn_mixed_forward)
 from . import synthetic
 from . import modules, pixel_decoder, sharding
 
@@ -27,6 +29,7 @@ __all__ = [
     "ms_deform_attn_forward", "ms_deform_attn_backward", "MSDeformAttnFunction", "debug_indices",
     "ms_deform_attn_fused_forward", "ms_deform_attn_fused_backward", "MSDeformAttnFusedFunction", "linear_tf32x3", "add_layernorm", "group_norm", "LinearTF32x3Function", "AddLayerNormFunction",
     "GroupNormFunction", "GroupNormRowsFunction",
+    "ms_deform_attn_mixed_forward", "ms_deform_attn_mixed_backward", "MSDeformAttnMixedFunction",
     "install_dropin", "set_option", "get_option", "launch_count", "synthetic", "modules", "pixel_decoder", "sharding",
 ]
 

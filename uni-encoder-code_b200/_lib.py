@@ -29,6 +29,12 @@ SYMBOLS = {
     "msda_b200_backward_deterministic_workspace_bytes": (ctypes.c_longlong, _DIMS + [_I]),
     "msda_b200_backward_deterministic_f32": (_I, [_P] * 6 + _DIMS + [_P, _P, _P, _P, _P]),
     "msda_b200_backward_deterministic_f64": (_I, [_P] * 6 + _DIMS + [_P, _P, _P, _P, _P]),
+    "msda_b200_forward_bf16": (_I, [_P] * 5 + _DIMS + [_P, _P]),
+    "msda_b200_forward_f16": (_I, [_P] * 5 + _DIMS + [_P, _P]),
+    "msda_b200_backward_bf16": (_I, [_P] * 6 + _DIMS + [_P] * 5),
+    "msda_b200_backward_f16": (_I, [_P] * 6 + _DIMS + [_P] * 5),
+    "msda_b200_backward_deterministic_bf16": (_I, [_P] * 6 + _DIMS + [_P] * 5),
+    "msda_b200_backward_deterministic_f16": (_I, [_P] * 6 + _DIMS + [_P] * 5),
     "msda_b200_debug_indices_f32": (_I, [_P] * 3 + _DIMS + [_P, _P, _P]),
     "msda_b200_fused_forward_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P, _P]),
     "msda_b200_fused_forward_strided_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _P, _I, _P, _I, _P, _P] + _DIMS + [_P, _P]),

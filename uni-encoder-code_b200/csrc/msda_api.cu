@@ -7,7 +7,8 @@
 //
 // The plain and the fused-producer MSDA entries differ only in the Producers they hand to the
 // launchers (reference points == nullptr: plain), so each backward has one body for both:
-// backward_f32() (kernel choice and "bwd_variant") and backward_deterministic().  Entries that
+// backward() (kernel choice and "bwd_variant") and backward_deterministic().  The fp32 and the mixed-precision
+// (bf16 / fp16 value) entries share the same bodies, templates over the value type.  Entries that
 // come as a default and a deterministic / training twin forward to one static body each.
 #include <atomic>
 #include <cstdint>
@@ -18,25 +19,32 @@
 
 namespace msda {
 
-// implemented in the kernel translation units
-cudaError_t launch_fwd_d32(const float *, const int64_t *, const int64_t *, const float *, const float *,
-                           const Producers &, const Dims &, float *, cudaStream_t, bool *handled);
-cudaError_t launch_bwd_d32(const float *, const float *, const int64_t *, const int64_t *, const float *,
+// implemented in the kernel translation units.  V: element type of value / output / grad_output (float, or
+// __nv_bfloat16 / __half for the mixed-precision entries); T: of the locations, weights and sums
+template <typename V>
+cudaError_t launch_fwd_d32(const V *, const int64_t *, const int64_t *, const float *, const float *,
+                           const Producers &, const Dims &, V *, cudaStream_t, bool *handled);
+template <typename V>
+cudaError_t launch_bwd_d32(const V *, const V *, const int64_t *, const int64_t *, const float *,
                            const float *, const Producers &, const Dims &, float *, float *, float *,
                            const DetRecords *, int gate, cudaStream_t, bool *handled);
-cudaError_t launch_bwd_sorted(const float *, const float *, const int64_t *, const int64_t *, const float *,
+template <typename V>
+cudaError_t launch_bwd_sorted(const V *, const V *, const int64_t *, const int64_t *, const float *,
                               const float *, const Producers &, const Dims &, float *, float *, float *, int gate,
                               cudaStream_t, bool *handled);
-bool bwd_sorted_applies(const float *value, const float *grad_value, const Dims &);
-template <typename T>
-cudaError_t launch_bwd_generic_records(const T *, const T *, const int64_t *, const int64_t *, const T *, const T *,
+template <typename V>
+bool bwd_sorted_applies(const V *value, const float *grad_value, const Dims &);
+template <typename V, typename T>
+cudaError_t launch_bwd_generic_records(const V *, const V *, const int64_t *, const int64_t *, const T *, const T *,
                                        const Dims &, T *, T *, const DetRecords &, cudaStream_t);
-template <typename T>
-cudaError_t launch_fwd_generic(const T *, const int64_t *, const int64_t *, const T *, const T *,
-                               const Dims &, T *, cudaStream_t);
-template <typename T>
-cudaError_t launch_bwd_generic(const T *, const T *, const int64_t *, const int64_t *, const T *,
+template <typename V, typename T>
+cudaError_t launch_fwd_generic(const V *, const int64_t *, const int64_t *, const T *, const T *,
+                               const Dims &, V *, cudaStream_t);
+template <typename V, typename T>
+cudaError_t launch_bwd_generic(const V *, const V *, const int64_t *, const int64_t *, const T *,
                                const T *, const Dims &, T *, T *, T *, cudaStream_t);
+template <typename V>
+cudaError_t launch_narrow(const float *, V *, long long, cudaStream_t);
 cudaError_t launch_linear_tf32x3(const float *, const float *, const float *, float *, int, int, int, int,
                                  float *, cudaStream_t, bool *handled, bool deterministic);
 cudaError_t launch_split_weight(const float *, float *, int, int, cudaStream_t, bool *handled);
@@ -121,19 +129,38 @@ static int option_index(const char *name) {
     return -1;
 }
 
-// The fp32 backward, plain (pr.ref == nullptr: `loc` / `attw` are the sampling locations and attention weights)
-// or fused (`loc` / `attw` are the raw sampling offsets and attention logits, and the gradients are taken with
-// respect to them).  Where no 32-channel kernel covers the problem (shape, or a view that is not aligned) the plain
-// op takes the generic kernel and the fused one returns MSDA_ERR_UNSUPPORTED.  "bwd_variant":
+// The forward of fp32 (V = float) and of the mixed-precision op (16-bit V, fp32 locations and weights): the
+// 32-channel kernel where it applies, the generic one otherwise.
+template <typename V>
+static int forward(const V *value, const int64_t *shapes, const int64_t *lstart, const float *loc,
+                   const float *attw, const Dims &d, V *output, cudaStream_t st) {
+    if (!value || !shapes || !lstart || !loc || !attw || !output) return MSDA_ERR_NULL_POINTER;
+    if (int rc = check_dims(d)) return rc;
+    bool handled = false;
+    cudaError_t e = cudaSuccess;
+    const bool fast_ok = aligned16(value) && aligned16(output) && aligned8(loc);
+    if (option_value(OPT_FWD_VARIANT) != 63 && fast_ok)   // 63 forces the generic kernel (tests)
+        e = launch_fwd_d32<V>(value, shapes, lstart, loc, attw, Producers{}, d, output, st, &handled);
+    if (e == cudaSuccess && !handled) e = launch_fwd_generic<V, float>(value, shapes, lstart, loc, attw, d, output, st);
+    return (int)e;
+}
+
+// The backward of fp32 (V = float) and of the mixed-precision op (16-bit V: `gv` is the caller's zero-filled fp32
+// accumulation buffer, rounded into the 16-bit grad_value by the entry afterwards), plain (pr.ref == nullptr: `loc`
+// / `attw` are the sampling locations and attention weights) or fused, fp32 only (`loc` / `attw` are the raw
+// sampling offsets and attention logits, and the gradients are taken with respect to them).  Where no 32-channel
+// kernel covers the problem (shape, or a view that is not aligned) the plain op takes the generic kernel and the
+// fused one returns MSDA_ERR_UNSUPPORTED.  "bwd_variant":
 //   0 (default): where the queries are the value pixels (encoder self-attention) the in-SM merging kernel (points
 //       near their query) and the per-row reduction kernel (points anywhere) are both launched; every CTA of both
 //       runs the same probe of the sampling locations first and the kernel the verdict goes against returns at
 //       once (msda_common.cuh);
 //   20..39: merging kernel forced (plain: and its tuning variants); 1..8: CTA shapes of the plain per-row kernel;
-//   63: generic kernel (plain only, tests)
-static int backward_f32(const float *grad_output, const float *value, const int64_t *shapes, const int64_t *lstart,
-                        const float *loc, const float *attw, const Producers &pr, const Dims &d, float *gv,
-                        float *gl, float *gw, cudaStream_t st) {
+//   63: generic kernel (plain only, tests).  16-bit V takes the same meanings, each kernel in its default shape.
+template <typename V>
+static int backward(const V *grad_output, const V *value, const int64_t *shapes, const int64_t *lstart,
+                    const float *loc, const float *attw, const Producers &pr, const Dims &d, float *gv,
+                    float *gl, float *gw, cudaStream_t st) {
     if (!grad_output || !value || !shapes || !lstart || !loc || !attw || !gv || !gl || !gw)
         return MSDA_ERR_NULL_POINTER;
     if (int rc = check_dims(d, pr.ref_bstride)) return rc;
@@ -145,8 +172,8 @@ static int backward_f32(const float *grad_output, const float *value, const int6
     cudaError_t e = cudaSuccess;
     if (aligned && (fused || variant != 63)) {
         int gate = GATE_NONE;
-        if ((variant == 0 || (variant >= 20 && variant < 40)) && bwd_sorted_applies(value, gv, d)) {
-            e = launch_bwd_sorted(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw,
+        if ((variant == 0 || (variant >= 20 && variant < 40)) && bwd_sorted_applies<V>(value, gv, d)) {
+            e = launch_bwd_sorted<V>(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw,
                                   variant == 0 ? GATE_RUN_IF_LOCAL : GATE_NONE, st, &handled);
             if (variant == 0) {                  // the per-row kernel follows, gated the other way
                 handled = false;
@@ -154,18 +181,32 @@ static int backward_f32(const float *grad_output, const float *value, const int6
             }
         }
         if (e == cudaSuccess && !handled)
-            e = launch_bwd_d32(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, nullptr, gate, st,
-                               &handled);
+            e = launch_bwd_d32<V>(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, nullptr, gate, st,
+                                  &handled);
     }
     if (e != cudaSuccess || handled || fused) return launch_rc(e, handled);
-    return (int)launch_bwd_generic<float>(grad_output, value, shapes, lstart, loc, attw, d, gv, gl, gw, st);
+    return (int)launch_bwd_generic<V, float>(grad_output, value, shapes, lstart, loc, attw, d, gv, gl, gw, st);
 }
 
-// Deterministic backward (msda_det.cu), plain or fused as in backward_f32 (fp64: plain only): the records kernel
-// of the path, then sort, bounds and gather into grad_value.
-template <typename T>
-static int backward_deterministic(const T *grad_output, const T *value, const int64_t *shapes, const int64_t *lstart,
-                                  const T *loc, const T *attw, const Producers &pr, const Dims &d, T *gv, T *gl,
+// The mixed-precision backward: backward() into the fp32 accumulation buffer `acc`, then the conversion into the
+// 16-bit grad_value
+template <typename V>
+static int backward_mixed(const V *grad_output, const V *value, const int64_t *shapes, const int64_t *lstart,
+                          const float *loc, const float *attw, const Dims &d, float *acc, V *gv, float *gl, float *gw,
+                          cudaStream_t st) {
+    if (!gv) return MSDA_ERR_NULL_POINTER;
+    const int rc = backward<V>(grad_output, value, shapes, lstart, loc, attw, Producers{}, d, acc, gl, gw, st);
+    if (rc != MSDA_OK) return rc;
+    return (int)launch_narrow<V>(acc, gv, (long long)d.N * d.S * d.M * d.D, st);
+}
+
+// Deterministic backward (msda_det.cu), plain or fused as in backward() (fp64 and 16-bit: plain only): the records
+// kernel of the path, then sort, bounds and gather into grad_value.  V: element type of value / grad_output /
+// grad_value, T: of the locations, weights, records and sums (16-bit V: float; the gather writes the 16-bit
+// grad_value directly, no accumulation buffer).
+template <typename V, typename T>
+static int backward_deterministic(const V *grad_output, const V *value, const int64_t *shapes, const int64_t *lstart,
+                                  const T *loc, const T *attw, const Producers &pr, const Dims &d, V *gv, T *gl,
                                   T *gw, void *workspace, cudaStream_t st) {
     if (!grad_output || !value || !shapes || !lstart || !loc || !attw || !gv || !gl || !gw || !workspace)
         return MSDA_ERR_NULL_POINTER;
@@ -176,18 +217,18 @@ static int backward_deterministic(const T *grad_output, const T *value, const in
     const DetRecords rec = det_records(workspace, l);
     bool handled = false;
     cudaError_t e = cudaSuccess;
-    if constexpr (sizeof(T) == 4) {
+    if constexpr (std::is_same<T, float>::value) {
         const bool aligned = aligned16(value) && aligned16(grad_output) && aligned8(loc) && aligned8(gl) &&
                              aligned8(pr.ref);
         if (aligned && (pr.ref != nullptr || option_value(OPT_BWD_VARIANT) != 63))
-            e = launch_bwd_d32(grad_output, value, shapes, lstart, loc, attw, pr, d, nullptr, gl, gw, &rec,
+            e = launch_bwd_d32<V>(grad_output, value, shapes, lstart, loc, attw, pr, d, nullptr, gl, gw, &rec,
                                GATE_NONE, st, &handled);
     }
     if (e == cudaSuccess && !handled) {
         if (pr.ref != nullptr) return MSDA_ERR_UNSUPPORTED;
-        e = launch_bwd_generic_records<T>(grad_output, value, shapes, lstart, loc, attw, d, gl, gw, rec, st);
+        e = launch_bwd_generic_records<V, T>(grad_output, value, shapes, lstart, loc, attw, d, gl, gw, rec, st);
     }
-    if (e == cudaSuccess) e = launch_det_reduce<T>(l, workspace, grad_output, gv, d, st);
+    if (e == cudaSuccess) e = launch_det_reduce<V, T>(l, workspace, grad_output, gv, d, st);
     return (int)e;
 }
 
@@ -307,21 +348,9 @@ int msda_b200_forward_f32(const float *value, const int64_t *spatial_shapes,
                           const float *attn_weight, int batch, int spatial_size, int num_heads,
                           int channels, int num_levels, int num_query, int num_point, float *output,
                           void *stream) {
-    if (!value || !spatial_shapes || !level_start || !sampling_loc || !attn_weight || !output)
-        return MSDA_ERR_NULL_POINTER;
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    if (int rc = check_dims(d)) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    bool handled = false;
-    cudaError_t e = cudaSuccess;
-    const bool fast_ok = aligned16(value) && aligned16(output) && aligned8(sampling_loc);
-    if (option_value(OPT_FWD_VARIANT) != 63 && fast_ok)   // 63 forces the generic kernel (tests)
-        e = launch_fwd_d32(value, spatial_shapes, level_start, sampling_loc, attn_weight, Producers{}, d, output, st,
-                           &handled);
-    if (e == cudaSuccess && !handled)
-        e = launch_fwd_generic<float>(value, spatial_shapes, level_start, sampling_loc, attn_weight, d,
-                                      output, st);
-    return (int)e;
+    return forward<float>(value, spatial_shapes, level_start, sampling_loc, attn_weight, d, output,
+                          (cudaStream_t)stream);
 }
 
 int msda_b200_forward_f64(const double *value, const int64_t *spatial_shapes,
@@ -333,7 +362,7 @@ int msda_b200_forward_f64(const double *value, const int64_t *spatial_shapes,
         return MSDA_ERR_NULL_POINTER;
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
     if (int rc = check_dims(d)) return rc;
-    return (int)launch_fwd_generic<double>(value, spatial_shapes, level_start, sampling_loc,
+    return (int)launch_fwd_generic<double, double>(value, spatial_shapes, level_start, sampling_loc,
                                            attn_weight, d, output, (cudaStream_t)stream);
 }
 
@@ -344,8 +373,8 @@ int msda_b200_backward_f32(const float *grad_output, const float *value,
                            int num_query, int num_point, float *grad_value,
                            float *grad_sampling_loc, float *grad_attn_weight, void *stream) {
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    return backward_f32(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight, Producers{}, d,
-                        grad_value, grad_sampling_loc, grad_attn_weight, (cudaStream_t)stream);
+    return backward<float>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight, Producers{}, d,
+                           grad_value, grad_sampling_loc, grad_attn_weight, (cudaStream_t)stream);
 }
 
 int msda_b200_backward_f64(const double *grad_output, const double *value,
@@ -359,7 +388,7 @@ int msda_b200_backward_f64(const double *grad_output, const double *value,
         return MSDA_ERR_NULL_POINTER;
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
     if (int rc = check_dims(d)) return rc;
-    return (int)launch_bwd_generic<double>(grad_output, value, spatial_shapes, level_start,
+    return (int)launch_bwd_generic<double, double>(grad_output, value, spatial_shapes, level_start,
                                            sampling_loc, attn_weight, d, grad_value,
                                            grad_sampling_loc, grad_attn_weight, (cudaStream_t)stream);
 }
@@ -417,9 +446,9 @@ int msda_b200_fused_backward_f32(const float *grad_output, const float *value,
                                  float *grad_sampling_offsets, float *grad_attn_logits, void *stream) {
     if (!reference_points) return MSDA_ERR_NULL_POINTER;      // (it selects the fused form)
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    return backward_f32(grad_output, value, spatial_shapes, level_start, sampling_offsets, attn_logits,
-                        Producers{reference_points, ref_batch_stride}, d, grad_value, grad_sampling_offsets,
-                        grad_attn_logits, (cudaStream_t)stream);
+    return backward<float>(grad_output, value, spatial_shapes, level_start, sampling_offsets, attn_logits,
+                           Producers{reference_points, ref_batch_stride}, d, grad_value, grad_sampling_offsets,
+                           grad_attn_logits, (cudaStream_t)stream);
 }
 
 long long msda_b200_backward_deterministic_workspace_bytes(int batch, int spatial_size, int num_heads, int channels,
@@ -427,7 +456,10 @@ long long msda_b200_backward_deterministic_workspace_bytes(int batch, int spatia
                                                           int value_bytes) {
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
     DetLayout l;
-    if (check_dims(d) != MSDA_OK || (value_bytes != 4 && value_bytes != 8) || !det_layout(d, value_bytes, &l)) return 0;
+    // 16-bit value (2 bytes): the records carry fp32 weights
+    if (check_dims(d) != MSDA_OK || (value_bytes != 2 && value_bytes != 4 && value_bytes != 8) ||
+        !det_layout(d, value_bytes == 2 ? 4 : value_bytes, &l))
+        return 0;
     return (long long)l.total;
 }
 
@@ -439,7 +471,7 @@ int msda_b200_backward_deterministic_f32(const float *grad_output, const float *
                                          float *grad_sampling_loc, float *grad_attn_weight, void *workspace,
                                          void *stream) {
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    return backward_deterministic<float>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
+    return backward_deterministic<float, float>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
                                          Producers{}, d, grad_value, grad_sampling_loc, grad_attn_weight, workspace,
                                          (cudaStream_t)stream);
 }
@@ -452,7 +484,7 @@ int msda_b200_backward_deterministic_f64(const double *grad_output, const double
                                          double *grad_sampling_loc, double *grad_attn_weight, void *workspace,
                                          void *stream) {
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    return backward_deterministic<double>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
+    return backward_deterministic<double, double>(grad_output, value, spatial_shapes, level_start, sampling_loc, attn_weight,
                                           Producers{}, d, grad_value, grad_sampling_loc, grad_attn_weight, workspace,
                                           (cudaStream_t)stream);
 }
@@ -467,10 +499,48 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
                                                void *workspace, void *stream) {
     if (!reference_points) return MSDA_ERR_NULL_POINTER;      // (it selects the fused form)
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    return backward_deterministic<float>(grad_output, value, spatial_shapes, level_start, sampling_offsets,
+    return backward_deterministic<float, float>(grad_output, value, spatial_shapes, level_start, sampling_offsets,
                                          attn_logits, Producers{reference_points, ref_batch_stride}, d, grad_value,
                                          grad_sampling_offsets, grad_attn_logits, workspace, (cudaStream_t)stream);
 }
+
+// ---- mixed precision: bf16 / fp16 value, output, grad_output and grad_value; fp32 locations, weights and their
+// gradients; fp32 sums ----
+#define MSDA_MIXED_ENTRIES(SUFFIX, V)                                                                                \
+    int msda_b200_forward_##SUFFIX(const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start,  \
+                                   const float *sampling_loc, const float *attn_weight, int batch, int spatial_size,  \
+                                   int num_heads, int channels, int num_levels, int num_query, int num_point,        \
+                                   uint16_t *output, void *stream) {                                                \
+        const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};                    \
+        return forward<V>(reinterpret_cast<const V *>(value), spatial_shapes, level_start, sampling_loc, attn_weight, \
+                          d, reinterpret_cast<V *>(output), (cudaStream_t)stream);                                   \
+    }                                                                                                                \
+    int msda_b200_backward_##SUFFIX(const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes, \
+                                    const int64_t *level_start, const float *sampling_loc, const float *attn_weight, \
+                                    int batch, int spatial_size, int num_heads, int channels, int num_levels,        \
+                                    int num_query, int num_point, float *grad_value_accum, uint16_t *grad_value,     \
+                                    float *grad_sampling_loc, float *grad_attn_weight, void *stream) {               \
+        const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};                    \
+        return backward_mixed<V>(reinterpret_cast<const V *>(grad_output), reinterpret_cast<const V *>(value),       \
+                                 spatial_shapes, level_start, sampling_loc, attn_weight, d, grad_value_accum,        \
+                                 reinterpret_cast<V *>(grad_value), grad_sampling_loc, grad_attn_weight,             \
+                                 (cudaStream_t)stream);                                                              \
+    }                                                                                                                \
+    int msda_b200_backward_deterministic_##SUFFIX(                                                                   \
+        const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start, \
+        const float *sampling_loc, const float *attn_weight, int batch, int spatial_size, int num_heads, int channels, \
+        int num_levels, int num_query, int num_point, uint16_t *grad_value, float *grad_sampling_loc,                \
+        float *grad_attn_weight, void *workspace, void *stream) {                                                   \
+        const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};                    \
+        return backward_deterministic<V, float>(reinterpret_cast<const V *>(grad_output),                           \
+                                                reinterpret_cast<const V *>(value), spatial_shapes, level_start,     \
+                                                sampling_loc, attn_weight, Producers{}, d,                           \
+                                                reinterpret_cast<V *>(grad_value), grad_sampling_loc,                \
+                                                grad_attn_weight, workspace, (cudaStream_t)stream);                  \
+    }
+MSDA_MIXED_ENTRIES(bf16, __nv_bfloat16)
+MSDA_MIXED_ENTRIES(f16, __half)
+#undef MSDA_MIXED_ENTRIES
 
 int msda_b200_linear_f32(const float *x, const float *weight, const float *bias, float *y, int rows,
                          int out_features, int in_features, int relu, float *workspace, void *stream) {

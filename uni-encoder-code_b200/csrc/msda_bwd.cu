@@ -1,4 +1,5 @@
-// msda_bwd.cu -- backward MSDA kernel for sm_100a, 32 fp32 channels per head.
+// msda_bwd.cu -- backward MSDA kernel for sm_100a, 32 channels per head (fp32 value rows, or bf16 / fp16
+// ones with fp32 locations, weights, sums and grad_value accumulation).
 //
 // Replaces the reference's col2im kernel that is hit at D = 32,
 // ms_deformable_col2im_gpu_kernel_shm_blocksize_aware_reduce_v1<T,32>
@@ -58,9 +59,11 @@ struct BwdCfg {
 // FUSED: `loc` / `attw` are the raw sampling offsets / attention logits and `grad_loc` / `grad_attw`
 // receive the gradients with respect to THEM (offset gradient = location gradient / (W, H);
 // softmax backward folded in), see phase1_records() in msda_common.cuh.
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED, bool RECORDS>
+// V: element type of grad_out / value (16-bit: 8-byte lane loads widened to fp32); grad_value is fp32 either way --
+// for 16-bit V the zero-filled accumulation buffer that msda_api.cu rounds into the 16-bit grad_value afterwards
+template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED, bool RECORDS>
 __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
-msda_bwd_d32_kernel(const float *__restrict__ grad_out, const float *__restrict__ value,
+msda_bwd_d32_kernel(const V *__restrict__ grad_out, const V *__restrict__ value,
                     const int64_t *__restrict__ shapes, const int64_t *__restrict__ lstart,
                     const float *__restrict__ loc, const float *__restrict__ attw,
                     const Producers pr, const Dims d, const int flags,
@@ -109,12 +112,12 @@ msda_bwd_d32_kernel(const float *__restrict__ grad_out, const float *__restrict_
 
         // ---- phase 2 ----
         const long long img = n * (long long)d.S * M * 8 + chunk;
-        const float4 *vb = reinterpret_cast<const float4 *>(value) + img;
+        const V *vb = value + img * 4;
         float4 *gvb = reinterpret_cast<float4 *>(grad_value) + img;
         const uint4 *plane = reinterpret_cast<const uint4 *>(rec + corner * Cfg::kPlane);
         for (int qi = 0; qi < cnt; ++qi) {
             const long long qrow = (n * d.Lq + q0 + qi) * M + m;
-            const float4 go = ldg_stream_f4(reinterpret_cast<const float4 *>(grad_out) + qrow * 8 + chunk);
+            const float4 go = ldg_stream_v4(grad_out + (qrow * 8 + chunk) * 4);
             const uint4 *rq = plane + qi * Cfg::kPairs;
             // RECORDS: this query-head's first slot, and the first grad_value row of image n
             const uint32_t slot0 = (uint32_t)qrow * (uint32_t)(LP * 4) + (uint32_t)corner;
@@ -131,8 +134,8 @@ msda_bwd_d32_kernel(const float *__restrict__ grad_out, const float *__restrict_
 #pragma unroll
                 for (int j = 0; j < kB; ++j) {                  // 2*BATCH independent loads in flight
                     if (pb + j < Cfg::kPairs) {
-                        va[j] = ldg_keep_f4_if(vb, e[j].x);
-                        vc[j] = ldg_keep_f4_if(vb, e[j].z);
+                        va[j] = ldg_keep_v4_if(vb, e[j].x);
+                        vc[j] = ldg_keep_v4_if(vb, e[j].z);
                     }
                 }
 #pragma unroll
@@ -261,13 +264,13 @@ msda_bwd_d32_kernel(const float *__restrict__ grad_out, const float *__restrict_
 // host side: launch_bwd_d32() serves the plain op, the fused producers (Producers::ref set) and
 // the deterministic records (msda_det.cu), the last two in the default CTA shape only
 // ---------------------------------------------------------------------------
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED, bool RECORDS>
-static cudaError_t launch_bwd_cfg(const float *grad_out, const float *value, const int64_t *shapes,
+template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED, bool RECORDS>
+static cudaError_t launch_bwd_cfg(const V *grad_out, const V *value, const int64_t *shapes,
                                   const int64_t *lstart, const float *loc, const float *attw, const Producers &pr,
                                   const Dims &d, float *grad_value, float *grad_loc, float *grad_attw,
                                   const DetRecords &det, int gate, cudaStream_t stream) {
     using Cfg = BwdCfg<LP, WARPS, TILE_W, QPW>;
-    constexpr auto kern = msda_bwd_d32_kernel<LP, WARPS, TILE_W, MIN_CTAS, BATCH, QPW, FUSED, RECORDS>;
+    constexpr auto kern = msda_bwd_d32_kernel<V, LP, WARPS, TILE_W, MIN_CTAS, BATCH, QPW, FUSED, RECORDS>;
     cudaError_t e;
     const int blocks = persistent_blocks<kern>(WARPS * 32, Cfg::kSmem, d, &e);
     if (blocks == 0) return e;
@@ -278,17 +281,20 @@ static cudaError_t launch_bwd_cfg(const float *grad_out, const float *value, con
     return cudaGetLastError();
 }
 
-template <int LP>
-static cudaError_t launch_bwd_lp(const float *grad_out, const float *value, const int64_t *shapes,
+template <typename V, int LP>
+static cudaError_t launch_bwd_lp(const V *grad_out, const V *value, const int64_t *shapes,
                                  const int64_t *lstart, const float *loc, const float *attw, const Producers &pr,
                                  const Dims &d, float *gv, float *gl, float *gw, const DetRecords *det, int gate,
                                  cudaStream_t st) {
     // variant = (warps, query tile width, min CTAs per SM -> register budget, load batch in pairs,
     //            queries per warp)
 #define MSDA_BWD(W, TW, C, B, Q, F, R) \
-    launch_bwd_cfg<LP, W, TW, C, B, Q, F, R>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, \
+    launch_bwd_cfg<V, LP, W, TW, C, B, Q, F, R>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, \
                                              R ? *det : DetRecords{}, gate, st)
-    // fused producers and the deterministic records: the default shape only
+    // 16-bit (plain only), fused producers and the deterministic records: the default shape only
+    if constexpr (is16<V>) {
+        return det != nullptr ? MSDA_BWD(16, 16, 2, 1, 8, false, true) : MSDA_BWD(16, 16, 2, 1, 8, false, false);
+    } else {
     if (det != nullptr)
         return pr.ref != nullptr ? MSDA_BWD(16, 16, 2, 1, 8, true, true) : MSDA_BWD(16, 16, 2, 1, 8, false, true);
     if (pr.ref != nullptr) return MSDA_BWD(16, 16, 2, 1, 8, true, false);
@@ -303,6 +309,7 @@ static cudaError_t launch_bwd_lp(const float *grad_out, const float *value, cons
         case 2:
         default: return MSDA_BWD(16, 16, 2, 1, 8, false, false);  // 16 warps, tile  8x16, 8 queries per warp (147 KB smem per SM)
     }
+    }
 #undef MSDA_BWD
 }
 
@@ -310,17 +317,27 @@ static cudaError_t launch_bwd_lp(const float *grad_out, const float *value, cons
 // attention logits (`attw`).  det != nullptr: deterministic mode (msda_det.cu), grad_value `gv` is not touched and
 // the corner records go to `det`.  `gate`: see msda_bwd_sorted.cu.  `handled` = false: the problem is outside
 // d32_applies() and nothing was launched.
-cudaError_t launch_bwd_d32(const float *grad_out, const float *value, const int64_t *shapes, const int64_t *lstart,
+template <typename V>
+cudaError_t launch_bwd_d32(const V *grad_out, const V *value, const int64_t *shapes, const int64_t *lstart,
                            const float *loc, const float *attw, const Producers &pr, const Dims &d, float *gv,
                            float *gl, float *gw, const DetRecords *det, int gate, cudaStream_t st, bool *handled) {
     *handled = d32_applies(d);
     if (!*handled) return cudaSuccess;
     switch (d.L * d.P) {       // 4, 8, 12 or 16 (d32_applies)
-        case 4: return launch_bwd_lp<4>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
-        case 8: return launch_bwd_lp<8>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
-        case 12: return launch_bwd_lp<12>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
-        default: return launch_bwd_lp<16>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        case 4: return launch_bwd_lp<V, 4>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        case 8: return launch_bwd_lp<V, 8>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        case 12: return launch_bwd_lp<V, 12>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        default: return launch_bwd_lp<V, 16>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
     }
 }
+
+#define MSDA_BWD_D32(V)                                                                                             \
+    template cudaError_t launch_bwd_d32<V>(const V *, const V *, const int64_t *, const int64_t *, const float *,    \
+                                           const float *, const Producers &, const Dims &, float *, float *, float *, \
+                                           const DetRecords *, int, cudaStream_t, bool *);
+MSDA_BWD_D32(float)
+MSDA_BWD_D32(__nv_bfloat16)
+MSDA_BWD_D32(__half)
+#undef MSDA_BWD_D32
 
 }  // namespace msda

@@ -1,4 +1,5 @@
-// msda_bwd_sorted.cu -- backward MSDA kernel for sm_100a (32 fp32 channels per head) that merges
+// msda_bwd_sorted.cu -- backward MSDA kernel for sm_100a (32 channels per head; fp32 value rows, or bf16 / fp16
+// ones with fp32 sums and an fp32 grad_value accumulation buffer) that merges
 // the grad_value contributions of a query tile INSIDE the SM before anything is sent to L2.
 //
 // Replaces ms_deformable_col2im_gpu_kernel_shm_blocksize_aware_reduce_v1<T,32>
@@ -309,6 +310,23 @@ template <typename P>
 __device__ __forceinline__ P xor64(P p) {       // the other 64-byte half of a 128-byte aligned row
     return reinterpret_cast<P>(reinterpret_cast<uintptr_t>(p) ^ (uintptr_t)64);
 }
+// a lane's 4-channel chunk of a value row as two packed fp32 pairs (16-bit V: 8 bytes, widened)
+template <typename V>
+__device__ __forceinline__ void ldg_value_chunk(const char *p, uint64_t &x, uint64_t &y) {
+    if constexpr (!is16<V>) {
+        ldg_2x64(p, x, y);
+    } else {
+        uint2 u;
+        asm volatile("ld.global.nc.v2.u32 {%0,%1}, [%2];" : "=r"(u.x), "=r"(u.y) : "l"(p));
+        const float4 f = widen4<V>(u);
+        x = (uint64_t)__float_as_uint(f.x) | ((uint64_t)__float_as_uint(f.y) << 32);
+        y = (uint64_t)__float_as_uint(f.z) | ((uint64_t)__float_as_uint(f.w) << 32);
+    }
+}
+template <typename V>
+__device__ __forceinline__ const char *other_half(const char *p) {   // the chunk 4 chunks away in an aligned row
+    return reinterpret_cast<const char *>(reinterpret_cast<uintptr_t>(p) ^ (uintptr_t)(4 * kChunkBytes<V>));
+}
 __device__ __forceinline__ void sts_f1(uint32_t a, float v) {
     asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory");
 }
@@ -321,9 +339,12 @@ __device__ __forceinline__ void red_add_f4(float4 *p, const float4 v) {
 //      receive the gradients with respect to THEM (SURVEY 8f.1, as in msda_bwd.cu): pass A forms
 //      location = ref + offset / (W, H) and the softmax of the (query, head)'s L*P logits (exchanged
 //      through shared memory), the epilogue applies 1 / (W, H) and the softmax backward.
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int TILE_Q, int SLOTS, int GW, bool FUSED>
+// V: element type of grad_out / value.  16-bit: the grad_output tile is widened to fp32 while it is staged (the merge
+// loop reads it as for fp32), a lane's value chunk is 8 bytes of a 64-byte row, and grad_value is the fp32
+// accumulation buffer (128-byte rows, as for fp32)
+template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int TILE_Q, int SLOTS, int GW, bool FUSED>
 __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
-msda_bwd_sorted_kernel(const float *__restrict__ grad_out, const float *__restrict__ value,
+msda_bwd_sorted_kernel(const V *__restrict__ grad_out, const V *__restrict__ value,
                        const int64_t *__restrict__ shapes, const int64_t *__restrict__ lstart,
                        const float *__restrict__ loc, const float *__restrict__ attw, const Producers pr, const Dims d,
                        const int flags, float *__restrict__ grad_value, float *__restrict__ grad_loc,
@@ -377,7 +398,7 @@ msda_bwd_sorted_kernel(const float *__restrict__ grad_out, const float *__restri
         if (tid == 0) tail_ctr = 0u;
         // rows of image n: 64-bit bases here, 32-bit offsets (query * M + m) * {8, LP} below
         // (Lq * M * 16 < 2^32: host check)
-        const float4 *go_n = reinterpret_cast<const float4 *>(grad_out) + n * Lq * (long long)M * 8;
+        const V *go_n = grad_out + n * Lq * (long long)M * 32;
         const float2 *loc_n = reinterpret_cast<const float2 *>(loc) + n * Lq * (long long)M * LP;
         const float *attw_n = attw + n * Lq * (long long)M * LP;
 
@@ -390,14 +411,39 @@ msda_bwd_sorted_kernel(const float *__restrict__ grad_out, const float *__restri
             // asynchronous copies, waited for at the end of pass B; empty query slots are zero-filled ----
             {
                 const uint32_t go_dst = smem_u32(go_sm);
+                if constexpr (!is16<V>) {
 #pragma unroll
-                for (int i = tid; i < kSortTile * 8; i += NT) {
-                    const int qg = tile_query<TILE_W>(tm, i >> 3, Lq);
-                    const float4 *src = go_n + (qg >= 0 ? (uint32_t)(qg * M + m) * 8u + (uint32_t)(i & 7) : 0u);
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;"
-                                 ::"r"(go_dst + 16u * (uint32_t)i), "l"(src), "r"(qg >= 0 ? 16 : 0) : "memory");
+                    for (int i = tid; i < kSortTile * 8; i += NT) {
+                        const int qg = tile_query<TILE_W>(tm, i >> 3, Lq);
+                        const float4 *src = reinterpret_cast<const float4 *>(go_n) +
+                                            (qg >= 0 ? (uint32_t)(qg * M + m) * 8u + (uint32_t)(i & 7) : 0u);
+                        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;"
+                                     ::"r"(go_dst + 16u * (uint32_t)i), "l"(src), "r"(qg >= 0 ? 16 : 0) : "memory");
+                    }
+                    asm volatile("cp.async.commit_group;" ::: "memory");
+                } else {
+                    // 16-bit: widened while staging (synchronous: all loads issued before the first store).  Measured
+                    // faster than staging the 16-bit rows with cp.async (8 KB) and widening them in the merge loop:
+                    // bf16, merging kernel, 0.599 against 0.622 ms at configs[1], 2.44 against 2.58 ms at the
+                    // configs[2] shape (DESIGN.md section 11, profiles/r5_staging.jsonl)
+                    constexpr int kPer = (kSortTile * 8 + NT - 1) / NT;
+                    float4 gs[kPer];
+#pragma unroll
+                    for (int k = 0; k < kPer; ++k) {
+                        const int i = tid + k * NT;
+                        const int qg = i < kSortTile * 8 ? tile_query<TILE_W>(tm, i >> 3, Lq) : -1;
+                        gs[k] = qg >= 0 ? ldg_stream_v4(at_chunk(go_n, (uint32_t)(qg * M + m) * 8u + (uint32_t)(i & 7)))
+                                        : make_float4(0.f, 0.f, 0.f, 0.f);
+                    }
+#pragma unroll
+                    for (int k = 0; k < kPer; ++k) {
+                        const int i = tid + k * NT;
+                        if (i < kSortTile * 8)
+                            asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};"
+                                         ::"r"(go_dst + 16u * (uint32_t)i), "f"(gs[k].x), "f"(gs[k].y), "f"(gs[k].z),
+                                           "f"(gs[k].w) : "memory");
+                    }
                 }
-                asm volatile("cp.async.commit_group;" ::: "memory");
             }
 
             // ---- pass A: load the points, count the in-window corners per pixel ----
@@ -528,7 +574,7 @@ msda_bwd_sorted_kernel(const float *__restrict__ grad_out, const float *__restri
                     place_point(bn[r], cnt_s, rec_sa, &tail_ctr, n_in, lt.W[lt.level_of[p]],
                                 ((uint32_t)q << 7) | (uint32_t)(p * 4), d.S, Cfg::kRecs, Cfg::kPixShift);
             }
-            asm volatile("cp.async.wait_group 0;" ::: "memory");
+            if constexpr (!is16<V>) asm volatile("cp.async.wait_group 0;" ::: "memory");
         }
         __syncthreads();                                                    // B4: records + grad_output tile complete
 
@@ -558,15 +604,18 @@ msda_bwd_sorted_kernel(const float *__restrict__ grad_out, const float *__restri
             const int i0 = (gl * WARPS + warp) * per;
             for (int i = max(i0, T) + cl; i < i0 + per; i += GW) rec[i] = make_uint2(0xffffffffu, 0u);
             __syncwarp();
-            // value / grad_value row of pixel 0 for this lane: + key * (M * 128) bytes per pixel; the
-            // lane's second chunk is the same address ^ 64 (rows are 128-byte aligned: host check)
-            const size_t lane_off = ((size_t)(n * (long long)d.S * M + m) * 8 + c0) * 16;
-            const char *v_lane = reinterpret_cast<const char *>(value) + lane_off;
-            char *gv_lane = reinterpret_cast<char *>(grad_value) + lane_off;
+            // value / grad_value row of pixel 0 for this lane: + key * (M * 128) bytes per pixel (value rows:
+            // M * 64 for 16-bit V); the lane's second chunk is the same address ^ 64 (value: ^ half a row).  Rows are
+            // aligned to their size: host check
+            const size_t lane_chunk = (size_t)(n * (long long)d.S * M + m) * 8 + c0;
+            const char *v_lane = reinterpret_cast<const char *>(value) + lane_chunk * kChunkBytes<V>;
+            char *gv_lane = reinterpret_cast<char *>(grad_value) + lane_chunk * 16;
             uint32_t row_bytes = (uint32_t)M * 128u;
             // keep the two 64-bit lane bases and the row stride as they are in registers: ptxas otherwise
             // splits them into a uniform and a per-lane part and re-adds / reloads them at every run start
             asm volatile("" : "+l"(v_lane), "+l"(gv_lane), "+r"(row_bytes));
+            // value row stride: row_bytes for fp32, half of it for 16-bit V
+            constexpr int kVShift = is16<V> ? 1 : 0;
             float4 acc[NCH];                                          // one 16-byte chunk each: leaves as one red.v4
             uint64_t v[2 * NCH];                                      // channel pairs: packed fp32x2 math
 #pragma unroll
@@ -602,9 +651,9 @@ msda_bwd_sorted_kernel(const float *__restrict__ grad_out, const float *__restri
                             if (NCH == 2) red_add_f4(reinterpret_cast<float4 *>(xor64(p)), acc[NCH - 1]);
                         }
                         if (key != kNoKey) {
-                            const char *p = v_lane + (size_t)key * row_bytes;
-                            ldg_2x64(p, v[0], v[1]);
-                            if (NCH == 2) ldg_2x64(xor64(p), v[2], v[3]);
+                            const char *p = v_lane + (size_t)key * (row_bytes >> kVShift);
+                            ldg_value_chunk<V>(p, v[0], v[1]);
+                            if (NCH == 2) ldg_value_chunk<V>(other_half<V>(p), v[2], v[3]);
                         }
                         cur = key;
 #pragma unroll
@@ -758,13 +807,13 @@ msda_bwd_sorted_kernel(const float *__restrict__ grad_out, const float *__restri
 // host side: launch_bwd_sorted() serves the plain op and the fused producers (Producers::ref set),
 // the latter in the default shapes only
 // ---------------------------------------------------------------------------
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int TILE_Q, int SLOTS, int GW, bool FUSED>
-static cudaError_t launch_bwd_sorted_cfg(const float *grad_out, const float *value, const int64_t *shapes,
+template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int TILE_Q, int SLOTS, int GW, bool FUSED>
+static cudaError_t launch_bwd_sorted_cfg(const V *grad_out, const V *value, const int64_t *shapes,
                                          const int64_t *lstart, const float *loc, const float *attw,
                                          const Producers &pr, const Dims &d, float *gv, float *gl, float *gw,
                                          int gate, cudaStream_t stream) {
     using Cfg = SortCfg<LP, WARPS, TILE_W, TILE_Q, SLOTS>;
-    constexpr auto kern = msda_bwd_sorted_kernel<LP, WARPS, TILE_W, MIN_CTAS, TILE_Q, SLOTS, GW, FUSED>;
+    constexpr auto kern = msda_bwd_sorted_kernel<V, LP, WARPS, TILE_W, MIN_CTAS, TILE_Q, SLOTS, GW, FUSED>;
     constexpr size_t kSmemBytes = Cfg::kSmem + (FUSED ? (size_t)Cfg::kPoints * sizeof(float) : 0);
     cudaError_t e;
     const int blocks = persistent_blocks<kern>(WARPS * 32, kSmemBytes, d, &e);
@@ -777,17 +826,21 @@ static cudaError_t launch_bwd_sorted_cfg(const float *grad_out, const float *val
 }
 
 // whether launch_bwd_sorted() covers this problem (shape + alignment)
-bool bwd_sorted_applies(const float *value, const float *gv, const Dims &d) {
-    // rows of value / grad_value must be 128-byte aligned (the merge loop addresses the two halves
-    // of a row as p and p ^ 64); torch allocations are, odd views take the other kernel
-    const bool rows_aligned = ((reinterpret_cast<uintptr_t>(value) | reinterpret_cast<uintptr_t>(gv)) & 127u) == 0;
+template <typename V>
+bool bwd_sorted_applies(const V *value, const float *gv, const Dims &d) {
+    // rows must be aligned to their size -- value: 32 * sizeof(V) bytes (128 fp32, 64 16-bit), grad_value (or the
+    // 16-bit op's fp32 accumulation buffer): 128 -- because the merge loop addresses the two halves of a row as
+    // p and p ^ (half a row); torch allocations are, odd views take the other kernel
+    const bool rows_aligned = (reinterpret_cast<uintptr_t>(value) & (32u * sizeof(V) - 1u)) == 0 &&
+                              (reinterpret_cast<uintptr_t>(gv) & 127u) == 0;
     return d32_applies(d) && d.Lq == d.S && (long long)d.S < (long long)kNoKey && rows_aligned;
 }
 
 // pr.ref == nullptr: plain; otherwise fused producers, gradients w.r.t. the raw sampling offsets (`loc`) and
 // attention logits (`attw`), default shapes only.  `handled` = false: shape outside this kernel's domain (the
 // caller falls back to msda_bwd.cu)
-cudaError_t launch_bwd_sorted(const float *grad_out, const float *value, const int64_t *shapes,
+template <typename V>
+cudaError_t launch_bwd_sorted(const V *grad_out, const V *value, const int64_t *shapes,
                               const int64_t *lstart, const float *loc, const float *attw, const Producers &pr,
                               const Dims &d, float *gv, float *gl, float *gw, int gate, cudaStream_t stream,
                               bool *handled) {
@@ -795,8 +848,16 @@ cudaError_t launch_bwd_sorted(const float *grad_out, const float *value, const i
     if (!*handled) return cudaSuccess;
     // (warps, tile width, min CTAs per SM, queries per tile, window slots, lanes per record)
 #define MSDA_SORTED(LPV, W, TW, C, TQ, SL, GWV, F) \
-    launch_bwd_sorted_cfg<LPV, W, TW, C, TQ, SL, GWV, F>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, \
+    launch_bwd_sorted_cfg<V, LPV, W, TW, C, TQ, SL, GWV, F>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, \
                                                          gw, gate, stream)
+    if constexpr (is16<V>) {   // 16-bit (plain only): the default shapes only
+        switch (d.L * d.P) {
+            case 4: return MSDA_SORTED(4, 16, 16, 2, 128, 4096, 8, false);
+            case 8: return MSDA_SORTED(8, 16, 16, 2, 128, 4096, 8, false);
+            case 12: return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 4, false);
+            default: return MSDA_SORTED(16, 16, 16, 1, 128, 4096, 8, false);
+        }
+    } else {
     if (pr.ref != nullptr) {
         switch (d.L * d.P) {   // 4, 8, 12 or 16 (d32_applies)
             case 4: return MSDA_SORTED(4, 16, 16, 2, 128, 4096, 4, true);
@@ -824,7 +885,18 @@ cudaError_t launch_bwd_sorted(const float *grad_out, const float *value, const i
             }
         default: return MSDA_SORTED(16, 16, 16, 1, 128, 4096, 8, false);
     }
+    }
 #undef MSDA_SORTED
 }
+
+#define MSDA_SORTED_V(V)                                                                                              \
+    template bool bwd_sorted_applies<V>(const V *, const float *, const Dims &);                                       \
+    template cudaError_t launch_bwd_sorted<V>(const V *, const V *, const int64_t *, const int64_t *, const float *,   \
+                                              const float *, const Producers &, const Dims &, float *, float *, float *, \
+                                              int, cudaStream_t, bool *);
+MSDA_SORTED_V(float)
+MSDA_SORTED_V(__nv_bfloat16)
+MSDA_SORTED_V(__half)
+#undef MSDA_SORTED_V
 
 }  // namespace msda

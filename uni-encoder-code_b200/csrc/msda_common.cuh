@@ -6,9 +6,13 @@
 // /root/reference/model/modeling/pixel_decoder/ops/src/cuda/) next to the code.
 #pragma once
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <atomic>
+#include <cstring>
+#include <type_traits>
 #ifdef MSDA_CHECK_BOUNDS
 #include <cassert>     // `make checked`: every corner offset is asserted to lie inside its image
 #endif
@@ -265,6 +269,100 @@ __device__ __forceinline__ void red_add_f4_if(float4 *base, uint32_t off16, floa
                  "@p red.global.add.v4.f32 [%0], {%1,%2,%3,%4};\n\t}"
                  ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "r"(off16)
                  : "memory");
+}
+
+// ---------------------------------------------------------------------------
+// Element type of value / output / grad_output.  V = float, or one of the 16-bit types
+// (__nv_bfloat16, __half) of the mixed-precision op: its rows are half as wide, but every
+// sum stays fp32 -- loads widen to fp32, and only the final store of a result rounds to V.
+// A "chunk" is 4 channels: the 16 (fp32) or 8 (16-bit) bytes a lane of the 32-channel
+// kernels owns; the record offsets count chunks, so their meaning does not depend on V.
+// ---------------------------------------------------------------------------
+template <typename V>
+constexpr bool is16 = sizeof(V) == 2;
+template <typename V>
+constexpr uint32_t kChunkBytes = 4 * sizeof(V);
+
+template <typename T, typename V>
+__device__ __forceinline__ T widen(V v) {
+    if constexpr (std::is_same<V, __nv_bfloat16>::value) return (T)__bfloat162float(v);
+    else if constexpr (std::is_same<V, __half>::value) return (T)__half2float(v);
+    else return (T)v;
+}
+template <typename V, typename T>
+__device__ __forceinline__ V narrow(T v) {
+    if constexpr (std::is_same<V, __nv_bfloat16>::value) return __float2bfloat16_rn((float)v);
+    else if constexpr (std::is_same<V, __half>::value) return __float2half_rn((float)v);   // overflow: +-inf
+    else return (V)v;
+}
+// four 16-bit channels (8 bytes) -> fp32: a shift / mask for bf16, cvt for fp16
+template <typename V>
+__device__ __forceinline__ float4 widen4(uint2 u) {
+    if constexpr (std::is_same<V, __nv_bfloat16>::value) {
+        return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xffff0000u),
+                           __uint_as_float(u.y << 16), __uint_as_float(u.y & 0xffff0000u));
+    } else {
+        __half2 a, b;
+        memcpy(&a, &u.x, 4);
+        memcpy(&b, &u.y, 4);
+        const float2 fa = __half22float2(a), fb = __half22float2(b);
+        return make_float4(fa.x, fa.y, fb.x, fb.y);
+    }
+}
+// address of chunk `off` from `base` in ONE instruction (see at_off16)
+template <typename V>
+__device__ __forceinline__ const V *at_chunk(const V *base, uint32_t off) {
+    unsigned long long r;
+    asm("mad.wide.u32 %0, %1, %2, %3;" : "=l"(r) : "r"(off), "n"(kChunkBytes<V>), "l"((unsigned long long)base));
+    return reinterpret_cast<const V *>(r);
+}
+// a value chunk, kept in L1 (LDG.128 fp32, LDG.64 16-bit)
+template <typename V>
+__device__ __forceinline__ float4 ldg_keep_v4(const V *base, uint32_t off) {
+    if constexpr (!is16<V>) {
+        return ldg_keep_f4(reinterpret_cast<const float4 *>(at_chunk(base, off)));
+    } else {
+        uint2 u;
+        asm("ld.global.nc.v2.u32 {%0,%1}, [%2];" : "=r"(u.x), "=r"(u.y) : "l"(at_chunk(base, off)));
+        return widen4<V>(u);
+    }
+}
+// the same, predicated on off != kNoCorner inside the asm (zeros otherwise), see ldg_keep_f4_if
+template <typename V>
+__device__ __forceinline__ float4 ldg_keep_v4_if(const V *base, uint32_t off) {
+    if constexpr (!is16<V>) {
+        return ldg_keep_f4_if(reinterpret_cast<const float4 *>(base), off);
+    } else {
+        uint2 u;
+        asm("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %3, 0xffffffff;\n\t"
+            "mov.b32 %0, 0;\n\tmov.b32 %1, 0;\n\t"
+            "@p ld.global.nc.v2.u32 {%0,%1}, [%2];\n\t}"
+            : "=r"(u.x), "=r"(u.y) : "l"(at_chunk(base, off)), "r"(off));
+        return widen4<V>(u);
+    }
+}
+// a chunk read once (grad_output rows)
+template <typename V>
+__device__ __forceinline__ float4 ldg_stream_v4(const V *p) {
+    if constexpr (!is16<V>) {
+        return ldg_stream_f4(reinterpret_cast<const float4 *>(p));
+    } else {
+        uint2 u;
+        asm("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(u.x), "=r"(u.y) : "l"(p));
+        return widen4<V>(u);
+    }
+}
+// one result element, rounded to V
+template <typename V>
+__device__ __forceinline__ void stg_stream_v1(V *p, float v) {
+    if constexpr (!is16<V>) {
+        stg_stream_f1(reinterpret_cast<float *>(p), v);
+    } else {
+        const V h = narrow<V>(v);
+        unsigned short bits;
+        memcpy(&bits, &h, 2);
+        asm volatile("st.global.L1::no_allocate.b16 [%0], %1;" ::"l"(p), "h"(bits) : "memory");
+    }
 }
 
 // ---------------------------------------------------------------------------
@@ -551,8 +649,9 @@ struct DetLayout {
 };
 bool det_layout(const Dims &d, int value_bytes, DetLayout *out);
 DetRecords det_records(void *ws, const DetLayout &l);
-template <typename T>
-cudaError_t launch_det_reduce(const DetLayout &l, void *ws, const T *grad_out, T *grad_value, const Dims &d,
+// V: element type of grad_output / grad_value; T: of the record weights and the sums (float for 16-bit V)
+template <typename V, typename T>
+cudaError_t launch_det_reduce(const DetLayout &l, void *ws, const V *grad_out, V *grad_value, const Dims &d,
                               cudaStream_t stream);
 
 void note_launch();                   // increments the library launch counter

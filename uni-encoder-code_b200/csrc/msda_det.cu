@@ -72,10 +72,11 @@ msda_det_bounds_kernel(const uint32_t *__restrict__ keys, long long records, uin
     }
 }
 
-template <typename T>
+// V: element type of grad_output / grad_value (16-bit: widened per term, the row rounded once at the store)
+template <typename V, typename T>
 __global__ void __launch_bounds__(256)
 msda_det_gather_kernel(const uint32_t *__restrict__ start, const uint32_t *__restrict__ ids,
-                       const T *__restrict__ w, const T *__restrict__ grad_out, T *__restrict__ grad_value,
+                       const T *__restrict__ w, const V *__restrict__ grad_out, V *__restrict__ grad_value,
                        uint32_t rows, int D, uint32_t rec_per_row) {
     const int lane = threadIdx.x & 31;
     const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
@@ -99,11 +100,11 @@ msda_det_gather_kernel(const uint32_t *__restrict__ start, const uint32_t *__res
                     if (j < n) {
                         const uint32_t s = __shfl_sync(kFullMask, sl, j);
                         const T ww = __shfl_sync(kFullMask, wl, j);
-                        if (c < D) acc = fma_rn(ww, grad_out[(long long)(s / rec_per_row) * D + c], acc);
+                        if (c < D) acc = fma_rn(ww, widen<T>(grad_out[(long long)(s / rec_per_row) * D + c]), acc);
                     }
                 }
             }
-            if (c < D) grad_value[row * D + c] = acc;
+            if (c < D) grad_value[row * D + c] = narrow<V>(acc);
         }
     }
 }
@@ -120,8 +121,8 @@ unsigned det_grid(long long work, int per_block) {
 
 // Steps 2-4 after the records kernel has filled the workspace.  Counts as three launches
 // (msda_b200_launch_count): the sort as one, whatever number of kernels CUB runs for it.
-template <typename T>
-cudaError_t launch_det_reduce(const DetLayout &l, void *ws, const T *grad_out, T *grad_value, const Dims &d,
+template <typename V, typename T>
+cudaError_t launch_det_reduce(const DetLayout &l, void *ws, const V *grad_out, V *grad_value, const Dims &d,
                               cudaStream_t stream) {
     char *b = static_cast<char *>(ws);
     cub::DoubleBuffer<uint32_t> k(reinterpret_cast<uint32_t *>(b + l.keys_a), reinterpret_cast<uint32_t *>(b + l.keys_b));
@@ -134,16 +135,20 @@ cudaError_t launch_det_reduce(const DetLayout &l, void *ws, const T *grad_out, T
     msda_det_bounds_kernel<<<det_grid(l.records + 1, 256), 256, 0, stream>>>(k.Current(), l.records, l.rows, start);
     note_launch();
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    msda_det_gather_kernel<T><<<det_grid(l.rows, 8), 256, 0, stream>>>(
+    msda_det_gather_kernel<V, T><<<det_grid(l.rows, 8), 256, 0, stream>>>(
         start, v.Current(), reinterpret_cast<const T *>(b + l.w), grad_out, grad_value, l.rows, d.D,
         (uint32_t)(d.L * d.P * 4));
     note_launch();
     return cudaGetLastError();
 }
 
-template cudaError_t launch_det_reduce<float>(const DetLayout &, void *, const float *, float *, const Dims &,
-                                              cudaStream_t);
-template cudaError_t launch_det_reduce<double>(const DetLayout &, void *, const double *, double *, const Dims &,
-                                               cudaStream_t);
+template cudaError_t launch_det_reduce<float, float>(const DetLayout &, void *, const float *, float *, const Dims &,
+                                                     cudaStream_t);
+template cudaError_t launch_det_reduce<double, double>(const DetLayout &, void *, const double *, double *,
+                                                       const Dims &, cudaStream_t);
+template cudaError_t launch_det_reduce<__nv_bfloat16, float>(const DetLayout &, void *, const __nv_bfloat16 *,
+                                                             __nv_bfloat16 *, const Dims &, cudaStream_t);
+template cudaError_t launch_det_reduce<__half, float>(const DetLayout &, void *, const __half *, __half *,
+                                                      const Dims &, cudaStream_t);
 
 }  // namespace msda

@@ -1,5 +1,6 @@
-// msda_fwd.cu -- forward MSDA kernel for sm_100a, specialised for 32 fp32
-// channels per head (the pixel-decoder shape: d_model 256 / 8 heads).
+// msda_fwd.cu -- forward MSDA kernel for sm_100a, specialised for 32 channels per head
+// (the pixel-decoder shape: d_model 256 / 8 heads); value rows in fp32, or bf16 / fp16
+// with fp32 locations, weights and sums (the mixed-precision op).
 //
 // Replaces the reference's ms_deformable_im2col_gpu_kernel
 // (ms_deform_im2col_cuda.cuh:242-304), which runs one thread per output element
@@ -46,12 +47,14 @@ struct FwdCfg {
     static_assert(TILE_W % QPW == 0 && kGroup % TILE_W == 0, "tile shape");
 };
 
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
+// V: element type of value / out (float, or 16-bit: a lane's chunk is then 8 bytes of a 64-byte row,
+// loaded as LDG.64 and widened to fp32; the sums are fp32 and only the output store rounds)
+template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
 __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
-msda_fwd_d32_kernel(const float *__restrict__ value, const int64_t *__restrict__ shapes,
+msda_fwd_d32_kernel(const V *__restrict__ value, const int64_t *__restrict__ shapes,
                     const int64_t *__restrict__ lstart, const float *__restrict__ loc,
                     const float *__restrict__ attw, const Producers pr, const Dims d,
-                    const int want_spatial, float *__restrict__ out) {
+                    const int want_spatial, V *__restrict__ out) {
     using Cfg = FwdCfg<LP, WARPS, TILE_W, QPW>;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ LevelTable lt;
@@ -83,7 +86,7 @@ msda_fwd_d32_kernel(const float *__restrict__ value, const int64_t *__restrict__
         __syncwarp();
 
         // ---- phase 2: gather + weighted reduction, one query at a time ----
-        const float4 *vb = reinterpret_cast<const float4 *>(value) + n * (long long)d.S * M * 8 + chunk;
+        const V *vb = value + (n * (long long)d.S * M * 8 + chunk) * 4;
         const uint4 *plane = reinterpret_cast<const uint4 *>(rec + corner * Cfg::kPlane);
         for (int qi = 0; qi < cnt; ++qi) {
             const uint4 *rq = plane + qi * (LP / 2);
@@ -92,7 +95,7 @@ msda_fwd_d32_kernel(const float *__restrict__ value, const int64_t *__restrict__
             for (int sp2 = 0; sp2 < LP / 2; ++sp2) {
                 const uint4 e = lds_u4(rq + sp2);           // this corner's records of 2 points
                 if (e.x != kNoCorner) {
-                    const float4 v = ldg_keep_f4(at_off16(vb, e.x));
+                    const float4 v = ldg_keep_v4(vb, e.x);
                     const float w = __uint_as_float(e.y);
                     acc.x = fmaf(w, v.x, acc.x);
                     acc.y = fmaf(w, v.y, acc.y);
@@ -100,7 +103,7 @@ msda_fwd_d32_kernel(const float *__restrict__ value, const int64_t *__restrict__
                     acc.w = fmaf(w, v.w, acc.w);
                 }
                 if (e.z != kNoCorner) {
-                    const float4 v = ldg_keep_f4(at_off16(vb, e.z));
+                    const float4 v = ldg_keep_v4(vb, e.z);
                     const float w = __uint_as_float(e.w);
                     acc.x = fmaf(w, v.x, acc.x);
                     acc.y = fmaf(w, v.y, acc.y);
@@ -116,8 +119,8 @@ msda_fwd_d32_kernel(const float *__restrict__ value, const int64_t *__restrict__
             a1 += __shfl_xor_sync(kFullMask, s1, 16);
             const float keep = up8 ? a1 : a0, send = up8 ? a0 : a1;
             const float res = keep + __shfl_xor_sync(kFullMask, send, 8);
-            float *o = out + ((n * d.Lq + q0 + qi) * M + m) * 32LL + chunk * 4 + corner;
-            stg_stream_f1(o, res);
+            V *o = out + ((n * d.Lq + q0 + qi) * M + m) * 32LL + chunk * 4 + corner;
+            stg_stream_v1(o, res);
         }
         __syncwarp();   // records are overwritten by the next item
     }
@@ -127,12 +130,12 @@ msda_fwd_d32_kernel(const float *__restrict__ value, const int64_t *__restrict__
 // host side: launch_fwd_d32() serves the plain op and the fused producers (Producers::ref set),
 // the latter in the default CTA shape only
 // ---------------------------------------------------------------------------
-template <int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
-static cudaError_t launch_fwd_cfg(const float *value, const int64_t *shapes, const int64_t *lstart,
+template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
+static cudaError_t launch_fwd_cfg(const V *value, const int64_t *shapes, const int64_t *lstart,
                                   const float *loc, const float *attw, const Producers &pr, const Dims &d,
-                                  float *out, cudaStream_t stream) {
+                                  V *out, cudaStream_t stream) {
     using Cfg = FwdCfg<LP, WARPS, TILE_W, QPW>;
-    constexpr auto kern = msda_fwd_d32_kernel<LP, WARPS, TILE_W, MIN_CTAS, QPW, FUSED>;
+    constexpr auto kern = msda_fwd_d32_kernel<V, LP, WARPS, TILE_W, MIN_CTAS, QPW, FUSED>;
     cudaError_t e;
     const int blocks = persistent_blocks<kern>(WARPS * 32, Cfg::kSmem, d, &e);
     if (blocks == 0) return e;
@@ -142,12 +145,15 @@ static cudaError_t launch_fwd_cfg(const float *value, const int64_t *shapes, con
     return cudaGetLastError();
 }
 
-template <int LP>
-static cudaError_t launch_fwd_lp(const float *value, const int64_t *shapes, const int64_t *lstart,
+template <typename V, int LP>
+static cudaError_t launch_fwd_lp(const V *value, const int64_t *shapes, const int64_t *lstart,
                                  const float *loc, const float *attw, const Producers &pr, const Dims &d,
-                                 float *out, cudaStream_t stream) {
+                                 V *out, cudaStream_t stream) {
     // variant = (warps, query tile width, min CTAs per SM -> register budget, queries per warp)
-#define MSDA_FWD(W, TW, C, Q, F) launch_fwd_cfg<LP, W, TW, C, Q, F>(value, shapes, lstart, loc, attw, pr, d, out, stream)
+#define MSDA_FWD(W, TW, C, Q, F) launch_fwd_cfg<V, LP, W, TW, C, Q, F>(value, shapes, lstart, loc, attw, pr, d, out, stream)
+    if constexpr (is16<V>) {
+        return MSDA_FWD(16, 16, 2, 8, false);                     // 16-bit (plain only): the default shape only
+    } else {
     if (pr.ref != nullptr) return MSDA_FWD(16, 16, 2, 8, true);   // fused producers: the default shape only
     switch (option_value(OPT_FWD_VARIANT)) {
         case 1: return MSDA_FWD(8, 8, 4, 8, false);     //  8 warps, tile  8x8
@@ -160,23 +166,33 @@ static cudaError_t launch_fwd_lp(const float *value, const int64_t *shapes, cons
         case 2:
         default: return MSDA_FWD(16, 16, 2, 8, false);  // 16 warps, tile  8x16, 8 queries per warp (98 KB smem per SM)
     }
+    }
 #undef MSDA_FWD
 }
 
 // pr.ref == nullptr: plain, `loc` / `attw` are the sampling locations and attention weights.  Otherwise fused
 // producers (SURVEY 8f.1): `loc` = raw sampling offsets, `attw` = raw attention logits, `pr.ref` = reference
 // points [N or 1, Lq, L, 2].  `handled` = false: the problem is outside d32_applies() and nothing was launched.
-cudaError_t launch_fwd_d32(const float *value, const int64_t *shapes, const int64_t *lstart, const float *loc,
-                           const float *attw, const Producers &pr, const Dims &d, float *out, cudaStream_t stream,
+template <typename V>
+cudaError_t launch_fwd_d32(const V *value, const int64_t *shapes, const int64_t *lstart, const float *loc,
+                           const float *attw, const Producers &pr, const Dims &d, V *out, cudaStream_t stream,
                            bool *handled) {
     *handled = d32_applies(d);
     if (!*handled) return cudaSuccess;
     switch (d.L * d.P) {       // 4, 8, 12 or 16 (d32_applies)
-        case 4: return launch_fwd_lp<4>(value, shapes, lstart, loc, attw, pr, d, out, stream);
-        case 8: return launch_fwd_lp<8>(value, shapes, lstart, loc, attw, pr, d, out, stream);
-        case 12: return launch_fwd_lp<12>(value, shapes, lstart, loc, attw, pr, d, out, stream);
-        default: return launch_fwd_lp<16>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        case 4: return launch_fwd_lp<V, 4>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        case 8: return launch_fwd_lp<V, 8>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        case 12: return launch_fwd_lp<V, 12>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        default: return launch_fwd_lp<V, 16>(value, shapes, lstart, loc, attw, pr, d, out, stream);
     }
 }
+
+#define MSDA_FWD_D32(V)                                                                                             \
+    template cudaError_t launch_fwd_d32<V>(const V *, const int64_t *, const int64_t *, const float *, const float *, \
+                                           const Producers &, const Dims &, V *, cudaStream_t, bool *);
+MSDA_FWD_D32(float)
+MSDA_FWD_D32(__nv_bfloat16)
+MSDA_FWD_D32(__half)
+#undef MSDA_FWD_D32
 
 }  // namespace msda

@@ -35,6 +35,30 @@ class MSDeformAttnFunction(Function):
         return grad_value, None, None, grad_loc, grad_w, None
 
 
+class MSDeformAttnMixedFunction(Function):
+    """``MSDeformAttnFunction`` for mixed precision (torch.autocast): same ``apply`` signature, a bf16 / fp16
+    ``value`` (output and grad_value in its dtype) with fp32 ``sampling_locations`` / ``attention_weights`` (and
+    fp32 gradients for them); every sum in fp32 (ops.ms_deform_attn_mixed_forward / _backward)."""
+
+    @staticmethod
+    def forward(ctx, value, value_spatial_shapes, value_level_start_index, sampling_locations,
+                attention_weights, im2col_step):
+        ctx.im2col_step = im2col_step
+        output = ops.ms_deform_attn_mixed_forward(value, value_spatial_shapes, value_level_start_index,
+                                                  sampling_locations, attention_weights, im2col_step)
+        ctx.save_for_backward(value, value_spatial_shapes, value_level_start_index,
+                              sampling_locations, attention_weights)
+        return output
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_output):
+        value, shapes, lsi, loc, w = ctx.saved_tensors
+        grad_value, grad_loc, grad_w = ops.ms_deform_attn_mixed_backward(
+            value, shapes, lsi, loc, w, grad_output.contiguous(), ctx.im2col_step)
+        return grad_value, None, None, grad_loc, grad_w, None
+
+
 class MSDeformAttnFusedFunction(Function):
     """``apply(value, spatial_shapes, level_start_index, reference_points, sampling_offsets,
     attn_logits)`` -- the op with its caller's softmax and location arithmetic

@@ -29,7 +29,8 @@ import torch.nn.functional as F
 from torch import nn
 
 from . import ops
-from .functions import AddLayerNormFunction, LinearTF32x3Function, MSDeformAttnFunction, MSDeformAttnFusedFunction
+from .functions import (AddLayerNormFunction, LinearTF32x3Function, MSDeformAttnFunction, MSDeformAttnFusedFunction,
+                        MSDeformAttnMixedFunction)
 
 CoreFn = Callable[..., torch.Tensor]
 
@@ -125,6 +126,10 @@ def _add_norm(norm: nn.LayerNorm, x, sublayer_out, impl: str):
 
 def _cuda_core(value, spatial_shapes, level_start_index, sampling_locations, attention_weights,
                im2col_step):
+    if value.dtype in (torch.bfloat16, torch.float16):
+        # mixed precision (autocast): 16-bit value rows, locations and weights in fp32 (upcasting them is exact)
+        return MSDeformAttnMixedFunction.apply(value, spatial_shapes, level_start_index, sampling_locations.float(),
+                                               attention_weights.float(), im2col_step)
     return MSDeformAttnFunction.apply(value, spatial_shapes, level_start_index, sampling_locations,
                                       attention_weights, im2col_step)
 
@@ -177,6 +182,9 @@ class MSDeformAttn(nn.Module):
         M, L, P = self.n_heads, self.n_levels, self.n_points
         offsets = _linear(self.sampling_offsets, query, self.linear).view(N, Lq, M, L, P, 2)
         weights = F.softmax(_linear(self.attention_weights, query, self.linear).view(N, Lq, M, L * P), -1).view(N, Lq, M, L, P)
+        if offsets.dtype in (torch.bfloat16, torch.float16):
+            offsets = offsets.float()       # autocast: the locations are formed in fp32 (a 16-bit one is off by up to
+            #                                 half a pixel at W = 256)
         if reference_points.shape[-1] == 2:
             wh = input_spatial_shapes.flip(-1).to(offsets.dtype)       # (W_l, H_l)
             loc = reference_points[:, :, None, :, None, :] + offsets / wh[None, None, None, :, None, :]
@@ -198,7 +206,8 @@ class MSDeformAttn(nn.Module):
     def forward(self, query, reference_points, input_flatten, input_spatial_shapes,
                 input_level_start_index, input_padding_mask=None):
         value = self.project_value(input_flatten, input_padding_mask)
-        if self.fused and self._core is _cuda_core and not reference_points.requires_grad:
+        if self.fused and self._core is _cuda_core and not reference_points.requires_grad \
+                and value.dtype == torch.float32:      # (the fused kernels are fp32; autocast takes the path below)
             N, Lq, _ = query.shape
             offsets = _linear(self.sampling_offsets, query, self.linear).view(
                 N, Lq, self.n_heads, self.n_levels, self.n_points, 2)

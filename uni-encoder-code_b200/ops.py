@@ -55,6 +55,11 @@ _FWD = {torch.float32: _lib.lib.msda_b200_forward_f32, torch.float64: _lib.lib.m
 _BWD = {torch.float32: _lib.lib.msda_b200_backward_f32, torch.float64: _lib.lib.msda_b200_backward_f64}
 _BWD_DET = {torch.float32: _lib.lib.msda_b200_backward_deterministic_f32,
             torch.float64: _lib.lib.msda_b200_backward_deterministic_f64}
+# the mixed-precision op: 16-bit value / output / grad_output / grad_value, fp32 locations and weights
+_MIXED_FWD = {torch.bfloat16: _lib.lib.msda_b200_forward_bf16, torch.float16: _lib.lib.msda_b200_forward_f16}
+_MIXED_BWD = {torch.bfloat16: _lib.lib.msda_b200_backward_bf16, torch.float16: _lib.lib.msda_b200_backward_f16}
+_MIXED_BWD_DET = {torch.bfloat16: _lib.lib.msda_b200_backward_deterministic_bf16,
+                  torch.float16: _lib.lib.msda_b200_backward_deterministic_f16}
 
 # With torch.use_deterministic_algorithms(True) every backward here takes its deterministic entry point.  The
 # MSDA backwards then sort one record per (sampling point, corner): the batch is processed in chunks of whole
@@ -97,18 +102,23 @@ def _require_cuda_contiguous(named):
             raise RuntimeError(f"{name} is on {t.device}, {first} is on {anchor.device}")
 
 
-def _check_common(named, im2col_step, opname):
+def _check_common(named, im2col_step, opname, mixed=False):
+    """The checks of the op over (name, tensor) pairs (value, spatial_shapes, level_start_index, sampling_loc,
+    attn_weight[, grad_output]) -> (N, S, M, D, L, Lq, P).  ``mixed``: the mixed-precision op's dtypes -- a 16-bit
+    value (and grad_output of the same type), fp32 sampling_loc and attn_weight."""
     _require_cuda_contiguous(named)
     value = named[0][1]
-    if value.dtype not in _FWD:
+    if value.dtype not in (_MIXED_FWD if mixed else _FWD):
         raise RuntimeError(f'"{opname}" not implemented for \'{value.dtype}\'')   # cu:69,139
     _, shapes, lsi, loc, w = (t for _, t in named[:5])
     for name, t in named[1:3]:
         if t.dtype != torch.int64:
             raise RuntimeError(f"expected scalar type Long but found {t.dtype} for {name}")
-    for name, t in named[3:]:
-        if t.dtype != value.dtype:
-            raise RuntimeError(f"expected scalar type {value.dtype} but found {t.dtype} for {name}")
+    for i, (name, t) in enumerate(named[3:], start=3):
+        want = torch.float32 if mixed and i < 5 else value.dtype
+        if t.dtype != want:
+            hint = " (the mixed-precision op keeps locations and weights in fp32)" if want == torch.float32 and mixed else ""
+            raise RuntimeError(f"expected scalar type {want} but found {t.dtype} for {name}{hint}")
     if value.dim() != 4 or loc.dim() != 6 or shapes.dim() != 2 or shapes.size(1) != 2:
         raise RuntimeError("value must be [N,S,M,D], sampling_loc [N,Lq,M,L,P,2], spatial_shapes [L,2]")
     N, S, M, D = value.shape
@@ -178,10 +188,12 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
     return [grad_value, grad_loc, grad_w]
 
 
-def _backward_deterministic(fn, opname, value, shapes, lsi, producers, grad_output, dims, ref=None, rs=0):
-    """A deterministic backward entry ``fn`` (msda_b200_backward_deterministic_f32/_f64, or with ``ref`` the fused
+def _backward_deterministic(fn, opname, value, shapes, lsi, producers, grad_output, dims, ref=None, rs=0,
+                            kind="backward"):
+    """A deterministic backward entry ``fn`` (msda_b200_backward_deterministic_f32/_f64/_bf16/_f16, or with ``ref`` the fused
     msda_b200_fused_backward_deterministic_f32) in chunks of whole images -> [grad_value, *grads of producers].
-    ``producers``: (sampling_loc, attn_weight), or for the fused op (sampling_offsets, attn_logits)."""
+    ``producers``: (sampling_loc, attn_weight), or for the fused op (sampling_offsets, attn_logits).  ``kind``: the
+    name of the call in ``enable_timing``'s list, the same as the default backward's."""
     N, S, M, D, L, Lq, P = dims
     chunks = _image_chunks(N, Lq * M * L * P * 4)
     with torch.cuda.device(value.device):
@@ -189,7 +201,7 @@ def _backward_deterministic(fn, opname, value, shapes, lsi, producers, grad_outp
         grads = [torch.empty_like(t) for t in producers]
         ws = _det_workspace(max(b - a for a, b in chunks), S, M, D, L, Lq, P, value.dtype, value.device)
         stream = torch.cuda.current_stream().cuda_stream
-        with _timed("backward"):
+        with _timed(kind):
             for a, b in chunks:
                 fused = ()
                 if ref is not None:                     # rs == 0: one set of reference points shared by the batch
@@ -199,6 +211,63 @@ def _backward_deterministic(fn, opname, value, shapes, lsi, producers, grad_outp
                         *(g[a:b].data_ptr() for g in grads), ws.data_ptr(), stream)
                 _lib.check(rc, opname)
     return [grad_value, *grads]
+
+
+# ----------------------------------------------------------------------------------------------
+# Mixed precision (torch.autocast): bf16 / fp16 value rows with fp32 locations, weights and sums.  Not part of the
+# drop-in boundary above, which keeps the reference's fp32 / fp64 dtype contract.
+# ----------------------------------------------------------------------------------------------
+def ms_deform_attn_mixed_forward(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, im2col_step):
+    """-> output [N, Lq, M*D] in value's dtype, for a bf16 / fp16 ``value`` and fp32 ``sampling_loc`` /
+    ``attn_weight``: the fp32 op on the widened value, rounded once to the 16-bit type (msda_b200_forward_bf16 /
+    _f16).  Arguments as ``ms_deform_attn_forward``; ``im2col_step`` is validated and ignored."""
+    named = [("value", value), ("spatial_shapes", spatial_shapes),
+             ("level_start_index", level_start_index), ("sampling_loc", sampling_loc),
+             ("attn_weight", attn_weight)]
+    N, S, M, D, L, Lq, P = _check_common(named, im2col_step, "ms_deform_attn_mixed_forward", mixed=True)
+    if N * Lq * M * D == 0 or S == 0 or L * P == 0:
+        return torch.zeros((N, Lq, M * D), dtype=value.dtype, device=value.device)
+    with torch.cuda.device(value.device):
+        output = torch.empty((N, Lq, M * D), dtype=value.dtype, device=value.device)
+        with _timed("forward_mixed"):
+            rc = _MIXED_FWD[value.dtype](
+                value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
+                sampling_loc.data_ptr(), attn_weight.data_ptr(), N, S, M, D, L, Lq, P,
+                output.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    _lib.check(rc, "ms_deform_attn_mixed_forward")
+    return output
+
+
+def ms_deform_attn_mixed_backward(value, spatial_shapes, level_start_index, sampling_loc, attn_weight,
+                                  grad_output, im2col_step):
+    """-> [grad_value (value's dtype), grad_sampling_loc, grad_attn_weight (fp32)] of the mixed-precision op.
+    grad_value is reduced in an fp32 buffer allocated here and rounded once (msda_b200_backward_bf16 / _f16); with
+    torch.use_deterministic_algorithms(True) the deterministic entries, in image chunks as for fp32."""
+    named = [("value", value), ("spatial_shapes", spatial_shapes),
+             ("level_start_index", level_start_index), ("sampling_loc", sampling_loc),
+             ("attn_weight", attn_weight), ("grad_output", grad_output)]
+    N, S, M, D, L, Lq, P = _check_common(named, im2col_step, "ms_deform_attn_mixed_backward", mixed=True)
+    if grad_output.numel() != N * Lq * M * D:
+        raise RuntimeError(f"grad_output has {grad_output.numel()} elements, expected {N * Lq * M * D}")
+    if N * Lq * M * D == 0 or S == 0 or L * P == 0:
+        return [torch.zeros_like(value), torch.zeros_like(sampling_loc), torch.zeros_like(attn_weight)]
+    if _deterministic():
+        return _backward_deterministic(_MIXED_BWD_DET[value.dtype], "ms_deform_attn_mixed_backward (deterministic)",
+                                       value, spatial_shapes, level_start_index, (sampling_loc, attn_weight),
+                                       grad_output, (N, S, M, D, L, Lq, P), kind="backward_mixed")
+    with torch.cuda.device(value.device):
+        accum = torch.zeros((N, S, M, D), dtype=torch.float32, device=value.device)   # fp32 reductions
+        grad_value = torch.empty_like(value)            # rounded from accum
+        grad_loc = torch.empty_like(sampling_loc)
+        grad_w = torch.empty_like(attn_weight)
+        with _timed("backward_mixed"):
+            rc = _MIXED_BWD[value.dtype](
+                grad_output.data_ptr(), value.data_ptr(), spatial_shapes.data_ptr(),
+                level_start_index.data_ptr(), sampling_loc.data_ptr(), attn_weight.data_ptr(),
+                N, S, M, D, L, Lq, P, accum.data_ptr(), grad_value.data_ptr(), grad_loc.data_ptr(),
+                grad_w.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    _lib.check(rc, "ms_deform_attn_mixed_backward")
+    return [grad_value, grad_loc, grad_w]
 
 
 def debug_indices(value_shape, spatial_shapes, level_start_index, sampling_loc):

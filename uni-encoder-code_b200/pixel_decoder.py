@@ -16,6 +16,7 @@ Differences, all from SURVEY.md section 8f.4 (input-independent work and host sy
 """
 from __future__ import annotations
 
+import contextlib
 import math
 from typing import Dict, List, Optional, Sequence, Tuple
 
@@ -123,8 +124,15 @@ class MSDeformAttnPixelDecoder(nn.Module):
                  transformer_nheads: int, transformer_dim_feedforward: int, transformer_enc_layers: int,
                  conv_dim: int, mask_dim: int, norm: Optional[str] = None,
                  transformer_in_features: Sequence[str], common_stride: int,
-                 core: Optional[CoreFn] = None, fused: bool = False, linear: str = "torch"):
+                 core: Optional[CoreFn] = None, fused: bool = False, linear: str = "torch", amp: bool = False):
+        """`amp=True` (not in the reference): `forward_features` runs inside the caller's torch.autocast context
+        instead of disabling it -- torch's 16-bit GEMMs and convolutions, and the mixed-precision MSDA op
+        (functions.MSDeformAttnMixedFunction).  `amp=False` is the reference's behaviour: autocast off, fp32."""
+        if amp and linear == "tf32x3":
+            raise ValueError('amp=True cannot be combined with linear="tf32x3": the 3xTF32 GEMMs and the fp32 '
+                             'GroupNorm / LayerNorm kernels are fp32 paths that autocast would bypass')
         super().__init__()
+        self.amp = amp
         by_stride = sorted(input_shape.items(), key=lambda kv: kv[1][1])
         self.in_features = [k for k, _ in by_stride]
         self.feature_channels = [v[0] for _, v in by_stride]
@@ -167,8 +175,10 @@ class MSDeformAttnPixelDecoder(nn.Module):
 
     def forward_features(self, features: Dict[str, torch.Tensor]):
         """-> (mask_features [N, mask_dim, H/4, W/4], lowest-resolution map, 3 multi-scale maps),
-        as msdeformattn.py:336-386 (autocast disabled, inputs promoted to fp32)."""
-        with torch.autocast(device_type=next(iter(features.values())).device.type, enabled=False):
+        as msdeformattn.py:336-386 (autocast disabled, inputs promoted to fp32; with `amp`, under the caller's
+        autocast, if any)."""
+        device_type = next(iter(features.values())).device.type
+        with contextlib.nullcontext() if self.amp else torch.autocast(device_type=device_type, enabled=False):
             fused_norm = self.linear == "tf32x3"        # the inference kernels of SURVEY 8f.3 / 8f.4
             names = self.transformer_in_features[::-1]
             levels = [(int(features[k].shape[2]), int(features[k].shape[3])) for k in names]
