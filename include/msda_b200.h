@@ -195,8 +195,9 @@ int msda_b200_backward_deterministic_f16(const uint16_t *grad_output, const uint
  *   attn_logits       [batch, num_query, num_heads, num_levels*num_point]      (raw Linear output)
  * The backward returns the gradients with respect to sampling_offsets and attn_logits (softmax
  * backward and the 1/(W,H) scaling folded in); reference_points get no gradient here.
- * Only the 32-channel fp32 fast path exists (num_levels*num_point in {4,8,12,16});
- * MSDA_ERR_UNSUPPORTED otherwise -- the caller then composes the unfused entry points.
+ * Only the 32-channel fast path exists (channels == 32, num_levels*num_point in {4,8,12,16}), in fp32
+ * and in mixed precision (the _bf16 / _f16 entries below); MSDA_ERR_UNSUPPORTED otherwise, and for views
+ * whose alignment the kernels cannot take -- the caller then composes the unfused entry points.
  */
 int msda_b200_fused_forward_f32(const float *value, const int64_t *spatial_shapes,
                                 const int64_t *level_start, const float *reference_points,
@@ -241,6 +242,63 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
                                                int batch, int spatial_size, int num_heads, int channels,
                                                int num_levels, int num_query, int num_point, float *grad_value,
                                                float *grad_sampling_offsets, float *grad_attn_logits,
+                                               void *workspace, void *stream);
+
+/*
+ * Mixed-precision fused producers (what torch.autocast hands the module: every Linear output is 16-bit):
+ * value, sampling_offsets, attn_logits, output, grad_output, grad_value, grad_sampling_offsets and
+ * grad_attn_logits all bf16 (_bf16) or all fp16 (_f16), as uint16_t bit patterns; reference_points stay
+ * fp32.  Everything in between is fp32 -- the widened offsets and logits, ref + offset / (W, H), the
+ * softmax and its backward, the 1/(W, H) scaling and every sum -- with the integer geometry of the fp32 op,
+ * and each output is rounded once (round-to-nearest-even; fp16 overflow gives +-inf).  For the same widened
+ * inputs output, grad_sampling_offsets, grad_attn_logits and the deterministic grad_value are therefore the
+ * fp32 fused entries' results rounded to 16 bits, bit for bit.
+ * msda_b200_fused_backward_{bf16,f16}: grad_value_accum is a zero-filled fp32 [batch, spatial_size,
+ * num_heads, channels] buffer that the kernels reduce into and that is then rounded into grad_value, as for
+ * msda_b200_backward_bf16.  The deterministic twins take a workspace of
+ * msda_b200_backward_deterministic_workspace_bytes(..., value_bytes = 2) bytes.
+ * Alignment: sampling_offsets 4 bytes, reference_points 8, value / output / grad_output 16 (and value 64
+ * for the merging backward kernel, otherwise the per-row one runs); MSDA_ERR_UNSUPPORTED otherwise.
+ */
+int msda_b200_fused_forward_bf16(const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start,
+                                 const float *reference_points, long long ref_batch_stride,
+                                 const uint16_t *sampling_offsets, const uint16_t *attn_logits, int batch,
+                                 int spatial_size, int num_heads, int channels, int num_levels, int num_query,
+                                 int num_point, uint16_t *output, void *stream);
+int msda_b200_fused_forward_f16(const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start,
+                                const float *reference_points, long long ref_batch_stride,
+                                const uint16_t *sampling_offsets, const uint16_t *attn_logits, int batch,
+                                int spatial_size, int num_heads, int channels, int num_levels, int num_query,
+                                int num_point, uint16_t *output, void *stream);
+int msda_b200_fused_backward_bf16(const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes,
+                                  const int64_t *level_start, const float *reference_points,
+                                  long long ref_batch_stride, const uint16_t *sampling_offsets,
+                                  const uint16_t *attn_logits, int batch, int spatial_size, int num_heads,
+                                  int channels, int num_levels, int num_query, int num_point,
+                                  float *grad_value_accum, uint16_t *grad_value, uint16_t *grad_sampling_offsets,
+                                  uint16_t *grad_attn_logits, void *stream);
+int msda_b200_fused_backward_f16(const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes,
+                                 const int64_t *level_start, const float *reference_points,
+                                 long long ref_batch_stride, const uint16_t *sampling_offsets,
+                                 const uint16_t *attn_logits, int batch, int spatial_size, int num_heads,
+                                 int channels, int num_levels, int num_query, int num_point,
+                                 float *grad_value_accum, uint16_t *grad_value, uint16_t *grad_sampling_offsets,
+                                 uint16_t *grad_attn_logits, void *stream);
+int msda_b200_fused_backward_deterministic_bf16(const uint16_t *grad_output, const uint16_t *value,
+                                                const int64_t *spatial_shapes, const int64_t *level_start,
+                                                const float *reference_points, long long ref_batch_stride,
+                                                const uint16_t *sampling_offsets, const uint16_t *attn_logits,
+                                                int batch, int spatial_size, int num_heads, int channels,
+                                                int num_levels, int num_query, int num_point, uint16_t *grad_value,
+                                                uint16_t *grad_sampling_offsets, uint16_t *grad_attn_logits,
+                                                void *workspace, void *stream);
+int msda_b200_fused_backward_deterministic_f16(const uint16_t *grad_output, const uint16_t *value,
+                                               const int64_t *spatial_shapes, const int64_t *level_start,
+                                               const float *reference_points, long long ref_batch_stride,
+                                               const uint16_t *sampling_offsets, const uint16_t *attn_logits,
+                                               int batch, int spatial_size, int num_heads, int channels,
+                                               int num_levels, int num_query, int num_point, uint16_t *grad_value,
+                                               uint16_t *grad_sampling_offsets, uint16_t *grad_attn_logits,
                                                void *workspace, void *stream);
 
 /*

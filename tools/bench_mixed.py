@@ -14,10 +14,18 @@ DIR defaults to $BENCH_OUT/mixed, and BENCH_OUT to bench_out/ in the repository 
     point) and their gradients once -- per query at configs[1] 3 200 (fp32) / 2 176 (16-bit) forward and
     5 376 / 3 840 backward; the accumulation buffer's zero-fill and conversion read (4 + 4 bytes per value
     element) are reported separately.
+(f) part (a)'s fused-producer arms at the same two shapes (raw offsets [N, Lq, M, L, P, 2] and logits [N, Lq, M, L*P]
+    as the Linear layers hand them over, fp32 reference points): per 16-bit type the fused 16-bit op against the
+    unfused 16-bit composition MSDeformAttn(fused=False) runs under autocast (torch's fp32 softmax and
+    `ref + off.float() / (W, H)`, then the mixed-precision op) and against the fp32 fused op; forward, backward and
+    both, through autograd (the backward arm's forward runs untimed just before it), arms alternating and the L2
+    evicted before every timed call as in (a).
 (b) the decoder forward (forward_features, no autograd) at the configs[2] shape with a Swin-T pyramid: the fastest
-    fp32 setting (fused=True, linear="tf32x3") against amp=True under bf16 autocast.
+    fp32 setting (fused=True, linear="tf32x3") against amp=True under bf16 autocast, with fused=True (the fused 16-bit
+    kernels) and fused=False (torch's producers around the mixed-precision op).
 (c) the decoder training step (forward_features -> loss -> backward -> AdamW) at 512x1024, batch 16, as
-    tools/bench_decoder_train.py: fp32 linear="tf32x3" against amp=True with bf16, and with fp16 + GradScaler.
+    tools/bench_decoder_train.py: fp32 linear="tf32x3" against amp=True with bf16, and with fp16 + GradScaler, each
+    with fused=True and fused=False.
 
 Every JSON line carries the card's name and power limit (read-only nvidia-smi query).
 """
@@ -114,6 +122,81 @@ def part_a(pkg, args, emit):
         torch.cuda.empty_cache()
 
 
+def part_f(pkg, args, emit):
+    dev = torch.device("cuda", 0)
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    tags = [t for t in args.dtypes.split(",") if t != "fp32"]
+    for name in ("cityscapes_512x1024_b8", "cityscapes_1024x2048_b8"):
+        w = pkg.synthetic.WORKLOADS[name]
+        levels, N, M, P = list(w.levels), w.batch, 8, 4
+        L, S = len(levels), sum(h * wd for h, wd in levels)
+        gen = torch.Generator(device=dev).manual_seed(1)
+        base = {"value": torch.randn(N, S, M, 32, device=dev, generator=gen),
+                "off": torch.randn(N, S, M, L, P, 2, device=dev, generator=gen) * 2.0,
+                "logits": torch.randn(N, S, M, L * P, device=dev, generator=gen),
+                "grad": torch.randn(N, S, M * 32, device=dev, generator=gen)}
+        shapes, lsi = pkg.synthetic.level_tensors(levels, device=dev)
+        ref = pkg.modules.reference_points_for(levels, dev)                 # [1, S, L, 2], fp32
+        wh = shapes.flip(-1).float()[None, None, None, :, None, :]
+        inputs = {"fp32": {k: v.bfloat16().float() for k, v in base.items()}}   # the values the 16-bit arms see
+        for t in tags:
+            inputs[t] = {k: v.to(DTYPES[t]) for k, v in base.items()}
+        del base
+
+        def fused(d):
+            leaves = [d[k].requires_grad_(True) for k in ("value", "off", "logits")]
+            return pkg.MSDeformAttnFusedFunction.apply(leaves[0], shapes, lsi, ref, leaves[1], leaves[2])
+
+        def unfused(d):          # MSDeformAttn(fused=False) under autocast: fp32 producers, then the mixed op
+            v, off, lg = (d[k].requires_grad_(True) for k in ("value", "off", "logits"))
+            wts = torch.softmax(lg.float(), -1).view(N, S, M, L, P)
+            loc = ref[:, :, None, :, None, :] + off.float() / wh
+            return pkg.MSDeformAttnMixedFunction.apply(v, shapes, lsi, loc.contiguous(), wts.contiguous(), 128)
+
+        arms = [("fp32", "fused", fused)] + [(t, kind, fn) for t in tags for kind, fn in (("fused", fused),
+                                                                                         ("unfused", unfused))]
+        times = {(t, k, op): [] for t, k, _ in arms for op in ("forward", "backward", "fwd+bwd")}
+
+        def one(t, fn, op):
+            d = inputs[t]
+            if op == "forward":
+                flush.zero_()
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                with torch.no_grad():
+                    e0.record()
+                    fn(d)
+                    e1.record()
+            else:
+                out = fn(d) if op == "backward" else None
+                flush.zero_()
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                if out is None:
+                    out = fn(d)
+                out.backward(d["grad"])
+                e1.record()
+                for k in ("value", "off", "logits"):
+                    d[k].grad = None
+            e1.synchronize()
+            return e0.elapsed_time(e1)
+
+        for t, _, fn in arms:                               # warm-up of every arm
+            for op in ("forward", "backward", "fwd+bwd"):
+                one(t, fn, op)
+        for _ in range(args.steps):
+            for op in ("forward", "backward", "fwd+bwd"):
+                for t, k, fn in arms:                       # the arms alternate
+                    times[(t, k, op)].append(one(t, fn, op))
+        for (t, k, op), ts in times.items():
+            emit({"part": "f", "label": args.label, "workload": name, "dtype": t, "producers": k, "op": op,
+                  "ms_median": statistics.median(ts), "ms_min": min(ts), "ms_max": max(ts), "timed_calls": len(ts),
+                  "what": "fused: MSDeformAttnFusedFunction on raw offsets / logits; unfused: torch fp32 softmax and "
+                          "locations + MSDeformAttnMixedFunction (autograd, L*P = 12, offsets ~ N(0, 2) px)",
+                  "l2": "evicted before every call (256 MB write)"})
+        del inputs
+        torch.cuda.empty_cache()
+
+
 def _decoder(pkg, fused, linear, amp, train):
     torch.manual_seed(0)
     m = pkg.pixel_decoder.MSDeformAttnPixelDecoder(
@@ -131,7 +214,8 @@ def _feats(batch, h, w, seed):
 def part_b(pkg, args, emit):
     feats = _feats(8, 1024, 2048, 3)
     arms = [("fp32 fused tf32x3", dict(fused=True, linear="tf32x3", amp=False), None),
-            ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16)]
+            ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16),
+            ("amp bf16 fused=False", dict(fused=False, linear="torch", amp=True), torch.bfloat16)]
     models = {tag: _decoder(pkg, train=False, **kw) for tag, kw, _ in arms}
     res = {tag: [] for tag, _, _ in arms}
     for _ in range(args.repeats):
@@ -151,7 +235,9 @@ def part_c(pkg, args, emit):
     feats = _feats(16, 512, 1024, 2)
     arms = [("fp32 fused tf32x3", dict(fused=True, linear="tf32x3", amp=False), None),
             ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16),
-            ("amp fp16 + GradScaler", dict(fused=True, linear="torch", amp=True), torch.float16)]
+            ("amp bf16 fused=False", dict(fused=False, linear="torch", amp=True), torch.bfloat16),
+            ("amp fp16 + GradScaler", dict(fused=True, linear="torch", amp=True), torch.float16),
+            ("amp fp16 + GradScaler fused=False", dict(fused=False, linear="torch", amp=True), torch.float16)]
     for tag, kw, dt in arms:
         m = _decoder(pkg, train=True, **kw)
         opt = torch.optim.AdamW(m.parameters(), lr=1e-4)
@@ -181,7 +267,7 @@ def part_c(pkg, args, emit):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--parts", default="a,b,c")
+    ap.add_argument("--parts", default="a,b,c", help="a, b, c: profiles/r5_mixed.jsonl; f, b, c: r6_fused_mixed.jsonl")
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--dtypes", default="fp32,bf16,fp16", help="part (a): element types of value")
@@ -204,7 +290,7 @@ def main():
         with open(path, "a") as f:
             f.write(json.dumps(rec) + "\n")
     for part in args.parts.split(","):
-        {"a": part_a, "b": part_b, "c": part_c}[part](pkg, args, emit)
+        {"a": part_a, "f": part_f, "b": part_b, "c": part_c}[part](pkg, args, emit)
 
 
 if __name__ == "__main__":

@@ -40,6 +40,12 @@ SYMBOLS = {
     "msda_b200_fused_forward_strided_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _P, _I, _P, _I, _P, _P] + _DIMS + [_P, _P]),
     "msda_b200_fused_backward_f32": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P, _P, _P, _P]),
     "msda_b200_fused_backward_deterministic_f32": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P] * 5),
+    "msda_b200_fused_forward_bf16": (_I, [_P] * 4 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P, _P]),
+    "msda_b200_fused_forward_f16": (_I, [_P] * 4 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P, _P]),
+    "msda_b200_fused_backward_bf16": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P] * 5),
+    "msda_b200_fused_backward_f16": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P] * 5),
+    "msda_b200_fused_backward_deterministic_bf16": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P] * 5),
+    "msda_b200_fused_backward_deterministic_f16": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P] * 5),
     "msda_b200_linear_f32": (_I, [_P] * 4 + [_I] * 4 + [_P, _P]),
     "msda_b200_linear_deterministic_f32": (_I, [_P] * 4 + [_I] * 4 + [_P, _P]),
     "msda_b200_split_weight_f32": (_I, [_P, _P, _I, _I, _P]),

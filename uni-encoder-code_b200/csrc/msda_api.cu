@@ -20,17 +20,19 @@
 namespace msda {
 
 // implemented in the kernel translation units.  V: element type of value / output / grad_output (float, or
-// __nv_bfloat16 / __half for the mixed-precision entries); T: of the locations, weights and sums
-template <typename V>
-cudaError_t launch_fwd_d32(const V *, const int64_t *, const int64_t *, const float *, const float *,
+// __nv_bfloat16 / __half for the mixed-precision entries); T: of the locations, weights and sums; P: of the
+// 32-channel kernels' locations / weights or raw offsets / logits and their gradients (float, or V for the
+// mixed-precision fused entries)
+template <typename V, typename P>
+cudaError_t launch_fwd_d32(const V *, const int64_t *, const int64_t *, const P *, const P *,
                            const Producers &, const Dims &, V *, cudaStream_t, bool *handled);
-template <typename V>
-cudaError_t launch_bwd_d32(const V *, const V *, const int64_t *, const int64_t *, const float *,
-                           const float *, const Producers &, const Dims &, float *, float *, float *,
+template <typename V, typename P>
+cudaError_t launch_bwd_d32(const V *, const V *, const int64_t *, const int64_t *, const P *,
+                           const P *, const Producers &, const Dims &, float *, P *, P *,
                            const DetRecords *, int gate, cudaStream_t, bool *handled);
-template <typename V>
-cudaError_t launch_bwd_sorted(const V *, const V *, const int64_t *, const int64_t *, const float *,
-                              const float *, const Producers &, const Dims &, float *, float *, float *, int gate,
+template <typename V, typename P>
+cudaError_t launch_bwd_sorted(const V *, const V *, const int64_t *, const int64_t *, const P *,
+                              const P *, const Producers &, const Dims &, float *, P *, P *, int gate,
                               cudaStream_t, bool *handled);
 template <typename V>
 bool bwd_sorted_applies(const V *value, const float *grad_value, const Dims &);
@@ -108,6 +110,9 @@ static int check_dims(const Dims &d, long long ref_bstride = 0) {
 // which accept any alignment like the reference's scalar kernels do
 static bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static bool aligned8(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 7u) == 0; }
+// the 32-channel kernels read and write an (x, y) pair of locations / offsets at once: 8 bytes in fp32, 4 in 16-bit
+template <typename P>
+static bool pair_aligned(const P *p) { return (reinterpret_cast<uintptr_t>(p) & (2 * sizeof(P) - 1)) == 0; }
 
 // the return code of a launcher that reports through `handled` whether it covers the problem
 static int launch_rc(cudaError_t e, bool handled) {
@@ -130,25 +135,30 @@ static int option_index(const char *name) {
 }
 
 // The forward of fp32 (V = float) and of the mixed-precision op (16-bit V, fp32 locations and weights): the
-// 32-channel kernel where it applies, the generic one otherwise.
-template <typename V>
-static int forward(const V *value, const int64_t *shapes, const int64_t *lstart, const float *loc,
-                   const float *attw, const Dims &d, V *output, cudaStream_t st) {
+// 32-channel kernel where it applies, the generic one otherwise.  With pr.ref set, the mixed-precision fused
+// producers (P = V: raw 16-bit offsets / logits, packed rows): the 32-channel kernel or MSDA_ERR_UNSUPPORTED.
+template <typename V, typename P = float>
+static int forward(const V *value, const int64_t *shapes, const int64_t *lstart, const P *loc,
+                   const P *attw, const Producers &pr, const Dims &d, V *output, cudaStream_t st) {
     if (!value || !shapes || !lstart || !loc || !attw || !output) return MSDA_ERR_NULL_POINTER;
-    if (int rc = check_dims(d)) return rc;
+    if (int rc = check_dims(d, pr.ref_bstride)) return rc;
+    const bool fused = pr.ref != nullptr;
     bool handled = false;
     cudaError_t e = cudaSuccess;
-    const bool fast_ok = aligned16(value) && aligned16(output) && aligned8(loc);
-    if (option_value(OPT_FWD_VARIANT) != 63 && fast_ok)   // 63 forces the generic kernel (tests)
-        e = launch_fwd_d32<V>(value, shapes, lstart, loc, attw, Producers{}, d, output, st, &handled);
-    if (e == cudaSuccess && !handled) e = launch_fwd_generic<V, float>(value, shapes, lstart, loc, attw, d, output, st);
+    const bool fast_ok = aligned16(value) && aligned16(output) && pair_aligned(loc) && aligned8(pr.ref);
+    if ((fused || option_value(OPT_FWD_VARIANT) != 63) && fast_ok)   // 63 forces the generic kernel (tests)
+        e = launch_fwd_d32<V, P>(value, shapes, lstart, loc, attw, pr, d, output, st, &handled);
+    if (e != cudaSuccess || handled || fused) return launch_rc(e, handled);
+    if constexpr (std::is_same<P, float>::value)
+        e = launch_fwd_generic<V, float>(value, shapes, lstart, loc, attw, d, output, st);
     return (int)e;
 }
 
 // The backward of fp32 (V = float) and of the mixed-precision op (16-bit V: `gv` is the caller's zero-filled fp32
 // accumulation buffer, rounded into the 16-bit grad_value by the entry afterwards), plain (pr.ref == nullptr: `loc`
 // / `attw` are the sampling locations and attention weights) or fused, fp32 only (`loc` / `attw` are the raw
-// sampling offsets and attention logits, and the gradients are taken with respect to them).  Where no 32-channel
+// sampling offsets and attention logits, and the gradients are taken with respect to them; P = V for the 16-bit
+// ones of the mixed-precision fused entries, float otherwise).  Where no 32-channel
 // kernel covers the problem (shape, or a view that is not aligned) the plain op takes the generic kernel and the
 // fused one returns MSDA_ERR_UNSUPPORTED.  "bwd_variant":
 //   0 (default): where the queries are the value pixels (encoder self-attention) the in-SM merging kernel (points
@@ -157,23 +167,23 @@ static int forward(const V *value, const int64_t *shapes, const int64_t *lstart,
 //       once (msda_common.cuh);
 //   20..39: merging kernel forced (plain: and its tuning variants); 1..8: CTA shapes of the plain per-row kernel;
 //   63: generic kernel (plain only, tests).  16-bit V takes the same meanings, each kernel in its default shape.
-template <typename V>
+template <typename V, typename P = float>
 static int backward(const V *grad_output, const V *value, const int64_t *shapes, const int64_t *lstart,
-                    const float *loc, const float *attw, const Producers &pr, const Dims &d, float *gv,
-                    float *gl, float *gw, cudaStream_t st) {
+                    const P *loc, const P *attw, const Producers &pr, const Dims &d, float *gv,
+                    P *gl, P *gw, cudaStream_t st) {
     if (!grad_output || !value || !shapes || !lstart || !loc || !attw || !gv || !gl || !gw)
         return MSDA_ERR_NULL_POINTER;
     if (int rc = check_dims(d, pr.ref_bstride)) return rc;
     const bool fused = pr.ref != nullptr;
     const int variant = option_value(OPT_BWD_VARIANT);
-    const bool aligned = aligned16(value) && aligned16(grad_output) && aligned16(gv) && aligned8(loc) &&
-                         aligned8(gl) && aligned8(pr.ref);
+    const bool aligned = aligned16(value) && aligned16(grad_output) && aligned16(gv) && pair_aligned(loc) &&
+                         pair_aligned(gl) && aligned8(pr.ref);
     bool handled = false;
     cudaError_t e = cudaSuccess;
     if (aligned && (fused || variant != 63)) {
         int gate = GATE_NONE;
         if ((variant == 0 || (variant >= 20 && variant < 40)) && bwd_sorted_applies<V>(value, gv, d)) {
-            e = launch_bwd_sorted<V>(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw,
+            e = launch_bwd_sorted<V, P>(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw,
                                   variant == 0 ? GATE_RUN_IF_LOCAL : GATE_NONE, st, &handled);
             if (variant == 0) {                  // the per-row kernel follows, gated the other way
                 handled = false;
@@ -181,33 +191,36 @@ static int backward(const V *grad_output, const V *value, const int64_t *shapes,
             }
         }
         if (e == cudaSuccess && !handled)
-            e = launch_bwd_d32<V>(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, nullptr, gate, st,
-                                  &handled);
+            e = launch_bwd_d32<V, P>(grad_output, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, nullptr, gate,
+                                     st, &handled);
     }
     if (e != cudaSuccess || handled || fused) return launch_rc(e, handled);
-    return (int)launch_bwd_generic<V, float>(grad_output, value, shapes, lstart, loc, attw, d, gv, gl, gw, st);
+    if constexpr (std::is_same<P, float>::value)
+        e = launch_bwd_generic<V, float>(grad_output, value, shapes, lstart, loc, attw, d, gv, gl, gw, st);
+    return (int)e;
 }
 
-// The mixed-precision backward: backward() into the fp32 accumulation buffer `acc`, then the conversion into the
-// 16-bit grad_value
-template <typename V>
+// The mixed-precision backward, plain or fused: backward() into the fp32 accumulation buffer `acc`, then the
+// conversion into the 16-bit grad_value
+template <typename V, typename P = float>
 static int backward_mixed(const V *grad_output, const V *value, const int64_t *shapes, const int64_t *lstart,
-                          const float *loc, const float *attw, const Dims &d, float *acc, V *gv, float *gl, float *gw,
-                          cudaStream_t st) {
+                          const P *loc, const P *attw, const Producers &pr, const Dims &d, float *acc, V *gv, P *gl,
+                          P *gw, cudaStream_t st) {
     if (!gv) return MSDA_ERR_NULL_POINTER;
-    const int rc = backward<V>(grad_output, value, shapes, lstart, loc, attw, Producers{}, d, acc, gl, gw, st);
+    const int rc = backward<V, P>(grad_output, value, shapes, lstart, loc, attw, pr, d, acc, gl, gw, st);
     if (rc != MSDA_OK) return rc;
     return (int)launch_narrow<V>(acc, gv, (long long)d.N * d.S * d.M * d.D, st);
 }
 
-// Deterministic backward (msda_det.cu), plain or fused as in backward() (fp64 and 16-bit: plain only): the records
-// kernel of the path, then sort, bounds and gather into grad_value.  V: element type of value / grad_output /
-// grad_value, T: of the locations, weights, records and sums (16-bit V: float; the gather writes the 16-bit
-// grad_value directly, no accumulation buffer).
-template <typename V, typename T>
+// Deterministic backward (msda_det.cu), plain or fused as in backward() (fp64: plain only): the records kernel of the
+// path, then sort, bounds and gather into grad_value.  V: element type of value / grad_output / grad_value, T: of the
+// records and sums (16-bit V: float; the gather writes the 16-bit grad_value directly, no accumulation buffer),
+// P: of the locations and weights or raw offsets and logits and their gradients (T, or V for the 16-bit fused
+// producers).
+template <typename V, typename T, typename P = T>
 static int backward_deterministic(const V *grad_output, const V *value, const int64_t *shapes, const int64_t *lstart,
-                                  const T *loc, const T *attw, const Producers &pr, const Dims &d, V *gv, T *gl,
-                                  T *gw, void *workspace, cudaStream_t st) {
+                                  const P *loc, const P *attw, const Producers &pr, const Dims &d, V *gv, P *gl,
+                                  P *gw, void *workspace, cudaStream_t st) {
     if (!grad_output || !value || !shapes || !lstart || !loc || !attw || !gv || !gl || !gw || !workspace)
         return MSDA_ERR_NULL_POINTER;
     if (int rc = check_dims(d, pr.ref_bstride)) return rc;
@@ -218,15 +231,16 @@ static int backward_deterministic(const V *grad_output, const V *value, const in
     bool handled = false;
     cudaError_t e = cudaSuccess;
     if constexpr (std::is_same<T, float>::value) {
-        const bool aligned = aligned16(value) && aligned16(grad_output) && aligned8(loc) && aligned8(gl) &&
+        const bool aligned = aligned16(value) && aligned16(grad_output) && pair_aligned(loc) && pair_aligned(gl) &&
                              aligned8(pr.ref);
         if (aligned && (pr.ref != nullptr || option_value(OPT_BWD_VARIANT) != 63))
-            e = launch_bwd_d32<V>(grad_output, value, shapes, lstart, loc, attw, pr, d, nullptr, gl, gw, &rec,
-                               GATE_NONE, st, &handled);
+            e = launch_bwd_d32<V, P>(grad_output, value, shapes, lstart, loc, attw, pr, d, nullptr, gl, gw, &rec,
+                                     GATE_NONE, st, &handled);
     }
     if (e == cudaSuccess && !handled) {
         if (pr.ref != nullptr) return MSDA_ERR_UNSUPPORTED;
-        e = launch_bwd_generic_records<V, T>(grad_output, value, shapes, lstart, loc, attw, d, gl, gw, rec, st);
+        if constexpr (std::is_same<P, T>::value)
+            e = launch_bwd_generic_records<V, T>(grad_output, value, shapes, lstart, loc, attw, d, gl, gw, rec, st);
     }
     if (e == cudaSuccess) e = launch_det_reduce<V, T>(l, workspace, grad_output, gv, d, st);
     return (int)e;
@@ -349,7 +363,7 @@ int msda_b200_forward_f32(const float *value, const int64_t *spatial_shapes,
                           int channels, int num_levels, int num_query, int num_point, float *output,
                           void *stream) {
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    return forward<float>(value, spatial_shapes, level_start, sampling_loc, attn_weight, d, output,
+    return forward<float>(value, spatial_shapes, level_start, sampling_loc, attn_weight, Producers{}, d, output,
                           (cudaStream_t)stream);
 }
 
@@ -505,7 +519,7 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
 }
 
 // ---- mixed precision: bf16 / fp16 value, output, grad_output and grad_value; fp32 locations, weights and their
-// gradients; fp32 sums ----
+// gradients; fp32 sums.  The fused entries: 16-bit raw offsets, logits and their gradients, fp32 reference points ----
 #define MSDA_MIXED_ENTRIES(SUFFIX, V)                                                                                \
     int msda_b200_forward_##SUFFIX(const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start,  \
                                    const float *sampling_loc, const float *attn_weight, int batch, int spatial_size,  \
@@ -513,7 +527,7 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
                                    uint16_t *output, void *stream) {                                                \
         const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};                    \
         return forward<V>(reinterpret_cast<const V *>(value), spatial_shapes, level_start, sampling_loc, attn_weight, \
-                          d, reinterpret_cast<V *>(output), (cudaStream_t)stream);                                   \
+                          Producers{}, d, reinterpret_cast<V *>(output), (cudaStream_t)stream);                      \
     }                                                                                                                \
     int msda_b200_backward_##SUFFIX(const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes, \
                                     const int64_t *level_start, const float *sampling_loc, const float *attn_weight, \
@@ -522,7 +536,8 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
                                     float *grad_sampling_loc, float *grad_attn_weight, void *stream) {               \
         const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};                    \
         return backward_mixed<V>(reinterpret_cast<const V *>(grad_output), reinterpret_cast<const V *>(value),       \
-                                 spatial_shapes, level_start, sampling_loc, attn_weight, d, grad_value_accum,        \
+                                 spatial_shapes, level_start, sampling_loc, attn_weight, Producers{}, d,             \
+                                 grad_value_accum,                                                                   \
                                  reinterpret_cast<V *>(grad_value), grad_sampling_loc, grad_attn_weight,             \
                                  (cudaStream_t)stream);                                                              \
     }                                                                                                                \
@@ -537,6 +552,49 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
                                                 sampling_loc, attn_weight, Producers{}, d,                           \
                                                 reinterpret_cast<V *>(grad_value), grad_sampling_loc,                \
                                                 grad_attn_weight, workspace, (cudaStream_t)stream);                  \
+    }                                                                                                                \
+    int msda_b200_fused_forward_##SUFFIX(const uint16_t *value, const int64_t *spatial_shapes,                       \
+                                         const int64_t *level_start, const float *reference_points,                  \
+                                         long long ref_batch_stride, const uint16_t *sampling_offsets,               \
+                                         const uint16_t *attn_logits, int batch, int spatial_size, int num_heads,    \
+                                         int channels, int num_levels, int num_query, int num_point,                 \
+                                         uint16_t *output, void *stream) {                                          \
+        if (!reference_points) return MSDA_ERR_NULL_POINTER;      /* (it selects the fused form) */                  \
+        const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};                    \
+        return forward<V, V>(reinterpret_cast<const V *>(value), spatial_shapes, level_start,                        \
+                             reinterpret_cast<const V *>(sampling_offsets), reinterpret_cast<const V *>(attn_logits), \
+                             Producers{reference_points, ref_batch_stride}, d, reinterpret_cast<V *>(output),        \
+                             (cudaStream_t)stream);                                                                  \
+    }                                                                                                                \
+    int msda_b200_fused_backward_##SUFFIX(                                                                           \
+        const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start, \
+        const float *reference_points, long long ref_batch_stride, const uint16_t *sampling_offsets,                 \
+        const uint16_t *attn_logits, int batch, int spatial_size, int num_heads, int channels, int num_levels,        \
+        int num_query, int num_point, float *grad_value_accum, uint16_t *grad_value, uint16_t *grad_sampling_offsets, \
+        uint16_t *grad_attn_logits, void *stream) {                                                                  \
+        if (!reference_points) return MSDA_ERR_NULL_POINTER;                                                         \
+        const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};                    \
+        return backward_mixed<V, V>(reinterpret_cast<const V *>(grad_output), reinterpret_cast<const V *>(value),    \
+                                    spatial_shapes, level_start, reinterpret_cast<const V *>(sampling_offsets),      \
+                                    reinterpret_cast<const V *>(attn_logits),                                        \
+                                    Producers{reference_points, ref_batch_stride}, d, grad_value_accum,              \
+                                    reinterpret_cast<V *>(grad_value), reinterpret_cast<V *>(grad_sampling_offsets), \
+                                    reinterpret_cast<V *>(grad_attn_logits), (cudaStream_t)stream);                  \
+    }                                                                                                                \
+    int msda_b200_fused_backward_deterministic_##SUFFIX(                                                             \
+        const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start, \
+        const float *reference_points, long long ref_batch_stride, const uint16_t *sampling_offsets,                 \
+        const uint16_t *attn_logits, int batch, int spatial_size, int num_heads, int channels, int num_levels,        \
+        int num_query, int num_point, uint16_t *grad_value, uint16_t *grad_sampling_offsets,                         \
+        uint16_t *grad_attn_logits, void *workspace, void *stream) {                                                 \
+        if (!reference_points) return MSDA_ERR_NULL_POINTER;                                                         \
+        const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};                    \
+        return backward_deterministic<V, float, V>(                                                                  \
+            reinterpret_cast<const V *>(grad_output), reinterpret_cast<const V *>(value), spatial_shapes, level_start, \
+            reinterpret_cast<const V *>(sampling_offsets), reinterpret_cast<const V *>(attn_logits),                 \
+            Producers{reference_points, ref_batch_stride}, d, reinterpret_cast<V *>(grad_value),                     \
+            reinterpret_cast<V *>(grad_sampling_offsets), reinterpret_cast<V *>(grad_attn_logits), workspace,        \
+            (cudaStream_t)stream);                                                                                   \
     }
 MSDA_MIXED_ENTRIES(bf16, __nv_bfloat16)
 MSDA_MIXED_ENTRIES(f16, __half)

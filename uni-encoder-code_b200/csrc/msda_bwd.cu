@@ -60,16 +60,24 @@ struct BwdCfg {
 // receive the gradients with respect to THEM (offset gradient = location gradient / (W, H);
 // softmax backward folded in), see phase1_records() in msda_common.cuh.
 // V: element type of grad_out / value (16-bit: 8-byte lane loads widened to fp32); grad_value is fp32 either way --
-// for 16-bit V the zero-filled accumulation buffer that msda_api.cu rounds into the 16-bit grad_value afterwards
+// for 16-bit V the zero-filled accumulation buffer that msda_api.cu rounds into the 16-bit grad_value afterwards.
+// FUSED with 16-bit V: the raw offsets / logits and their gradients are of type V too (ProducerT), widened as they
+// are loaded and rounded once as they are stored
 template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED, bool RECORDS>
 __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
 msda_bwd_d32_kernel(const V *__restrict__ grad_out, const V *__restrict__ value,
                     const int64_t *__restrict__ shapes, const int64_t *__restrict__ lstart,
-                    const float *__restrict__ loc, const float *__restrict__ attw,
+                    const float *__restrict__ loc_arg, const float *__restrict__ attw_arg,
                     const Producers pr, const Dims d, const int flags,
-                    float *__restrict__ grad_value, float *__restrict__ grad_loc,
-                    float *__restrict__ grad_attw, const int gate, const DetRecords det) {
+                    float *__restrict__ grad_value, float *__restrict__ grad_loc_arg,
+                    float *__restrict__ grad_attw_arg, const int gate, const DetRecords det) {
     using Cfg = BwdCfg<LP, WARPS, TILE_W, QPW>;
+    // the raw tensors are passed as float pointers whatever their type, so that the fp32 kernels keep their names
+    using PT = ProducerT<V, FUSED>;
+    const PT *__restrict__ loc = reinterpret_cast<const PT *>(loc_arg);
+    const PT *__restrict__ attw = reinterpret_cast<const PT *>(attw_arg);
+    PT *__restrict__ grad_loc = reinterpret_cast<PT *>(grad_loc_arg);
+    PT *__restrict__ grad_attw = reinterpret_cast<PT *>(grad_attw_arg);
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ LevelTable lt;
 
@@ -197,7 +205,7 @@ msda_bwd_d32_kernel(const V *__restrict__ grad_out, const V *__restrict__ value,
             float t1[Cfg::kT1], t2[Cfg::kT2];
             rs_step<Cfg::kT0>(t0, t1, c1, 16);
             rs_step<Cfg::kT1>(t1, t2, c0, 8);
-            if (!FUSED) {
+            if constexpr (!FUSED) {
 #pragma unroll
                 for (int i = 0; i < Cfg::kT2; ++i) {
                     const int u1 = i + (c0 ? Cfg::kT2 : 0);
@@ -250,8 +258,8 @@ msda_bwd_d32_kernel(const V *__restrict__ grad_out, const V *__restrict__ value,
                 for (int i = 0; i < Cfg::kT2; ++i) {
                     if (sp_of[i] >= 0) {
                         const long long sidx = qrow * LP + sp_of[i];
-                        if (comp_of[i] == 2) stg_stream_f1(grad_attw + sidx, prob[i] * (t2[i] - dot_a));
-                        else stg_stream_f1(grad_loc + 2 * sidx + comp_of[i], __fdiv_rn(t2[i], div[i]));
+                        if (comp_of[i] == 2) stg_stream_v1<PT>(grad_attw + sidx, prob[i] * (t2[i] - dot_a));
+                        else stg_stream_v1<PT>(grad_loc + 2 * sidx + comp_of[i], __fdiv_rn(t2[i], div[i]));
                     }
                 }
             }
@@ -265,34 +273,42 @@ msda_bwd_d32_kernel(const V *__restrict__ grad_out, const V *__restrict__ value,
 // the deterministic records (msda_det.cu), the last two in the default CTA shape only
 // ---------------------------------------------------------------------------
 template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int BATCH, int QPW, bool FUSED, bool RECORDS>
-static cudaError_t launch_bwd_cfg(const V *grad_out, const V *value, const int64_t *shapes,
-                                  const int64_t *lstart, const float *loc, const float *attw, const Producers &pr,
-                                  const Dims &d, float *grad_value, float *grad_loc, float *grad_attw,
-                                  const DetRecords &det, int gate, cudaStream_t stream) {
+static cudaError_t launch_bwd_cfg(const V *grad_out, const V *value, const int64_t *shapes, const int64_t *lstart,
+                                  const ProducerT<V, FUSED> *loc, const ProducerT<V, FUSED> *attw, const Producers &pr,
+                                  const Dims &d, float *grad_value, ProducerT<V, FUSED> *grad_loc,
+                                  ProducerT<V, FUSED> *grad_attw, const DetRecords &det, int gate,
+                                  cudaStream_t stream) {
     using Cfg = BwdCfg<LP, WARPS, TILE_W, QPW>;
     constexpr auto kern = msda_bwd_d32_kernel<V, LP, WARPS, TILE_W, MIN_CTAS, BATCH, QPW, FUSED, RECORDS>;
     cudaError_t e;
     const int blocks = persistent_blocks<kern>(WARPS * 32, Cfg::kSmem, d, &e);
     if (blocks == 0) return e;
     const int flags = (option_value(OPT_TILE_ORDER) != 1 ? 1 : 0) | (whatif_value(OPT_WHATIF_DROP_REDS) << 1);
-    kern<<<blocks, WARPS * 32, Cfg::kSmem, stream>>>(grad_out, value, shapes, lstart, loc, attw, pr, d, flags,
-                                                     grad_value, grad_loc, grad_attw, gate, det);
+    kern<<<blocks, WARPS * 32, Cfg::kSmem, stream>>>(grad_out, value, shapes, lstart, reinterpret_cast<const float *>(loc),
+                                                     reinterpret_cast<const float *>(attw), pr, d, flags, grad_value,
+                                                     reinterpret_cast<float *>(grad_loc),
+                                                     reinterpret_cast<float *>(grad_attw), gate, det);
     note_launch();
     return cudaGetLastError();
 }
 
-template <typename V, int LP>
+template <typename V, typename P, int LP>
 static cudaError_t launch_bwd_lp(const V *grad_out, const V *value, const int64_t *shapes,
-                                 const int64_t *lstart, const float *loc, const float *attw, const Producers &pr,
-                                 const Dims &d, float *gv, float *gl, float *gw, const DetRecords *det, int gate,
+                                 const int64_t *lstart, const P *loc, const P *attw, const Producers &pr,
+                                 const Dims &d, float *gv, P *gl, P *gw, const DetRecords *det, int gate,
                                  cudaStream_t st) {
     // variant = (warps, query tile width, min CTAs per SM -> register budget, load batch in pairs,
     //            queries per warp)
 #define MSDA_BWD(W, TW, C, B, Q, F, R) \
     launch_bwd_cfg<V, LP, W, TW, C, B, Q, F, R>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, \
                                              R ? *det : DetRecords{}, gate, st)
-    // 16-bit (plain only), fused producers and the deterministic records: the default shape only
-    if constexpr (is16<V>) {
+    // 16-bit, fused producers and the deterministic records: the default shape only (16-bit fused at L*P = 16: below)
+    if constexpr (is16<P>) {          // 16-bit fused producers
+        if constexpr (LP == 16)       // 12 warps (85 registers): in the default shape they spill
+            return det != nullptr ? MSDA_BWD(12, 16, 2, 1, 8, true, true) : MSDA_BWD(12, 16, 2, 1, 8, true, false);
+        else
+            return det != nullptr ? MSDA_BWD(16, 16, 2, 1, 8, true, true) : MSDA_BWD(16, 16, 2, 1, 8, true, false);
+    } else if constexpr (is16<V>) {   // 16-bit plain
         return det != nullptr ? MSDA_BWD(16, 16, 2, 1, 8, false, true) : MSDA_BWD(16, 16, 2, 1, 8, false, false);
     } else {
     if (det != nullptr)
@@ -314,30 +330,33 @@ static cudaError_t launch_bwd_lp(const V *grad_out, const V *value, const int64_
 }
 
 // pr.ref == nullptr: plain; otherwise fused producers, gradients w.r.t. the raw sampling offsets (`loc`) and
-// attention logits (`attw`).  det != nullptr: deterministic mode (msda_det.cu), grad_value `gv` is not touched and
+// attention logits (`attw`).  P: element type of `loc` / `attw` / `gl` / `gw` -- float, or V for the 16-bit fused
+// producers.  det != nullptr: deterministic mode (msda_det.cu), grad_value `gv` is not touched and
 // the corner records go to `det`.  `gate`: see msda_bwd_sorted.cu.  `handled` = false: the problem is outside
 // d32_applies() and nothing was launched.
-template <typename V>
+template <typename V, typename P>
 cudaError_t launch_bwd_d32(const V *grad_out, const V *value, const int64_t *shapes, const int64_t *lstart,
-                           const float *loc, const float *attw, const Producers &pr, const Dims &d, float *gv,
-                           float *gl, float *gw, const DetRecords *det, int gate, cudaStream_t st, bool *handled) {
+                           const P *loc, const P *attw, const Producers &pr, const Dims &d, float *gv,
+                           P *gl, P *gw, const DetRecords *det, int gate, cudaStream_t st, bool *handled) {
     *handled = d32_applies(d);
     if (!*handled) return cudaSuccess;
     switch (d.L * d.P) {       // 4, 8, 12 or 16 (d32_applies)
-        case 4: return launch_bwd_lp<V, 4>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
-        case 8: return launch_bwd_lp<V, 8>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
-        case 12: return launch_bwd_lp<V, 12>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
-        default: return launch_bwd_lp<V, 16>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        case 4: return launch_bwd_lp<V, P, 4>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        case 8: return launch_bwd_lp<V, P, 8>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        case 12: return launch_bwd_lp<V, P, 12>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
+        default: return launch_bwd_lp<V, P, 16>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, gw, det, gate, st);
     }
 }
 
-#define MSDA_BWD_D32(V)                                                                                             \
-    template cudaError_t launch_bwd_d32<V>(const V *, const V *, const int64_t *, const int64_t *, const float *,    \
-                                           const float *, const Producers &, const Dims &, float *, float *, float *, \
-                                           const DetRecords *, int, cudaStream_t, bool *);
-MSDA_BWD_D32(float)
-MSDA_BWD_D32(__nv_bfloat16)
-MSDA_BWD_D32(__half)
+#define MSDA_BWD_D32(V, P)                                                                                       \
+    template cudaError_t launch_bwd_d32<V, P>(const V *, const V *, const int64_t *, const int64_t *, const P *, \
+                                              const P *, const Producers &, const Dims &, float *, P *, P *,     \
+                                              const DetRecords *, int, cudaStream_t, bool *);
+MSDA_BWD_D32(float, float)
+MSDA_BWD_D32(__nv_bfloat16, float)
+MSDA_BWD_D32(__half, float)
+MSDA_BWD_D32(__nv_bfloat16, __nv_bfloat16)
+MSDA_BWD_D32(__half, __half)
 #undef MSDA_BWD_D32
 
 }  // namespace msda

@@ -341,15 +341,22 @@ __device__ __forceinline__ void red_add_f4(float4 *p, const float4 v) {
 //      through shared memory), the epilogue applies 1 / (W, H) and the softmax backward.
 // V: element type of grad_out / value.  16-bit: the grad_output tile is widened to fp32 while it is staged (the merge
 // loop reads it as for fp32), a lane's value chunk is 8 bytes of a 64-byte row, and grad_value is the fp32
-// accumulation buffer (128-byte rows, as for fp32)
+// accumulation buffer (128-byte rows, as for fp32).  FUSED with 16-bit V: the raw offsets / logits and their
+// gradients are of type V too (ProducerT), widened in pass A and the epilogue, rounded once as they are stored
 template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int TILE_Q, int SLOTS, int GW, bool FUSED>
 __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
 msda_bwd_sorted_kernel(const V *__restrict__ grad_out, const V *__restrict__ value,
                        const int64_t *__restrict__ shapes, const int64_t *__restrict__ lstart,
-                       const float *__restrict__ loc, const float *__restrict__ attw, const Producers pr, const Dims d,
-                       const int flags, float *__restrict__ grad_value, float *__restrict__ grad_loc,
-                       float *__restrict__ grad_attw, const int gate) {
+                       const float *__restrict__ loc_arg, const float *__restrict__ attw_arg, const Producers pr,
+                       const Dims d, const int flags, float *__restrict__ grad_value,
+                       float *__restrict__ grad_loc_arg, float *__restrict__ grad_attw_arg, const int gate) {
     using Cfg = SortCfg<LP, WARPS, TILE_W, TILE_Q, SLOTS>;
+    // the raw tensors are passed as float pointers whatever their type, so that the fp32 kernels keep their names
+    using PT = ProducerT<V, FUSED>;
+    const PT *__restrict__ loc = reinterpret_cast<const PT *>(loc_arg);
+    const PT *__restrict__ attw = reinterpret_cast<const PT *>(attw_arg);
+    PT *__restrict__ grad_loc = reinterpret_cast<PT *>(grad_loc_arg);
+    PT *__restrict__ grad_attw = reinterpret_cast<PT *>(grad_attw_arg);
     constexpr int NT = Cfg::kThreads;
     constexpr int kSortTile = Cfg::kSortTile, kSortSlots = Cfg::kSortSlots;
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -399,8 +406,8 @@ msda_bwd_sorted_kernel(const V *__restrict__ grad_out, const V *__restrict__ val
         // rows of image n: 64-bit bases here, 32-bit offsets (query * M + m) * {8, LP} below
         // (Lq * M * 16 < 2^32: host check)
         const V *go_n = grad_out + n * Lq * (long long)M * 32;
-        const float2 *loc_n = reinterpret_cast<const float2 *>(loc) + n * Lq * (long long)M * LP;
-        const float *attw_n = attw + n * Lq * (long long)M * LP;
+        const Pair<PT> *loc_n = reinterpret_cast<const Pair<PT> *>(loc) + n * Lq * (long long)M * LP;
+        const PT *attw_n = attw + n * Lq * (long long)M * LP;
 
         uint32_t n_in;
         {
@@ -463,9 +470,9 @@ msda_bwd_sorted_kernel(const V *__restrict__ grad_out, const V *__restrict__ val
                         const int qg = tile_query<TILE_W>(tm, q, Lq);
                         if (qg >= 0) {
                             const uint32_t row = (uint32_t)(qg * M + m) * (uint32_t)LP + (uint32_t)p;
-                            const float2 xy = ldg_stream_f2(loc_n + row);
+                            const float2 xy = ldg_stream_pair<PT>(loc_n + row);
                             px[r] = xy.x; py[r] = xy.y;
-                            pw[r] = ldg_stream_f1(attw_n + row);
+                            pw[r] = ldg_stream_one<PT>(attw_n + row);
                             if (FUSED)
                                 rp[r] = ldg_stream_f2(reinterpret_cast<const float2 *>(
                                     pr.ref + n * pr.ref_bstride + ((long long)qg * L + lt.level_of[p]) * 2));
@@ -713,8 +720,8 @@ msda_bwd_sorted_kernel(const V *__restrict__ grad_out, const V *__restrict__ val
         // loads are issued before the barrier so that they fly while the warp waits)
         {
             const TileMap te = tile_of<TILE_W, Cfg::kTileH>(lt, L, g);
-            float2 *gloc_n = reinterpret_cast<float2 *>(grad_loc) + n * Lq * (long long)M * LP;
-            float *gattw_n = grad_attw + n * Lq * (long long)M * LP;
+            Pair<PT> *gloc_n = reinterpret_cast<Pair<PT> *>(grad_loc) + n * Lq * (long long)M * LP;
+            PT *gattw_n = grad_attw + n * Lq * (long long)M * LP;
             float2 exy[Cfg::kRounds];
             float2 erp[FUSED ? Cfg::kRounds : 1];
             float eaw[Cfg::kRounds];
@@ -731,12 +738,12 @@ msda_bwd_sorted_kernel(const V *__restrict__ grad_out, const V *__restrict__ val
                 eaw[r] = 0.f;
                 if (FUSED) erp[r] = make_float2(0.f, 0.f);
                 if (elive[r]) {
-                    exy[r] = ldg_stream_f2(loc_n + erow[r]);
+                    exy[r] = ldg_stream_pair<PT>(loc_n + erow[r]);
                     if (FUSED)
                         erp[r] = ldg_stream_f2(reinterpret_cast<const float2 *>(
                             pr.ref + n * pr.ref_bstride + ((long long)qg * L + lt.level_of[p]) * 2));
                     else
-                        eaw[r] = ldg_stream_f1(attw_n + erow[r]);
+                        eaw[r] = ldg_stream_one<PT>(attw_n + erow[r]);
                 }
             }
             __syncthreads();                                                // B5: D complete
@@ -794,9 +801,8 @@ msda_bwd_sorted_kernel(const V *__restrict__ grad_out, const V *__restrict__ val
 #pragma unroll
             for (int r = 0; r < Cfg::kRounds; ++r) {
                 if (elive[r]) {
-                    asm volatile("st.global.L1::no_allocate.v2.f32 [%0], {%1,%2};"
-                                 ::"l"(gloc_n + erow[r]), "f"(egx[r]), "f"(egy[r]) : "memory");
-                    stg_stream_f1(gattw_n + erow[r], ega[r]);
+                    stg_stream_pair<PT>(gloc_n + erow[r], egx[r], egy[r]);
+                    stg_stream_v1<PT>(gattw_n + erow[r], ega[r]);
                 }
             }
         }
@@ -809,9 +815,10 @@ msda_bwd_sorted_kernel(const V *__restrict__ grad_out, const V *__restrict__ val
 // ---------------------------------------------------------------------------
 template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int TILE_Q, int SLOTS, int GW, bool FUSED>
 static cudaError_t launch_bwd_sorted_cfg(const V *grad_out, const V *value, const int64_t *shapes,
-                                         const int64_t *lstart, const float *loc, const float *attw,
-                                         const Producers &pr, const Dims &d, float *gv, float *gl, float *gw,
-                                         int gate, cudaStream_t stream) {
+                                         const int64_t *lstart, const ProducerT<V, FUSED> *loc,
+                                         const ProducerT<V, FUSED> *attw, const Producers &pr, const Dims &d,
+                                         float *gv, ProducerT<V, FUSED> *gl, ProducerT<V, FUSED> *gw, int gate,
+                                         cudaStream_t stream) {
     using Cfg = SortCfg<LP, WARPS, TILE_W, TILE_Q, SLOTS>;
     constexpr auto kern = msda_bwd_sorted_kernel<V, LP, WARPS, TILE_W, MIN_CTAS, TILE_Q, SLOTS, GW, FUSED>;
     constexpr size_t kSmemBytes = Cfg::kSmem + (FUSED ? (size_t)Cfg::kPoints * sizeof(float) : 0);
@@ -819,8 +826,9 @@ static cudaError_t launch_bwd_sorted_cfg(const V *grad_out, const V *value, cons
     const int blocks = persistent_blocks<kern>(WARPS * 32, kSmemBytes, d, &e);
     if (blocks == 0) return e;
     const int flags = option_value(OPT_TILE_ORDER) != 1 ? 1 : 0;
-    kern<<<blocks, WARPS * 32, kSmemBytes, stream>>>(grad_out, value, shapes, lstart, loc, attw, pr, d, flags, gv,
-                                                     gl, gw, gate);
+    kern<<<blocks, WARPS * 32, kSmemBytes, stream>>>(grad_out, value, shapes, lstart, reinterpret_cast<const float *>(loc),
+                                                     reinterpret_cast<const float *>(attw), pr, d, flags, gv,
+                                                     reinterpret_cast<float *>(gl), reinterpret_cast<float *>(gw), gate);
     note_launch();
     return cudaGetLastError();
 }
@@ -837,12 +845,13 @@ bool bwd_sorted_applies(const V *value, const float *gv, const Dims &d) {
 }
 
 // pr.ref == nullptr: plain; otherwise fused producers, gradients w.r.t. the raw sampling offsets (`loc`) and
-// attention logits (`attw`), default shapes only.  `handled` = false: shape outside this kernel's domain (the
-// caller falls back to msda_bwd.cu)
-template <typename V>
+// attention logits (`attw`), default shapes only (16-bit at L*P = 8: see below).  P: element type of `loc` / `attw` / `gl` / `gw` -- float, or V
+// for the 16-bit fused producers.  `handled` = false: shape outside this kernel's domain (the caller falls back to
+// msda_bwd.cu)
+template <typename V, typename P>
 cudaError_t launch_bwd_sorted(const V *grad_out, const V *value, const int64_t *shapes,
-                              const int64_t *lstart, const float *loc, const float *attw, const Producers &pr,
-                              const Dims &d, float *gv, float *gl, float *gw, int gate, cudaStream_t stream,
+                              const int64_t *lstart, const P *loc, const P *attw, const Producers &pr,
+                              const Dims &d, float *gv, P *gl, P *gw, int gate, cudaStream_t stream,
                               bool *handled) {
     *handled = bwd_sorted_applies(value, gv, d);
     if (!*handled) return cudaSuccess;
@@ -850,7 +859,15 @@ cudaError_t launch_bwd_sorted(const V *grad_out, const V *value, const int64_t *
 #define MSDA_SORTED(LPV, W, TW, C, TQ, SL, GWV, F) \
     launch_bwd_sorted_cfg<V, LPV, W, TW, C, TQ, SL, GWV, F>(grad_out, value, shapes, lstart, loc, attw, pr, d, gv, gl, \
                                                          gw, gate, stream)
-    if constexpr (is16<V>) {   // 16-bit (plain only): the default shapes only
+    if constexpr (is16<P>) {   // 16-bit fused producers: 4 lanes per record, as fp32 fused (the same D summation order)
+        switch (d.L * d.P) {
+            case 4: return MSDA_SORTED(4, 16, 16, 2, 128, 4096, 4, true);
+            // 8 warps, 64-query tiles, 3 CTAs per SM (85 registers): in the fp32 fused shape it spills
+            case 8: return MSDA_SORTED(8, 8, 8, 3, 64, 2048, 4, true);
+            case 12: return MSDA_SORTED(12, 16, 16, 2, 128, 4096, 4, true);
+            default: return MSDA_SORTED(16, 16, 16, 1, 128, 4096, 4, true);
+        }
+    } else if constexpr (is16<V>) {   // 16-bit plain: the default shapes only
         switch (d.L * d.P) {
             case 4: return MSDA_SORTED(4, 16, 16, 2, 128, 4096, 8, false);
             case 8: return MSDA_SORTED(8, 16, 16, 2, 128, 4096, 8, false);
@@ -889,14 +906,18 @@ cudaError_t launch_bwd_sorted(const V *grad_out, const V *value, const int64_t *
 #undef MSDA_SORTED
 }
 
-#define MSDA_SORTED_V(V)                                                                                              \
-    template bool bwd_sorted_applies<V>(const V *, const float *, const Dims &);                                       \
-    template cudaError_t launch_bwd_sorted<V>(const V *, const V *, const int64_t *, const int64_t *, const float *,   \
-                                              const float *, const Producers &, const Dims &, float *, float *, float *, \
-                                              int, cudaStream_t, bool *);
-MSDA_SORTED_V(float)
-MSDA_SORTED_V(__nv_bfloat16)
-MSDA_SORTED_V(__half)
+#define MSDA_SORTED_V(V, P)                                                                                         \
+    template cudaError_t launch_bwd_sorted<V, P>(const V *, const V *, const int64_t *, const int64_t *, const P *, \
+                                                 const P *, const Producers &, const Dims &, float *, P *, P *, int, \
+                                                 cudaStream_t, bool *);
+template bool bwd_sorted_applies<float>(const float *, const float *, const Dims &);
+template bool bwd_sorted_applies<__nv_bfloat16>(const __nv_bfloat16 *, const float *, const Dims &);
+template bool bwd_sorted_applies<__half>(const __half *, const float *, const Dims &);
+MSDA_SORTED_V(float, float)
+MSDA_SORTED_V(__nv_bfloat16, float)
+MSDA_SORTED_V(__half, float)
+MSDA_SORTED_V(__nv_bfloat16, __nv_bfloat16)
+MSDA_SORTED_V(__half, __half)
 #undef MSDA_SORTED_V
 
 }  // namespace msda

@@ -366,6 +366,84 @@ __device__ __forceinline__ void stg_stream_v1(V *p, float v) {
 }
 
 // ---------------------------------------------------------------------------
+// Element type of the fused producers' raw tensors (sampling offsets, attention logits and their
+// gradients): fp32, or -- in the mixed-precision fused op -- the value's 16-bit type, widened to fp32 on
+// load and rounded once at the store.  The plain op's locations and weights are fp32 for every V.
+// ---------------------------------------------------------------------------
+template <typename V, bool FUSED>
+using ProducerT = std::conditional_t<FUSED, V, float>;
+// one (x, y) pair of offsets / locations: float2, or two 16-bit values in one 32-bit word
+template <typename P>
+using Pair = std::conditional_t<is16<P>, uint32_t, float2>;
+
+template <typename P>
+__device__ __forceinline__ float widen1(unsigned short bits) {
+    if constexpr (std::is_same<P, __nv_bfloat16>::value) return __uint_as_float((uint32_t)bits << 16);
+    else return __half2float(__ushort_as_half(bits));
+}
+template <typename P>
+__device__ __forceinline__ float2 widen2(uint32_t u) {
+    if constexpr (std::is_same<P, __nv_bfloat16>::value) {
+        return make_float2(__uint_as_float(u << 16), __uint_as_float(u & 0xffff0000u));
+    } else {
+        __half2 h;
+        memcpy(&h, &u, 4);
+        return __half22float2(h);
+    }
+}
+template <typename P>
+__device__ __forceinline__ float2 widen_pair(Pair<P> v) {
+    if constexpr (!is16<P>) return v;
+    else return widen2<P>(v);
+}
+// a pair read once (LDG.64 fp32, one 4-byte load 16-bit), as loaded: 16-bit pairs take one register until widened
+template <typename P>
+__device__ __forceinline__ Pair<P> ldg_stream_pair_raw(const Pair<P> *p) {
+    if constexpr (!is16<P>) {
+        return ldg_stream_f2(p);
+    } else {
+        uint32_t u;
+        asm("ld.global.nc.L1::no_allocate.b32 %0, [%1];" : "=r"(u) : "l"(p));
+        return u;
+    }
+}
+template <typename P>
+__device__ __forceinline__ float2 ldg_stream_pair(const Pair<P> *p) {
+    return widen_pair<P>(ldg_stream_pair_raw<P>(p));
+}
+// the same through the default cache path (the backward kernels' location probe)
+template <typename P>
+__device__ __forceinline__ float2 ld_pair(const Pair<P> *p) {
+    if constexpr (!is16<P>) return *p;
+    else return widen2<P>(*p);
+}
+// one element read once (a logit / attention weight)
+template <typename P>
+__device__ __forceinline__ float ldg_stream_one(const P *p) {
+    if constexpr (!is16<P>) {
+        return ldg_stream_f1(p);
+    } else {
+        unsigned short u;
+        asm("ld.global.nc.L1::no_allocate.b16 %0, [%1];" : "=h"(u) : "l"(p));
+        return widen1<P>(u);
+    }
+}
+// one pair of results, each rounded to P (one 8-byte / 4-byte store)
+template <typename P>
+__device__ __forceinline__ void stg_stream_pair(Pair<P> *p, float x, float y) {
+    if constexpr (!is16<P>) {
+        asm volatile("st.global.L1::no_allocate.v2.f32 [%0], {%1,%2};" ::"l"(p), "f"(x), "f"(y) : "memory");
+    } else {
+        const P hx = narrow<P>(x), hy = narrow<P>(y);
+        unsigned short bx, by;
+        memcpy(&bx, &hx, 2);
+        memcpy(&by, &hy, 2);
+        asm volatile("st.global.L1::no_allocate.b32 [%0], %1;" ::"l"(p), "r"((uint32_t)bx | ((uint32_t)by << 16))
+                     : "memory");
+    }
+}
+
+// ---------------------------------------------------------------------------
 // Warp reduce-scatter: n per-lane values are summed across the two lanes that
 // differ in one lane-id bit; each lane keeps ceil(n/2) of the sums.  Repeating it
 // over k bits sums across 2^k lanes with ~n shuffles in total instead of n*k.
@@ -427,24 +505,27 @@ struct Producers {
     const float *logit_table;
 };
 
-template <bool FUSED, int LP, int QPW, int PLANE, bool WITH_AUX>
+// PT: element type of `loc` / `attw` (ProducerT: 16-bit only for the mixed-precision fused op, whose rows are packed:
+// the row strides and tables of Producers are the fp32 packed forward's)
+template <bool FUSED, int LP, int QPW, int PLANE, bool WITH_AUX, typename PT>
 __device__ __forceinline__ void phase1_records(const LevelTable &lt, uint2 *rec, float4 *aux,
-                                               const float *__restrict__ loc,
-                                               const float *__restrict__ attw, const Producers pr,
+                                               const PT *__restrict__ loc,
+                                               const PT *__restrict__ attw, const Producers pr,
                                                long long n, int q0, int cnt, int m, int M, int Lq,
                                                int L, uint32_t pix_stride, uint32_t image_f4, int lane) {
     constexpr int kRounds = (QPW * LP + 31) / 32;
-    float2 xy[kRounds];
+    constexpr bool kStrided = FUSED && !is16<PT>;   // row strides / tables may be set
+    Pair<PT> xy[kRounds];       // as loaded (16-bit: widened where used, one register per pair until then)
     float aw[kRounds];          // attention weight; FUSED: the raw logit until the softmax below
     float2 txy[FUSED ? kRounds : 1];   // FUSED with tables: the table entries, added once ALL loads are in flight
     float taw[FUSED ? kRounds : 1];
-    const long long tab_li = FUSED ? n * Lq * (long long)((pr.off_qstride != 0 ? pr.off_qstride : M * LP * 2) >> 1) : 0;
-    const long long tab_ai = FUSED ? n * Lq * (long long)(pr.logit_qstride != 0 ? pr.logit_qstride : M * LP) : 0;
+    const long long tab_li = kStrided ? n * Lq * (long long)((pr.off_qstride != 0 ? pr.off_qstride : M * LP * 2) >> 1) : 0;
+    const long long tab_ai = kStrided ? n * Lq * (long long)(pr.logit_qstride != 0 ? pr.logit_qstride : M * LP) : 0;
 #pragma unroll
     for (int r = 0; r < kRounds; ++r) {          // all global loads first
         const int s = r * 32 + lane;
         const int qi = s / LP, sp = s - qi * LP;
-        xy[r] = make_float2(0.f, 0.f);
+        xy[r] = Pair<PT>{};
         aw[r] = 0.f;
         if (FUSED) {
             txy[r] = make_float2(0.f, 0.f);
@@ -453,14 +534,14 @@ __device__ __forceinline__ void phase1_records(const LevelTable &lt, uint2 *rec,
         if (qi < cnt) {                           // also false for the padding lanes of the last round
             const long long qrow = (n * Lq + q0 + qi) * M + m;
             long long li = qrow * LP + sp, ai = li;
-            if (FUSED && pr.off_qstride != 0) {
+            if (kStrided && pr.off_qstride != 0) {
                 const long long q = n * Lq + q0 + qi;
                 li = q * (pr.off_qstride >> 1) + m * LP + sp;
                 ai = q * pr.logit_qstride + m * LP + sp;
             }
-            xy[r] = ldg_stream_f2(reinterpret_cast<const float2 *>(loc) + li);
-            aw[r] = ldg_stream_f1(attw + ai);
-            if (FUSED && pr.off_table != nullptr) {
+            xy[r] = ldg_stream_pair_raw<PT>(reinterpret_cast<const Pair<PT> *>(loc) + li);
+            aw[r] = ldg_stream_one<PT>(attw + ai);
+            if (kStrided && pr.off_table != nullptr) {
                 // the tables have Lq rows with the projections' row strides: entry = the projection's index
                 // minus the image's n * Lq rows (tab_li / tab_ai below).  Reused by every image, but by one warp
                 // per image: kept out of L1 (whose lines phase 2's value rows live on), served by L2
@@ -469,12 +550,14 @@ __device__ __forceinline__ void phase1_records(const LevelTable &lt, uint2 *rec,
             }
         }
     }
-    if (FUSED && pr.off_table != nullptr) {
+    if constexpr (kStrided) {
+        if (pr.off_table != nullptr) {
 #pragma unroll
-        for (int r = 0; r < kRounds; ++r) {
-            xy[r].x += txy[r].x;
-            xy[r].y += txy[r].y;
-            aw[r] += taw[r];
+            for (int r = 0; r < kRounds; ++r) {
+                xy[r].x += txy[r].x;
+                xy[r].y += txy[r].y;
+                aw[r] += taw[r];
+            }
         }
     }
     if (FUSED) {
@@ -529,7 +612,8 @@ __device__ __forceinline__ void phase1_records(const LevelTable &lt, uint2 *rec,
         if (qi < cnt) {
             const int l = lt.level_of[sp];
             const int4 lv = lt.hws[l];            // {H, W, start, -}
-            float x = xy[r].x, y = xy[r].y;
+            const float2 xyf = widen_pair<PT>(xy[r]);
+            float x = xyf.x, y = xyf.y;
             if (FUSED) {
                 const long long rrow = n * pr.ref_bstride + ((long long)(q0 + qi) * L + l) * 2;
                 const float2 rp = ldg_stream_f2(reinterpret_cast<const float2 *>(pr.ref + rrow));
@@ -572,8 +656,8 @@ enum { GATE_NONE = 0, GATE_RUN_IF_LOCAL = 1, GATE_RUN_IF_SPREAD = 2 };
 
 // FUSED: `loc` holds the raw sampling offsets, which ARE the distance from the query's own position in
 // pixels of the sampled level (location = ref + offset / (W, H), mod.py:110-112).
-template <bool FUSED = false>
-__device__ __forceinline__ bool probe_points_stay_local(const LevelTable &lt, const float *__restrict__ loc,
+template <bool FUSED = false, typename PT = float>
+__device__ __forceinline__ bool probe_points_stay_local(const LevelTable &lt, const PT *__restrict__ loc,
                                                         int N, int Lq, int M, int L, int P) {
     __shared__ int probe_in, probe_all;
     if (threadIdx.x == 0) { probe_in = 0; probe_all = 0; }
@@ -590,7 +674,7 @@ __device__ __forceinline__ bool probe_points_stay_local(const LevelTable &lt, co
             h = h * 1664525u + 1013904223u;
             const int m = (int)((h >> 8) % (uint32_t)M), sp = (int)((h >> 16) % (uint32_t)LP);
             if (FUSED) {
-                const float2 off = reinterpret_cast<const float2 *>(loc)[(((long long)n * Lq + q) * M + m) * LP + sp];
+                const float2 off = ld_pair<PT>(reinterpret_cast<const Pair<PT> *>(loc) + ((((long long)n * Lq + q) * M + m) * LP + sp));
                 ++n_all;
                 if (fabsf(off.x) <= kProbeMarginPx && fabsf(off.y) <= kProbeMarginPx) ++n_in;
                 continue;

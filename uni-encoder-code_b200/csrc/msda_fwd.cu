@@ -48,14 +48,19 @@ struct FwdCfg {
 };
 
 // V: element type of value / out (float, or 16-bit: a lane's chunk is then 8 bytes of a 64-byte row,
-// loaded as LDG.64 and widened to fp32; the sums are fp32 and only the output store rounds)
+// loaded as LDG.64 and widened to fp32; the sums are fp32 and only the output store rounds).  FUSED with 16-bit V:
+// the raw offsets / logits are of type V too (ProducerT), widened as they are loaded
 template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
 __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
 msda_fwd_d32_kernel(const V *__restrict__ value, const int64_t *__restrict__ shapes,
-                    const int64_t *__restrict__ lstart, const float *__restrict__ loc,
-                    const float *__restrict__ attw, const Producers pr, const Dims d,
+                    const int64_t *__restrict__ lstart, const float *__restrict__ loc_arg,
+                    const float *__restrict__ attw_arg, const Producers pr, const Dims d,
                     const int want_spatial, V *__restrict__ out) {
     using Cfg = FwdCfg<LP, WARPS, TILE_W, QPW>;
+    // the raw tensors are passed as float pointers whatever their type, so that the fp32 kernels keep their names
+    using PT = ProducerT<V, FUSED>;
+    const PT *__restrict__ loc = reinterpret_cast<const PT *>(loc_arg);
+    const PT *__restrict__ attw = reinterpret_cast<const PT *>(attw_arg);
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ LevelTable lt;
 
@@ -132,27 +137,30 @@ msda_fwd_d32_kernel(const V *__restrict__ value, const int64_t *__restrict__ sha
 // ---------------------------------------------------------------------------
 template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
 static cudaError_t launch_fwd_cfg(const V *value, const int64_t *shapes, const int64_t *lstart,
-                                  const float *loc, const float *attw, const Producers &pr, const Dims &d,
-                                  V *out, cudaStream_t stream) {
+                                  const ProducerT<V, FUSED> *loc, const ProducerT<V, FUSED> *attw, const Producers &pr,
+                                  const Dims &d, V *out, cudaStream_t stream) {
     using Cfg = FwdCfg<LP, WARPS, TILE_W, QPW>;
     constexpr auto kern = msda_fwd_d32_kernel<V, LP, WARPS, TILE_W, MIN_CTAS, QPW, FUSED>;
     cudaError_t e;
     const int blocks = persistent_blocks<kern>(WARPS * 32, Cfg::kSmem, d, &e);
     if (blocks == 0) return e;
     const int want_spatial = option_value(OPT_TILE_ORDER) != 1;
-    kern<<<blocks, WARPS * 32, Cfg::kSmem, stream>>>(value, shapes, lstart, loc, attw, pr, d, want_spatial, out);
+    kern<<<blocks, WARPS * 32, Cfg::kSmem, stream>>>(value, shapes, lstart, reinterpret_cast<const float *>(loc),
+                                                     reinterpret_cast<const float *>(attw), pr, d, want_spatial, out);
     note_launch();
     return cudaGetLastError();
 }
 
-template <typename V, int LP>
+template <typename V, typename P, int LP>
 static cudaError_t launch_fwd_lp(const V *value, const int64_t *shapes, const int64_t *lstart,
-                                 const float *loc, const float *attw, const Producers &pr, const Dims &d,
+                                 const P *loc, const P *attw, const Producers &pr, const Dims &d,
                                  V *out, cudaStream_t stream) {
     // variant = (warps, query tile width, min CTAs per SM -> register budget, queries per warp)
 #define MSDA_FWD(W, TW, C, Q, F) launch_fwd_cfg<V, LP, W, TW, C, Q, F>(value, shapes, lstart, loc, attw, pr, d, out, stream)
-    if constexpr (is16<V>) {
-        return MSDA_FWD(16, 16, 2, 8, false);                     // 16-bit (plain only): the default shape only
+    if constexpr (is16<P>) {
+        return MSDA_FWD(16, 16, 2, 8, true);                      // 16-bit fused producers: the default shape only
+    } else if constexpr (is16<V>) {
+        return MSDA_FWD(16, 16, 2, 8, false);                     // 16-bit plain: the default shape only
     } else {
     if (pr.ref != nullptr) return MSDA_FWD(16, 16, 2, 8, true);   // fused producers: the default shape only
     switch (option_value(OPT_FWD_VARIANT)) {
@@ -173,26 +181,29 @@ static cudaError_t launch_fwd_lp(const V *value, const int64_t *shapes, const in
 // pr.ref == nullptr: plain, `loc` / `attw` are the sampling locations and attention weights.  Otherwise fused
 // producers (SURVEY 8f.1): `loc` = raw sampling offsets, `attw` = raw attention logits, `pr.ref` = reference
 // points [N or 1, Lq, L, 2].  `handled` = false: the problem is outside d32_applies() and nothing was launched.
-template <typename V>
-cudaError_t launch_fwd_d32(const V *value, const int64_t *shapes, const int64_t *lstart, const float *loc,
-                           const float *attw, const Producers &pr, const Dims &d, V *out, cudaStream_t stream,
+// P: element type of `loc` / `attw` -- float, or V for the 16-bit fused producers (pr.ref set).
+template <typename V, typename P>
+cudaError_t launch_fwd_d32(const V *value, const int64_t *shapes, const int64_t *lstart, const P *loc,
+                           const P *attw, const Producers &pr, const Dims &d, V *out, cudaStream_t stream,
                            bool *handled) {
     *handled = d32_applies(d);
     if (!*handled) return cudaSuccess;
     switch (d.L * d.P) {       // 4, 8, 12 or 16 (d32_applies)
-        case 4: return launch_fwd_lp<V, 4>(value, shapes, lstart, loc, attw, pr, d, out, stream);
-        case 8: return launch_fwd_lp<V, 8>(value, shapes, lstart, loc, attw, pr, d, out, stream);
-        case 12: return launch_fwd_lp<V, 12>(value, shapes, lstart, loc, attw, pr, d, out, stream);
-        default: return launch_fwd_lp<V, 16>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        case 4: return launch_fwd_lp<V, P, 4>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        case 8: return launch_fwd_lp<V, P, 8>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        case 12: return launch_fwd_lp<V, P, 12>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        default: return launch_fwd_lp<V, P, 16>(value, shapes, lstart, loc, attw, pr, d, out, stream);
     }
 }
 
-#define MSDA_FWD_D32(V)                                                                                             \
-    template cudaError_t launch_fwd_d32<V>(const V *, const int64_t *, const int64_t *, const float *, const float *, \
-                                           const Producers &, const Dims &, V *, cudaStream_t, bool *);
-MSDA_FWD_D32(float)
-MSDA_FWD_D32(__nv_bfloat16)
-MSDA_FWD_D32(__half)
+#define MSDA_FWD_D32(V, P)                                                                                         \
+    template cudaError_t launch_fwd_d32<V, P>(const V *, const int64_t *, const int64_t *, const P *, const P *,  \
+                                              const Producers &, const Dims &, V *, cudaStream_t, bool *);
+MSDA_FWD_D32(float, float)
+MSDA_FWD_D32(__nv_bfloat16, float)
+MSDA_FWD_D32(__half, float)
+MSDA_FWD_D32(__nv_bfloat16, __nv_bfloat16)
+MSDA_FWD_D32(__half, __half)
 #undef MSDA_FWD_D32
 
 }  // namespace msda

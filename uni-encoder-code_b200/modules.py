@@ -206,8 +206,9 @@ class MSDeformAttn(nn.Module):
     def forward(self, query, reference_points, input_flatten, input_spatial_shapes,
                 input_level_start_index, input_padding_mask=None):
         value = self.project_value(input_flatten, input_padding_mask)
+        # fp32, or under autocast a 16-bit value whose offsets / logits come out in the same type (fused_supported)
         if self.fused and self._core is _cuda_core and not reference_points.requires_grad \
-                and value.dtype == torch.float32:      # (the fused kernels are fp32; autocast takes the path below)
+                and value.dtype in (torch.float32, torch.bfloat16, torch.float16):
             N, Lq, _ = query.shape
             offsets = _linear(self.sampling_offsets, query, self.linear).view(
                 N, Lq, self.n_heads, self.n_levels, self.n_points, 2)

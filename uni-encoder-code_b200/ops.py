@@ -191,7 +191,7 @@ def ms_deform_attn_backward(value, spatial_shapes, level_start_index, sampling_l
 def _backward_deterministic(fn, opname, value, shapes, lsi, producers, grad_output, dims, ref=None, rs=0,
                             kind="backward"):
     """A deterministic backward entry ``fn`` (msda_b200_backward_deterministic_f32/_f64/_bf16/_f16, or with ``ref`` the fused
-    msda_b200_fused_backward_deterministic_f32) in chunks of whole images -> [grad_value, *grads of producers].
+    msda_b200_fused_backward_deterministic_f32/_bf16/_f16) in chunks of whole images -> [grad_value, *grads of producers].
     ``producers``: (sampling_loc, attn_weight), or for the fused op (sampling_offsets, attn_logits).  ``kind``: the
     name of the call in ``enable_timing``'s list, the same as the default backward's."""
     N, S, M, D, L, Lq, P = dims
@@ -292,10 +292,27 @@ def debug_indices(value_shape, spatial_shapes, level_start_index, sampling_loc):
 # Fused producers (SURVEY.md 8f.1): softmax over the L*P logits and `ref + offset / (W, H)` inside
 # the kernels (ops/modules/ms_deform_attn.py:105-112).  No counterpart in the reference's extension.
 # ----------------------------------------------------------------------------------------------
+# the mixed-precision fused op (torch.autocast): 16-bit value, raw offsets / logits and their gradients, fp32 reference
+# points, fp32 arithmetic in between
+_FUSED_MIXED_FWD = {torch.bfloat16: _lib.lib.msda_b200_fused_forward_bf16,
+                    torch.float16: _lib.lib.msda_b200_fused_forward_f16}
+_FUSED_MIXED_BWD = {torch.bfloat16: _lib.lib.msda_b200_fused_backward_bf16,
+                    torch.float16: _lib.lib.msda_b200_fused_backward_f16}
+_FUSED_MIXED_BWD_DET = {torch.bfloat16: _lib.lib.msda_b200_fused_backward_deterministic_bf16,
+                        torch.float16: _lib.lib.msda_b200_fused_backward_deterministic_f16}
+
+
 def fused_supported(value, reference_points, sampling_offsets, attn_logits):
-    """The fused kernels cover the pixel-decoder shape only: fp32, 32 channels per head,
-    L*P in {4, 8, 12, 16}, 2-d reference points shared by the batch or per image."""
-    if not (isinstance(value, torch.Tensor) and value.is_cuda and value.dtype == torch.float32):
+    """The fused kernels cover the pixel-decoder shape only: 32 channels per head, L*P in {4, 8, 12, 16}, 2-d
+    reference points shared by the batch or per image; fp32, or -- what torch.autocast hands the module -- a bf16 /
+    fp16 value with sampling_offsets and attn_logits of the same type and fp32 reference points."""
+    if not (isinstance(value, torch.Tensor) and value.is_cuda):
+        return False
+    if value.dtype in _FUSED_MIXED_FWD:
+        if not (sampling_offsets.dtype == attn_logits.dtype == value.dtype
+                and reference_points.dtype == torch.float32):
+            return False
+    elif value.dtype != torch.float32:
         return False
     if value.dim() != 4 or value.size(3) != 32 or sampling_offsets.dim() != 6:
         return False
@@ -307,29 +324,52 @@ def fused_supported(value, reference_points, sampling_offsets, attn_logits):
 
 
 def _check_fused(value, shapes, lsi, ref, off, logits, extra=()):
+    """The fused op's checks: fp32 throughout, or a bf16 / fp16 value with every other tensor but the fp32
+    reference points of the same type (the mixed-precision fused op) -> (N, S, M, D, L, Lq, P, ref batch stride)."""
     named = [("value", value), ("spatial_shapes", shapes), ("level_start_index", lsi),
              ("reference_points", ref), ("sampling_offsets", off), ("attn_logits", logits)] + list(extra)
     _require_cuda_contiguous(named)
+    mixed = value.dtype in _FUSED_MIXED_FWD
+    if mixed:
+        for name, t in [("sampling_offsets", off), ("attn_logits", logits)] + list(extra):
+            if t.dtype != value.dtype:
+                raise RuntimeError(f"fused MSDA: {name} is {t.dtype} but value is {value.dtype} (the mixed-precision "
+                                   "fused op takes one 16-bit type)")
+        if ref.dtype != torch.float32:
+            raise RuntimeError(f"fused MSDA: reference_points must be float32, found {ref.dtype}")
     if not fused_supported(value, ref, off, logits):
-        raise RuntimeError("fused MSDA covers fp32, 32 channels per head, L*P in {4,8,12,16}, 2-d "
-                           "reference points only; compose the unfused op for other shapes")
+        raise RuntimeError("fused MSDA covers fp32 or bf16 / fp16 (with fp32 reference points), 32 channels per "
+                           "head, L*P in {4,8,12,16}, 2-d reference points only; compose the unfused op for other "
+                           "shapes")
     N, S, M, D = value.shape
     _, Lq, _, L, P, _ = off.shape
     if tuple(off.shape) != (N, Lq, M, L, P, 2) or logits.numel() != N * Lq * M * L * P \
             or tuple(ref.shape[1:]) != (Lq, L, 2) or shapes.size(0) != L:
         raise RuntimeError("inconsistent shapes for fused MSDA")
-    for t in (ref, off, logits) + tuple(t for _, t in extra):
-        if t.dtype != torch.float32:
-            raise RuntimeError("fused MSDA is float32 only")
+    if not mixed:
+        for name, t in [("reference_points", ref), ("sampling_offsets", off), ("attn_logits", logits)] + list(extra):
+            if t.dtype != torch.float32:
+                raise RuntimeError(f"fused MSDA is float32 only: {name} is {t.dtype}")
     ref_stride = 0 if ref.size(0) == 1 and N > 1 else Lq * L * 2
     return N, S, M, D, L, Lq, P, ref_stride
 
 
 def ms_deform_attn_fused_forward(value, spatial_shapes, level_start_index, reference_points,
                                  sampling_offsets, attn_logits):
-    """output [N, Lq, M*D] from raw offsets / logits (msda_b200_fused_forward_strided_f32 on packed rows)."""
+    """output [N, Lq, M*D] in value's dtype from raw offsets / logits (msda_b200_fused_forward_strided_f32 on packed
+    rows; bf16 / fp16: msda_b200_fused_forward_bf16 / _f16, fp32 arithmetic and one rounding of the output)."""
     N, S, M, D, L, Lq, P, rs = _check_fused(value, spatial_shapes, level_start_index, reference_points,
                                             sampling_offsets, attn_logits)
+    if value.dtype in _FUSED_MIXED_FWD:
+        with torch.cuda.device(value.device):
+            output = torch.empty((N, Lq, M * D), dtype=value.dtype, device=value.device)
+            with _timed("forward_mixed"):
+                rc = _FUSED_MIXED_FWD[value.dtype](
+                    value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
+                    reference_points.data_ptr(), rs, sampling_offsets.data_ptr(), attn_logits.data_ptr(),
+                    N, S, M, D, L, Lq, P, output.data_ptr(), torch.cuda.current_stream().cuda_stream)
+        _lib.check(rc, "ms_deform_attn_fused_forward")
+        return output
     return _fused_forward("ms_deform_attn_fused_forward", value, spatial_shapes, level_start_index, reference_points,
                           rs, sampling_offsets, 2 * M * L * P, attn_logits, M * L * P, None, None,
                           (N, S, M, D, L, Lq, P))
@@ -387,9 +427,31 @@ def ms_deform_attn_fused_forward_packed(value, spatial_shapes, level_start_index
 
 def ms_deform_attn_fused_backward(value, spatial_shapes, level_start_index, reference_points,
                                   sampling_offsets, attn_logits, grad_output):
-    """[grad_value, grad_sampling_offsets, grad_attn_logits] (msda_b200_fused_backward_f32)."""
+    """[grad_value, grad_sampling_offsets, grad_attn_logits] in the inputs' dtypes (msda_b200_fused_backward_f32;
+    bf16 / fp16: msda_b200_fused_backward_bf16 / _f16, grad_value reduced in an fp32 buffer allocated here and
+    rounded once, as in ms_deform_attn_mixed_backward)."""
     N, S, M, D, L, Lq, P, rs = _check_fused(value, spatial_shapes, level_start_index, reference_points,
                                             sampling_offsets, attn_logits, [("grad_output", grad_output)])
+    if value.dtype in _FUSED_MIXED_FWD:
+        if _deterministic():
+            return _backward_deterministic(_FUSED_MIXED_BWD_DET[value.dtype],
+                                           "ms_deform_attn_fused_backward (deterministic)", value, spatial_shapes,
+                                           level_start_index, (sampling_offsets, attn_logits), grad_output,
+                                           (N, S, M, D, L, Lq, P), reference_points, rs, kind="backward_mixed")
+        with torch.cuda.device(value.device):
+            accum = torch.zeros((N, S, M, D), dtype=torch.float32, device=value.device)   # fp32 reductions
+            grad_value = torch.empty_like(value)            # rounded from accum
+            grad_off = torch.empty_like(sampling_offsets)
+            grad_logits = torch.empty_like(attn_logits)
+            with _timed("backward_mixed"):
+                rc = _FUSED_MIXED_BWD[value.dtype](
+                    grad_output.data_ptr(), value.data_ptr(), spatial_shapes.data_ptr(),
+                    level_start_index.data_ptr(), reference_points.data_ptr(), rs,
+                    sampling_offsets.data_ptr(), attn_logits.data_ptr(), N, S, M, D, L, Lq, P,
+                    accum.data_ptr(), grad_value.data_ptr(), grad_off.data_ptr(), grad_logits.data_ptr(),
+                    torch.cuda.current_stream().cuda_stream)
+        _lib.check(rc, "ms_deform_attn_fused_backward")
+        return [grad_value, grad_off, grad_logits]
     if _deterministic():
         return _backward_deterministic(_lib.lib.msda_b200_fused_backward_deterministic_f32,
                                        "ms_deform_attn_fused_backward (deterministic)", value, spatial_shapes,

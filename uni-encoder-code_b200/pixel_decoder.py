@@ -127,7 +127,9 @@ class MSDeformAttnPixelDecoder(nn.Module):
                  core: Optional[CoreFn] = None, fused: bool = False, linear: str = "torch", amp: bool = False):
         """`amp=True` (not in the reference): `forward_features` runs inside the caller's torch.autocast context
         instead of disabling it -- torch's 16-bit GEMMs and convolutions, and the mixed-precision MSDA op
-        (functions.MSDeformAttnMixedFunction).  `amp=False` is the reference's behaviour: autocast off, fp32."""
+        (functions.MSDeformAttnMixedFunction; with `fused=True` the 16-bit fused-producer kernels,
+        functions.MSDeformAttnFusedFunction, which take the softmax and the location arithmetic off torch).
+        `amp=False` is the reference's behaviour: autocast off, fp32."""
         if amp and linear == "tf32x3":
             raise ValueError('amp=True cannot be combined with linear="tf32x3": the 3xTF32 GEMMs and the fp32 '
                              'GroupNorm / LayerNorm kernels are fp32 paths that autocast would bypass')
