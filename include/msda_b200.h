@@ -270,6 +270,26 @@ int msda_b200_fused_forward_f16(const uint16_t *value, const int64_t *spatial_sh
                                 const uint16_t *sampling_offsets, const uint16_t *attn_logits, int batch,
                                 int spatial_size, int num_heads, int channels, int num_levels, int num_query,
                                 int num_point, uint16_t *output, void *stream);
+/* The 16-bit fused forward with row strides and per-query tables, as msda_b200_fused_forward_strided_f32: the raw
+ * offsets / logits are 16-bit rows (strides in elements, offsets_row_stride even), e.g. of one [rows, 3*M*L*P]
+ * projection output; offsets_table / logits_table (both or neither) stay fp32.  Each raw value is widened first
+ * and then gets its table entry added in fp32, so output is bit-identical to msda_b200_fused_forward_strided_f32 run
+ * on the widened rows, the widened value and the same tables, rounded once to 16 bits.  Error codes and
+ * alignment as for that entry, with sampling_offsets 4-byte aligned. */
+int msda_b200_fused_forward_strided_bf16(const uint16_t *value, const int64_t *spatial_shapes,
+                                         const int64_t *level_start, const float *reference_points,
+                                         long long ref_batch_stride, const uint16_t *sampling_offsets,
+                                         int offsets_row_stride, const uint16_t *attn_logits, int logits_row_stride,
+                                         const float *offsets_table, const float *logits_table, int batch,
+                                         int spatial_size, int num_heads, int channels, int num_levels, int num_query,
+                                         int num_point, uint16_t *output, void *stream);
+int msda_b200_fused_forward_strided_f16(const uint16_t *value, const int64_t *spatial_shapes,
+                                        const int64_t *level_start, const float *reference_points,
+                                        long long ref_batch_stride, const uint16_t *sampling_offsets,
+                                        int offsets_row_stride, const uint16_t *attn_logits, int logits_row_stride,
+                                        const float *offsets_table, const float *logits_table, int batch,
+                                        int spatial_size, int num_heads, int channels, int num_levels, int num_query,
+                                        int num_point, uint16_t *output, void *stream);
 int msda_b200_fused_backward_bf16(const uint16_t *grad_output, const uint16_t *value, const int64_t *spatial_shapes,
                                   const int64_t *level_start, const float *reference_points,
                                   long long ref_batch_stride, const uint16_t *sampling_offsets,
@@ -367,6 +387,49 @@ int msda_b200_add_layernorm_backward_deterministic_f32(const float *grad_y, cons
                                                        float *grad_beta, long long rows, int cols, float eps,
                                                        void *workspace, void *stream);
 long long msda_b200_add_layernorm_backward_deterministic_workspace_bytes(long long rows, int cols);
+
+/*
+ * Mixed precision (torch.autocast: the sublayer's Linear output is 16-bit, the residual stream fp32):
+ * y = LayerNorm(x + widen(residual)) * gamma + beta with x, gamma, beta, y fp32 and residual bf16 (_bf16) or fp16
+ * (_f16), as uint16_t bit patterns.  y is bit-identical to msda_b200_add_layernorm_f32(x, widen(residual)): the
+ * fp32 arithmetic is that kernel's, residual is widened once on load.  y16 (may be NULL) receives the same rows
+ * rounded to the 16-bit type (round-to-nearest-even, == y.to(dtype); fp16 overflow gives +-inf) -- the copy the
+ * next GEMMs read.  residual is required.  cols in {128, 256, 384, 512}; x, gamma, beta, y 16-byte aligned,
+ * residual and y16 8-byte aligned; MSDA_ERR_UNSUPPORTED otherwise.
+ */
+int msda_b200_add_layernorm_mixed_bf16(const float *x, const uint16_t *residual, const float *gamma,
+                                       const float *beta, float *y, uint16_t *y16, long long rows, int cols,
+                                       float eps, void *stream);
+int msda_b200_add_layernorm_mixed_f16(const float *x, const uint16_t *residual, const float *gamma,
+                                      const float *beta, float *y, uint16_t *y16, long long rows, int cols,
+                                      float eps, void *stream);
+/* Backward of the entries above with respect to y (grad_y, fp32) and y16 (grad_y16, 16-bit), either of which may
+ * be NULL (not both): g = grad_y + widen(grad_y16), one fp32 add per element.  grad_x (fp32) is bit-identical to
+ * msda_b200_add_layernorm_backward_f32(g, x, widen(residual)); grad_residual (16-bit) is grad_x rounded once;
+ * grad_gamma / grad_beta (fp32, overwritten) are reduced as in that entry.  cols in {128, 256}; alignment as in the
+ * forward (grad_y and grad_x 16 bytes, grad_y16 and grad_residual 8); MSDA_ERR_UNSUPPORTED otherwise.  The
+ * deterministic twins take the workspace of msda_b200_add_layernorm_backward_deterministic_workspace_bytes(rows,
+ * cols) and are bit-identical to msda_b200_add_layernorm_backward_deterministic_f32 fed g. */
+int msda_b200_add_layernorm_mixed_backward_bf16(const float *grad_y, const uint16_t *grad_y16, const float *x,
+                                                const uint16_t *residual, const float *gamma, float *grad_x,
+                                                uint16_t *grad_residual, float *grad_gamma, float *grad_beta,
+                                                long long rows, int cols, float eps, void *stream);
+int msda_b200_add_layernorm_mixed_backward_f16(const float *grad_y, const uint16_t *grad_y16, const float *x,
+                                               const uint16_t *residual, const float *gamma, float *grad_x,
+                                               uint16_t *grad_residual, float *grad_gamma, float *grad_beta,
+                                               long long rows, int cols, float eps, void *stream);
+int msda_b200_add_layernorm_mixed_backward_deterministic_bf16(const float *grad_y, const uint16_t *grad_y16,
+                                                              const float *x, const uint16_t *residual,
+                                                              const float *gamma, float *grad_x,
+                                                              uint16_t *grad_residual, float *grad_gamma,
+                                                              float *grad_beta, long long rows, int cols, float eps,
+                                                              void *workspace, void *stream);
+int msda_b200_add_layernorm_mixed_backward_deterministic_f16(const float *grad_y, const uint16_t *grad_y16,
+                                                             const float *x, const uint16_t *residual,
+                                                             const float *gamma, float *grad_x,
+                                                             uint16_t *grad_residual, float *grad_gamma,
+                                                             float *grad_beta, long long rows, int cols, float eps,
+                                                             void *workspace, void *stream);
 
 /*
  * GroupNorm over an NCHW fp32 map with the pixel decoder's epilogues fused in (SURVEY 8f.4;

@@ -27,6 +27,17 @@ DIR defaults to $BENCH_OUT/mixed, and BENCH_OUT to bench_out/ in the repository 
     tools/bench_decoder_train.py: fp32 linear="tf32x3" against amp=True with bf16, and with fp16 + GradScaler, each
     with fused=True and fused=False.
 
+(l) the residual + LayerNorm site of the encoder alone at 344 064 x 256 (configs[2]'s rows), bf16 and fp16, forward and
+    backward: the mixed-precision kernels (fp32 x, 16-bit residual -> fp32 y and its 16-bit copy; backward from both
+    gradients) against torch's autocast composition of the same site (add, layer_norm, the cast for the next GEMM;
+    autograd for the backward) and against the fp32 kernels (fp32 residual, no copy).  Arms alternate, the L2 is
+    evicted before every call.  Algorithmic bytes per element: forward 4 + 2 in, 4 + 2 out; backward 4 + 2 + 4 + 2 in,
+    4 + 2 out (fp32 kernels: 4 + 4 in, 4 out; 4 + 4 + 4 in, 4 out), and their share of the measured HBM figure.
+(p) the 16-bit packed / per-query-table forward (one [N, Lq, 3*M*L*P] projection output and the fp32 table) against
+    the 16-bit fused forward on separate offset / logit tensors and the fp32 packed forward with the table, at
+    configs[1] and the configs[2] shape; arms alternate, L2 evicted before every call.
+Parts (b) and (c) carry linear="autocast" arms next to the others; the arms of (b) and (c) alternate.
+
 Every JSON line carries the card's name and power limit (read-only nvidia-smi query).
 """
 import argparse
@@ -45,6 +56,7 @@ from __graft_entry__ import load_package  # noqa: E402
 from bench_decoder_train import card, timed  # noqa: E402
 
 DTYPES = {"fp32": torch.float32, "bf16": torch.bfloat16, "fp16": torch.float16}
+HBM_GBS = 6540.8          # the project's measured HBM bandwidth on the B200 (DESIGN.md section 10)
 SWIN_T = {"res2": (96, 4), "res3": (192, 8), "res4": (384, 16), "res5": (768, 32)}
 
 
@@ -197,6 +209,124 @@ def part_f(pkg, args, emit):
         torch.cuda.empty_cache()
 
 
+def _evicted(flush, fn):
+    """Time one call of `fn` after a 256 MB write that evicts the L2 (events bracket the call only)."""
+    flush.zero_()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    fn()
+    e1.record()
+    e1.synchronize()
+    return e0.elapsed_time(e1)
+
+
+def part_l(pkg, args, emit):
+    dev = torch.device("cuda", 0)
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    rows, cols = 344064, 256
+    gen = torch.Generator(device=dev).manual_seed(4)
+    x = torch.randn(rows, cols, device=dev, generator=gen)
+    w = torch.rand(cols, device=dev, generator=gen) + 0.5
+    b = torch.randn(cols, device=dev, generator=gen) * 0.1
+    gy = torch.randn(rows, cols, device=dev, generator=gen)
+    base_r = torch.randn(rows, cols, device=dev, generator=gen)
+    base_g16 = torch.randn(rows, cols, device=dev, generator=gen)
+    norm = torch.nn.LayerNorm(cols).to(dev)
+    with torch.no_grad():
+        norm.weight.copy_(w)
+        norm.bias.copy_(b)
+    for tag in ("bf16", "fp16"):
+        dt = DTYPES[tag]
+        r16, gy16 = base_r.to(dt), base_g16.to(dt)
+        r32 = r16.float()
+
+        def composition_fwd():
+            with torch.no_grad(), torch.autocast("cuda", dtype=dt):
+                y = norm(x + r16)
+                y.to(dt)
+
+        def composition_bwd():
+            xl, rl = x.detach().requires_grad_(True), r16.detach().requires_grad_(True)
+            with torch.autocast("cuda", dtype=dt):
+                y = norm(xl + rl)
+                y16 = y.to(dt)
+            return lambda: torch.autograd.backward([y, y16], [gy, gy16])
+
+        arms = {
+            ("mixed kernels", "forward"): lambda: pkg.add_layernorm_mixed(x, r16, w, b),
+            ("torch autocast composition", "forward"): composition_fwd,
+            ("fp32 kernels", "forward"): lambda: pkg.add_layernorm(x, r32, w, b),
+            ("mixed kernels", "backward"): lambda: pkg.ops.add_layernorm_mixed_backward(gy, gy16, x, r16, w),
+            ("torch autocast composition", "backward"): None,
+            ("fp32 kernels", "backward"): lambda: pkg.ops.add_layernorm_backward(gy, x, r32, w),
+        }
+        nbytes = {("mixed kernels", "forward"): 12, ("torch autocast composition", "forward"): 12,
+                  ("fp32 kernels", "forward"): 12, ("mixed kernels", "backward"): 18,
+                  ("torch autocast composition", "backward"): 18, ("fp32 kernels", "backward"): 16}
+        times = {k: [] for k in arms}
+
+        def one(k):
+            if k == ("torch autocast composition", "backward"):
+                bwd = composition_bwd()            # the forward runs untimed just before
+                return _evicted(flush, bwd)
+            return _evicted(flush, arms[k])
+        for k in arms:
+            for _ in range(2):
+                one(k)
+        for _ in range(args.steps):
+            for k in arms:                                  # the arms alternate
+                times[k].append(one(k))
+        for (arm, op), ts in times.items():
+            ms = statistics.median(ts)
+            byt = nbytes[(arm, op)] * rows * cols
+            emit({"part": "l", "what": "residual + LayerNorm site, 344064 x 256", "dtype": tag, "arm": arm, "op": op,
+                  "ms_median": ms, "ms_min": min(ts), "ms_max": max(ts), "timed_calls": len(ts),
+                  "algorithmic_bytes": byt, "algorithmic_GBs": byt / ms / 1e6,
+                  "hbm_share": byt / ms / 1e6 / HBM_GBS, "hbm_GBs_reference": HBM_GBS,
+                  "l2": "evicted before every call (256 MB write)"})
+
+
+def part_p(pkg, args, emit):
+    dev = torch.device("cuda", 0)
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    for name in ("cityscapes_512x1024_b8", "cityscapes_1024x2048_b8"):
+        w = pkg.synthetic.WORKLOADS[name]
+        levels, N, M, P = list(w.levels), w.batch, 8, 4
+        L, S = len(levels), sum(h * wd for h, wd in levels)
+        gen = torch.Generator(device=dev).manual_seed(1)
+        value = torch.randn(N, S, M, 32, device=dev, generator=gen)
+        proj = torch.cat((torch.randn(N, S, 2 * M * L * P, device=dev, generator=gen) * 2.0,
+                          torch.randn(N, S, M * L * P, device=dev, generator=gen)), -1)
+        table = torch.randn(S, 3 * M * L * P, device=dev, generator=gen) * 0.3
+        shapes, lsi = pkg.synthetic.level_tensors(levels, device=dev)
+        ref = pkg.modules.reference_points_for(levels, dev)
+        arms = {}
+        v32, p32 = value.bfloat16().float(), proj.bfloat16().float()
+        arms["fp32 packed + table"] = lambda: pkg.ops.ms_deform_attn_fused_forward_packed(
+            v32, shapes, lsi, ref, p32, L, P, query_table=table)
+        for tag in ("bf16", "fp16"):
+            dt = DTYPES[tag]
+            v16, p16 = value.to(dt), proj.to(dt)
+            off16 = p16[..., :2 * M * L * P].reshape(N, S, M, L, P, 2).contiguous()
+            lg16 = p16[..., 2 * M * L * P:].reshape(N, S, M, L * P).contiguous()
+            arms[f"{tag} packed + table"] = (lambda v16=v16, p16=p16: pkg.ops.ms_deform_attn_fused_mixed_forward_packed(
+                v16, shapes, lsi, ref, p16, L, P, query_table=table))
+            arms[f"{tag} fused, separate tensors"] = (lambda v16=v16, o=off16, g=lg16: pkg.ms_deform_attn_fused_forward(
+                v16, shapes, lsi, ref, o, g))
+        times = {k: [] for k in arms}
+        for k, fn in arms.items():
+            for _ in range(2):
+                fn()
+        for _ in range(args.steps):
+            for k, fn in arms.items():                      # the arms alternate
+                times[k].append(_evicted(flush, fn))
+        for k, ts in times.items():
+            emit({"part": "p", "workload": name, "arm": k, "ms_median": statistics.median(ts), "ms_min": min(ts),
+                  "ms_max": max(ts), "timed_calls": len(ts), "l2": "evicted before every call (256 MB write)"})
+        del arms, value, proj, v32, p32
+        torch.cuda.empty_cache()
+
+
 def _decoder(pkg, fused, linear, amp, train):
     torch.manual_seed(0)
     m = pkg.pixel_decoder.MSDeformAttnPixelDecoder(
@@ -215,7 +345,8 @@ def part_b(pkg, args, emit):
     feats = _feats(8, 1024, 2048, 3)
     arms = [("fp32 fused tf32x3", dict(fused=True, linear="tf32x3", amp=False), None),
             ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16),
-            ("amp bf16 fused=False", dict(fused=False, linear="torch", amp=True), torch.bfloat16)]
+            ("amp bf16 fused=False", dict(fused=False, linear="torch", amp=True), torch.bfloat16),
+            ("amp bf16 linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.bfloat16)]
     models = {tag: _decoder(pkg, train=False, **kw) for tag, kw, _ in arms}
     res = {tag: [] for tag, _, _ in arms}
     for _ in range(args.repeats):
@@ -236,15 +367,18 @@ def part_c(pkg, args, emit):
     arms = [("fp32 fused tf32x3", dict(fused=True, linear="tf32x3", amp=False), None),
             ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16),
             ("amp bf16 fused=False", dict(fused=False, linear="torch", amp=True), torch.bfloat16),
+            ("amp bf16 linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.bfloat16),
             ("amp fp16 + GradScaler", dict(fused=True, linear="torch", amp=True), torch.float16),
-            ("amp fp16 + GradScaler fused=False", dict(fused=False, linear="torch", amp=True), torch.float16)]
+            ("amp fp16 + GradScaler fused=False", dict(fused=False, linear="torch", amp=True), torch.float16),
+            ("amp fp16 + GradScaler linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.float16)]
+    steps = {}
     for tag, kw, dt in arms:
         m = _decoder(pkg, train=True, **kw)
         opt = torch.optim.AdamW(m.parameters(), lr=1e-4)
         scaler = torch.amp.GradScaler("cuda") if dt == torch.float16 else None
-        ctx = (lambda: torch.autocast("cuda", dtype=dt)) if dt is not None else contextlib.nullcontext
+        ctx = (lambda dt=dt: torch.autocast("cuda", dtype=dt)) if dt is not None else contextlib.nullcontext
 
-        def step():
+        def step(m=m, opt=opt, scaler=scaler, ctx=ctx):
             opt.zero_grad(set_to_none=True)
             with ctx():
                 mask, low, multi = m.forward_features(feats)
@@ -256,24 +390,31 @@ def part_c(pkg, args, emit):
                 scaler.scale(loss).backward()
                 scaler.step(opt)
                 scaler.update()
-        ms = timed(step, args.steps // 2, args.warmup)
+        steps[tag] = step
+    res, peak = {tag: [] for tag, _, _ in arms}, {}
+    for r in range(args.repeats):
+        for tag, _, _ in arms:                               # the arms alternate
+            torch.cuda.reset_peak_memory_stats()
+            res[tag].append(timed(steps[tag], max(2, args.steps // 4), args.warmup if r == 0 else 1))
+            peak[tag] = max(peak.get(tag, 0.0), torch.cuda.max_memory_allocated() / 2 ** 30)
+    for tag, _, _ in arms:
+        ms = min(res[tag])
         emit({"part": "c", "what": "pixel-decoder training step (forward_features + loss + backward + AdamW), "
                                    "512x1024, batch 16, Swin-T pyramid, 6 encoder layers", "arm": tag, "ms": ms,
-              "images_per_s": 16 / ms * 1e3, "peak_mem_gib": torch.cuda.max_memory_allocated() / 2 ** 30})
-        del m, opt
-        torch.cuda.empty_cache()
-        torch.cuda.reset_peak_memory_stats()
+              "ms_all_repeats": res[tag], "images_per_s": 16 / ms * 1e3, "peak_mem_gib": peak[tag],
+              "note": "peak memory includes the parameters and optimizer state of all arms' models"})
 
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--parts", default="a,b,c", help="a, b, c: profiles/r5_mixed.jsonl; f, b, c: r6_fused_mixed.jsonl")
+    ap.add_argument("--parts", default="a,b,c", help="a, b, c: profiles/r5_mixed.jsonl; f, b, c: r6_fused_mixed.jsonl; "
+                                                  "l, p, b, c: r7_autocast_encoder.jsonl")
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--dtypes", default="fp32,bf16,fp16", help="part (a): element types of value")
     ap.add_argument("--ops", default="forward,backward,fwd+bwd", help="part (a): calls timed")
     ap.add_argument("--label", default="", help="part (a): recorded in every line (e.g. the library build)")
-    ap.add_argument("--repeats", type=int, default=3, help="part (b): alternating repeats of each arm (min reported)")
+    ap.add_argument("--repeats", type=int, default=3, help="parts (b), (c): alternating repeats of each arm (min reported)")
     ap.add_argument("--out", default=os.path.join(os.environ.get("BENCH_OUT") or os.path.join(ROOT, "bench_out"),
                                                   "mixed"))
     args = ap.parse_args()
@@ -290,7 +431,7 @@ def main():
         with open(path, "a") as f:
             f.write(json.dumps(rec) + "\n")
     for part in args.parts.split(","):
-        {"a": part_a, "f": part_f, "b": part_b, "c": part_c}[part](pkg, args, emit)
+        {"a": part_a, "f": part_f, "b": part_b, "c": part_c, "l": part_l, "p": part_p}[part](pkg, args, emit)
 
 
 if __name__ == "__main__":

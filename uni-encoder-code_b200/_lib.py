@@ -46,6 +46,8 @@ SYMBOLS = {
     "msda_b200_fused_backward_f16": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P] * 5),
     "msda_b200_fused_backward_deterministic_bf16": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P] * 5),
     "msda_b200_fused_backward_deterministic_f16": (_I, [_P] * 5 + [ctypes.c_longlong, _P, _P] + _DIMS + [_P] * 5),
+    "msda_b200_fused_forward_strided_bf16": (_I, [_P] * 4 + [ctypes.c_longlong, _P, _I, _P, _I, _P, _P] + _DIMS + [_P, _P]),
+    "msda_b200_fused_forward_strided_f16": (_I, [_P] * 4 + [ctypes.c_longlong, _P, _I, _P, _I, _P, _P] + _DIMS + [_P, _P]),
     "msda_b200_linear_f32": (_I, [_P] * 4 + [_I] * 4 + [_P, _P]),
     "msda_b200_linear_deterministic_f32": (_I, [_P] * 4 + [_I] * 4 + [_P, _P]),
     "msda_b200_split_weight_f32": (_I, [_P, _P, _I, _I, _P]),
@@ -55,6 +57,14 @@ SYMBOLS = {
     "msda_b200_add_layernorm_backward_f32": (_I, [_P] * 7 + [ctypes.c_longlong, _I, ctypes.c_float, _P]),
     "msda_b200_add_layernorm_backward_deterministic_f32": (_I, [_P] * 7 + [ctypes.c_longlong, _I, ctypes.c_float, _P, _P]),
     "msda_b200_add_layernorm_backward_deterministic_workspace_bytes": (ctypes.c_longlong, [ctypes.c_longlong, _I]),
+    "msda_b200_add_layernorm_mixed_bf16": (_I, [_P] * 6 + [ctypes.c_longlong, _I, ctypes.c_float, _P]),
+    "msda_b200_add_layernorm_mixed_f16": (_I, [_P] * 6 + [ctypes.c_longlong, _I, ctypes.c_float, _P]),
+    "msda_b200_add_layernorm_mixed_backward_bf16": (_I, [_P] * 9 + [ctypes.c_longlong, _I, ctypes.c_float, _P]),
+    "msda_b200_add_layernorm_mixed_backward_f16": (_I, [_P] * 9 + [ctypes.c_longlong, _I, ctypes.c_float, _P]),
+    "msda_b200_add_layernorm_mixed_backward_deterministic_bf16": (_I, [_P] * 9 + [ctypes.c_longlong, _I, ctypes.c_float,
+                                                                                 _P, _P]),
+    "msda_b200_add_layernorm_mixed_backward_deterministic_f16": (_I, [_P] * 9 + [ctypes.c_longlong, _I, ctypes.c_float,
+                                                                                _P, _P]),
     "msda_b200_linear_wgrad_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _I, _I, _P]),
     "msda_b200_linear_wgrad_deterministic_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _I, _I, _P, _P]),
     "msda_b200_linear_wgrad_deterministic_workspace_bytes": (ctypes.c_longlong, [ctypes.c_longlong, _I, _I]),

@@ -55,6 +55,13 @@ cudaError_t launch_add_layernorm(const float *, const float *, const float *, co
 cudaError_t launch_add_layernorm_bwd(const float *, const float *, const float *, const float *, float *, float *,
                                      float *, long long, int, float, cudaStream_t, bool *handled, float *partials);
 long long add_layernorm_bwd_partials(long long rows, int cols);
+template <typename R>
+cudaError_t launch_add_layernorm_mixed(const float *, const R *, const float *, const float *, float *, R *, long long,
+                                       int, float, cudaStream_t, bool *handled);
+template <typename R>
+cudaError_t launch_add_layernorm_mixed_bwd(const float *, const R *, const float *, const R *, const float *, float *,
+                                           R *, float *, float *, long long, int, float, cudaStream_t, bool *handled,
+                                           float *partials);
 cudaError_t launch_linear_wgrad(const float *, const float *, float *, float *, long long, int, int, cudaStream_t,
                                 bool *handled, float *partials);
 long long linear_wgrad_partials(long long rows, int out_f, int in_f);
@@ -246,6 +253,58 @@ static int backward_deterministic(const V *grad_output, const V *value, const in
     return (int)e;
 }
 
+// The fused forward with row strides and per-query tables: fp32 (V = float), or 16-bit V with 16-bit raw offsets /
+// logits (P = V) and fp32 tables.  Strides in elements of P.
+template <typename V>
+static int fused_forward_strided(const V *value, const int64_t *shapes, const int64_t *lstart, const float *ref,
+                                 long long ref_bstride, const V *offsets, int offsets_stride, const V *logits,
+                                 int logits_stride, const float *offsets_table, const float *logits_table,
+                                 const Dims &d, V *output, cudaStream_t st) {
+    if (!value || !shapes || !lstart || !ref || !offsets || !logits || !output) return MSDA_ERR_NULL_POINTER;
+    if (int rc = check_dims(d, ref_bstride)) return rc;
+    const long long packed = (long long)d.M * d.L * d.P;
+    if (offsets_stride < 2 * packed || logits_stride < packed || (offsets_stride & 1)) return MSDA_ERR_BAD_SHAPE;
+    if ((offsets_table != nullptr) != (logits_table != nullptr)) return MSDA_ERR_NULL_POINTER;
+    if (!aligned16(value) || !aligned16(output) || !pair_aligned(offsets) || !aligned8(ref) || !aligned8(offsets_table))
+        return MSDA_ERR_UNSUPPORTED;
+    // the kernel reads packed rows (row strides 2*M*L*P and M*L*P) as stride 0
+    const bool rows_packed = offsets_stride == 2 * packed && logits_stride == packed;
+    const Producers pr{ref, ref_bstride, rows_packed ? 0 : offsets_stride, rows_packed ? 0 : logits_stride,
+                       offsets_table, logits_table};
+    bool handled = false;
+    const cudaError_t e = launch_fwd_d32<V, V>(value, shapes, lstart, offsets, logits, pr, d, output, st, &handled);
+    return launch_rc(e, handled);
+}
+
+// mixed-precision residual + LayerNorm (16-bit R) and its backward; partials: the deterministic twin's workspace
+template <typename R>
+static int add_layernorm_mixed(const float *x, const R *residual, const float *gamma, const float *beta, float *y,
+                               R *y16, long long rows, int cols, float eps, void *stream) {
+    if (!x || !residual || !gamma || !beta || !y) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || cols <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_add_layernorm_mixed<R>(x, residual, gamma, beta, y, y16, rows, cols, eps,
+                                                        (cudaStream_t)stream, &handled);
+    return launch_rc(e, handled);
+}
+
+template <typename R>
+static int add_layernorm_mixed_backward(const float *grad_y, const R *grad_y16, const float *x, const R *residual,
+                                        const float *gamma, float *grad_x, R *grad_residual, float *grad_gamma,
+                                        float *grad_beta, long long rows, int cols, float eps, void *workspace,
+                                        void *stream, bool deterministic) {
+    if ((!grad_y && !grad_y16) || !x || !residual || !gamma || !grad_x || !grad_residual || !grad_gamma ||
+        !grad_beta || (deterministic && !workspace))
+        return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || cols <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_add_layernorm_mixed_bwd<R>(grad_y, grad_y16, x, residual, gamma, grad_x, grad_residual,
+                                                            grad_gamma, grad_beta, rows, cols, eps,
+                                                            (cudaStream_t)stream, &handled,
+                                                            static_cast<float *>(workspace));
+    return launch_rc(e, handled);
+}
+
 // the bodies of the entries that come in a default and a deterministic (or training) form: `deterministic` /
 // `train` select the form's null-pointer rule, the workspace / mean_rstd pointer selects the launch
 static int linear(const float *x, const float *weight, const float *bias, float *y, int rows, int out_f, int in_f,
@@ -415,26 +474,10 @@ int msda_b200_fused_forward_strided_f32(const float *value, const int64_t *spati
                                         const float *logits_table, int batch, int spatial_size, int num_heads,
                                         int channels, int num_levels, int num_query, int num_point,
                                         float *output, void *stream) {
-    if (!value || !spatial_shapes || !level_start || !reference_points || !sampling_offsets ||
-        !attn_logits || !output)
-        return MSDA_ERR_NULL_POINTER;
     const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-    if (int rc = check_dims(d, ref_batch_stride)) return rc;
-    const long long packed = (long long)num_heads * num_levels * num_point;
-    if (offsets_row_stride < 2 * packed || logits_row_stride < packed || (offsets_row_stride & 1))
-        return MSDA_ERR_BAD_SHAPE;
-    if ((offsets_table != nullptr) != (logits_table != nullptr)) return MSDA_ERR_NULL_POINTER;
-    if (!aligned16(value) || !aligned16(output) || !aligned8(sampling_offsets) || !aligned8(reference_points) ||
-        !aligned8(offsets_table))
-        return MSDA_ERR_UNSUPPORTED;
-    // the kernel reads packed rows (row strides 2*M*L*P and M*L*P) as stride 0
-    const bool rows_packed = offsets_row_stride == 2 * packed && logits_row_stride == packed;
-    const Producers pr{reference_points, ref_batch_stride, rows_packed ? 0 : offsets_row_stride,
-                       rows_packed ? 0 : logits_row_stride, offsets_table, logits_table};
-    bool handled = false;
-    const cudaError_t e = launch_fwd_d32(value, spatial_shapes, level_start, sampling_offsets, attn_logits, pr, d,
-                                         output, (cudaStream_t)stream, &handled);
-    return launch_rc(e, handled);
+    return fused_forward_strided<float>(value, spatial_shapes, level_start, reference_points, ref_batch_stride,
+                                        sampling_offsets, offsets_row_stride, attn_logits, logits_row_stride,
+                                        offsets_table, logits_table, d, output, (cudaStream_t)stream);
 }
 
 int msda_b200_fused_forward_f32(const float *value, const int64_t *spatial_shapes,
@@ -595,6 +638,43 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
             Producers{reference_points, ref_batch_stride}, d, reinterpret_cast<V *>(grad_value),                     \
             reinterpret_cast<V *>(grad_sampling_offsets), reinterpret_cast<V *>(grad_attn_logits), workspace,        \
             (cudaStream_t)stream);                                                                                   \
+    }                                                                                                                \
+    int msda_b200_fused_forward_strided_##SUFFIX(                                                                   \
+        const uint16_t *value, const int64_t *spatial_shapes, const int64_t *level_start, const float *reference_points, \
+        long long ref_batch_stride, const uint16_t *sampling_offsets, int offsets_row_stride,                         \
+        const uint16_t *attn_logits, int logits_row_stride, const float *offsets_table, const float *logits_table,    \
+        int batch, int spatial_size, int num_heads, int channels, int num_levels, int num_query, int num_point,       \
+        uint16_t *output, void *stream) {                                                                            \
+        const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};                    \
+        return fused_forward_strided<V>(reinterpret_cast<const V *>(value), spatial_shapes, level_start,             \
+                                        reference_points, ref_batch_stride,                                          \
+                                        reinterpret_cast<const V *>(sampling_offsets), offsets_row_stride,           \
+                                        reinterpret_cast<const V *>(attn_logits), logits_row_stride, offsets_table,  \
+                                        logits_table, d, reinterpret_cast<V *>(output), (cudaStream_t)stream);       \
+    }                                                                                                                \
+    int msda_b200_add_layernorm_mixed_##SUFFIX(const float *x, const uint16_t *residual, const float *gamma,         \
+                                               const float *beta, float *y, uint16_t *y16, long long rows, int cols, \
+                                               float eps, void *stream) {                                            \
+        return add_layernorm_mixed<V>(x, reinterpret_cast<const V *>(residual), gamma, beta, y,                      \
+                                      reinterpret_cast<V *>(y16), rows, cols, eps, stream);                         \
+    }                                                                                                                \
+    int msda_b200_add_layernorm_mixed_backward_##SUFFIX(                                                             \
+        const float *grad_y, const uint16_t *grad_y16, const float *x, const uint16_t *residual, const float *gamma,  \
+        float *grad_x, uint16_t *grad_residual, float *grad_gamma, float *grad_beta, long long rows, int cols,        \
+        float eps, void *stream) {                                                                                   \
+        return add_layernorm_mixed_backward<V>(grad_y, reinterpret_cast<const V *>(grad_y16), x,                     \
+                                               reinterpret_cast<const V *>(residual), gamma, grad_x,                 \
+                                               reinterpret_cast<V *>(grad_residual), grad_gamma, grad_beta, rows,    \
+                                               cols, eps, nullptr, stream, false);                                   \
+    }                                                                                                                \
+    int msda_b200_add_layernorm_mixed_backward_deterministic_##SUFFIX(                                               \
+        const float *grad_y, const uint16_t *grad_y16, const float *x, const uint16_t *residual, const float *gamma,  \
+        float *grad_x, uint16_t *grad_residual, float *grad_gamma, float *grad_beta, long long rows, int cols,        \
+        float eps, void *workspace, void *stream) {                                                                  \
+        return add_layernorm_mixed_backward<V>(grad_y, reinterpret_cast<const V *>(grad_y16), x,                     \
+                                               reinterpret_cast<const V *>(residual), gamma, grad_x,                 \
+                                               reinterpret_cast<V *>(grad_residual), grad_gamma, grad_beta, rows,    \
+                                               cols, eps, workspace, stream, true);                                  \
     }
 MSDA_MIXED_ENTRIES(bf16, __nv_bfloat16)
 MSDA_MIXED_ENTRIES(f16, __half)

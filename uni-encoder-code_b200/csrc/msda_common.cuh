@@ -505,17 +505,20 @@ struct Producers {
     const float *logit_table;
 };
 
-// PT: element type of `loc` / `attw` (ProducerT: 16-bit only for the mixed-precision fused op, whose rows are packed:
-// the row strides and tables of Producers are the fp32 packed forward's)
-template <bool FUSED, int LP, int QPW, int PLANE, bool WITH_AUX, typename PT>
+// PT: element type of `loc` / `attw` (ProducerT: 16-bit only for the mixed-precision fused op).  STRIDED: the row
+// strides and tables of Producers may be set -- every fp32 fused kernel, and the 16-bit strided forward, whose raw
+// values are widened first and then get their fp32 table entries added
+template <bool FUSED, int LP, int QPW, int PLANE, bool WITH_AUX, typename PT, bool STRIDED = FUSED && !is16<PT>>
 __device__ __forceinline__ void phase1_records(const LevelTable &lt, uint2 *rec, float4 *aux,
                                                const PT *__restrict__ loc,
                                                const PT *__restrict__ attw, const Producers pr,
                                                long long n, int q0, int cnt, int m, int M, int Lq,
                                                int L, uint32_t pix_stride, uint32_t image_f4, int lane) {
     constexpr int kRounds = (QPW * LP + 31) / 32;
-    constexpr bool kStrided = FUSED && !is16<PT>;   // row strides / tables may be set
-    Pair<PT> xy[kRounds];       // as loaded (16-bit: widened where used, one register per pair until then)
+    constexpr bool kStrided = STRIDED;             // row strides / tables may be set
+    constexpr bool kWidened = STRIDED && is16<PT>;  // 16-bit pairs widened as loaded (a table entry may be added)
+    // as loaded (16-bit: widened where used, one register per pair until then -- unless kWidened)
+    std::conditional_t<kWidened, float2, Pair<PT>> xy[kRounds];
     float aw[kRounds];          // attention weight; FUSED: the raw logit until the softmax below
     float2 txy[FUSED ? kRounds : 1];   // FUSED with tables: the table entries, added once ALL loads are in flight
     float taw[FUSED ? kRounds : 1];
@@ -525,7 +528,7 @@ __device__ __forceinline__ void phase1_records(const LevelTable &lt, uint2 *rec,
     for (int r = 0; r < kRounds; ++r) {          // all global loads first
         const int s = r * 32 + lane;
         const int qi = s / LP, sp = s - qi * LP;
-        xy[r] = Pair<PT>{};
+        xy[r] = {};
         aw[r] = 0.f;
         if (FUSED) {
             txy[r] = make_float2(0.f, 0.f);
@@ -539,7 +542,8 @@ __device__ __forceinline__ void phase1_records(const LevelTable &lt, uint2 *rec,
                 li = q * (pr.off_qstride >> 1) + m * LP + sp;
                 ai = q * pr.logit_qstride + m * LP + sp;
             }
-            xy[r] = ldg_stream_pair_raw<PT>(reinterpret_cast<const Pair<PT> *>(loc) + li);
+            if constexpr (kWidened) xy[r] = ldg_stream_pair<PT>(reinterpret_cast<const Pair<PT> *>(loc) + li);
+            else xy[r] = ldg_stream_pair_raw<PT>(reinterpret_cast<const Pair<PT> *>(loc) + li);
             aw[r] = ldg_stream_one<PT>(attw + ai);
             if (kStrided && pr.off_table != nullptr) {
                 // the tables have Lq rows with the projections' row strides: entry = the projection's index
@@ -612,7 +616,9 @@ __device__ __forceinline__ void phase1_records(const LevelTable &lt, uint2 *rec,
         if (qi < cnt) {
             const int l = lt.level_of[sp];
             const int4 lv = lt.hws[l];            // {H, W, start, -}
-            const float2 xyf = widen_pair<PT>(xy[r]);
+            float2 xyf;
+            if constexpr (kWidened) xyf = xy[r];
+            else xyf = widen_pair<PT>(xy[r]);
             float x = xyf.x, y = xyf.y;
             if (FUSED) {
                 const long long rrow = n * pr.ref_bstride + ((long long)(q0 + qi) * L + l) * 2;

@@ -50,19 +50,19 @@ struct FwdCfg {
 // V: element type of value / out (float, or 16-bit: a lane's chunk is then 8 bytes of a 64-byte row,
 // loaded as LDG.64 and widened to fp32; the sums are fp32 and only the output store rounds).  FUSED with 16-bit V:
 // the raw offsets / logits are of type V too (ProducerT), widened as they are loaded
-template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
-__global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
-msda_fwd_d32_kernel(const V *__restrict__ value, const int64_t *__restrict__ shapes,
-                    const int64_t *__restrict__ lstart, const float *__restrict__ loc_arg,
-                    const float *__restrict__ attw_arg, const Producers pr, const Dims d,
-                    const int want_spatial, V *__restrict__ out) {
+// The body of both forward kernels.  STRIDED (phase1_records): the row strides / tables of `pr` may be set.  The
+// shared memory is the kernel's.
+template <typename V, int LP, int WARPS, int TILE_W, int QPW, bool FUSED, bool STRIDED>
+__device__ __forceinline__ void fwd_d32_items(const V *__restrict__ value, const int64_t *__restrict__ shapes,
+                                              const int64_t *__restrict__ lstart, const float *__restrict__ loc_arg,
+                                              const float *__restrict__ attw_arg, const Producers pr, const Dims d,
+                                              const int want_spatial, V *__restrict__ out, unsigned char *smem_raw,
+                                              LevelTable &lt) {
     using Cfg = FwdCfg<LP, WARPS, TILE_W, QPW>;
     // the raw tensors are passed as float pointers whatever their type, so that the fp32 kernels keep their names
     using PT = ProducerT<V, FUSED>;
     const PT *__restrict__ loc = reinterpret_cast<const PT *>(loc_arg);
     const PT *__restrict__ attw = reinterpret_cast<const PT *>(attw_arg);
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    __shared__ LevelTable lt;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int corner = lane >> 3, chunk = lane & 7;
@@ -86,7 +86,7 @@ msda_fwd_d32_kernel(const V *__restrict__ value, const int64_t *__restrict__ sha
         warp_queries(lt, d.L, g, warp, Cfg::kGroup, Cfg::kTileH, TILE_W, d.Lq, Cfg::kQPW, q0, cnt);
 
         // ---- phase 1: one sampling point per lane per round -> records ----
-        phase1_records<FUSED, LP, Cfg::kQPW, Cfg::kPlane, false>(lt, rec, nullptr, loc, attw, pr, n, q0, cnt, m,
+        phase1_records<FUSED, LP, Cfg::kQPW, Cfg::kPlane, false, PT, STRIDED>(lt, rec, nullptr, loc, attw, pr, n, q0, cnt, m,
                                                                  M, d.Lq, d.L, pix_stride, (uint32_t)d.S * pix_stride, lane);
         __syncwarp();
 
@@ -131,16 +131,46 @@ msda_fwd_d32_kernel(const V *__restrict__ value, const int64_t *__restrict__ sha
     }
 }
 
+template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
+__global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
+msda_fwd_d32_kernel(const V *__restrict__ value, const int64_t *__restrict__ shapes,
+                    const int64_t *__restrict__ lstart, const float *__restrict__ loc_arg,
+                    const float *__restrict__ attw_arg, const Producers pr, const Dims d,
+                    const int want_spatial, V *__restrict__ out) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ LevelTable lt;
+    fwd_d32_items<V, LP, WARPS, TILE_W, QPW, FUSED, FUSED && !is16<V>>(value, shapes, lstart, loc_arg, attw_arg, pr, d,
+                                                                      want_spatial, out, smem_raw, lt);
+}
+
+// the mixed-precision fused forward with row strides and / or per-query tables (16-bit V, raw 16-bit offsets / logits
+// in rows of a [rows, 3*M*L*P] projection output, fp32 tables)
+template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW>
+__global__ void __launch_bounds__(WARPS * 32, MIN_CTAS)
+msda_fwd_d32_strided_kernel(const V *__restrict__ value, const int64_t *__restrict__ shapes,
+                            const int64_t *__restrict__ lstart, const float *__restrict__ loc_arg,
+                            const float *__restrict__ attw_arg, const Producers pr, const Dims d,
+                            const int want_spatial, V *__restrict__ out) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ LevelTable lt;
+    fwd_d32_items<V, LP, WARPS, TILE_W, QPW, true, true>(value, shapes, lstart, loc_arg, attw_arg, pr, d, want_spatial,
+                                                         out, smem_raw, lt);
+}
+
 // ---------------------------------------------------------------------------
 // host side: launch_fwd_d32() serves the plain op and the fused producers (Producers::ref set),
 // the latter in the default CTA shape only
 // ---------------------------------------------------------------------------
-template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED>
+// STRIDED: the 16-bit strided kernel (FUSED, 16-bit V)
+template <typename V, int LP, int WARPS, int TILE_W, int MIN_CTAS, int QPW, bool FUSED, bool STRIDED = false>
 static cudaError_t launch_fwd_cfg(const V *value, const int64_t *shapes, const int64_t *lstart,
                                   const ProducerT<V, FUSED> *loc, const ProducerT<V, FUSED> *attw, const Producers &pr,
                                   const Dims &d, V *out, cudaStream_t stream) {
     using Cfg = FwdCfg<LP, WARPS, TILE_W, QPW>;
-    constexpr auto kern = msda_fwd_d32_kernel<V, LP, WARPS, TILE_W, MIN_CTAS, QPW, FUSED>;
+    constexpr auto kern = [] {       // (only the kernel that is launched is instantiated)
+        if constexpr (STRIDED) return msda_fwd_d32_strided_kernel<V, LP, WARPS, TILE_W, MIN_CTAS, QPW>;
+        else return msda_fwd_d32_kernel<V, LP, WARPS, TILE_W, MIN_CTAS, QPW, FUSED>;
+    }();
     cudaError_t e;
     const int blocks = persistent_blocks<kern>(WARPS * 32, Cfg::kSmem, d, &e);
     if (blocks == 0) return e;
@@ -157,8 +187,10 @@ static cudaError_t launch_fwd_lp(const V *value, const int64_t *shapes, const in
                                  V *out, cudaStream_t stream) {
     // variant = (warps, query tile width, min CTAs per SM -> register budget, queries per warp)
 #define MSDA_FWD(W, TW, C, Q, F) launch_fwd_cfg<V, LP, W, TW, C, Q, F>(value, shapes, lstart, loc, attw, pr, d, out, stream)
-    if constexpr (is16<P>) {
-        return MSDA_FWD(16, 16, 2, 8, true);                      // 16-bit fused producers: the default shape only
+    if constexpr (is16<P>) {                                   // 16-bit fused producers: the default shape only
+        if (pr.off_qstride != 0 || pr.off_table != nullptr)
+            return launch_fwd_cfg<V, LP, 16, 16, 2, 8, true, true>(value, shapes, lstart, loc, attw, pr, d, out, stream);
+        return MSDA_FWD(16, 16, 2, 8, true);
     } else if constexpr (is16<V>) {
         return MSDA_FWD(16, 16, 2, 8, false);                     // 16-bit plain: the default shape only
     } else {

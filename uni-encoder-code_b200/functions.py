@@ -174,6 +174,37 @@ class AddLayerNormFunction(Function):
         return gv, gv, gg, gb, None
 
 
+class AddLayerNormMixedFunction(Function):
+    """``apply(x, residual16, weight, bias, eps)`` -> ``(y, y16)`` with ``y = F.layer_norm(x + residual16.float(), (C,),
+    weight, bias, eps)`` (fp32: the residual stream under torch.autocast) and ``y16 = y.to(residual16.dtype)`` (the copy
+    the next GEMMs read) -- one kernel each way (ops.add_layernorm_mixed / add_layernorm_mixed_backward); C in {128,
+    256}.  Either output may go unused: its gradient is then absent, and the backward adds the two gradients in fp32
+    where both are present, as autograd does for torch's composition.  Returns an fp32 grad_x and a grad_residual of
+    residual16's dtype."""
+
+    @staticmethod
+    def supported(x, residual, weight) -> bool:
+        return ops.add_layernorm_mixed_backward_supported(x, residual, weight)
+
+    @staticmethod
+    def forward(ctx, x, residual, weight, bias, eps):
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(x, residual, weight)
+        ctx.eps = eps
+        return ops.add_layernorm_mixed(x, residual, weight, bias, eps)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_y, grad_y16):
+        if grad_y is None and grad_y16 is None:
+            return None, None, None, None, None
+        x, residual, weight = ctx.saved_tensors
+        gx, gr, gg, gb = ops.add_layernorm_mixed_backward(
+            _aligned(grad_y) if grad_y is not None else None,
+            _aligned(grad_y16) if grad_y16 is not None else None, x, residual, weight, ctx.eps)
+        return gx, gr, gg, gb, None
+
+
 def _aligned(t):
     """`t` contiguous and 16-byte aligned (the kernels' 128-bit accesses); copies only when it is not."""
     t = t.contiguous()

@@ -29,8 +29,8 @@ import torch.nn.functional as F
 from torch import nn
 
 from . import ops
-from .functions import (AddLayerNormFunction, LinearTF32x3Function, MSDeformAttnFunction, MSDeformAttnFusedFunction,
-                        MSDeformAttnMixedFunction)
+from .functions import (AddLayerNormFunction, AddLayerNormMixedFunction, LinearTF32x3Function, MSDeformAttnFunction,
+                        MSDeformAttnFusedFunction, MSDeformAttnMixedFunction)
 
 CoreFn = Callable[..., torch.Tensor]
 
@@ -94,19 +94,37 @@ def _presplit_of(layer: nn.Linear):
     return hit[1]
 
 
+def _autocast_dtype():
+    """The 16-bit type of the active CUDA torch.autocast, or None (no context, a disabled one, or another type)."""
+    if not torch.is_autocast_enabled("cuda"):
+        return None
+    dtype = torch.get_autocast_dtype("cuda")
+    return dtype if dtype in (torch.bfloat16, torch.float16) else None
+
+
+def _resolve(impl: str) -> str:
+    """linear="autocast" is linear="tf32x3" unless a bf16 / fp16 CUDA autocast is active; then it stays "autocast":
+    torch's autocast GEMMs and the mixed-precision residual + LayerNorm kernels (`_add_norm_mixed`)."""
+    if impl == "autocast" and _autocast_dtype() is None:
+        return "tf32x3"
+    return impl
+
+
 def _linear(layer: nn.Linear, x, impl: str, relu: bool = False):
     """``layer(x)`` (+ ReLU).  impl == "tf32x3" selects the inference kernels of SURVEY 8f.3 (this GEMM and the
     fused residual + LayerNorm of `_add_norm`): in inference (autograd off) the fp32 GEMM runs on the
     tensor cores as an error-compensated 3xTF32 product (ops.linear_tf32x3, SURVEY 8f.3); with autograd
     on, the forward and the input-gradient GEMMs do (LinearTF32x3Function; the weight gradient stays a
-    torch GEMM); for any shape the kernel does not cover torch's own fp32 GEMM is used as in the reference."""
+    torch GEMM); for any shape the kernel does not cover torch's own fp32 GEMM is used as in the reference.
+    impl == "autocast": see `_resolve` (under autocast, torch's own 16-bit GEMM)."""
+    impl = _resolve(impl)
     if impl == "tf32x3" and not torch.is_grad_enabled() and x.is_contiguous() \
             and ops.linear_tf32x3_supported(x, layer.weight):
         return ops.linear_tf32x3(x, layer.weight, layer.bias, relu=relu, presplit=_presplit_of(layer))
     if impl == "tf32x3" and torch.is_grad_enabled() and LinearTF32x3Function.supported(x, layer.weight):
         # all three GEMMs on the tensor cores; the ReLU rides in the forward GEMM's epilogue
         return LinearTF32x3Function.apply(x, layer.weight, layer.bias, relu)
-    if impl not in ("torch", "tf32x3"):
+    if impl not in ("torch", "tf32x3", "autocast"):
         raise ValueError(f"unknown linear implementation {impl!r}")
     y = layer(x)
     return F.relu(y) if relu else y
@@ -114,6 +132,7 @@ def _linear(layer: nn.Linear, x, impl: str, relu: bool = False):
 
 def _add_norm(norm: nn.LayerNorm, x, sublayer_out, impl: str):
     """``norm(x + sublayer_out)``; impl == "tf32x3" (inference): one fused pass (ops.add_layernorm)."""
+    impl = _resolve(impl)
     if impl == "tf32x3" and not torch.is_grad_enabled() and norm.elementwise_affine \
             and ops.add_layernorm_supported(x, sublayer_out, norm.weight, norm.bias, need_bias=True):
         return ops.add_layernorm(x, sublayer_out, norm.weight, norm.bias, norm.eps)
@@ -122,6 +141,21 @@ def _add_norm(norm: nn.LayerNorm, x, sublayer_out, impl: str):
             and AddLayerNormFunction.supported(x, sublayer_out, norm.weight):
         return AddLayerNormFunction.apply(x, sublayer_out, norm.weight, norm.bias, norm.eps)
     return norm(x + sublayer_out)
+
+
+def _add_norm_mixed(norm: nn.LayerNorm, x, sublayer_out):
+    """Under a 16-bit autocast: (``norm(x + sublayer_out)``, its 16-bit copy for the next GEMMs or None).  An fp32
+    residual stream ``x`` and a 16-bit ``sublayer_out`` go through the mixed-precision kernels (ops.add_layernorm_mixed
+    without autograd, AddLayerNormMixedFunction with it), which also write the copy autocast's own cast would give;
+    whatever they do not cover takes torch's composition (no copy: the GEMMs cast)."""
+    if norm.elementwise_affine and norm.bias is not None and sublayer_out.dtype == _autocast_dtype():
+        if not torch.is_grad_enabled() \
+                and ops.add_layernorm_mixed_supported(x, sublayer_out, norm.weight, norm.bias, need_bias=True):
+            return ops.add_layernorm_mixed(x, sublayer_out, norm.weight, norm.bias, norm.eps)
+        if torch.is_grad_enabled() and AddLayerNormMixedFunction.supported(x, sublayer_out, norm.weight) \
+                and ops.add_layernorm_mixed_supported(x, sublayer_out, norm.weight, norm.bias, need_bias=True):
+            return AddLayerNormMixedFunction.apply(x, sublayer_out, norm.weight, norm.bias, norm.eps)
+    return norm(x + sublayer_out), None
 
 
 def _cuda_core(value, spatial_shapes, level_start_index, sampling_locations, attention_weights,
@@ -141,7 +175,7 @@ class MSDeformAttn(nn.Module):
                  fused: bool = False, linear: str = "torch"):
         """`fused=True` (not in the reference): softmax and location arithmetic run inside the
         kernels whenever the shapes allow (SURVEY 8f.1); results agree to rounding.
-        `linear="tf32x3"` (not in the reference): see `_linear`."""
+        `linear="tf32x3"` (not in the reference): see `_linear`; `linear="autocast"`: see `_resolve`."""
         super().__init__()
         self.fused = fused
         self.linear = linear
@@ -232,7 +266,9 @@ class MSDeformAttn(nn.Module):
         """Whether `forward_shared_pos` applies: inference kernels on, no mask, 2-d reference points, and
         `pos` [N or 1, S, C] holding the same rows for every image (batch stride 0, as the pixel decoder's
         sine embedding + level embedding is)."""
-        return (self.fused and self.linear == "tf32x3" and self._core is _cuda_core
+        if _resolve(self.linear) == "autocast":
+            return self._can_fold_pos_mixed(src, pos, reference_points, padding_mask)
+        return (self.fused and _resolve(self.linear) == "tf32x3" and self._core is _cuda_core
                 and not torch.is_grad_enabled() and padding_mask is None and pos is not None
                 and pos.dim() == 3 and (pos.size(0) == 1 or pos.stride(0) == 0)
                 and pos.shape[1:] == src.shape[1:] and pos[0].is_contiguous()
@@ -242,6 +278,19 @@ class MSDeformAttn(nn.Module):
                 and not reference_points.requires_grad
                 and self.d_model // self.n_heads == 32 and self.n_levels * self.n_points in (4, 8, 12, 16)
                 and ops.linear_tf32x3_supported(src, self.sampling_offsets.weight)
+                and self.sampling_offsets.bias is not None and self.attention_weights.bias is not None)
+
+    def _can_fold_pos_mixed(self, src, pos, reference_points, padding_mask) -> bool:
+        """`can_fold_pos` under a 16-bit autocast (linear="autocast"): the same conditions, with the query GEMM run by
+        autocast and the fused forward the 16-bit packed one (ops.ms_deform_attn_fused_mixed_forward_packed)."""
+        return (self.fused and self._core is _cuda_core and not torch.is_grad_enabled() and padding_mask is None
+                and pos is not None and pos.dim() == 3 and (pos.size(0) == 1 or pos.stride(0) == 0)
+                and pos.shape[1:] == src.shape[1:] and pos[0].is_contiguous()
+                and src.is_cuda and src.dtype == torch.float32 and pos.dtype == torch.float32
+                and pos.device == src.device and reference_points.dim() == 4 and reference_points.size(-1) == 2
+                and not reference_points.requires_grad
+                and self.d_model // self.n_heads == 32 and self.n_levels * self.n_points in (4, 8, 12, 16)
+                and ops.linear_tf32x3_supported(pos[0], self.sampling_offsets.weight)
                 and self.sampling_offsets.bias is not None and self.attention_weights.bias is not None)
 
     def _query_projection(self, pos_rows):
@@ -263,13 +312,18 @@ class MSDeformAttn(nn.Module):
         return self._qproj[0], self._qproj[1], self._qproj[3]
 
     def forward_shared_pos(self, src, pos, reference_points, input_spatial_shapes, input_level_start_index,
-                           value=None):
+                           value=None, src16=None):
         """`forward(src + pos, reference_points, src, ...)` without forming `src + pos`: the two query
         projections run as ONE GEMM on `src`; the fused kernel reads offsets and logits in place from its
         [N, S, 3*M*L*P] output and adds the cached `pos @ W^T + b` row of the query
         ((src + pos) W^T + b = src W^T + (pos W^T + b)).  `value`: a callable returning the projected value
         [N, S, M, D] (query-range sharding: `src` holds this rank's rows only and the value rows of the other
-        ranks are still in flight while the query GEMM runs); default: `project_value(src)`."""
+        ranks are still in flight while the query GEMM runs); default: `project_value(src)`.
+        Under a 16-bit autocast (linear="autocast"): the query GEMM and the value projection read `src16`, the 16-bit
+        copy of `src` (default: `src` cast), and the 16-bit packed forward adds the same fp32 table."""
+        if _resolve(self.linear) == "autocast":
+            return self._forward_shared_pos_mixed(src, pos, reference_points, input_spatial_shapes,
+                                                  input_level_start_index, value, src16)
         if value is None:
             value = self.project_value(src)
         weight, table, split = self._query_projection(pos[0])
@@ -282,6 +336,30 @@ class MSDeformAttn(nn.Module):
         out = ops.ms_deform_attn_fused_forward_packed(value, input_spatial_shapes, input_level_start_index,
                                                       ref.contiguous(), proj, self.n_levels, self.n_points,
                                                       query_table=table)
+        return _linear(self.output_proj, out, self.linear)
+
+    def _forward_shared_pos_mixed(self, src, pos, reference_points, input_spatial_shapes, input_level_start_index,
+                                  value, src16):
+        if src16 is None:
+            src16 = src.to(_autocast_dtype())
+        if value is None:
+            value = self.project_value(src16)
+        weight, table, _ = self._query_projection(pos[0])
+        proj = F.linear(src16, weight)                     # autocast's 16-bit GEMM; the bias is in the table
+        if callable(value):
+            value = value()
+        ref = reference_points
+        if ref.stride(0) == 0:
+            ref = ref[:1]
+        ref = ref.contiguous()
+        if ops.ms_deform_attn_fused_mixed_forward_packed_supported(value, ref, proj, self.n_levels, self.n_points,
+                                                                   table):
+            out = ops.ms_deform_attn_fused_mixed_forward_packed(value, input_spatial_shapes, input_level_start_index,
+                                                                ref, proj, self.n_levels, self.n_points,
+                                                                query_table=table)
+        else:                                              # e.g. a value view the kernel cannot take
+            q = src + pos
+            return self.forward(q, reference_points, src16, input_spatial_shapes, input_level_start_index)
         return _linear(self.output_proj, out, self.linear)
 
 
@@ -308,7 +386,7 @@ class MSDeformAttnTransformerEncoderLayer(nn.Module):
 
     def forward_ffn(self, src):
         p = self.dropout2.p if self.dropout2.training else 0.0
-        if (self.activation is F.relu and self.linear == "tf32x3" and torch.is_grad_enabled() and 0.0 < p < 1.0
+        if (self.activation is F.relu and _resolve(self.linear) == "tf32x3" and torch.is_grad_enabled() and 0.0 < p < 1.0
                 and LinearTF32x3Function.supported(src, self.linear1.weight)):
             # training: linear1 + ReLU + dropout2 as one autograd node (one pass over the hidden gradient)
             hidden = LinearTF32x3Function.apply(src, self.linear1.weight, self.linear1.bias, True, p)
@@ -321,12 +399,41 @@ class MSDeformAttnTransformerEncoderLayer(nn.Module):
         return _add_norm(self.norm2, src, self.dropout3(_linear(self.linear2, hidden, self.linear)), self.linear)
 
     def forward(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask=None):
+        return self._forward_pair(src, None, pos, reference_points, spatial_shapes, level_start_index, padding_mask)[0]
+
+    def _forward_pair(self, src, src16, pos, reference_points, spatial_shapes, level_start_index, padding_mask=None):
+        """-> (output, its 16-bit copy or None).  `src16`: the 16-bit copy of `src` that the previous layer's mixed
+        residual + LayerNorm kernel wrote, or None.  Under a 16-bit autocast with linear="autocast" the two norms go
+        through `_add_norm_mixed`, and the GEMMs that read a norm's output (value_proj, linear1, and the next layer's)
+        read its copy instead of casting it again; otherwise `forward`'s computation, and no copy."""
+        if _resolve(self.linear) != "autocast":
+            if self.self_attn.can_fold_pos(src, pos, reference_points, padding_mask):
+                attn = self.self_attn.forward_shared_pos(src, pos, reference_points, spatial_shapes, level_start_index)
+            else:
+                q = src if pos is None else src + pos
+                attn = self.self_attn(q, reference_points, src, spatial_shapes, level_start_index, padding_mask)
+            return self.forward_ffn(_add_norm(self.norm1, src, self.dropout1(attn), self.linear)), None
+        if src16 is None and src.dtype == torch.float32:
+            src16 = src.to(_autocast_dtype())              # the first layer's input: a plain cast
+        value_in = src16 if src16 is not None else src
         if self.self_attn.can_fold_pos(src, pos, reference_points, padding_mask):
-            attn = self.self_attn.forward_shared_pos(src, pos, reference_points, spatial_shapes, level_start_index)
+            attn = self.self_attn.forward_shared_pos(src, pos, reference_points, spatial_shapes, level_start_index,
+                                                     src16=src16)
         else:
             q = src if pos is None else src + pos
-            attn = self.self_attn(q, reference_points, src, spatial_shapes, level_start_index, padding_mask)
-        return self.forward_ffn(_add_norm(self.norm1, src, self.dropout1(attn), self.linear))
+            attn = self.self_attn(q, reference_points, value_in, spatial_shapes, level_start_index, padding_mask)
+        y, y16 = _add_norm_mixed(self.norm1, src, self.dropout1(attn))
+        return self._forward_ffn_mixed(y, y16)
+
+    def _forward_ffn_mixed(self, src, src16):
+        """`forward_ffn` under a 16-bit autocast: linear1 reads `src16` when there is one -> (output, its copy)."""
+        x = src16 if src16 is not None else src
+        if self.activation is F.relu:
+            hidden = F.relu(self.linear1(x))
+        else:
+            hidden = self.activation(self.linear1(x))
+        hidden = self.dropout2(hidden)
+        return _add_norm_mixed(self.norm2, src, self.dropout3(self.linear2(hidden)))
 
 
 _REF_CACHE = ShapeCache()
@@ -395,9 +502,13 @@ class MSDeformAttnTransformerEncoder(nn.Module):
             ref = reference_points_for(levels, src.device).expand(src.shape[0], -1, -1, -1)
         else:
             ref = self.get_reference_points(spatial_shapes, valid_ratios, src.device)
-        out = src
+        out, out16 = src, None
         for layer in self.layers:
-            out = layer(out, pos, ref, spatial_shapes, level_start_index, padding_mask)
+            if _resolve(layer.linear) == "autocast":
+                # under autocast each layer hands the 16-bit copy of its output to the next
+                out, out16 = layer._forward_pair(out, out16, pos, ref, spatial_shapes, level_start_index, padding_mask)
+            else:
+                out = layer(out, pos, ref, spatial_shapes, level_start_index, padding_mask)
         return out
 
 

@@ -425,6 +425,74 @@ def ms_deform_attn_fused_forward_packed(value, spatial_shapes, level_start_index
                           query_table[:, 2 * M * L * P:] if query_table is not None else None, (N, S, M, D, L, Lq, P))
 
 
+_FUSED_MIXED_FWD_STRIDED = {torch.bfloat16: _lib.lib.msda_b200_fused_forward_strided_bf16,
+                            torch.float16: _lib.lib.msda_b200_fused_forward_strided_f16}
+
+
+def ms_deform_attn_fused_mixed_forward_packed_supported(value, reference_points, projections, n_levels, n_points,
+                                                        query_table=None) -> bool:
+    """Whether ``ms_deform_attn_fused_mixed_forward_packed`` covers these tensors: what the 16-bit fused forward
+    covers (``fused_supported``), ``projections`` a contiguous [N, Lq, 3*M*L*P] tensor of value's 16-bit type,
+    4-byte aligned, fp32 reference points with Lq rows, and ``query_table`` None or a contiguous fp32 [Lq, 3*M*L*P]
+    tensor, 8-byte aligned, on value's device."""
+    if not (isinstance(value, torch.Tensor) and value.is_cuda and value.dtype in _FUSED_MIXED_FWD_STRIDED
+            and value.dim() == 4 and isinstance(projections, torch.Tensor) and projections.dim() == 3):
+        return False
+    N, S, M, D = value.shape
+    L, P = int(n_levels), int(n_points)
+    width = 3 * M * L * P
+    if not (projections.dtype == value.dtype and projections.size(0) == N and projections.size(2) == width
+            and projections.is_contiguous() and projections.device == value.device and projections.data_ptr() % 4 == 0
+            and value.is_contiguous() and value.data_ptr() % 16 == 0):
+        return False
+    Lq = projections.size(1)
+    if query_table is not None and not (
+            isinstance(query_table, torch.Tensor) and query_table.dtype == torch.float32
+            and tuple(query_table.shape) == (Lq, width) and query_table.is_contiguous()
+            and query_table.device == value.device and query_table.data_ptr() % 8 == 0):
+        return False
+    off = projections[..., :2 * M * L * P]
+    return (isinstance(reference_points, torch.Tensor) and reference_points.dtype == torch.float32
+            and reference_points.is_contiguous() and reference_points.device == value.device
+            and fused_supported(value, reference_points, off.view(N, Lq, M, L, P, 2), projections[..., 2 * M * L * P:])
+            and tuple(reference_points.shape[1:]) == (Lq, L, 2))
+
+
+def ms_deform_attn_fused_mixed_forward_packed(value, spatial_shapes, level_start_index, reference_points,
+                                              projections, n_levels, n_points, query_table=None):
+    """``ms_deform_attn_fused_forward_packed`` for mixed precision: a bf16 / fp16 ``value`` and ``projections``
+    [N, Lq, 3*M*L*P] (the stacked query GEMM run under torch.autocast), fp32 ``reference_points`` and fp32
+    ``query_table`` [Lq, 3*M*L*P] (optional).  Each raw offset / logit is widened, then gets its table entry added in
+    fp32; output [N, Lq, M*D] in value's dtype is the fp32 strided forward on the widened inputs rounded once
+    (msda_b200_fused_forward_strided_bf16 / _f16).  Inference only."""
+    N, S, M, D = value.shape
+    L, P = int(n_levels), int(n_points)
+    named = [("value", value), ("spatial_shapes", spatial_shapes), ("level_start_index", level_start_index),
+             ("reference_points", reference_points), ("projections", projections)]
+    if query_table is not None:
+        named.append(("query_table", query_table))
+    _require_cuda_contiguous(named)
+    if not ms_deform_attn_fused_mixed_forward_packed_supported(value, reference_points, projections, L, P, query_table) \
+            or spatial_shapes.size(0) != L:
+        raise RuntimeError("ms_deform_attn_fused_mixed_forward_packed covers a bf16 / fp16 value and projections "
+                           "[N, Lq, 3*M*L*P] of the same type, fp32 reference points and query_table [Lq, 3*M*L*P], "
+                           "32 channels per head, L*P in {4,8,12,16}")
+    Lq = projections.size(1)
+    width = 3 * M * L * P
+    rs = 0 if reference_points.size(0) == 1 and N > 1 else Lq * L * 2
+    with torch.cuda.device(value.device):
+        output = torch.empty((N, Lq, M * D), dtype=value.dtype, device=value.device)
+        with _timed("forward_mixed"):
+            rc = _FUSED_MIXED_FWD_STRIDED[value.dtype](
+                value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(), reference_points.data_ptr(),
+                rs, projections.data_ptr(), width, projections.data_ptr() + 2 * M * L * P * projections.element_size(),
+                width, _ptr(query_table),
+                query_table.data_ptr() + 2 * M * L * P * 4 if query_table is not None else None,
+                N, S, M, D, L, Lq, P, output.data_ptr(), torch.cuda.current_stream().cuda_stream)
+    _lib.check(rc, "ms_deform_attn_fused_mixed_forward_packed")
+    return output
+
+
 def ms_deform_attn_fused_backward(value, spatial_shapes, level_start_index, reference_points,
                                   sampling_offsets, attn_logits, grad_output):
     """[grad_value, grad_sampling_offsets, grad_attn_logits] in the inputs' dtypes (msda_b200_fused_backward_f32;
@@ -573,6 +641,96 @@ def add_layernorm(x, residual, weight, bias, eps=1e-5):
             torch.cuda.current_stream(x.device).cuda_stream)
     _lib.check(rc, "add_layernorm")
     return y
+
+
+# ---------------------------------------------------------------- mixed precision (torch.autocast) residual + LayerNorm
+_LN_MIXED = {torch.bfloat16: _lib.lib.msda_b200_add_layernorm_mixed_bf16,
+             torch.float16: _lib.lib.msda_b200_add_layernorm_mixed_f16}
+_LN_MIXED_BWD = {torch.bfloat16: _lib.lib.msda_b200_add_layernorm_mixed_backward_bf16,
+                 torch.float16: _lib.lib.msda_b200_add_layernorm_mixed_backward_f16}
+_LN_MIXED_BWD_DET = {torch.bfloat16: _lib.lib.msda_b200_add_layernorm_mixed_backward_deterministic_bf16,
+                     torch.float16: _lib.lib.msda_b200_add_layernorm_mixed_backward_deterministic_f16}
+
+
+def _rows16_ok(t, x) -> bool:
+    """`t` a contiguous bf16 / fp16 tensor shaped like `x` on x's device, 8-byte aligned (the kernels' 4-element
+    accesses)."""
+    return (isinstance(t, torch.Tensor) and t.dtype in _LN_MIXED and t.shape == x.shape and t.is_contiguous()
+            and t.device == x.device and t.data_ptr() % 8 == 0)
+
+
+def add_layernorm_mixed_supported(x, residual, weight, bias=None, need_bias=False) -> bool:
+    """Whether the mixed-precision residual + LayerNorm kernels cover these tensors: ``x`` what ``add_layernorm``
+    takes and 16-byte aligned, ``residual`` a contiguous bf16 / fp16 tensor of x's shape, 8-byte aligned (an unaligned
+    view takes torch's path in the modules)."""
+    return (add_layernorm_supported(x, None, weight, bias, need_bias) and x.data_ptr() % 16 == 0
+            and weight.data_ptr() % 16 == 0 and (bias is None or bias.data_ptr() % 16 == 0)
+            and _rows16_ok(residual, x))
+
+
+def add_layernorm_mixed(x, residual, weight, bias, eps=1e-5, want_y16=True):
+    """``(y, y16)``: ``y = F.layer_norm(x + residual.float(), (C,), weight, bias, eps)`` (fp32, bit-identical to
+    ``add_layernorm(x, residual.float(), ...)``) and ``y16 = y.to(residual.dtype)`` (None unless ``want_y16``), for an
+    fp32 ``x`` and a bf16 / fp16 ``residual`` -- torch.autocast's ``layer_norm(x + sublayer)`` and the cast of its
+    result for the next GEMM, in one pass (msda_b200_add_layernorm_mixed_bf16 / _f16).  Inference only (no autograd:
+    functions.AddLayerNormMixedFunction)."""
+    if not x.is_cuda:
+        raise RuntimeError("Not implemented on the CPU")
+    if not add_layernorm_mixed_supported(x, residual, weight, bias, need_bias=True):
+        raise RuntimeError("add_layernorm_mixed needs a contiguous fp32 CUDA x (16-byte aligned) with a last dimension of "
+                           "128, 256, 384 or 512, a contiguous bf16 / fp16 residual of its shape (8-byte aligned) and "
+                           "fp32 affine parameters")
+    y = torch.empty_like(x)
+    y16 = torch.empty_like(residual) if want_y16 else None
+    cols = x.size(-1)
+    with torch.cuda.device(x.device):
+        with _timed("add_layernorm_mixed"):
+            rc = _LN_MIXED[residual.dtype](x.data_ptr(), residual.data_ptr(), weight.data_ptr(), bias.data_ptr(),
+                                           y.data_ptr(), _ptr(y16), x.numel() // cols, cols, float(eps),
+                                           torch.cuda.current_stream(x.device).cuda_stream)
+    _lib.check(rc, "add_layernorm_mixed")
+    return y, y16
+
+
+def add_layernorm_mixed_backward_supported(x, residual, weight) -> bool:
+    """Whether ``add_layernorm_mixed_backward`` covers these tensors: those of ``add_layernorm_mixed_supported`` with a
+    last dimension of 128 or 256."""
+    return add_layernorm_mixed_supported(x, residual, weight) and x.size(-1) in (128, 256)
+
+
+def add_layernorm_mixed_backward(grad_y, grad_y16, x, residual, weight, eps=1e-5):
+    """``(grad_x, grad_residual, grad_weight, grad_bias)`` of ``add_layernorm_mixed`` from the gradients of ``y`` (fp32)
+    and ``y16`` (residual's dtype); either may be None.  With ``g = grad_y + grad_y16.float()``, ``grad_x`` (fp32) is
+    bit-identical to ``add_layernorm_backward(g, x, residual.float(), weight)[0]`` and ``grad_residual`` is
+    ``grad_x.to(residual.dtype)``: what autograd computes for torch.autocast's composition.  With
+    torch.use_deterministic_algorithms(True) the deterministic entries (per-CTA partials added in CTA order)."""
+    if grad_y is None and grad_y16 is None:
+        raise RuntimeError("add_layernorm_mixed_backward needs grad_y or grad_y16")
+    if not add_layernorm_mixed_backward_supported(x, residual, weight) \
+            or (grad_y is not None and not (grad_y.shape == x.shape and grad_y.is_contiguous()
+                                            and grad_y.dtype == torch.float32 and grad_y.device == x.device
+                                            and grad_y.data_ptr() % 16 == 0)) \
+            or (grad_y16 is not None and not (_rows16_ok(grad_y16, x) and grad_y16.dtype == residual.dtype)):
+        raise RuntimeError("add_layernorm_mixed_backward needs what add_layernorm_mixed needs, a last dimension of 128 or "
+                           "256, a contiguous fp32 grad_y (16-byte aligned) and a contiguous grad_y16 of residual's "
+                           "dtype (8-byte aligned)")
+    gx = torch.empty_like(x)
+    gr = torch.empty_like(residual)
+    gg, gb = torch.empty_like(weight), torch.empty_like(weight)
+    cols = x.size(-1)
+    rows = x.numel() // cols
+    with torch.cuda.device(x.device):
+        args = (_ptr(grad_y), _ptr(grad_y16), x.data_ptr(), residual.data_ptr(), weight.data_ptr(), gx.data_ptr(),
+                gr.data_ptr(), gg.data_ptr(), gb.data_ptr(), rows, cols, float(eps))
+        stream = torch.cuda.current_stream(x.device).cuda_stream
+        with _timed("add_layernorm_mixed_backward"):
+            if _deterministic():
+                ws = _workspace(_lib.lib.msda_b200_add_layernorm_backward_deterministic_workspace_bytes(rows, cols), x)
+                rc = _LN_MIXED_BWD_DET[residual.dtype](*args, ws.data_ptr(), stream)
+            else:
+                rc = _LN_MIXED_BWD[residual.dtype](*args, stream)
+    _lib.check(rc, "add_layernorm_mixed_backward")
+    return gx, gr, gg, gb
 
 
 def _vec_ok(t, x) -> bool:

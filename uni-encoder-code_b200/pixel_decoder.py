@@ -26,7 +26,7 @@ from torch import nn
 
 from . import ops
 from .functions import GroupNormFunction, GroupNormRowsFunction
-from .modules import CoreFn, MSDeformAttnTransformerEncoderOnly, ShapeCache, _capturing
+from .modules import CoreFn, MSDeformAttnTransformerEncoderOnly, ShapeCache, _capturing, _resolve
 
 
 class PositionEmbeddingSine(nn.Module):
@@ -129,7 +129,11 @@ class MSDeformAttnPixelDecoder(nn.Module):
         instead of disabling it -- torch's 16-bit GEMMs and convolutions, and the mixed-precision MSDA op
         (functions.MSDeformAttnMixedFunction; with `fused=True` the 16-bit fused-producer kernels,
         functions.MSDeformAttnFusedFunction, which take the softmax and the location arithmetic off torch).
-        `amp=False` is the reference's behaviour: autocast off, fp32."""
+        `amp=False` is the reference's behaviour: autocast off, fp32.
+        `linear="autocast"` (not in the reference): `linear="tf32x3"` where no bf16 / fp16 autocast is active (with
+        `amp=False` always); under one, torch's autocast GEMMs, convolutions and GroupNorms as with `linear="torch"`,
+        except the encoder's residual + LayerNorm steps and the batch-shared position embedding's query projection,
+        which run on the mixed-precision kernels (modules._add_norm_mixed, MSDeformAttn.forward_shared_pos)."""
         if amp and linear == "tf32x3":
             raise ValueError('amp=True cannot be combined with linear="tf32x3": the 3xTF32 GEMMs and the fp32 '
                              'GroupNorm / LayerNorm kernels are fp32 paths that autocast would bypass')
@@ -181,7 +185,8 @@ class MSDeformAttnPixelDecoder(nn.Module):
         autocast, if any)."""
         device_type = next(iter(features.values())).device.type
         with contextlib.nullcontext() if self.amp else torch.autocast(device_type=device_type, enabled=False):
-            fused_norm = self.linear == "tf32x3"        # the inference kernels of SURVEY 8f.3 / 8f.4
+            # the inference kernels of SURVEY 8f.3 / 8f.4 (linear="autocast": when no 16-bit autocast is active)
+            fused_norm = _resolve(self.linear) == "tf32x3"
             names = self.transformer_in_features[::-1]
             levels = [(int(features[k].shape[2]), int(features[k].shape[3])) for k in names]
             srcs, src_flat = self._input_proj([features[k].float() for k in names], levels, fused_norm)
