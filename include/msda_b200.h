@@ -507,6 +507,95 @@ int msda_b200_add_channel_bias_nchw_f32(float *x, const float *bias, int batch, 
                                         long long plane, void *stream);
 
 /*
+ * Mixed precision (torch.autocast: the convolution in front of each GroupNorm writes bf16 / fp16): the GroupNorms
+ * above on a bf16 (_bf16) or fp16 (_f16) map x, passed as uint16_t bit patterns.  channel_bias, gamma, beta, up,
+ * mean_rstd and every `float *` output stay fp32; the workspaces are those of the fp32 entries.  Contract: bit
+ * identity with the fp32 entry of the same name fed the widened map (the fp32 arithmetic and its grouping are that
+ * entry's; x is widened on load):
+ *   y, y_rows, mean_rstd, grad_gamma, grad_beta, grad_channel_bias, grad_up == the fp32 entry's on widen(x) and the
+ *                      widened incoming gradient;
+ *   y16                == y rounded to the 16-bit type (round-to-nearest-even, == y.to(dtype); fp16 overflow gives
+ *                      +-inf): the copy the next convolution reads;
+ *   grad_x (16-bit)    == the fp32 entry's grad_x rounded once.
+ * The NCHW forwards write y and / or y16 (either may be NULL, not both: MSDA_ERR_NULL_POINTER).  The NCHW backward
+ * takes the gradient of whichever output the forward wrote: exactly one of grad_y (fp32) and grad_y16 (16-bit);
+ * neither gives MSDA_ERR_NULL_POINTER, both MSDA_ERR_UNSUPPORTED.  Requirements are the fp32 twins', with x, y16,
+ * grad_y16 and grad_x 8-byte aligned (the fp32 maps 16-byte aligned); MSDA_ERR_UNSUPPORTED otherwise.  Launches as
+ * in fp32: two forward, three backward (four with grad_up).
+ */
+int msda_b200_group_norm_nchw_mixed_bf16(const uint16_t *x, const float *channel_bias, const float *gamma,
+                                         const float *beta, float *y, uint16_t *y16, int batch, int channels,
+                                         int height, int width, int groups, float eps, int relu, const float *up,
+                                         int up_h, int up_w, void *workspace, void *stream);
+int msda_b200_group_norm_nchw_mixed_f16(const uint16_t *x, const float *channel_bias, const float *gamma,
+                                        const float *beta, float *y, uint16_t *y16, int batch, int channels,
+                                        int height, int width, int groups, float eps, int relu, const float *up,
+                                        int up_h, int up_w, void *workspace, void *stream);
+int msda_b200_group_norm_nchw_mixed_train_bf16(const uint16_t *x, const float *channel_bias, const float *gamma,
+                                               const float *beta, float *y, uint16_t *y16, float *mean_rstd,
+                                               int batch, int channels, int height, int width, int groups, float eps,
+                                               int relu, const float *up, int up_h, int up_w, void *workspace,
+                                               void *stream);
+int msda_b200_group_norm_nchw_mixed_train_f16(const uint16_t *x, const float *channel_bias, const float *gamma,
+                                              const float *beta, float *y, uint16_t *y16, float *mean_rstd,
+                                              int batch, int channels, int height, int width, int groups, float eps,
+                                              int relu, const float *up, int up_h, int up_w, void *workspace,
+                                              void *stream);
+/* fp32 rows (the encoder's [N, S, C] input) from a 16-bit NCHW map; strides and requirements of
+ * msda_b200_group_norm_nchw_to_rows_f32, x 8-byte aligned. */
+int msda_b200_group_norm_nchw_to_rows_mixed_bf16(const uint16_t *x, const float *channel_bias, const float *gamma,
+                                                 const float *beta, float *y_rows, long long row_stride,
+                                                 long long image_stride, int batch, int channels, long long plane,
+                                                 int groups, float eps, int relu, void *workspace, void *stream);
+int msda_b200_group_norm_nchw_to_rows_mixed_f16(const uint16_t *x, const float *channel_bias, const float *gamma,
+                                                const float *beta, float *y_rows, long long row_stride,
+                                                long long image_stride, int batch, int channels, long long plane,
+                                                int groups, float eps, int relu, void *workspace, void *stream);
+int msda_b200_group_norm_nchw_to_rows_mixed_train_bf16(const uint16_t *x, const float *channel_bias,
+                                                       const float *gamma, const float *beta, float *y_rows,
+                                                       float *mean_rstd, long long row_stride, long long image_stride,
+                                                       int batch, int channels, long long plane, int groups, float eps,
+                                                       int relu, void *workspace, void *stream);
+int msda_b200_group_norm_nchw_to_rows_mixed_train_f16(const uint16_t *x, const float *channel_bias,
+                                                      const float *gamma, const float *beta, float *y_rows,
+                                                      float *mean_rstd, long long row_stride, long long image_stride,
+                                                      int batch, int channels, long long plane, int groups, float eps,
+                                                      int relu, void *workspace, void *stream);
+int msda_b200_group_norm_backward_nchw_mixed_bf16(const float *grad_y, const uint16_t *grad_y16, const uint16_t *x,
+                                                  const float *channel_bias, const float *gamma, const float *beta,
+                                                  const float *mean_rstd, uint16_t *grad_x, float *grad_gamma,
+                                                  float *grad_beta, float *grad_channel_bias, float *grad_up,
+                                                  int batch, int channels, int height, int width, int groups,
+                                                  int relu, int up_h, int up_w, void *workspace, void *stream);
+int msda_b200_group_norm_backward_nchw_mixed_f16(const float *grad_y, const uint16_t *grad_y16, const uint16_t *x,
+                                                 const float *channel_bias, const float *gamma, const float *beta,
+                                                 const float *mean_rstd, uint16_t *grad_x, float *grad_gamma,
+                                                 float *grad_beta, float *grad_channel_bias, float *grad_up,
+                                                 int batch, int channels, int height, int width, int groups,
+                                                 int relu, int up_h, int up_w, void *workspace, void *stream);
+/* Backward of the rows forwards: fp32 gradient rows, 16-bit x and grad_x (NCHW). */
+int msda_b200_group_norm_rows_backward_mixed_bf16(const float *grad_y_rows, long long row_stride,
+                                                  long long image_stride, const uint16_t *x,
+                                                  const float *channel_bias, const float *gamma, const float *beta,
+                                                  const float *mean_rstd, uint16_t *grad_x, float *grad_gamma,
+                                                  float *grad_beta, float *grad_channel_bias, int batch, int channels,
+                                                  long long plane, int groups, int relu, void *workspace,
+                                                  void *stream);
+int msda_b200_group_norm_rows_backward_mixed_f16(const float *grad_y_rows, long long row_stride,
+                                                 long long image_stride, const uint16_t *x,
+                                                 const float *channel_bias, const float *gamma, const float *beta,
+                                                 const float *mean_rstd, uint16_t *grad_x, float *grad_gamma,
+                                                 float *grad_beta, float *grad_channel_bias, int batch, int channels,
+                                                 long long plane, int groups, int relu, void *workspace,
+                                                 void *stream);
+/* x[n, c, :] = round16(widen(x[n, c, :]) + bias[c]) in place over a 16-bit NCHW map with an fp32 bias
+ * (== (x.float() + bias).to(dtype)); plane % 4 == 0, x 8-byte aligned; MSDA_ERR_UNSUPPORTED otherwise. */
+int msda_b200_add_channel_bias_nchw_bf16(uint16_t *x, const float *bias, int batch, int channels, long long plane,
+                                         void *stream);
+int msda_b200_add_channel_bias_nchw_f16(uint16_t *x, const float *bias, int batch, int channels, long long plane,
+                                        void *stream);
+
+/*
  * Weight and bias gradient of the same Linear (torch autograd semantics), 3 x TF32 on the tensor cores
  * without transposing the operands in memory:
  *     grad_weight[out_features, in_features] = grad_y[rows, out_features]^T * x[rows, in_features]

@@ -36,7 +36,18 @@ DIR defaults to $BENCH_OUT/mixed, and BENCH_OUT to bench_out/ in the repository 
 (p) the 16-bit packed / per-query-table forward (one [N, Lq, 3*M*L*P] projection output and the fp32 table) against
     the 16-bit fused forward on separate offset / logit tensors and the fp32 packed forward with the table, at
     configs[1] and the configs[2] shape; arms alternate, L2 evicted before every call.
-Parts (b) and (c) carry linear="autocast" arms next to the others; the arms of (b) and (c) alternate.
+(g) the decoder's GroupNorm sites at the configs[2] shape (1024x2048, batch 8, Swin-T, conv_dim 256), bf16 and fp16:
+    the FPN lateral (GroupNorm + the up-sampled fp32 encoder level, [8, 256, 256, 512] with up [8, 256, 128, 256]) and
+    output (GroupNorm + ReLU) maps, both returning the 16-bit copy, and the three input projections written as fp32
+    rows of one [8, S, 256] tensor (with the convolution bias added on the fly); forward and backward (from the 16-bit
+    gradient for the two FPN maps, the fp32 rows gradient for the projections).  Arms: the 16-bit kernels, torch's
+    autocast composition (autograd for the backward; its forward runs untimed just before), and the fp32 kernels on
+    the widened map.  Arms alternate, the L2 is evicted before every call.  Algorithmic bytes per element of the map
+    (16-bit kernels): forward 2 + 2 read, 2 written (rows: 4 written), + 4 per element of `up`; backward 2 + 2 + 2 + 2
+    read, 2 written (rows: 4 + 2 + 4 + 2 read), + 2 read and 4 written per element of `up` for its gradient; the fp32
+    kernels 4 for every 2.  Torch's arm is charged the 16-bit kernels' bytes (the site's minimum).
+Parts (b) and (c) carry linear="autocast" arms next to the others, and the linear="autocast" arms with the 16-bit
+GroupNorm kernels off (the predicates patched to refuse 16-bit maps); the arms of (b) and (c) alternate.
 
 Every JSON line carries the card's name and power limit (read-only nvidia-smi query).
 """
@@ -48,6 +59,7 @@ import statistics
 import sys
 
 import torch
+import torch.nn.functional as F
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -327,6 +339,139 @@ def part_p(pkg, args, emit):
         torch.cuda.empty_cache()
 
 
+def part_g(pkg, args, emit):
+    dev = torch.device("cuda", 0)
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    N, C, G, eps = 8, 256, 32, 1e-5
+    gen = torch.Generator(device=dev).manual_seed(6)
+    w = torch.rand(C, device=dev, generator=gen) + 0.5
+    b = torch.randn(C, device=dev, generator=gen) * 0.1
+    cb = torch.randn(C, device=dev, generator=gen) * 0.1
+    base = torch.randn(N, C, 256, 512, device=dev, generator=gen) * 2 + 0.5
+    up = torch.randn(N, C, 128, 256, device=dev, generator=gen)
+    cot = torch.randn(N, C, 256, 512, device=dev, generator=gen)
+    levels = [(128, 256), (64, 128), (32, 64)]
+    S = sum(h * wd for h, wd in levels)
+    proj = [torch.randn(N, C, h, wd, device=dev, generator=gen) for h, wd in levels]
+    rows_cot = torch.randn(N, S, C, device=dev, generator=gen)
+    norm = torch.nn.GroupNorm(G, C, eps=eps).to(dev)
+    with torch.no_grad():
+        norm.weight.copy_(w)
+        norm.bias.copy_(b)
+    for tag in ("bf16", "fp16"):
+        dt = DTYPES[tag]
+        x16, g16 = base.to(dt), cot.to(dt)
+        x32, g32 = x16.float(), g16.float()
+        p16 = [p.to(dt) for p in proj]
+        p32 = [p.float() for p in p16]
+        rows = torch.empty(N, S, C, device=dev)
+        starts = [0]
+        for h, wd in levels:
+            starts.append(starts[-1] + h * wd)
+        slices = [rows[:, a:z] for a, z in zip(starts, starts[1:])]
+        gslices = [rows_cot[:, a:z] for a, z in zip(starts, starts[1:])]
+        sites = {}
+        for site, relu, u in (("lateral", False, up), ("output", True, None)):
+            _, st16 = pkg.ops.group_norm_train(x16, w, b, G, eps, relu=relu, up=u)
+            ups = tuple(u.shape[-2:]) if u is not None else None
+
+            def comp(relu=relu, u=u):
+                xl = x16.detach().requires_grad_(True)
+                ul = u.detach().requires_grad_(True) if u is not None else None
+                wl, bl = w.detach().requires_grad_(True), b.detach().requires_grad_(True)
+                with torch.autocast("cuda", dtype=dt):
+                    y = F.group_norm(xl, G, wl, bl, eps)
+                    y = torch.relu(y) if relu else y
+                    if ul is not None:
+                        y = y + F.interpolate(ul, size=xl.shape[-2:], mode="bilinear", align_corners=False)
+                    y = y.to(dt)
+                return y
+            sites[site] = {
+                ("16-bit kernels", "forward"): lambda relu=relu, u=u: pkg.ops.group_norm_train(
+                    x16, w, b, G, eps, relu=relu, up=u, out_dtype=dt),
+                ("torch autocast composition", "forward"): lambda comp=comp: comp(),
+                ("fp32 kernels", "forward"): lambda relu=relu, u=u: pkg.ops.group_norm_train(x32, w, b, G, eps,
+                                                                                            relu=relu, up=u),
+                ("16-bit kernels", "backward"): lambda relu=relu, st=st16, ups=ups: pkg.ops.group_norm_backward(
+                    g16, x16, w, b, st, G, relu=relu, up_shape=ups),
+                ("torch autocast composition", "backward"): ("graph", lambda comp=comp: comp(), g16),
+                ("fp32 kernels", "backward"): lambda relu=relu, st=st16, ups=ups: pkg.ops.group_norm_backward(
+                    g32, x32, w, b, st, G, relu=relu, up_shape=ups),
+            }
+        stats16 = [pkg.ops.group_norm_rows_train(p, w, b, G, eps, r, channel_bias=cb) for p, r in zip(p16, slices)]
+
+        def rows_comp():
+            leaves = [p.detach().requires_grad_(True) for p in p16]
+            wl, bl = w.detach().requires_grad_(True), b.detach().requires_grad_(True)
+            with torch.autocast("cuda", dtype=dt):
+                return torch.cat([F.group_norm(p, G, wl, bl, eps).flatten(2).transpose(1, 2) for p in leaves], 1)
+        sites["input projections"] = {
+            ("16-bit kernels", "forward"): lambda: [pkg.ops.group_norm_rows_train(p, w, b, G, eps, r, channel_bias=cb)
+                                                    for p, r in zip(p16, slices)],
+            ("torch autocast composition", "forward"): rows_comp,
+            ("fp32 kernels", "forward"): lambda: [pkg.ops.group_norm_rows_train(p, w, b, G, eps, r, channel_bias=cb)
+                                                  for p, r in zip(p32, slices)],
+            ("16-bit kernels", "backward"): lambda: [pkg.ops.group_norm_rows_backward(
+                g, p, w, b, st, G, channel_bias=cb, with_channel_bias=True) for g, p, st in zip(gslices, p16, stats16)],
+            ("torch autocast composition", "backward"): ("graph", rows_comp, rows_cot),
+            ("fp32 kernels", "backward"): lambda: [pkg.ops.group_norm_rows_backward(
+                g, p, w, b, st, G, channel_bias=cb, with_channel_bias=True) for g, p, st in zip(gslices, p32, stats16)],
+        }
+        elems = {"lateral": x16.numel(), "output": x16.numel(), "input projections": N * S * C}
+        upel = up.numel()
+        # bytes of the 16-bit kernels and of the fp32 kernels per site and op (see the docstring)
+        nbytes = {("lateral", "forward"): (6 * elems["lateral"] + 4 * upel, 12 * elems["lateral"] + 4 * upel),
+                  ("output", "forward"): (6 * elems["output"], 12 * elems["output"]),
+                  ("input projections", "forward"): (8 * elems["input projections"], 12 * elems["input projections"]),
+                  ("lateral", "backward"): (10 * elems["lateral"] + 6 * upel, 20 * elems["lateral"] + 8 * upel),
+                  ("output", "backward"): (10 * elems["output"], 20 * elems["output"]),
+                  ("input projections", "backward"): (16 * elems["input projections"],
+                                                      20 * elems["input projections"])}
+        for site, arms in sites.items():
+            def one(k, arms=arms):
+                fn = arms[k]
+                if isinstance(fn, tuple):                      # autograd: the forward untimed, then the backward
+                    y = fn[1]()
+                    return _evicted(flush, lambda: y.backward(fn[2]))
+                return _evicted(flush, fn)
+            times = {k: [] for k in arms}
+            for k in arms:
+                for _ in range(2):
+                    one(k)
+            for _ in range(args.steps):
+                for k in arms:                              # the arms alternate
+                    times[k].append(one(k))
+            for (arm, op), ts in times.items():
+                ms = statistics.median(ts)
+                byt = nbytes[(site, op)][1 if arm == "fp32 kernels" else 0]
+                emit({"part": "g", "what": f"GroupNorm site '{site}', 1024x2048 batch 8, Swin-T, conv_dim 256",
+                      "dtype": tag, "arm": arm, "op": op, "ms_median": ms, "ms_min": min(ts), "ms_max": max(ts),
+                      "timed_calls": len(ts), "algorithmic_bytes": byt,
+                      "bytes_per_element": byt / elems[site], "algorithmic_GBs": byt / ms / 1e6,
+                      "hbm_share": byt / ms / 1e6 / HBM_GBS, "hbm_GBs_reference": HBM_GBS,
+                      "l2": "evicted before every call (256 MB write)"})
+        del sites, x16, g16, x32, g32, p16, p32, rows
+        torch.cuda.empty_cache()
+
+
+@contextlib.contextmanager
+def gn16_off(pkg):
+    """The 16-bit GroupNorm kernels off: the predicates refuse bf16 / fp16 maps, so the decoder's linear="autocast"
+    path runs torch's GroupNorms as before those kernels."""
+    names = ("group_norm_supported", "group_norm_rows_supported", "channel_bias_supported")
+    saved = {n: getattr(pkg.ops, n) for n in names}
+    for n, f in saved.items():
+        setattr(pkg.ops, n, lambda x, *a, _f=f, **k: x.dtype == torch.float32 and _f(x, *a, **k))
+    try:
+        yield
+    finally:
+        for n, f in saved.items():
+            setattr(pkg.ops, n, f)
+
+
+OFF = ", 16-bit GroupNorm kernels off"
+
+
 def _decoder(pkg, fused, linear, amp, train):
     torch.manual_seed(0)
     m = pkg.pixel_decoder.MSDeformAttnPixelDecoder(
@@ -346,15 +491,16 @@ def part_b(pkg, args, emit):
     arms = [("fp32 fused tf32x3", dict(fused=True, linear="tf32x3", amp=False), None),
             ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16),
             ("amp bf16 fused=False", dict(fused=False, linear="torch", amp=True), torch.bfloat16),
-            ("amp bf16 linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.bfloat16)]
+            ("amp bf16 linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.bfloat16),
+            ("amp bf16 linear=autocast" + OFF, dict(fused=True, linear="autocast", amp=True), torch.bfloat16)]
     models = {tag: _decoder(pkg, train=False, **kw) for tag, kw, _ in arms}
     res = {tag: [] for tag, _, _ in arms}
     for _ in range(args.repeats):
         for tag, _, dt in arms:
             ctx = torch.autocast("cuda", dtype=dt) if dt is not None else contextlib.nullcontext()
 
-            def fwd(m=models[tag], ctx=ctx):
-                with torch.no_grad(), ctx:
+            def fwd(m=models[tag], ctx=ctx, off=tag.endswith(OFF)):
+                with torch.no_grad(), ctx, gn16_off(pkg) if off else contextlib.nullcontext():
                     m.forward_features(feats)
             res[tag].append(timed(fwd, max(2, args.steps // 4), 2))
     for tag, _, _ in arms:
@@ -368,9 +514,12 @@ def part_c(pkg, args, emit):
             ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16),
             ("amp bf16 fused=False", dict(fused=False, linear="torch", amp=True), torch.bfloat16),
             ("amp bf16 linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.bfloat16),
+            ("amp bf16 linear=autocast" + OFF, dict(fused=True, linear="autocast", amp=True), torch.bfloat16),
             ("amp fp16 + GradScaler", dict(fused=True, linear="torch", amp=True), torch.float16),
             ("amp fp16 + GradScaler fused=False", dict(fused=False, linear="torch", amp=True), torch.float16),
-            ("amp fp16 + GradScaler linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.float16)]
+            ("amp fp16 + GradScaler linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.float16),
+            ("amp fp16 + GradScaler linear=autocast" + OFF, dict(fused=True, linear="autocast", amp=True),
+             torch.float16)]
     steps = {}
     for tag, kw, dt in arms:
         m = _decoder(pkg, train=True, **kw)
@@ -378,9 +527,9 @@ def part_c(pkg, args, emit):
         scaler = torch.amp.GradScaler("cuda") if dt == torch.float16 else None
         ctx = (lambda dt=dt: torch.autocast("cuda", dtype=dt)) if dt is not None else contextlib.nullcontext
 
-        def step(m=m, opt=opt, scaler=scaler, ctx=ctx):
+        def step(m=m, opt=opt, scaler=scaler, ctx=ctx, off=tag.endswith(OFF)):
             opt.zero_grad(set_to_none=True)
-            with ctx():
+            with ctx(), gn16_off(pkg) if off else contextlib.nullcontext():
                 mask, low, multi = m.forward_features(feats)
                 loss = sum(o.float().square().mean() for o in (mask, low, *multi))
             if scaler is None:
@@ -408,7 +557,7 @@ def part_c(pkg, args, emit):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--parts", default="a,b,c", help="a, b, c: profiles/r5_mixed.jsonl; f, b, c: r6_fused_mixed.jsonl; "
-                                                  "l, p, b, c: r7_autocast_encoder.jsonl")
+                                                  "l, p, b, c: r7_autocast_encoder.jsonl; g, b, c: r8_group_norm_mixed.jsonl")
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--dtypes", default="fp32,bf16,fp16", help="part (a): element types of value")
@@ -431,7 +580,7 @@ def main():
         with open(path, "a") as f:
             f.write(json.dumps(rec) + "\n")
     for part in args.parts.split(","):
-        {"a": part_a, "f": part_f, "b": part_b, "c": part_c, "l": part_l, "p": part_p}[part](pkg, args, emit)
+        {"a": part_a, "f": part_f, "b": part_b, "c": part_c, "l": part_l, "p": part_p, "g": part_g}[part](pkg, args, emit)
 
 
 if __name__ == "__main__":

@@ -81,6 +81,17 @@ SYMBOLS = {
     "msda_b200_group_norm_backward_workspace_bytes": (ctypes.c_longlong, [_I, _I]),
     "msda_b200_group_norm_rows_backward_f32": (_I, [_P, ctypes.c_longlong, ctypes.c_longlong] + [_P] * 9
                                                + [_I, _I, ctypes.c_longlong, _I, _I, _P, _P]),
+    **{f"msda_b200_{name}_{sfx}": sig for sfx in ("bf16", "f16") for name, sig in (
+        ("group_norm_nchw_mixed", (_I, [_P] * 6 + [_I] * 5 + [ctypes.c_float, _I, _P, _I, _I, _P, _P])),
+        ("group_norm_nchw_mixed_train", (_I, [_P] * 7 + [_I] * 5 + [ctypes.c_float, _I, _P, _I, _I, _P, _P])),
+        ("group_norm_nchw_to_rows_mixed", (_I, [_P] * 5 + [ctypes.c_longlong, ctypes.c_longlong, _I, _I,
+                                                           ctypes.c_longlong, _I, ctypes.c_float, _I, _P, _P])),
+        ("group_norm_nchw_to_rows_mixed_train", (_I, [_P] * 6 + [ctypes.c_longlong, ctypes.c_longlong, _I, _I,
+                                                                 ctypes.c_longlong, _I, ctypes.c_float, _I, _P, _P])),
+        ("group_norm_backward_nchw_mixed", (_I, [_P] * 12 + [_I] * 8 + [_P, _P])),
+        ("group_norm_rows_backward_mixed", (_I, [_P, ctypes.c_longlong, ctypes.c_longlong] + [_P] * 9
+                                            + [_I, _I, ctypes.c_longlong, _I, _I, _P, _P])),
+        ("add_channel_bias_nchw", (_I, [_P, _P, _I, _I, ctypes.c_longlong, _P])))},
     "msda_b200_set_option": (_I, [ctypes.c_char_p, _I]),
     "msda_b200_get_option": (_I, [ctypes.c_char_p, ctypes.POINTER(_I)]),
 }

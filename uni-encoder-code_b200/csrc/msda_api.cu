@@ -66,19 +66,25 @@ cudaError_t launch_linear_wgrad(const float *, const float *, float *, float *, 
                                 bool *handled, float *partials);
 long long linear_wgrad_partials(long long rows, int out_f, int in_f);
 cudaError_t launch_transpose(const float *, float *, long long, int, cudaStream_t);
-cudaError_t launch_group_norm(const float *, const float *, const float *, const float *, float *, int, int, int, int,
-                              int, float, int, const float *, int, int, double *, float *mean_rstd, cudaStream_t,
+// GroupNorm: V = type of the map x (and of y16 / grad_x), float or 16-bit; G = type of grad_y (float or V)
+template <typename V>
+cudaError_t launch_group_norm(const V *, const float *, const float *, const float *, float *, V *y16, int, int, int,
+                              int, int, float, int, const float *, int, int, double *, float *mean_rstd, cudaStream_t,
                               bool *handled);
-cudaError_t launch_channel_bias(float *, const float *, int, int, long long, cudaStream_t, bool *handled);
-cudaError_t launch_group_norm_rows(const float *, const float *, const float *, const float *, float *, int, int,
+template <typename V>
+cudaError_t launch_channel_bias(V *, const float *, int, int, long long, cudaStream_t, bool *handled);
+template <typename V>
+cudaError_t launch_group_norm_rows(const V *, const float *, const float *, const float *, float *, int, int,
                                    long long, int, float, int, long long, long long, double *, float *mean_rstd,
                                    cudaStream_t, bool *handled);
 int group_norm_workspace_doubles(int N, int groups);
-cudaError_t launch_group_norm_bwd(const float *, const float *, const float *, const float *, const float *,
-                                  const float *, float *, float *, float *, float *, float *, int, int, int, int, int,
-                                  int, int, int, double *, cudaStream_t, bool *handled);
-cudaError_t launch_group_norm_rows_bwd(const float *, long long, long long, const float *, const float *, const float *,
-                                       const float *, const float *, float *, float *, float *, float *, int, int,
+template <typename G, typename V>
+cudaError_t launch_group_norm_bwd(const G *, const V *, const float *, const float *, const float *, const float *,
+                                  V *, float *, float *, float *, float *, int, int, int, int, int, int, int, int,
+                                  double *, cudaStream_t, bool *handled);
+template <typename V>
+cudaError_t launch_group_norm_rows_bwd(const float *, long long, long long, const V *, const float *, const float *,
+                                       const float *, const float *, V *, float *, float *, float *, int, int,
                                        long long, int, int, double *, cudaStream_t, bool *handled);
 long long group_norm_bwd_workspace_doubles(int N, int C);
 cudaError_t launch_debug_indices(const int64_t *, const int64_t *, const float *, const Dims &,
@@ -352,19 +358,23 @@ static int linear_wgrad(const float *grad_y, const float *x, float *grad_weight,
     return launch_rc(e, handled);
 }
 
-static int group_norm_nchw(const float *x, const float *channel_bias, const float *gamma, const float *beta, float *y,
-                           float *mean_rstd, int batch, int channels, int height, int width, int groups, float eps,
-                           int relu, const float *up, int up_h, int up_w, void *workspace, void *stream, bool train) {
-    if (!x || !gamma || !beta || !y || (train && !mean_rstd) || !workspace) return MSDA_ERR_NULL_POINTER;
+// V = float: y required (the fp32 entries pass y16 = NULL); 16-bit V: y and / or y16
+template <typename V>
+static int group_norm_nchw(const V *x, const float *channel_bias, const float *gamma, const float *beta, float *y,
+                           V *y16, float *mean_rstd, int batch, int channels, int height, int width, int groups,
+                           float eps, int relu, const float *up, int up_h, int up_w, void *workspace, void *stream,
+                           bool train) {
+    if (!x || !gamma || !beta || (!y && !y16) || (train && !mean_rstd) || !workspace) return MSDA_ERR_NULL_POINTER;
     if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
-    const cudaError_t e = launch_group_norm(x, channel_bias, gamma, beta, y, batch, channels, height, width, groups,
-                                            eps, relu, up, up_h, up_w, static_cast<double *>(workspace), mean_rstd,
-                                            (cudaStream_t)stream, &handled);
+    const cudaError_t e = launch_group_norm<V>(x, channel_bias, gamma, beta, y, y16, batch, channels, height, width,
+                                               groups, eps, relu, up, up_h, up_w, static_cast<double *>(workspace),
+                                               mean_rstd, (cudaStream_t)stream, &handled);
     return launch_rc(e, handled);
 }
 
-static int group_norm_nchw_to_rows(const float *x, const float *channel_bias, const float *gamma, const float *beta,
+template <typename V>
+static int group_norm_nchw_to_rows(const V *x, const float *channel_bias, const float *gamma, const float *beta,
                                    float *y_rows, float *mean_rstd, long long row_stride, long long image_stride,
                                    int batch, int channels, long long plane, int groups, float eps, int relu,
                                    void *workspace, void *stream, bool train) {
@@ -372,10 +382,68 @@ static int group_norm_nchw_to_rows(const float *x, const float *channel_bias, co
     if (batch <= 0 || channels <= 0 || plane <= 0 || groups <= 0 || row_stride < channels || image_stride < 0)
         return MSDA_ERR_BAD_SHAPE;
     bool handled = false;
-    const cudaError_t e = launch_group_norm_rows(x, channel_bias, gamma, beta, y_rows, batch, channels, plane, groups,
-                                                 eps, relu, row_stride, image_stride,
-                                                 static_cast<double *>(workspace), mean_rstd, (cudaStream_t)stream,
-                                                 &handled);
+    const cudaError_t e = launch_group_norm_rows<V>(x, channel_bias, gamma, beta, y_rows, batch, channels, plane,
+                                                    groups, eps, relu, row_stride, image_stride,
+                                                    static_cast<double *>(workspace), mean_rstd, (cudaStream_t)stream,
+                                                    &handled);
+    return launch_rc(e, handled);
+}
+
+// The NCHW backward: fp32 (V = float, grad_y), or 16-bit x / grad_x with exactly one of grad_y (fp32) and grad_y16
+// (V), the gradient of whichever output the forward wrote
+template <typename V>
+static int group_norm_backward_nchw(const float *grad_y, const V *grad_y16, const V *x, const float *channel_bias,
+                                    const float *gamma, const float *beta, const float *mean_rstd, V *grad_x,
+                                    float *grad_gamma, float *grad_beta, float *grad_channel_bias, float *grad_up,
+                                    int batch, int channels, int height, int width, int groups, int relu, int up_h,
+                                    int up_w, void *workspace, void *stream) {
+    if ((!grad_y && !grad_y16) || !x || !gamma || !beta || !mean_rstd || !grad_x || !grad_gamma || !grad_beta ||
+        !workspace)
+        return MSDA_ERR_NULL_POINTER;
+    if (grad_y && grad_y16) return MSDA_ERR_UNSUPPORTED;
+    if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    cudaError_t e;
+    if (grad_y)
+        e = launch_group_norm_bwd<float, V>(grad_y, x, channel_bias, gamma, beta, mean_rstd, grad_x, grad_gamma,
+                                            grad_beta, grad_channel_bias, grad_up, batch, channels, height, width,
+                                            groups, relu, up_h, up_w, static_cast<double *>(workspace),
+                                            (cudaStream_t)stream, &handled);
+    else if constexpr (is16<V>)
+        e = launch_group_norm_bwd<V, V>(grad_y16, x, channel_bias, gamma, beta, mean_rstd, grad_x, grad_gamma,
+                                        grad_beta, grad_channel_bias, grad_up, batch, channels, height, width, groups,
+                                        relu, up_h, up_w, static_cast<double *>(workspace), (cudaStream_t)stream,
+                                        &handled);
+    else
+        return MSDA_ERR_NULL_POINTER;
+    return launch_rc(e, handled);
+}
+
+template <typename V>
+static int group_norm_rows_backward(const float *grad_y_rows, long long row_stride, long long image_stride,
+                                    const V *x, const float *channel_bias, const float *gamma, const float *beta,
+                                    const float *mean_rstd, V *grad_x, float *grad_gamma, float *grad_beta,
+                                    float *grad_channel_bias, int batch, int channels, long long plane, int groups,
+                                    int relu, void *workspace, void *stream) {
+    if (!grad_y_rows || !x || !gamma || !beta || !mean_rstd || !grad_x || !grad_gamma || !grad_beta || !workspace)
+        return MSDA_ERR_NULL_POINTER;
+    if (batch <= 0 || channels <= 0 || plane <= 0 || groups <= 0 || row_stride < channels || image_stride < 0)
+        return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_group_norm_rows_bwd<V>(grad_y_rows, row_stride, image_stride, x, channel_bias, gamma,
+                                                        beta, mean_rstd, grad_x, grad_gamma, grad_beta,
+                                                        grad_channel_bias, batch, channels, plane, groups, relu,
+                                                        static_cast<double *>(workspace), (cudaStream_t)stream,
+                                                        &handled);
+    return launch_rc(e, handled);
+}
+
+template <typename V>
+static int add_channel_bias_nchw(V *x, const float *bias, int batch, int channels, long long plane, void *stream) {
+    if (!x || !bias) return MSDA_ERR_NULL_POINTER;
+    if (batch <= 0 || channels <= 0 || plane <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_channel_bias<V>(x, bias, batch, channels, plane, (cudaStream_t)stream, &handled);
     return launch_rc(e, handled);
 }
 
@@ -675,6 +743,62 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
                                                reinterpret_cast<const V *>(residual), gamma, grad_x,                 \
                                                reinterpret_cast<V *>(grad_residual), grad_gamma, grad_beta, rows,    \
                                                cols, eps, workspace, stream, true);                                  \
+    }                                                                                                                \
+    int msda_b200_group_norm_nchw_mixed_##SUFFIX(                                                                    \
+        const uint16_t *x, const float *channel_bias, const float *gamma, const float *beta, float *y, uint16_t *y16,\
+        int batch, int channels, int height, int width, int groups, float eps, int relu, const float *up, int up_h,  \
+        int up_w, void *workspace, void *stream) {                                                                   \
+        return group_norm_nchw<V>(reinterpret_cast<const V *>(x), channel_bias, gamma, beta, y, reinterpret_cast<V *>(y16),\
+                                  nullptr, batch, channels, height, width, groups, eps, relu, up, up_h, up_w, workspace,\
+                                  stream, false);                                                                    \
+    }                                                                                                                \
+    int msda_b200_group_norm_nchw_mixed_train_##SUFFIX(                                                              \
+        const uint16_t *x, const float *channel_bias, const float *gamma, const float *beta, float *y, uint16_t *y16,\
+        float *mean_rstd, int batch, int channels, int height, int width, int groups, float eps, int relu,           \
+        const float *up, int up_h, int up_w, void *workspace, void *stream) {                                        \
+        return group_norm_nchw<V>(reinterpret_cast<const V *>(x), channel_bias, gamma, beta, y, reinterpret_cast<V *>(y16),\
+                                  mean_rstd, batch, channels, height, width, groups, eps, relu, up, up_h, up_w, workspace,\
+                                  stream, true);                                                                     \
+    }                                                                                                                \
+    int msda_b200_group_norm_nchw_to_rows_mixed_##SUFFIX(                                                            \
+        const uint16_t *x, const float *channel_bias, const float *gamma, const float *beta, float *y_rows,          \
+        long long row_stride, long long image_stride, int batch, int channels, long long plane, int groups, float eps,\
+        int relu, void *workspace, void *stream) {                                                                   \
+        return group_norm_nchw_to_rows<V>(reinterpret_cast<const V *>(x), channel_bias, gamma, beta, y_rows, nullptr,\
+                                          row_stride, image_stride, batch, channels, plane, groups, eps, relu, workspace,\
+                                          stream, false);                                                            \
+    }                                                                                                                \
+    int msda_b200_group_norm_nchw_to_rows_mixed_train_##SUFFIX(                                                      \
+        const uint16_t *x, const float *channel_bias, const float *gamma, const float *beta, float *y_rows,          \
+        float *mean_rstd, long long row_stride, long long image_stride, int batch, int channels, long long plane,    \
+        int groups, float eps, int relu, void *workspace, void *stream) {                                            \
+        return group_norm_nchw_to_rows<V>(reinterpret_cast<const V *>(x), channel_bias, gamma, beta, y_rows, mean_rstd,\
+                                          row_stride, image_stride, batch, channels, plane, groups, eps, relu, workspace,\
+                                          stream, true);                                                             \
+    }                                                                                                                \
+    int msda_b200_group_norm_backward_nchw_mixed_##SUFFIX(                                                           \
+        const float *grad_y, const uint16_t *grad_y16, const uint16_t *x, const float *channel_bias, const float *gamma,\
+        const float *beta, const float *mean_rstd, uint16_t *grad_x, float *grad_gamma, float *grad_beta,            \
+        float *grad_channel_bias, float *grad_up, int batch, int channels, int height, int width, int groups, int relu,\
+        int up_h, int up_w, void *workspace, void *stream) {                                                         \
+        return group_norm_backward_nchw<V>(grad_y, reinterpret_cast<const V *>(grad_y16), reinterpret_cast<const V *>(x),\
+                                           channel_bias, gamma, beta, mean_rstd, reinterpret_cast<V *>(grad_x),      \
+                                           grad_gamma, grad_beta, grad_channel_bias, grad_up, batch, channels, height,\
+                                           width, groups, relu, up_h, up_w, workspace, stream);                      \
+    }                                                                                                                \
+    int msda_b200_group_norm_rows_backward_mixed_##SUFFIX(                                                           \
+        const float *grad_y_rows, long long row_stride, long long image_stride, const uint16_t *x,                   \
+        const float *channel_bias, const float *gamma, const float *beta, const float *mean_rstd, uint16_t *grad_x,  \
+        float *grad_gamma, float *grad_beta, float *grad_channel_bias, int batch, int channels, long long plane,     \
+        int groups, int relu, void *workspace, void *stream) {                                                       \
+        return group_norm_rows_backward<V>(grad_y_rows, row_stride, image_stride, reinterpret_cast<const V *>(x),    \
+                                           channel_bias, gamma, beta, mean_rstd, reinterpret_cast<V *>(grad_x), grad_gamma,\
+                                           grad_beta, grad_channel_bias, batch, channels, plane, groups, relu, workspace,\
+                                           stream);                                                                  \
+    }                                                                                                                \
+    int msda_b200_add_channel_bias_nchw_##SUFFIX(uint16_t *x, const float *bias, int batch, int channels,            \
+                                                 long long plane, void *stream) {                                    \
+        return add_channel_bias_nchw<V>(reinterpret_cast<V *>(x), bias, batch, channels, plane, stream);             \
     }
 MSDA_MIXED_ENTRIES(bf16, __nv_bfloat16)
 MSDA_MIXED_ENTRIES(f16, __half)
@@ -759,24 +883,26 @@ long long msda_b200_linear_wgrad_deterministic_workspace_bytes(long long rows, i
 int msda_b200_group_norm_nchw_f32(const float *x, const float *channel_bias, const float *gamma, const float *beta,
                                   float *y, int batch, int channels, int height, int width, int groups, float eps,
                                   int relu, const float *up, int up_h, int up_w, void *workspace, void *stream) {
-    return group_norm_nchw(x, channel_bias, gamma, beta, y, nullptr, batch, channels, height, width, groups, eps, relu,
-                           up, up_h, up_w, workspace, stream, false);
+    if (!y) return MSDA_ERR_NULL_POINTER;
+    return group_norm_nchw<float>(x, channel_bias, gamma, beta, y, nullptr, nullptr, batch, channels, height, width,
+                                  groups, eps, relu, up, up_h, up_w, workspace, stream, false);
 }
 
 int msda_b200_group_norm_nchw_to_rows_f32(const float *x, const float *channel_bias, const float *gamma,
                                           const float *beta, float *y_rows, long long row_stride,
                                           long long image_stride, int batch, int channels, long long plane,
                                           int groups, float eps, int relu, void *workspace, void *stream) {
-    return group_norm_nchw_to_rows(x, channel_bias, gamma, beta, y_rows, nullptr, row_stride, image_stride, batch,
-                                   channels, plane, groups, eps, relu, workspace, stream, false);
+    return group_norm_nchw_to_rows<float>(x, channel_bias, gamma, beta, y_rows, nullptr, row_stride, image_stride,
+                                          batch, channels, plane, groups, eps, relu, workspace, stream, false);
 }
 
 int msda_b200_group_norm_nchw_train_f32(const float *x, const float *channel_bias, const float *gamma,
                                         const float *beta, float *y, float *mean_rstd, int batch, int channels,
                                         int height, int width, int groups, float eps, int relu, const float *up,
                                         int up_h, int up_w, void *workspace, void *stream) {
-    return group_norm_nchw(x, channel_bias, gamma, beta, y, mean_rstd, batch, channels, height, width, groups, eps,
-                           relu, up, up_h, up_w, workspace, stream, true);
+    if (!y) return MSDA_ERR_NULL_POINTER;
+    return group_norm_nchw<float>(x, channel_bias, gamma, beta, y, nullptr, mean_rstd, batch, channels, height, width,
+                                  groups, eps, relu, up, up_h, up_w, workspace, stream, true);
 }
 
 int msda_b200_group_norm_nchw_to_rows_train_f32(const float *x, const float *channel_bias, const float *gamma,
@@ -784,8 +910,8 @@ int msda_b200_group_norm_nchw_to_rows_train_f32(const float *x, const float *cha
                                                 long long row_stride, long long image_stride, int batch,
                                                 int channels, long long plane, int groups, float eps, int relu,
                                                 void *workspace, void *stream) {
-    return group_norm_nchw_to_rows(x, channel_bias, gamma, beta, y_rows, mean_rstd, row_stride, image_stride, batch,
-                                   channels, plane, groups, eps, relu, workspace, stream, true);
+    return group_norm_nchw_to_rows<float>(x, channel_bias, gamma, beta, y_rows, mean_rstd, row_stride, image_stride,
+                                          batch, channels, plane, groups, eps, relu, workspace, stream, true);
 }
 
 int msda_b200_group_norm_backward_nchw_f32(const float *grad_y, const float *x, const float *channel_bias,
@@ -794,15 +920,9 @@ int msda_b200_group_norm_backward_nchw_f32(const float *grad_y, const float *x, 
                                            float *grad_channel_bias, float *grad_up, int batch, int channels,
                                            int height, int width, int groups, int relu, int up_h, int up_w,
                                            void *workspace, void *stream) {
-    if (!grad_y || !x || !gamma || !beta || !mean_rstd || !grad_x || !grad_gamma || !grad_beta || !workspace)
-        return MSDA_ERR_NULL_POINTER;
-    if (batch <= 0 || channels <= 0 || height <= 0 || width <= 0 || groups <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    const cudaError_t e = launch_group_norm_bwd(grad_y, x, channel_bias, gamma, beta, mean_rstd, grad_x, grad_gamma,
-                                                grad_beta, grad_channel_bias, grad_up, batch, channels, height, width,
-                                                groups, relu, up_h, up_w, static_cast<double *>(workspace),
-                                                (cudaStream_t)stream, &handled);
-    return launch_rc(e, handled);
+    return group_norm_backward_nchw<float>(grad_y, nullptr, x, channel_bias, gamma, beta, mean_rstd, grad_x,
+                                           grad_gamma, grad_beta, grad_channel_bias, grad_up, batch, channels, height,
+                                           width, groups, relu, up_h, up_w, workspace, stream);
 }
 
 int msda_b200_group_norm_rows_backward_f32(const float *grad_y_rows, long long row_stride, long long image_stride,
@@ -811,25 +931,14 @@ int msda_b200_group_norm_rows_backward_f32(const float *grad_y_rows, long long r
                                            float *grad_gamma, float *grad_beta, float *grad_channel_bias, int batch,
                                            int channels, long long plane, int groups, int relu, void *workspace,
                                            void *stream) {
-    if (!grad_y_rows || !x || !gamma || !beta || !mean_rstd || !grad_x || !grad_gamma || !grad_beta || !workspace)
-        return MSDA_ERR_NULL_POINTER;
-    if (batch <= 0 || channels <= 0 || plane <= 0 || groups <= 0 || row_stride < channels || image_stride < 0)
-        return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    const cudaError_t e = launch_group_norm_rows_bwd(grad_y_rows, row_stride, image_stride, x, channel_bias, gamma,
-                                                     beta, mean_rstd, grad_x, grad_gamma, grad_beta, grad_channel_bias,
-                                                     batch, channels, plane, groups, relu,
-                                                     static_cast<double *>(workspace), (cudaStream_t)stream, &handled);
-    return launch_rc(e, handled);
+    return group_norm_rows_backward<float>(grad_y_rows, row_stride, image_stride, x, channel_bias, gamma, beta,
+                                           mean_rstd, grad_x, grad_gamma, grad_beta, grad_channel_bias, batch,
+                                           channels, plane, groups, relu, workspace, stream);
 }
 
 int msda_b200_add_channel_bias_nchw_f32(float *x, const float *bias, int batch, int channels, long long plane,
                                         void *stream) {
-    if (!x || !bias) return MSDA_ERR_NULL_POINTER;
-    if (batch <= 0 || channels <= 0 || plane <= 0) return MSDA_ERR_BAD_SHAPE;
-    bool handled = false;
-    const cudaError_t e = launch_channel_bias(x, bias, batch, channels, plane, (cudaStream_t)stream, &handled);
-    return launch_rc(e, handled);
+    return add_channel_bias_nchw<float>(x, bias, batch, channels, plane, stream);
 }
 
 long long msda_b200_group_norm_workspace_bytes(int batch, int groups) {

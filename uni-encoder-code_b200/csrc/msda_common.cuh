@@ -365,6 +365,19 @@ __device__ __forceinline__ void stg_stream_v1(V *p, float v) {
     }
 }
 
+// four consecutive results rounded to the 16-bit type H (round-to-nearest-even; fp16 overflow gives +-inf), one
+// 8-byte store
+template <typename H>
+__device__ __forceinline__ void st_round4(H *p, float4 o) {
+    const H a = narrow<H>(o.x), b = narrow<H>(o.y), c = narrow<H>(o.z), d = narrow<H>(o.w);
+    unsigned short ba, bb, bc, bd;
+    memcpy(&ba, &a, 2);
+    memcpy(&bb, &b, 2);
+    memcpy(&bc, &c, 2);
+    memcpy(&bd, &d, 2);
+    *reinterpret_cast<uint2 *>(p) = make_uint2((uint32_t)ba | ((uint32_t)bb << 16), (uint32_t)bc | ((uint32_t)bd << 16));
+}
+
 // ---------------------------------------------------------------------------
 // Element type of the fused producers' raw tensors (sampling offsets, attention logits and their
 // gradients): fp32, or -- in the mixed-precision fused op -- the value's 16-bit type, widened to fp32 on

@@ -218,11 +218,16 @@ class GroupNormFunction(Function):
     GroupNorm epilogues (msdeformattn.py:233-248, :369-379) -- with the fused kernels both ways: two launches forward
     (ops.group_norm_train, bit-identical to ops.group_norm), three backward, four with the gradient of ``up``
     (ops.group_norm_backward).  ``channel_bias`` and ``up`` may be None.  Saves x and the [N, groups, 2] statistics,
-    not the output; the ReLU mask is rebuilt from x with the forward's own arithmetic."""
+    not the output; the ReLU mask is rebuilt from x with the forward's own arithmetic.
+
+    A bf16 / fp16 ``x`` (torch.autocast) is saved as it is, not widened; the result is fp32 (``out_dtype`` None, what
+    autocast's ``F.group_norm`` returns) or its copy rounded to x's type (``out_dtype=x.dtype``), and grad_x has x's
+    type."""
 
     @staticmethod
-    def forward(ctx, x, weight, bias, channel_bias, up, groups, eps, relu):
-        y, mean_rstd = ops.group_norm_train(x, weight, bias, groups, eps, relu=relu, up=up, channel_bias=channel_bias)
+    def forward(ctx, x, weight, bias, channel_bias, up, groups, eps, relu, out_dtype=None):
+        y, mean_rstd = ops.group_norm_train(x, weight, bias, groups, eps, relu=relu, up=up, channel_bias=channel_bias,
+                                            out_dtype=out_dtype)
         ctx.save_for_backward(x, weight, bias, channel_bias, mean_rstd)
         ctx.groups, ctx.relu = groups, bool(relu)
         ctx.up_shape = tuple(up.shape[-2:]) if up is not None else None
@@ -236,7 +241,8 @@ class GroupNormFunction(Function):
         gx, gw, gb, gcb, gup = ops.group_norm_backward(
             _aligned(grad_y), x, weight, bias, mean_rstd, ctx.groups, relu=ctx.relu, channel_bias=channel_bias,
             up_shape=ctx.up_shape if need[4] else None, with_channel_bias=channel_bias is not None and need[3])
-        return (gx if need[0] else None, gw if need[1] else None, gb if need[2] else None, gcb, gup, None, None, None)
+        return (gx if need[0] else None, gw if need[1] else None, gb if need[2] else None, gcb, gup, None, None, None,
+                None)
 
 
 class GroupNormRowsFunction(Function):
@@ -246,14 +252,17 @@ class GroupNormRowsFunction(Function):
     autograd node: every level's GroupNorm writes its rows of the concatenated tensor (ops.group_norm_rows_train) and
     its backward reads them back from the concatenated gradient (ops.group_norm_rows_backward), so neither the
     transposing ``cat`` nor its backward runs.  ``channel_bias_i`` may be None.  Two launches per level forward,
-    three backward."""
+    three backward.  The levels may be bf16 / fp16 (torch.autocast), all of one type: the output stays fp32 and each
+    grad_x has its level's type."""
 
     @staticmethod
     def forward(ctx, groups, eps, *level_args):
         levels = [level_args[i:i + 4] for i in range(0, len(level_args), 4)]
         x0 = levels[0][0]
+        if any(x.dtype != x0.dtype for x, _, _, _ in levels):
+            raise RuntimeError("GroupNormRowsFunction: all levels must have one dtype")
         sizes = [x.size(2) * x.size(3) for x, _, _, _ in levels]
-        out = x0.new_empty((x0.size(0), sum(sizes), x0.size(1)))
+        out = x0.new_empty((x0.size(0), sum(sizes), x0.size(1)), dtype=torch.float32)
         saved, start = [], 0
         for (x, weight, bias, channel_bias), hw in zip(levels, sizes):
             mean_rstd = ops.group_norm_rows_train(x, weight, bias, groups, eps, out[:, start:start + hw],

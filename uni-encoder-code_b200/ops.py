@@ -738,13 +738,24 @@ def _vec_ok(t, x) -> bool:
             and t.shape == (x.size(1),))
 
 
+# the GroupNorm maps' element types and the alignment their 4-element accesses need: fp32, or the bf16 / fp16 map a
+# convolution writes under torch.autocast (the mixed-precision kernels, DESIGN.md 11.3)
+_MAP_ALIGN = {torch.float32: 16, torch.bfloat16: 8, torch.float16: 8}
+_GN_MIXED = {dtype: {name: getattr(_lib.lib, f"msda_b200_{name}_{sfx}")
+                     for name in ("group_norm_nchw_mixed", "group_norm_nchw_mixed_train", "group_norm_nchw_to_rows_mixed",
+                                  "group_norm_nchw_to_rows_mixed_train", "group_norm_backward_nchw_mixed",
+                                  "group_norm_rows_backward_mixed", "add_channel_bias_nchw")}
+             for dtype, sfx in ((torch.bfloat16, "bf16"), (torch.float16, "f16"))}
+
+
 def _map_ok(x, weight, bias, groups, up=None) -> bool:
-    """What every GroupNorm kernel needs of an NCHW map: x contiguous fp32 on a CUDA device, 16-byte aligned, with H*W
-    a multiple of 4 (the planes are walked as float4); weight and bias contiguous fp32 [C] on x's device; C divisible
-    by groups; with `up` (the map the forward up-samples and adds): W a multiple of 4 as well, and `up` a contiguous
-    fp32 map with x's batch and channels on x's device."""
-    return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and x.dim() == 4
-            and x.is_contiguous() and x.numel() > 0 and (x.size(2) * x.size(3)) % 4 == 0 and x.data_ptr() % 16 == 0
+    """What every GroupNorm kernel needs of an NCHW map: x contiguous fp32 (16-byte aligned) or bf16 / fp16 (8-byte
+    aligned) on a CUDA device, with H*W a multiple of 4 (the planes are walked 4 elements at a time); weight and bias
+    contiguous fp32 [C] on x's device; C divisible by groups; with `up` (the map the forward up-samples and adds): W a
+    multiple of 4 as well, and `up` a contiguous fp32 map with x's batch and channels on x's device."""
+    return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype in _MAP_ALIGN and x.dim() == 4
+            and x.is_contiguous() and x.numel() > 0 and (x.size(2) * x.size(3)) % 4 == 0
+            and x.data_ptr() % _MAP_ALIGN[x.dtype] == 0
             and isinstance(groups, int) and groups > 0 and x.size(1) % groups == 0 and _vec_ok(weight, x)
             and _vec_ok(bias, x)
             and (up is None or (isinstance(up, torch.Tensor) and up.dtype == torch.float32 and up.dim() == 4
@@ -782,8 +793,8 @@ def _workspace(nbytes, x):
 
 
 def group_norm_supported(x, norm, up=None) -> bool:
-    """Whether the fused GroupNorm kernels cover `norm(x)` (x: NCHW fp32 CUDA, contiguous; `norm` an affine
-    nn.GroupNorm whose parameters are contiguous fp32 [C] tensors on x's device)."""
+    """Whether the fused GroupNorm kernels cover `norm(x)` (x: NCHW fp32, bf16 or fp16 CUDA, contiguous; `norm` an
+    affine nn.GroupNorm whose parameters are contiguous fp32 [C] tensors on x's device)."""
     return isinstance(norm, torch.nn.GroupNorm) and _map_ok(x, norm.weight, norm.bias, norm.num_groups, up)
 
 
@@ -793,23 +804,39 @@ def group_norm_rows_supported(x, norm, out_rows) -> bool:
     return group_norm_supported(x, norm) and _rows_view_ok(out_rows, x)
 
 
-def _group_norm_nchw(name, x, weight, bias, groups, eps, relu, up, channel_bias, stats):
-    """The NCHW forward -> (y, mean_rstd [N, groups, 2] when `stats`, else None)."""
+def _out_dtype(x, out_dtype):
+    """The output type of a GroupNorm of `x`: fp32 (None: what F.group_norm returns under torch.autocast), or -- for a
+    16-bit x -- x's own type, the rounded copy the next convolution reads."""
+    if out_dtype is None or out_dtype == torch.float32 or out_dtype == x.dtype:
+        return torch.float32 if out_dtype is None else out_dtype
+    raise RuntimeError(f"out_dtype must be None, torch.float32 or the map's dtype {x.dtype}, not {out_dtype}")
+
+
+def _group_norm_nchw(name, x, weight, bias, groups, eps, relu, up, channel_bias, stats, out_dtype=None):
+    """The NCHW forward -> (y, mean_rstd [N, groups, 2] when `stats`, else None); y of type `out_dtype` (None: fp32)."""
     if not _map_ok(x, weight, bias, groups, up):
         raise RuntimeError(f"{name} needs a contiguous NCHW fp32 CUDA map with H*W (and, with `up`, W) a multiple of 4, "
                            "contiguous fp32 [C] weight and bias on the same device, C divisible by groups and, if "
                            "given, a contiguous `up` map with the same batch and channels")
     _check_channel_bias(channel_bias, x)
+    out_dtype = _out_dtype(x, out_dtype)
     N, C, H, W = x.shape
-    y = torch.empty_like(x)
+    y = torch.empty_like(x, dtype=out_dtype)
     mean_rstd = torch.empty(N, groups, 2, dtype=torch.float32, device=x.device) if stats else None
     with torch.cuda.device(x.device):
         ws = _workspace(_lib.lib.msda_b200_group_norm_workspace_bytes(N, groups), x)
-        head = (x.data_ptr(), _ptr(channel_bias), weight.data_ptr(), bias.data_ptr(), y.data_ptr())
         tail = (N, C, H, W, groups, float(eps), int(bool(relu)), _ptr(up), up.size(2) if up is not None else 0,
                 up.size(3) if up is not None else 0, ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)
-        rc = (_lib.lib.msda_b200_group_norm_nchw_train_f32(*head, mean_rstd.data_ptr(), *tail) if stats
-              else _lib.lib.msda_b200_group_norm_nchw_f32(*head, *tail))
+        if x.dtype == torch.float32:
+            head = (x.data_ptr(), _ptr(channel_bias), weight.data_ptr(), bias.data_ptr(), y.data_ptr())
+            rc = (_lib.lib.msda_b200_group_norm_nchw_train_f32(*head, mean_rstd.data_ptr(), *tail) if stats
+                  else _lib.lib.msda_b200_group_norm_nchw_f32(*head, *tail))
+        else:                      # a 16-bit map: the fp32 y or its 16-bit copy y16
+            y32, y16 = (y, None) if out_dtype == torch.float32 else (None, y)
+            head = (x.data_ptr(), _ptr(channel_bias), weight.data_ptr(), bias.data_ptr(), _ptr(y32), _ptr(y16))
+            entries = _GN_MIXED[x.dtype]
+            rc = (entries["group_norm_nchw_mixed_train"](*head, mean_rstd.data_ptr(), *tail) if stats
+                  else entries["group_norm_nchw_mixed"](*head, *tail))
     _lib.check(rc, name)
     return y, mean_rstd
 
@@ -827,28 +854,39 @@ def _group_norm_rows(name, x, weight, bias, groups, eps, out_rows, channel_bias,
         head = (x.data_ptr(), _ptr(channel_bias), weight.data_ptr(), bias.data_ptr(), out_rows.data_ptr())
         tail = (out_rows.stride(1), out_rows.stride(0), N, C, H * W, groups, float(eps), int(bool(relu)), ws.data_ptr(),
                 torch.cuda.current_stream(x.device).cuda_stream)
-        rc = (_lib.lib.msda_b200_group_norm_nchw_to_rows_train_f32(*head, mean_rstd.data_ptr(), *tail) if stats
-              else _lib.lib.msda_b200_group_norm_nchw_to_rows_f32(*head, *tail))
+        if x.dtype == torch.float32:
+            rc = (_lib.lib.msda_b200_group_norm_nchw_to_rows_train_f32(*head, mean_rstd.data_ptr(), *tail) if stats
+                  else _lib.lib.msda_b200_group_norm_nchw_to_rows_f32(*head, *tail))
+        else:                      # a 16-bit map, fp32 rows
+            entries = _GN_MIXED[x.dtype]
+            rc = (entries["group_norm_nchw_to_rows_mixed_train"](*head, mean_rstd.data_ptr(), *tail) if stats
+                  else entries["group_norm_nchw_to_rows_mixed"](*head, *tail))
     _lib.check(rc, name)
     return mean_rstd
 
 
-def group_norm(x, norm, relu=False, up=None, channel_bias=None):
+def group_norm(x, norm, relu=False, up=None, channel_bias=None, out_dtype=None):
     """``norm(x)`` (``norm(x + channel_bias[None, :, None, None])`` when the producing convolution ran without
     its bias) for an ``nn.GroupNorm`` on an NCHW fp32 CUDA map, optionally followed by ReLU and by
     ``+ F.interpolate(up, size=x.shape[-2:], mode="bilinear", align_corners=False)`` -- the epilogues of the
     pixel decoder's input projections and FPN level (msdeformattn.py:233-248, :369-379) -- in two passes
     over x (statistics, apply) instead of torch's four to six kernels.  No autograd: training goes through
-    functions.GroupNormFunction (group_norm_train / group_norm_backward)."""
+    functions.GroupNormFunction (group_norm_train / group_norm_backward).
+
+    A bf16 / fp16 ``x`` (a convolution's output under torch.autocast) is widened on load; ``up``, the affine
+    parameters and ``channel_bias`` stay fp32.  The result is fp32 (``out_dtype`` None: what torch.autocast's
+    ``F.group_norm(x.float(), ...)`` composition returns), bit-identical to the fp32 kernels on ``x.float()``; with
+    ``out_dtype=x.dtype`` it is that result rounded to x's type, the copy the next convolution reads."""
     return _group_norm_nchw("group_norm", x, norm.weight, norm.bias, norm.num_groups, norm.eps, relu, up, channel_bias,
-                            False)[0]
+                            False, out_dtype)[0]
 
 
 def group_norm_rows(x, norm, out_rows, channel_bias=None, relu=False):
     """``out_rows[n, p, c] = norm(x + channel_bias)[n, c, p]`` (p = flattened pixel): GroupNorm of an NCHW map written
     straight into the ``[N, pixels, C]`` layout of the deformable encoder (``src.flatten(2).transpose(1, 2)``),
     e.g. into the level's rows of the concatenated tensor.  No autograd: training goes through
-    functions.GroupNormRowsFunction (group_norm_rows_train / group_norm_rows_backward).  Returns out_rows."""
+    functions.GroupNormRowsFunction (group_norm_rows_train / group_norm_rows_backward).  Returns out_rows.  x may be
+    bf16 / fp16 (widened on load); out_rows is fp32."""
     _group_norm_rows("group_norm_rows", x, norm.weight, norm.bias, norm.num_groups, norm.eps, out_rows, channel_bias,
                      relu, False)
     return out_rows
@@ -861,13 +899,15 @@ def channel_bias_supported(x, bias) -> bool:
 
 def add_channel_bias_(x, bias):
     """``x += bias[None, :, None, None]`` in place on a contiguous NCHW fp32 CUDA map (the bias of a convolution
-    that ran without one: torch's own broadcast add runs at less than half of the memory roofline)."""
+    that ran without one: torch's own broadcast add runs at less than half of the memory roofline).  A bf16 / fp16
+    map with the fp32 bias: ``x.copy_((x.float() + bias).to(x.dtype))``, one rounding per element."""
     if not channel_bias_supported(x, bias):
         raise RuntimeError("add_channel_bias_ needs a contiguous NCHW fp32 CUDA map with H*W % 4 == 0 and a [C] bias")
+    entry = (_lib.lib.msda_b200_add_channel_bias_nchw_f32 if x.dtype == torch.float32
+             else _GN_MIXED[x.dtype]["add_channel_bias_nchw"])
     with torch.cuda.device(x.device):
-        rc = _lib.lib.msda_b200_add_channel_bias_nchw_f32(x.data_ptr(), bias.data_ptr(), x.size(0), x.size(1),
-                                                          x.size(2) * x.size(3),
-                                                          torch.cuda.current_stream(x.device).cuda_stream)
+        rc = entry(x.data_ptr(), bias.data_ptr(), x.size(0), x.size(1), x.size(2) * x.size(3),
+                   torch.cuda.current_stream(x.device).cuda_stream)
     _lib.check(rc, "add_channel_bias_")
     return x
 
@@ -943,11 +983,11 @@ def add_layernorm_backward(grad_y, x, residual, weight, eps=1e-5):
 
 
 # ---------------------------------------------------------------- GroupNorm training (forward + backward)
-def group_norm_train(x, weight, bias, groups, eps, relu=False, up=None, channel_bias=None):
+def group_norm_train(x, weight, bias, groups, eps, relu=False, up=None, channel_bias=None, out_dtype=None):
     """Training forward of ``group_norm``: ``(y, mean_rstd)`` with ``y`` bit-identical to ``group_norm`` on the same
     inputs and ``mean_rstd`` [N, groups, 2] the (mean, rstd) of ``x + channel_bias`` that the backward needs.  The
     affine parameters are passed as tensors (weight, bias [C]) so that autograd can follow them."""
-    return _group_norm_nchw("group_norm_train", x, weight, bias, groups, eps, relu, up, channel_bias, True)
+    return _group_norm_nchw("group_norm_train", x, weight, bias, groups, eps, relu, up, channel_bias, True, out_dtype)
 
 
 def group_norm_rows_train(x, weight, bias, groups, eps, out_rows, channel_bias=None, relu=False):
@@ -961,9 +1001,13 @@ def group_norm_backward(grad_y, x, weight, bias, mean_rstd, groups, relu=False, 
     """Gradients of ``group_norm_train``: ``(grad_x, grad_weight, grad_bias, grad_channel_bias, grad_up)`` from
     ``grad_y`` and the forward's inputs and ``mean_rstd``.  ``grad_channel_bias`` is computed when
     ``with_channel_bias`` (else None); ``grad_up`` [N, C, *up_shape] when ``up_shape`` (the up-sampled map's (h, w))
-    is given (else None).  Three launches, four with ``grad_up``; deterministic."""
-    # grad_y: a map like x; with up_shape, the forward's `up` requirement on W
+    is given (else None).  Three launches, four with ``grad_up``; deterministic.  For a bf16 / fp16 ``x``, ``grad_y``
+    is fp32 or of x's type (the gradient of whichever output the forward returned) and ``grad_x`` is of x's type: the
+    fp32 kernels' grad_x on the widened inputs rounded once; the other gradients are fp32 and bit-identical to
+    theirs."""
+    # grad_y: a map like x (16-bit x: or an fp32 one); with up_shape, the forward's `up` requirement on W
     if not (_map_ok(x, weight, bias, groups) and _map_ok(grad_y, weight, bias, groups) and grad_y.shape == x.shape
+            and (grad_y.dtype == x.dtype or grad_y.dtype == torch.float32)
             and (up_shape is None or x.size(3) % 4 == 0)):
         raise RuntimeError("group_norm_backward needs contiguous NCHW fp32 CUDA grad_y and x of the same shape with H*W "
                            "(and, with up_shape, W) a multiple of 4, and contiguous fp32 [C] weight and bias")
@@ -973,11 +1017,17 @@ def group_norm_backward(grad_y, x, weight, bias, mean_rstd, groups, relu=False, 
     gx = torch.empty_like(x)
     gw, gb = torch.empty_like(weight), torch.empty_like(bias)
     gcb = torch.empty_like(bias) if with_channel_bias else None
-    gup = torch.empty(N, C, int(up_shape[0]), int(up_shape[1]), dtype=x.dtype, device=x.device) if up_shape else None
+    gup = (torch.empty(N, C, int(up_shape[0]), int(up_shape[1]), dtype=torch.float32, device=x.device) if up_shape
+           else None)
     with torch.cuda.device(x.device):
         ws = _workspace(_lib.lib.msda_b200_group_norm_backward_workspace_bytes(N, C), x)
-        rc = _lib.lib.msda_b200_group_norm_backward_nchw_f32(
-            grad_y.data_ptr(), x.data_ptr(), _ptr(channel_bias), weight.data_ptr(), bias.data_ptr(),
+        if x.dtype == torch.float32:
+            entry, grads = _lib.lib.msda_b200_group_norm_backward_nchw_f32, (grad_y.data_ptr(),)
+        else:                      # exactly one of grad_y (fp32) and grad_y16
+            entry = _GN_MIXED[x.dtype]["group_norm_backward_nchw_mixed"]
+            grads = (grad_y.data_ptr(), None) if grad_y.dtype == torch.float32 else (None, grad_y.data_ptr())
+        rc = entry(
+            *grads, x.data_ptr(), _ptr(channel_bias), weight.data_ptr(), bias.data_ptr(),
             mean_rstd.data_ptr(), gx.data_ptr(), gw.data_ptr(), gb.data_ptr(), _ptr(gcb), _ptr(gup), N, C, H, W,
             groups, int(bool(relu)), gup.size(2) if gup is not None else 0, gup.size(3) if gup is not None else 0,
             ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)
@@ -988,8 +1038,8 @@ def group_norm_backward(grad_y, x, weight, bias, mean_rstd, groups, relu=False, 
 def group_norm_rows_backward(grad_rows, x, weight, bias, mean_rstd, groups, relu=False, channel_bias=None,
                              with_channel_bias=False):
     """Gradients of ``group_norm_rows_train``: ``(grad_x, grad_weight, grad_bias, grad_channel_bias)`` with ``grad_rows``
-    an fp32 [N, H*W, C] view in the rows layout (e.g. the level's slice of the concatenated gradient) and grad_x NCHW.
-    Three launches; deterministic."""
+    an fp32 [N, H*W, C] view in the rows layout (e.g. the level's slice of the concatenated gradient) and grad_x NCHW
+    of x's type (bf16 / fp16 x: the fp32 kernels' grad_x rounded once).  Three launches; deterministic."""
     if not (_map_ok(x, weight, bias, groups) and _rows_view_ok(grad_rows, x)):
         raise RuntimeError("group_norm_rows_backward needs what group_norm_backward needs, channels % 32 == 0 and an "
                            "fp32 [N, H*W, C] grad_rows view with unit channel stride on the same device")
@@ -1001,7 +1051,9 @@ def group_norm_rows_backward(grad_rows, x, weight, bias, mean_rstd, groups, relu
     gcb = torch.empty_like(bias) if with_channel_bias else None
     with torch.cuda.device(x.device):
         ws = _workspace(_lib.lib.msda_b200_group_norm_backward_workspace_bytes(N, C), x)
-        rc = _lib.lib.msda_b200_group_norm_rows_backward_f32(
+        entry = (_lib.lib.msda_b200_group_norm_rows_backward_f32 if x.dtype == torch.float32
+                 else _GN_MIXED[x.dtype]["group_norm_rows_backward_mixed"])
+        rc = entry(
             grad_rows.data_ptr(), grad_rows.stride(1), grad_rows.stride(0), x.data_ptr(), _ptr(channel_bias),
             weight.data_ptr(), bias.data_ptr(), mean_rstd.data_ptr(), gx.data_ptr(), gw.data_ptr(), gb.data_ptr(),
             _ptr(gcb), N, C, H * W, groups, int(bool(relu)), ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)

@@ -26,7 +26,7 @@ from torch import nn
 
 from . import ops
 from .functions import GroupNormFunction, GroupNormRowsFunction
-from .modules import CoreFn, MSDeformAttnTransformerEncoderOnly, ShapeCache, _capturing, _resolve
+from .modules import CoreFn, MSDeformAttnTransformerEncoderOnly, ShapeCache, _autocast_dtype, _capturing, _resolve
 
 
 class PositionEmbeddingSine(nn.Module):
@@ -74,13 +74,15 @@ class _ConvNormAct(nn.Conv2d):
         super().__init__(*args, **kwargs)
         self.norm, self.activation = norm, activation
 
-    def forward(self, x, up=None, fused_norm=False):
+    def forward(self, x, up=None, fused_norm=False, out_dtype=None):
         """conv -> norm -> activation (-> + bilinear up-sampling of `up`, the FPN top-down add of
         msdeformattn.py:372-376).  `fused_norm` (GroupNorm): the norm, the ReLU and the up-sampled add through
-        `_group_norm`."""
+        `_group_norm`; `out_dtype` (under torch.autocast, the convolution's 16-bit type): the result rounded to it, the
+        copy the next convolution reads."""
         x = super().forward(x)
         if fused_norm and isinstance(self.norm, nn.GroupNorm) and self.activation in (None, F.relu):
-            return _group_norm(self.norm, x, relu=self.activation is F.relu, up=up)
+            return _group_norm(self.norm, x, relu=self.activation is F.relu, up=up,
+                               out_dtype=out_dtype if x.dtype == out_dtype else None)
         if self.norm is not None:
             x = self.norm(x)
         x = x if self.activation is None else self.activation(x)
@@ -89,15 +91,17 @@ class _ConvNormAct(nn.Conv2d):
         return x
 
 
-def _group_norm(norm: nn.GroupNorm, x, relu=False, up=None, channel_bias=None):
+def _group_norm(norm: nn.GroupNorm, x, relu=False, up=None, channel_bias=None, out_dtype=None):
     """``norm(x + channel_bias[None, :, None, None])`` [-> ReLU] [+ bilinear up-sampling of `up`] (`channel_bias`: the
     bias of the convolution that produced x and ran without it).  Where ops.group_norm_supported holds, one statistics
     + one apply kernel (SURVEY 8f.4): ops.group_norm with autograd off, GroupNormFunction, whose backward also runs on
-    the library's kernels, with it on; torch otherwise."""
+    the library's kernels, with it on; torch otherwise.  A 16-bit x (torch.autocast) gives an fp32 result, or with
+    `out_dtype=x.dtype` and the kernels its 16-bit copy."""
     if ops.group_norm_supported(x, norm, up):
         if not torch.is_grad_enabled():
-            return ops.group_norm(x, norm, relu=relu, up=up, channel_bias=channel_bias)
-        return GroupNormFunction.apply(x, norm.weight, norm.bias, channel_bias, up, norm.num_groups, norm.eps, relu)
+            return ops.group_norm(x, norm, relu=relu, up=up, channel_bias=channel_bias, out_dtype=out_dtype)
+        return GroupNormFunction.apply(x, norm.weight, norm.bias, channel_bias, up, norm.num_groups, norm.eps, relu,
+                                       out_dtype)
     x = norm(x if channel_bias is None else x + channel_bias.view(1, -1, 1, 1))
     x = F.relu(x) if relu else x
     if up is not None:
@@ -131,9 +135,13 @@ class MSDeformAttnPixelDecoder(nn.Module):
         functions.MSDeformAttnFusedFunction, which take the softmax and the location arithmetic off torch).
         `amp=False` is the reference's behaviour: autocast off, fp32.
         `linear="autocast"` (not in the reference): `linear="tf32x3"` where no bf16 / fp16 autocast is active (with
-        `amp=False` always); under one, torch's autocast GEMMs, convolutions and GroupNorms as with `linear="torch"`,
-        except the encoder's residual + LayerNorm steps and the batch-shared position embedding's query projection,
-        which run on the mixed-precision kernels (modules._add_norm_mixed, MSDeformAttn.forward_shared_pos)."""
+        `amp=False` always); under one, torch's autocast GEMMs and convolutions as with `linear="torch"`, with the
+        encoder's residual + LayerNorm steps and the batch-shared position embedding's query projection on the
+        mixed-precision kernels (modules._add_norm_mixed, MSDeformAttn.forward_shared_pos), and the five GroupNorms
+        on the 16-bit GroupNorm kernels, as `linear="tf32x3"` routes them: the input projections' convolutions run
+        without their bias and the rows kernels write the fp32 encoder input, adding it in fp32; the FPN lateral and
+        output GroupNorms (with the up-sampled fp32 encoder level, the ReLU) return the 16-bit copy the next
+        convolution reads; in inference `mask_features` adds its bias to its 16-bit output in one pass."""
         if amp and linear == "tf32x3":
             raise ValueError('amp=True cannot be combined with linear="tf32x3": the 3xTF32 GEMMs and the fp32 '
                              'GroupNorm / LayerNorm kernels are fp32 paths that autocast would bypass')
@@ -185,8 +193,10 @@ class MSDeformAttnPixelDecoder(nn.Module):
         autocast, if any)."""
         device_type = next(iter(features.values())).device.type
         with contextlib.nullcontext() if self.amp else torch.autocast(device_type=device_type, enabled=False):
-            # the inference kernels of SURVEY 8f.3 / 8f.4 (linear="autocast": when no 16-bit autocast is active)
-            fused_norm = _resolve(self.linear) == "tf32x3"
+            # the inference kernels of SURVEY 8f.3 / 8f.4 (linear="autocast": when no 16-bit autocast is active), and
+            # the GroupNorm kernels on the 16-bit maps of the convolutions under one (DESIGN.md 11.3)
+            fused_norm = _resolve(self.linear) in ("tf32x3", "autocast")
+            out16 = _autocast_dtype() if _resolve(self.linear) == "autocast" else None
             names = self.transformer_in_features[::-1]
             levels = [(int(features[k].shape[2]), int(features[k].shape[3])) for k in names]
             srcs, src_flat = self._input_proj([features[k].float() for k in names], levels, fused_norm)
@@ -197,8 +207,8 @@ class MSDeformAttnPixelDecoder(nn.Module):
                                        zip(memory.split([h * w for h, w in levels], dim=1), levels)]
             for idx, name in enumerate(self.in_features[:self.num_fpn_levels][::-1]):
                 y = self.lateral_convs[idx](features[name].float(), up=self._nchw(out[-1], memory, fused_norm),
-                                            fused_norm=fused_norm)
-                out.append(self.output_convs[idx](y, fused_norm=fused_norm))
+                                            fused_norm=fused_norm, out_dtype=out16)
+                out.append(self.output_convs[idx](y, fused_norm=fused_norm, out_dtype=out16))
             return self._mask_features(out[-1], fused_norm), out[0], out[:self.oneformer_num_feature_levels]
 
     def _input_proj(self, xs, levels, fused_norm):
@@ -207,7 +217,8 @@ class MSDeformAttnPixelDecoder(nn.Module):
         convolutions run without their bias (torch adds it in a separate pass over the map) and the GroupNorms add it
         on the fly.  When ops.group_norm_rows_supported holds for every level, each level's GroupNorm writes its rows
         of src_flat (no transposing `cat`): ops.group_norm_rows with autograd off, ONE GroupNormRowsFunction node for
-        all levels with it on.  Otherwise every level goes through `_group_norm`."""
+        all levels with it on.  Otherwise every level goes through `_group_norm`.  Under torch.autocast the
+        convolutions write 16-bit maps and src_flat stays fp32."""
         if not fused_norm:
             return [proj[1](proj[0](x)) for proj, x in zip(self.input_proj, xs)], None
         convs, norms = [proj[0] for proj in self.input_proj], [proj[1] for proj in self.input_proj]
@@ -215,7 +226,7 @@ class MSDeformAttnPixelDecoder(nn.Module):
         starts = [0]
         for h, w in levels:
             starts.append(starts[-1] + h * w)
-        src_flat = ys[0].new_empty((ys[0].shape[0], starts[-1], ys[0].shape[1]))
+        src_flat = ys[0].new_empty((ys[0].shape[0], starts[-1], ys[0].shape[1]), dtype=torch.float32)
         rows = [src_flat[:, a:b] for a, b in zip(starts, starts[1:])]
         if not (all(ops.group_norm_rows_supported(y, n, r) for y, n, r in zip(ys, norms, rows))
                 and len({(n.num_groups, n.eps) for n in norms}) == 1):
@@ -252,5 +263,5 @@ class MSDeformAttnPixelDecoder(nn.Module):
             y = F.conv2d(x, conv.weight, None, conv.stride, conv.padding, conv.dilation, conv.groups)
             if ops.channel_bias_supported(y, conv.bias):
                 return ops.add_channel_bias_(y, conv.bias)
-            return y + conv.bias.view(1, -1, 1, 1)
+            return (y + conv.bias.view(1, -1, 1, 1)).to(y.dtype)
         return conv(x)
