@@ -613,6 +613,32 @@ int msda_b200_linear_wgrad_deterministic_f32(const float *grad_y, const float *x
                                              void *workspace, void *stream);
 long long msda_b200_linear_wgrad_deterministic_workspace_bytes(long long rows, int out_features, int in_features);
 
+/*
+ * The same Linear under torch.autocast, on bf16 (_bf16) or fp16 (_f16) operands passed as uint16_t bit patterns:
+ *     y[rows, out_features] = round16(x[rows, in_features] * weight16[out_features, in_features]^T + bias)
+ * (then ReLU if relu != 0).  bias is fp32 (may be NULL) and is added to the fp32 accumulator; the result is rounded
+ * once to nearest-even (fp16 overflow gives +-inf).  The input gradient is the same call with grad_y as x and the
+ * transposed weight [in_features, out_features].  in_features % 8 == 0, out_features % 8 == 0 and 16-byte aligned
+ * x, weight16 and y; MSDA_ERR_UNSUPPORTED otherwise.  One launch.
+ */
+int msda_b200_linear_mixed_bf16(const uint16_t *x, const uint16_t *weight16, const float *bias, uint16_t *y, int rows,
+                                int out_features, int in_features, int relu, void *stream);
+int msda_b200_linear_mixed_f16(const uint16_t *x, const uint16_t *weight16, const float *bias, uint16_t *y, int rows,
+                               int out_features, int in_features, int relu, void *stream);
+/* Weight and bias gradient of that Linear, in fp32 from 16-bit operands:
+ *     grad_weight[out_features, in_features] = grad_y[rows, out_features]^T * x[rows, in_features]
+ *     grad_bias[out_features] = column sums of grad_y                      (grad_bias may be NULL)
+ * Deterministic by construction: each work item (a chunk of rows of one output tile) stores its partial tile and
+ * bias sums in `workspace` (msda_b200_linear_mixed_wgrad_workspace_bytes(rows, out_features, in_features) bytes) and a
+ * second launch adds the chunks in chunk order; the chunking depends on the shapes only.  out_features % 8 == 0,
+ * in_features % 8 == 0, 16-byte aligned grad_y, x, grad_weight and workspace; MSDA_ERR_UNSUPPORTED otherwise. */
+int msda_b200_linear_mixed_wgrad_bf16(const uint16_t *grad_y, const uint16_t *x, float *grad_weight, float *grad_bias,
+                                      long long rows, int out_features, int in_features, void *workspace,
+                                      void *stream);
+int msda_b200_linear_mixed_wgrad_f16(const uint16_t *grad_y, const uint16_t *x, float *grad_weight, float *grad_bias,
+                                     long long rows, int out_features, int in_features, void *workspace, void *stream);
+long long msda_b200_linear_mixed_wgrad_workspace_bytes(long long rows, int out_features, int in_features);
+
 /* y[cols, rows] = x[rows, cols]^T, fp32 (operand preparation for weight-gradient GEMMs). */
 int msda_b200_transpose_f32(const float *x, float *y, long long rows, int cols, void *stream);
 

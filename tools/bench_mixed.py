@@ -470,6 +470,27 @@ def gn16_off(pkg):
 
 
 OFF = ", 16-bit GroupNorm kernels off"
+LIN_OFF = ", 16-bit Linear kernels off"
+
+
+@contextlib.contextmanager
+def linear16_off(pkg):
+    """The 16-bit Linear kernels off: their predicates refuse every shape, so linear="autocast" runs torch's autocast
+    GEMMs (and the FFN's separate ReLU) as before those kernels."""
+    fn, op = pkg.functions.LinearMixedFunction, pkg.ops.linear_mixed_supported
+    saved = fn.__dict__["supported"]
+    fn.supported = staticmethod(lambda *a, **k: False)
+    pkg.ops.linear_mixed_supported = lambda *a, **k: False
+    try:
+        yield
+    finally:
+        fn.supported = saved
+        pkg.ops.linear_mixed_supported = op
+
+
+def _switch(pkg, tag):
+    return gn16_off(pkg) if tag.endswith(OFF) else linear16_off(pkg) if tag.endswith(LIN_OFF) \
+        else contextlib.nullcontext()
 
 
 def _decoder(pkg, fused, linear, amp, train):
@@ -492,15 +513,16 @@ def part_b(pkg, args, emit):
             ("amp bf16", dict(fused=True, linear="torch", amp=True), torch.bfloat16),
             ("amp bf16 fused=False", dict(fused=False, linear="torch", amp=True), torch.bfloat16),
             ("amp bf16 linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.bfloat16),
-            ("amp bf16 linear=autocast" + OFF, dict(fused=True, linear="autocast", amp=True), torch.bfloat16)]
+            ("amp bf16 linear=autocast" + OFF, dict(fused=True, linear="autocast", amp=True), torch.bfloat16),
+            ("amp bf16 linear=autocast" + LIN_OFF, dict(fused=True, linear="autocast", amp=True), torch.bfloat16)]
     models = {tag: _decoder(pkg, train=False, **kw) for tag, kw, _ in arms}
     res = {tag: [] for tag, _, _ in arms}
     for _ in range(args.repeats):
         for tag, _, dt in arms:
             ctx = torch.autocast("cuda", dtype=dt) if dt is not None else contextlib.nullcontext()
 
-            def fwd(m=models[tag], ctx=ctx, off=tag.endswith(OFF)):
-                with torch.no_grad(), ctx, gn16_off(pkg) if off else contextlib.nullcontext():
+            def fwd(m=models[tag], ctx=ctx, tag=tag):
+                with torch.no_grad(), ctx, _switch(pkg, tag):
                     m.forward_features(feats)
             res[tag].append(timed(fwd, max(2, args.steps // 4), 2))
     for tag, _, _ in arms:
@@ -515,10 +537,13 @@ def part_c(pkg, args, emit):
             ("amp bf16 fused=False", dict(fused=False, linear="torch", amp=True), torch.bfloat16),
             ("amp bf16 linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.bfloat16),
             ("amp bf16 linear=autocast" + OFF, dict(fused=True, linear="autocast", amp=True), torch.bfloat16),
+            ("amp bf16 linear=autocast" + LIN_OFF, dict(fused=True, linear="autocast", amp=True), torch.bfloat16),
             ("amp fp16 + GradScaler", dict(fused=True, linear="torch", amp=True), torch.float16),
             ("amp fp16 + GradScaler fused=False", dict(fused=False, linear="torch", amp=True), torch.float16),
             ("amp fp16 + GradScaler linear=autocast", dict(fused=True, linear="autocast", amp=True), torch.float16),
             ("amp fp16 + GradScaler linear=autocast" + OFF, dict(fused=True, linear="autocast", amp=True),
+             torch.float16),
+            ("amp fp16 + GradScaler linear=autocast" + LIN_OFF, dict(fused=True, linear="autocast", amp=True),
              torch.float16)]
     steps = {}
     for tag, kw, dt in arms:
@@ -527,9 +552,9 @@ def part_c(pkg, args, emit):
         scaler = torch.amp.GradScaler("cuda") if dt == torch.float16 else None
         ctx = (lambda dt=dt: torch.autocast("cuda", dtype=dt)) if dt is not None else contextlib.nullcontext
 
-        def step(m=m, opt=opt, scaler=scaler, ctx=ctx, off=tag.endswith(OFF)):
+        def step(m=m, opt=opt, scaler=scaler, ctx=ctx, tag=tag):
             opt.zero_grad(set_to_none=True)
-            with ctx(), gn16_off(pkg) if off else contextlib.nullcontext():
+            with ctx(), _switch(pkg, tag):
                 mask, low, multi = m.forward_features(feats)
                 loss = sum(o.float().square().mean() for o in (mask, low, *multi))
             if scaler is None:
@@ -554,10 +579,78 @@ def part_c(pkg, args, emit):
               "note": "peak memory includes the parameters and optimizer state of all arms' models"})
 
 
+# the encoder's Linear sites (d = 256, 8 heads, 4 levels x 4 points, FFN 1024): (name, in, out, relu)
+LINEAR_SITES = [("value / output projection", 256, 256, False), ("query GEMM (offsets + logits)", 256, 288, False),
+                ("sampling offsets", 256, 192, False), ("attention weights", 256, 96, False),
+                ("linear1 + ReLU", 256, 1024, True), ("linear2", 1024, 256, False)]
+
+
+def part_m(pkg, args, emit):
+    """The 16-bit Linear kernels against torch's autocast composition at the encoder's Linear sites: forward, input
+    gradient, weight + bias gradient; median of `--steps` alternating calls, the L2 evicted before each."""
+    dev = torch.device("cuda", 0)
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    for rows in (344064, 172032):
+        for tag in ("bf16", "fp16"):
+            dt = DTYPES[tag]
+            for name, k, n, relu in LINEAR_SITES:
+                gen = torch.Generator(device=dev).manual_seed(k + n)
+                x16 = torch.randn(rows, k, device=dev, generator=gen).to(dt)
+                g16 = (torch.randn(rows, n, device=dev, generator=gen) * 1e-2).to(dt)
+                w = torch.randn(n, k, device=dev, generator=gen) / k ** 0.5
+                b = torch.randn(n, device=dev, generator=gen) * 0.1
+                w16, wt16 = w.to(dt), w.t().contiguous().to(dt)
+
+                def torch_fwd():
+                    with torch.no_grad(), torch.autocast("cuda", dtype=dt):
+                        y = F.linear(x16, w, b)
+                        return F.relu(y) if relu else y
+
+                def addmm_act():
+                    with torch.no_grad(), torch.autocast("cuda", dtype=dt):
+                        return torch._addmm_activation(b.to(dt), x16, w16.t())
+
+                def torch_wgrad():
+                    return (g16.t() @ x16).float(), g16.sum(0).float()
+
+                arms = {("16-bit kernels", "forward"): lambda: pkg.ops.linear_mixed(x16, w16, b, relu=relu),
+                        ("torch autocast composition", "forward"): torch_fwd,
+                        ("16-bit kernels", "input gradient"): lambda: pkg.ops.linear_mixed(g16, wt16),
+                        ("torch autocast composition", "input gradient"): lambda: g16 @ w16,
+                        ("16-bit kernels", "weight + bias gradient"): lambda: pkg.ops.linear_mixed_wgrad(g16, x16),
+                        ("torch autocast composition", "weight + bias gradient"): torch_wgrad}
+                if relu:
+                    try:
+                        addmm_act()
+                        arms[("torch._addmm_activation (cuBLASLt ReLU epilogue)", "forward")] = addmm_act
+                    except RuntimeError as e:
+                        emit({"part": "m", "site": name, "dtype": tag, "note": f"_addmm_activation: {e}"[:300]})
+                act = rows * (k + n) * 2
+                nbytes = {"forward": act + n * k * 2, "input gradient": act + n * k * 2,
+                          "weight + bias gradient": act + n * k * 4 + n * 4}
+                times = {a: [] for a in arms}
+                for a in arms:
+                    for _ in range(2):
+                        _evicted(flush, arms[a])
+                for _ in range(args.steps):
+                    for a in arms:                                  # the arms alternate
+                        times[a].append(_evicted(flush, arms[a]))
+                for (arm, op), ts in times.items():
+                    ms = statistics.median(ts)
+                    emit({"part": "m", "site": name, "rows": rows, "in": k, "out": n, "relu": relu, "dtype": tag,
+                          "arm": arm, "op": op, "ms_median": ms, "ms_min": min(ts), "ms_max": max(ts),
+                          "timed_calls": len(ts), "algorithmic_bytes": nbytes[op],
+                          "algorithmic_GBs": nbytes[op] / ms / 1e6, "hbm_share": nbytes[op] / ms / 1e6 / HBM_GBS,
+                          "hbm_GBs_reference": HBM_GBS, "l2": "evicted before every call (256 MB write)"})
+                del x16, g16
+                torch.cuda.empty_cache()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--parts", default="a,b,c", help="a, b, c: profiles/r5_mixed.jsonl; f, b, c: r6_fused_mixed.jsonl; "
-                                                  "l, p, b, c: r7_autocast_encoder.jsonl; g, b, c: r8_group_norm_mixed.jsonl")
+                                                  "l, p, b, c: r7_autocast_encoder.jsonl; g, b, c: r8_group_norm_mixed.jsonl; "
+                                                  "m, b, c: r9_linear_mixed.jsonl")
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--dtypes", default="fp32,bf16,fp16", help="part (a): element types of value")
@@ -580,7 +673,7 @@ def main():
         with open(path, "a") as f:
             f.write(json.dumps(rec) + "\n")
     for part in args.parts.split(","):
-        {"a": part_a, "f": part_f, "b": part_b, "c": part_c, "l": part_l, "p": part_p, "g": part_g}[part](pkg, args, emit)
+        {"a": part_a, "f": part_f, "b": part_b, "c": part_c, "l": part_l, "p": part_p, "g": part_g, "m": part_m}[part](pkg, args, emit)
 
 
 if __name__ == "__main__":

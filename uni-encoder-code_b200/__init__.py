@@ -17,9 +17,9 @@ import sys
 
 from . import _lib
 from ._lib import get_option, launch_count, set_option
-from .functions import (AddLayerNormFunction, AddLayerNormMixedFunction, GroupNormFunction, GroupNormRowsFunction, LinearTF32x3Function,
-                        MSDeformAttnFunction, MSDeformAttnFusedFunction, MSDeformAttnMixedFunction)
-from .ops import (add_layernorm, add_layernorm_mixed, debug_indices, group_norm, linear_tf32x3, ms_deform_attn_backward, ms_deform_attn_forward,
+from .functions import (AddLayerNormFunction, AddLayerNormMixedFunction, GroupNormFunction, GroupNormRowsFunction, LinearMixedFunction,
+                        LinearTF32x3Function, MSDeformAttnFunction, MSDeformAttnFusedFunction, MSDeformAttnMixedFunction)
+from .ops import (add_layernorm, add_layernorm_mixed, debug_indices, group_norm, linear_mixed, linear_tf32x3, ms_deform_attn_backward, ms_deform_attn_forward,
                   ms_deform_attn_fused_backward, ms_deform_attn_fused_forward, ms_deform_attn_mixed_backward,
                   ms_deform_attn_mixed_forward)
 from . import synthetic
@@ -30,7 +30,7 @@ __all__ = [
     "ms_deform_attn_fused_forward", "ms_deform_attn_fused_backward", "MSDeformAttnFusedFunction", "linear_tf32x3", "add_layernorm", "group_norm", "LinearTF32x3Function", "AddLayerNormFunction",
     "GroupNormFunction", "GroupNormRowsFunction",
     "ms_deform_attn_mixed_forward", "ms_deform_attn_mixed_backward", "MSDeformAttnMixedFunction",
-    "add_layernorm_mixed", "AddLayerNormMixedFunction",
+    "add_layernorm_mixed", "AddLayerNormMixedFunction", "linear_mixed", "LinearMixedFunction",
     "install_dropin", "set_option", "get_option", "launch_count", "synthetic", "modules", "pixel_decoder", "sharding",
 ]
 

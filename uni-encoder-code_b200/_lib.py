@@ -69,6 +69,11 @@ SYMBOLS = {
     "msda_b200_linear_wgrad_deterministic_f32": (_I, [_P] * 4 + [ctypes.c_longlong, _I, _I, _P, _P]),
     "msda_b200_linear_wgrad_deterministic_workspace_bytes": (ctypes.c_longlong, [ctypes.c_longlong, _I, _I]),
     "msda_b200_transpose_f32": (_I, [_P, _P, ctypes.c_longlong, _I, _P]),
+    "msda_b200_linear_mixed_bf16": (_I, [_P] * 4 + [_I] * 4 + [_P]),
+    "msda_b200_linear_mixed_f16": (_I, [_P] * 4 + [_I] * 4 + [_P]),
+    "msda_b200_linear_mixed_wgrad_bf16": (_I, [_P] * 4 + [ctypes.c_longlong, _I, _I, _P, _P]),
+    "msda_b200_linear_mixed_wgrad_f16": (_I, [_P] * 4 + [ctypes.c_longlong, _I, _I, _P, _P]),
+    "msda_b200_linear_mixed_wgrad_workspace_bytes": (ctypes.c_longlong, [ctypes.c_longlong, _I, _I]),
     "msda_b200_group_norm_nchw_f32": (_I, [_P] * 5 + [_I] * 5 + [ctypes.c_float, _I, _P, _I, _I, _P, _P]),
     "msda_b200_group_norm_nchw_to_rows_f32": (_I, [_P] * 5 + [ctypes.c_longlong, ctypes.c_longlong, _I, _I, ctypes.c_longlong, _I,
                                                     ctypes.c_float, _I, _P, _P]),

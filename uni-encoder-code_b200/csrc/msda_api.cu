@@ -66,6 +66,14 @@ cudaError_t launch_linear_wgrad(const float *, const float *, float *, float *, 
                                 bool *handled, float *partials);
 long long linear_wgrad_partials(long long rows, int out_f, int in_f);
 cudaError_t launch_transpose(const float *, float *, long long, int, cudaStream_t);
+// 16-bit Linear (linear_mixed.cu): T = __nv_bfloat16 or __half
+template <typename T>
+cudaError_t launch_linear_mixed(const T *, const T *, const float *, T *, int, int, int, int, cudaStream_t,
+                                bool *handled);
+template <typename T>
+cudaError_t launch_linear_mixed_wgrad(const T *, const T *, float *, float *, long long, int, int, float *,
+                                      cudaStream_t, bool *handled);
+long long linear_mixed_wgrad_workspace_floats(long long rows, int out_f, int in_f);
 // GroupNorm: V = type of the map x (and of y16 / grad_x), float or 16-bit; G = type of grad_y (float or V)
 template <typename V>
 cudaError_t launch_group_norm(const V *, const float *, const float *, const float *, float *, V *y16, int, int, int,
@@ -355,6 +363,28 @@ static int linear_wgrad(const float *grad_y, const float *x, float *grad_weight,
     bool handled = false;
     const cudaError_t e = launch_linear_wgrad(grad_y, x, grad_weight, grad_bias, rows, out_f, in_f,
                                               (cudaStream_t)stream, &handled, static_cast<float *>(workspace));
+    return launch_rc(e, handled);
+}
+
+template <typename T>
+static int linear_mixed(const T *x, const T *weight, const float *bias, T *y, int rows, int out_f, int in_f, int relu,
+                        void *stream) {
+    if (!x || !weight || !y) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || out_f <= 0 || in_f <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_linear_mixed<T>(x, weight, bias, y, rows, out_f, in_f, relu, (cudaStream_t)stream,
+                                                 &handled);
+    return launch_rc(e, handled);
+}
+
+template <typename T>
+static int linear_mixed_wgrad(const T *grad_y, const T *x, float *grad_weight, float *grad_bias, long long rows,
+                              int out_f, int in_f, void *workspace, void *stream) {
+    if (!grad_y || !x || !grad_weight || !workspace) return MSDA_ERR_NULL_POINTER;
+    if (rows <= 0 || out_f <= 0 || in_f <= 0) return MSDA_ERR_BAD_SHAPE;
+    bool handled = false;
+    const cudaError_t e = launch_linear_mixed_wgrad<T>(grad_y, x, grad_weight, grad_bias, rows, out_f, in_f,
+                                                       static_cast<float *>(workspace), (cudaStream_t)stream, &handled);
     return launch_rc(e, handled);
 }
 
@@ -803,6 +833,28 @@ int msda_b200_fused_backward_deterministic_f32(const float *grad_output, const f
 MSDA_MIXED_ENTRIES(bf16, __nv_bfloat16)
 MSDA_MIXED_ENTRIES(f16, __half)
 #undef MSDA_MIXED_ENTRIES
+
+// ---- 16-bit Linear under torch.autocast: bf16 / fp16 operands, fp32 bias, accumulation and weight gradient ----
+#define MSDA_LINEAR_MIXED_ENTRIES(SUFFIX, T)                                                                         \
+    int msda_b200_linear_mixed_##SUFFIX(const uint16_t *x, const uint16_t *weight16, const float *bias, uint16_t *y, \
+                                        int rows, int out_features, int in_features, int relu, void *stream) {      \
+        return linear_mixed<T>(reinterpret_cast<const T *>(x), reinterpret_cast<const T *>(weight16), bias,          \
+                               reinterpret_cast<T *>(y), rows, out_features, in_features, relu, stream);             \
+    }                                                                                                                \
+    int msda_b200_linear_mixed_wgrad_##SUFFIX(const uint16_t *grad_y, const uint16_t *x, float *grad_weight,         \
+                                              float *grad_bias, long long rows, int out_features, int in_features,   \
+                                              void *workspace, void *stream) {                                       \
+        return linear_mixed_wgrad<T>(reinterpret_cast<const T *>(grad_y), reinterpret_cast<const T *>(x),            \
+                                     grad_weight, grad_bias, rows, out_features, in_features, workspace, stream);    \
+    }
+MSDA_LINEAR_MIXED_ENTRIES(bf16, __nv_bfloat16)
+MSDA_LINEAR_MIXED_ENTRIES(f16, __half)
+#undef MSDA_LINEAR_MIXED_ENTRIES
+
+long long msda_b200_linear_mixed_wgrad_workspace_bytes(long long rows, int out_features, int in_features) {
+    if (rows <= 0 || out_features <= 0 || in_features <= 0) return 0;
+    return linear_mixed_wgrad_workspace_floats(rows, out_features, in_features) * (long long)sizeof(float);
+}
 
 int msda_b200_linear_f32(const float *x, const float *weight, const float *bias, float *y, int rows,
                          int out_features, int in_features, int relu, float *workspace, void *stream) {

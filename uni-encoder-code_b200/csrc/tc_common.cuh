@@ -1,4 +1,4 @@
-// tc_common.cuh -- PTX wrappers shared by the tensor-core kernels (linear_tf32x3.cu, linear_wgrad.cu):
+// tc_common.cuh -- PTX wrappers shared by the tensor-core kernels (linear_tf32x3.cu, linear_wgrad.cu, linear_mixed.cu):
 // mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (MMA with A in shared or tensor memory, commit, ld, st),
 // shared-memory / instruction descriptors, and the host-side tensor-map helper.
 #pragma once
@@ -109,6 +109,30 @@ __device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[32
         : "memory");
 }
 
+// ---- 16-bit operands (linear_mixed.cu): a k-block is 64 elements, one 128-byte swizzle span ----
+constexpr int kBK16 = 64;
+constexpr int kUmmaK16 = 16;      // kind::f16 MMA depth
+
+// instruction descriptor for kind::f16: fp32 accumulate, A and B bf16 (bf16 = true) or fp16; a_mn / b_mn: the
+// operand is MN-major in shared memory (bits 15 / 16), K-major otherwise
+__device__ __forceinline__ constexpr uint32_t umma_idesc_f16(int m, int n, bool bf16, bool a_mn, bool b_mn) {
+    return (1u << 4) | ((bf16 ? 1u : 0u) << 7) | ((bf16 ? 1u : 0u) << 10) | ((a_mn ? 1u : 0u) << 15) |
+           ((b_mn ? 1u : 0u) << 16) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+// shared-memory descriptor of an MN-major tile with 128-byte swizzle: rows of 64 MN-elements (one swizzle span)
+// along K, 8-row (1024-byte) atoms SBO = 1024 bytes apart in K, the next 64 MN-elements LBO bytes further
+// (the canonical ((8,n),(8,k)) : ((1,LBO),(8,SBO)) layout in 16-byte units)
+__device__ __forceinline__ uint64_t umma_desc_mn(uint32_t smem_addr, uint32_t lbo) {
+    return (uint64_t)((smem_addr & 0x3ffffu) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(1024 >> 4) << 32) |
+           (1ull << 46) | (2ull << 61);
+}
+__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate) : "memory");
+}
+
 // ---- host side ----
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
@@ -151,6 +175,20 @@ inline bool make_map_plain(CUtensorMap *map, const float *ptr, long long rows, i
     return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float *>(ptr), dims, strides, box, estr,
                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+// row-major 16-bit matrix [rows x cols] (bf16 = true: bfloat16, else float16), box = box_rows x 64 columns
+// (128 bytes: one swizzle span), 128-byte swizzle, zero fill outside; cols % 8 == 0 (16-byte row stride)
+inline bool make_map16(CUtensorMap *map, const void *ptr, long long rows, int cols, int box_rows, bool bf16) {
+    EncodeTiledFn enc = encode_tiled();
+    if (!enc) return false;
+    const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+    const cuuint64_t strides[1] = {(cuuint64_t)cols * 2};
+    const cuuint32_t box[2] = {(cuuint32_t)kBK16, (cuuint32_t)box_rows};
+    const cuuint32_t estr[2] = {1, 1};
+    return enc(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void *>(ptr),
+               dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+               CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
 }  // namespace tc

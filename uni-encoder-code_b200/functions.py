@@ -152,6 +152,69 @@ class LinearTF32x3Function(Function):
         return grad_x, grad_w, grad_b, None, None
 
 
+class LinearMixedFunction(Function):
+    """``apply(x16, weight, bias, relu=False, dropout_p=0.0)``: ``LinearTF32x3Function`` under torch.autocast.  ``x16``
+    is bf16 / fp16, ``weight`` and ``bias`` (may be None) the fp32 parameters; the weight is cast to x16's dtype once
+    per call.  = ``F.linear(x16, weight, bias)`` as autocast computes it (bias added to the fp32 accumulator, one
+    rounding; ops.linear_mixed), with ``relu`` in the GEMM's epilogue and ``dropout_p`` drawn by torch's own dropout
+    kernel on the 16-bit output.  Backward: one ``threshold_backward`` when ``relu`` is set, the input gradient (in x16's
+    dtype) as torch's 16-bit GEMM -- faster than the library kernel at every measured shape (ops.linear_mixed_preferred)
+    -- or, with torch.use_deterministic_algorithms(True), on the library kernel, and the fp32 weight and bias gradients
+    of ops.linear_mixed_wgrad, which go to the fp32 parameters without a 16-bit rounding; the 1/(1-p) scale is applied
+    to the transposed weight and to those."""
+
+    @staticmethod
+    def supported(x16, weight, bias=None) -> bool:
+        """Whether the kernels cover ``x16`` with the fp32 parameters ``weight`` [out, in] and ``bias``."""
+        return (isinstance(weight, torch.Tensor) and weight.dtype == torch.float32 and weight.dim() == 2
+                and weight.is_contiguous()
+                and ops.linear_mixed_shapes_supported(x16, weight.size(0), weight.size(1), bias)
+                and weight.device == x16.device)
+
+    @staticmethod
+    def forward(ctx, x16, weight, bias, relu=False, dropout_p=0.0):
+        if dropout_p and not (relu and 0.0 < dropout_p < 1.0):
+            raise ValueError("dropout_p needs relu=True and 0 < p < 1")
+        w16 = weight.detach().to(x16.dtype)
+        y = ops.linear_mixed(x16, w16, bias, relu=relu)
+        ctx.has_bias = bias is not None
+        ctx.relu = bool(relu)
+        ctx.scale = 1.0
+        if dropout_p:
+            y, _ = torch.native_dropout(y, float(dropout_p), True)       # y * mask / (1 - p)
+            ctx.scale = 1.0 / (1.0 - float(dropout_p))
+        ctx.save_for_backward(x16, w16, y if relu else None, weight if dropout_p else None)
+        return y
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_y):
+        x16, w16, y, weight = ctx.saved_tensors
+        grad_y = grad_y.to(x16.dtype)
+        if ctx.relu:
+            # F.relu's backward; with dropout, y > 0 exactly where the element was kept AND the ReLU was active
+            grad_y = torch.ops.aten.threshold_backward(grad_y, y, 0)
+        g2 = _aligned(grad_y.reshape(-1, grad_y.size(-1)))
+        scale = ctx.scale
+        grad_x = grad_w = grad_b = None
+        if ctx.needs_input_grad[0]:
+            w_in = w16 if scale == 1.0 else (weight * scale).to(x16.dtype)          # [out, in]
+            if ops._deterministic() or ops.linear_mixed_preferred(g2.size(0), w_in.size(1), w_in.size(0), False,
+                                                                   "input_gradient"):
+                grad_x = ops.linear_mixed(g2, w_in.t().contiguous()).view(x16.shape)
+            else:
+                grad_x = (g2 @ w_in).view(x16.shape)
+        want_b = ctx.has_bias and ctx.needs_input_grad[2]
+        if ctx.needs_input_grad[1] or want_b:
+            grad_w, grad_b = ops.linear_mixed_wgrad(g2, x16.reshape(-1, x16.size(-1)), with_bias=want_b)
+            if not ctx.needs_input_grad[1]:
+                grad_w = None
+        if scale != 1.0:
+            grad_w = grad_w * scale if grad_w is not None else None
+            grad_b = grad_b * scale if grad_b is not None else None
+        return grad_x, grad_w, grad_b, None, None
+
+
 class AddLayerNormFunction(Function):
     """``apply(x, residual, weight, bias, eps)`` = ``F.layer_norm(x + residual, (C,), weight, bias, eps)`` with one
     fused kernel each way (ops.add_layernorm / add_layernorm_backward); C in {128, 256}."""

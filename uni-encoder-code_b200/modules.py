@@ -22,6 +22,7 @@ from __future__ import annotations
 
 import copy
 import math
+import weakref
 from typing import Callable, List, Optional, Sequence, Tuple
 
 import torch
@@ -29,8 +30,8 @@ import torch.nn.functional as F
 from torch import nn
 
 from . import ops
-from .functions import (AddLayerNormFunction, AddLayerNormMixedFunction, LinearTF32x3Function, MSDeformAttnFunction,
-                        MSDeformAttnFusedFunction, MSDeformAttnMixedFunction)
+from .functions import (AddLayerNormFunction, AddLayerNormMixedFunction, LinearMixedFunction, LinearTF32x3Function,
+                        MSDeformAttnFunction, MSDeformAttnFusedFunction, MSDeformAttnMixedFunction)
 
 CoreFn = Callable[..., torch.Tensor]
 
@@ -94,6 +95,19 @@ def _presplit_of(layer: nn.Linear):
     return hit[1]
 
 
+def _weight16_of(w: torch.Tensor, owner: dict, dtype):
+    """`w` cast to `dtype` for the inference GEMM under autocast, kept in `owner` (a module's __dict__) per weight
+    version and per weight tensor (a new tensor at the old address with an equal version is not served the old copy);
+    not kept while a CUDA graph is captured."""
+    key = (w.data_ptr(), _version_of(w), tuple(w.shape), str(w.device), dtype)
+    hit = owner.get("_weight16")
+    if hit is None or hit[0] != key or hit[1]() is not w:
+        hit = (key, weakref.ref(w), w.detach().to(dtype))
+        if not _capturing(w):
+            owner["_weight16"] = hit
+    return hit[2]
+
+
 def _autocast_dtype():
     """The 16-bit type of the active CUDA torch.autocast, or None (no context, a disabled one, or another type)."""
     if not torch.is_autocast_enabled("cuda"):
@@ -116,8 +130,13 @@ def _linear(layer: nn.Linear, x, impl: str, relu: bool = False):
     tensor cores as an error-compensated 3xTF32 product (ops.linear_tf32x3, SURVEY 8f.3); with autograd
     on, the forward and the input-gradient GEMMs do (LinearTF32x3Function; the weight gradient stays a
     torch GEMM); for any shape the kernel does not cover torch's own fp32 GEMM is used as in the reference.
-    impl == "autocast": see `_resolve` (under autocast, torch's own 16-bit GEMM)."""
+    impl == "autocast": see `_resolve`; under a 16-bit autocast the 16-bit GEMM of `_linear_mixed`, or torch's
+    autocast GEMM for shapes it does not cover."""
     impl = _resolve(impl)
+    if impl == "autocast":
+        y = _linear_mixed(layer, x, relu)
+        if y is not None:
+            return y
     if impl == "tf32x3" and not torch.is_grad_enabled() and x.is_contiguous() \
             and ops.linear_tf32x3_supported(x, layer.weight):
         return ops.linear_tf32x3(x, layer.weight, layer.bias, relu=relu, presplit=_presplit_of(layer))
@@ -128,6 +147,31 @@ def _linear(layer: nn.Linear, x, impl: str, relu: bool = False):
         raise ValueError(f"unknown linear implementation {impl!r}")
     y = layer(x)
     return F.relu(y) if relu else y
+
+
+def _to_autocast16(x):
+    """`x` as the active autocast's 16-bit type: an fp32 tensor is cast (once, for every GEMM that reads it)."""
+    dtype = _autocast_dtype()
+    return x.to(dtype) if dtype is not None and x.dtype == torch.float32 else x
+
+
+def _linear_mixed(layer: nn.Linear, x, relu: bool = False, dropout_p: float = 0.0):
+    """Under a 16-bit autocast: ``layer(x)`` (+ ReLU, + dropout: autograd only) on the library's 16-bit GEMM with
+    the fp32 bias in its epilogue -- ops.linear_mixed with the 16-bit weight cached per version in inference,
+    LinearMixedFunction (fp32 weight and bias gradients) with autograd -- or None where it does not apply."""
+    dtype = _autocast_dtype()
+    w, b = layer.weight, layer.bias
+    if dtype is None or w.dtype != torch.float32 or (b is not None and b.dtype != torch.float32):
+        return None
+    x16 = _to_autocast16(x)
+    if x16.dtype != dtype or not LinearMixedFunction.supported(x16, w, b):
+        return None
+    if torch.is_grad_enabled():
+        # the whole node (forward, input and weight gradients) is faster than torch's at every measured site
+        return LinearMixedFunction.apply(x16, w, b, relu, dropout_p)
+    if not ops.linear_mixed_preferred(x16.numel() // x16.size(-1), w.size(0), w.size(1), relu, "forward"):
+        return None                         # measured slower than torch's GEMM at this shape
+    return ops.linear_mixed(x16, _weight16_of(w, layer.__dict__, dtype), b, relu=relu)
 
 
 def _add_norm(norm: nn.LayerNorm, x, sublayer_out, impl: str):
@@ -240,6 +284,8 @@ class MSDeformAttn(nn.Module):
     def forward(self, query, reference_points, input_flatten, input_spatial_shapes,
                 input_level_start_index, input_padding_mask=None):
         value = self.project_value(input_flatten, input_padding_mask)
+        if _resolve(self.linear) == "autocast":
+            query = _to_autocast16(query)      # read by two GEMMs: cast once
         # fp32, or under autocast a 16-bit value whose offsets / logits come out in the same type (fused_supported)
         if self.fused and self._core is _cuda_core and not reference_points.requires_grad \
                 and value.dtype in (torch.float32, torch.bfloat16, torch.float16):
@@ -345,7 +391,9 @@ class MSDeformAttn(nn.Module):
         if value is None:
             value = self.project_value(src16)
         weight, table, _ = self._query_projection(pos[0])
-        proj = F.linear(src16, weight)                     # autocast's 16-bit GEMM; the bias is in the table
+        # the 16-bit query GEMM, cached 16-bit stacked weight; the bias is in the table
+        w16 = _weight16_of(weight, self.__dict__, src16.dtype)
+        proj = ops.linear_mixed(src16, w16) if ops.linear_mixed_supported(src16, w16) else F.linear(src16, weight)
         if callable(value):
             value = value()
         ref = reference_points
@@ -428,12 +476,18 @@ class MSDeformAttnTransformerEncoderLayer(nn.Module):
     def _forward_ffn_mixed(self, src, src16):
         """`forward_ffn` under a 16-bit autocast: linear1 reads `src16` when there is one -> (output, its copy)."""
         x = src16 if src16 is not None else src
-        if self.activation is F.relu:
-            hidden = F.relu(self.linear1(x))
-        else:
-            hidden = self.activation(self.linear1(x))
-        hidden = self.dropout2(hidden)
-        return _add_norm_mixed(self.norm2, src, self.dropout3(self.linear2(hidden)))
+        p = self.dropout2.p if self.dropout2.training else 0.0
+        hidden = None
+        if self.activation is F.relu and torch.is_grad_enabled() and 0.0 < p < 1.0:
+            # training: linear1 + ReLU + dropout2 as one autograd node (one pass over the hidden gradient)
+            hidden = _linear_mixed(self.linear1, x, relu=True, dropout_p=p)
+        if hidden is None:
+            if self.activation is F.relu:      # the ReLU rides in the 16-bit GEMM's epilogue
+                hidden = _linear(self.linear1, x, self.linear, relu=True)
+            else:
+                hidden = self.activation(_linear(self.linear1, x, self.linear))
+            hidden = self.dropout2(hidden)
+        return _add_norm_mixed(self.norm2, src, self.dropout3(_linear(self.linear2, hidden, self.linear)))
 
 
 _REF_CACHE = ShapeCache()

@@ -959,6 +959,104 @@ def linear_wgrad(grad_y, x, with_bias=True):
     return gw, gb
 
 
+# ---------------------------------------------------------------- 16-bit Linear under torch.autocast (DESIGN.md 11.4)
+_LIN_MIXED = {torch.bfloat16: _lib.lib.msda_b200_linear_mixed_bf16, torch.float16: _lib.lib.msda_b200_linear_mixed_f16}
+_LIN_MIXED_WGRAD = {torch.bfloat16: _lib.lib.msda_b200_linear_mixed_wgrad_bf16,
+                    torch.float16: _lib.lib.msda_b200_linear_mixed_wgrad_f16}
+
+
+def _mat16_ok(t, dtype, device) -> bool:
+    """`t` a contiguous tensor of `dtype` on `device` whose data is 16-byte aligned (the kernels' TMA loads)."""
+    return (isinstance(t, torch.Tensor) and t.dtype == dtype and t.device == device and t.is_contiguous()
+            and t.numel() > 0 and t.data_ptr() % 16 == 0)
+
+
+def linear_mixed_shapes_supported(x, out_features, in_features, bias=None) -> bool:
+    """Whether the 16-bit GEMM covers ``x`` [..., in_features] -> [..., out_features]: x a contiguous 16-byte aligned
+    bf16 / fp16 CUDA tensor, in % 8 == 0 and out % 8 == 0; ``bias`` None or a contiguous fp32 [out] on x's device."""
+    return (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype in _LIN_MIXED and x.dim() >= 1
+            and _mat16_ok(x, x.dtype, x.device) and x.size(-1) == in_features
+            and out_features % 8 == 0 and in_features % 8 == 0 and x.numel() // in_features < 2 ** 31
+            and (bias is None or (isinstance(bias, torch.Tensor) and bias.dtype == torch.float32
+                                  and bias.device == x.device and bias.is_contiguous()
+                                  and tuple(bias.shape) == (out_features,))))
+
+
+def linear_mixed_supported(x, weight16, bias=None) -> bool:
+    """Whether ``linear_mixed`` covers these tensors: ``x`` [..., in] a contiguous bf16 / fp16 CUDA tensor and
+    ``weight16`` [out, in] a contiguous one of x's dtype, both 16-byte aligned, with in % 8 == 0 and out % 8 == 0;
+    ``bias`` None or a contiguous fp32 [out] tensor on x's device."""
+    return (isinstance(weight16, torch.Tensor) and weight16.dim() == 2 and isinstance(x, torch.Tensor)
+            and _mat16_ok(weight16, x.dtype, x.device)
+            and linear_mixed_shapes_supported(x, weight16.size(0), weight16.size(1), bias))
+
+
+def linear_mixed_preferred(rows, out_features, in_features, relu, op) -> bool:
+    """Whether the 16-bit kernel is measured at least as fast as torch's 16-bit GEMM for `op` ("forward" or
+    "input_gradient") of a Linear with these shapes (NVIDIA B200, profiles/r9_linear_mixed.jsonl, DESIGN.md 11.4):
+    * the input gradient is 4-29 % slower than cuBLAS at every measured site (in_features = 256 with out_features
+      96 ... 1024, 172 032 and 344 064 rows);
+    * the forward is faster or level everywhere except in = out = 256 without ReLU above 262 144 rows (0.076 against
+      0.071 ms at 344 064 rows; 0.046 against 0.048 ms at 172 032).
+    Callers take torch's GEMM where this is False, unless determinism is asked for."""
+    if op == "input_gradient":
+        return False
+    if op == "forward":
+        return not (in_features == out_features == 256 and not relu and rows > 262144)
+    raise ValueError(f"unknown op {op!r}")
+
+
+def linear_mixed(x, weight16, bias=None, relu=False):
+    """``F.linear(x, weight16, bias)`` (then ReLU if ``relu``) as torch.autocast computes it, for a bf16 / fp16 ``x``
+    and ``weight16`` of one type and an fp32 ``bias``: the bias is added to the fp32 accumulator and the result rounded
+    once to x's dtype (msda_b200_linear_mixed_bf16 / _f16).  Also the input gradient ``grad_y @ weight16`` with the
+    transposed weight.  Inference only (no autograd: functions.LinearMixedFunction)."""
+    if not isinstance(x, torch.Tensor) or not x.is_cuda:
+        raise RuntimeError("Not implemented on the CPU")
+    if not linear_mixed_supported(x, weight16, bias):
+        raise RuntimeError("linear_mixed needs contiguous 16-byte aligned bf16 / fp16 CUDA tensors x [..., in] and "
+                           "weight16 [out, in] of one dtype with in % 8 == 0 and out % 8 == 0, and an fp32 bias [out] "
+                           "or None")
+    out_f, in_f = weight16.shape
+    y = torch.empty(x.shape[:-1] + (out_f,), dtype=x.dtype, device=x.device)
+    with torch.cuda.device(x.device):
+        with _timed("linear_mixed"):
+            rc = _LIN_MIXED[x.dtype](x.data_ptr(), weight16.data_ptr(), _ptr(bias), y.data_ptr(), x.numel() // in_f,
+                                     out_f, in_f, 1 if relu else 0, torch.cuda.current_stream(x.device).cuda_stream)
+    _lib.check(rc, "linear_mixed")
+    return y
+
+
+def linear_mixed_wgrad_supported(grad_y, x) -> bool:
+    """Whether ``linear_mixed_wgrad`` covers these tensors: contiguous 16-byte aligned bf16 / fp16 CUDA matrices
+    ``grad_y`` [rows, out] and ``x`` [rows, in] of one dtype, out % 8 == 0 and in % 8 == 0."""
+    return (isinstance(grad_y, torch.Tensor) and grad_y.is_cuda and grad_y.dtype in _LIN_MIXED_WGRAD
+            and grad_y.dim() == 2 and isinstance(x, torch.Tensor) and x.dim() == 2 and grad_y.size(0) == x.size(0)
+            and _mat16_ok(grad_y, grad_y.dtype, grad_y.device) and _mat16_ok(x, grad_y.dtype, grad_y.device)
+            and grad_y.size(1) % 8 == 0 and x.size(1) % 8 == 0 and grad_y.size(0) < 2 ** 31)
+
+
+def linear_mixed_wgrad(grad_y, x, with_bias=True):
+    """(grad_weight [out, in], grad_bias [out] or None), both fp32, of ``F.linear`` from 16-bit ``grad_y`` [rows, out]
+    and ``x`` [rows, in]: grad_y^T @ x and the column sums of grad_y with fp32 accumulation, never rounded to 16 bits.
+    Deterministic by construction (per-chunk partials in a workspace, added in chunk order by a second launch)."""
+    if not isinstance(grad_y, torch.Tensor) or not grad_y.is_cuda:
+        raise RuntimeError("Not implemented on the CPU")
+    if not linear_mixed_wgrad_supported(grad_y, x):
+        raise RuntimeError("linear_mixed_wgrad needs contiguous 16-byte aligned bf16 / fp16 CUDA matrices grad_y "
+                           "[rows, out] and x [rows, in] of one dtype with out % 8 == 0 and in % 8 == 0")
+    rows, out_f, in_f = grad_y.size(0), grad_y.size(1), x.size(1)
+    gw = torch.empty(out_f, in_f, dtype=torch.float32, device=x.device)
+    gb = torch.empty(out_f, dtype=torch.float32, device=x.device) if with_bias else None
+    with torch.cuda.device(x.device):
+        ws = _workspace(_lib.lib.msda_b200_linear_mixed_wgrad_workspace_bytes(rows, out_f, in_f), x)
+        with _timed("linear_mixed_wgrad"):
+            rc = _LIN_MIXED_WGRAD[grad_y.dtype](grad_y.data_ptr(), x.data_ptr(), gw.data_ptr(), _ptr(gb), rows, out_f,
+                                                in_f, ws.data_ptr(), torch.cuda.current_stream(x.device).cuda_stream)
+    _lib.check(rc, "linear_mixed_wgrad")
+    return gw, gb
+
+
 def add_layernorm_backward(grad_y, x, residual, weight, eps=1e-5):
     """(grad_v, grad_weight, grad_bias) of ``layer_norm(x + residual)``; grad_v is the gradient of both x and
     residual.  Last dimension 128 or 256."""
